@@ -42,6 +42,7 @@ import torch  # noqa: E402
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the modules imported from it leave no __pycache__ there
 
 METRIC = "rendered_views_per_sec_fwd_bwd"
 UNIT = "views/s"
@@ -67,7 +68,16 @@ def parse():
     ap.add_argument("--extras", default="auto", choices=["auto", "all", "none", "tiny"],
                     help="auto: the BASELINE sub-records when the main workload is the default one; tiny: shrunken (tests)")
     ap.add_argument("--only", default=None, help="comma list of extra record names to run (default: all of them)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the main record, write what its last step returned as DIR/<name>.npy: images "
+                         "and fragment indices (every k-th view, k the smallest stride that keeps the dump under 64 MB), cameras "
+                         "R / T / C and the gradients w.r.t. azim / elev / dist (a CUDA-graph replay returns images and gradients only)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -189,6 +199,43 @@ def traffic_table():
         return {}
 
 
+DUMP_LIMIT = 64_000_000      # bytes --dump-outputs may write in all
+
+
+def dump_outputs(out_dir, img, cams, frag, g_azim, g_elev, g_dist):
+    """--dump-outputs: what the caller of the timed step received from its last step, as out_dir/<name>.npy.  Floating-point
+    tensors are written as float32, fragment indices as float64 (exact for every int32).  Of the per-view arrays (images,
+    fragment indices) views 0, k, 2k, ... are kept, k the smallest stride that keeps the dump under DUMP_LIMIT; the inputs are
+    seeded, so the same arguments dump the same views of the same work, and two builds can be compared array by array."""
+    import numpy as np
+    from mvtn_b200 import ops
+    small = {"grad_azim": g_azim, "grad_elev": g_elev, "grad_dist": g_dist}
+    per_view = {"images": img}
+    if cams is not None:
+        small.update(R=cams[0], T=cams[1], C=cams[2])
+    if isinstance(frag, ops._PointFragments):      # densify a copy: covered_fraction() reads the sparse form of the original
+        per_view["idx"] = ops._PointFragments(*frag._raw)["idx"]
+    elif frag is not None:
+        per_view["pix_to_face"] = frag["pix_to_face"]
+
+    def host(t):
+        t = t.detach()
+        return (t.float() if t.is_floating_point() else t.double()).cpu().numpy()
+
+    small = {k: host(t) for k, t in small.items()}
+    budget = DUMP_LIMIT - sum(v.nbytes for v in small.values()) - 4096      # 4096: room for the .npy headers
+    view_bytes = sum(t[0].numel() * (4 if t.is_floating_point() else 8) for t in per_view.values())
+    if view_bytes > budget:
+        raise SystemExit(f"--dump-outputs: the outputs of one view ({view_bytes} bytes) do not fit {DUMP_LIMIT} bytes")
+    n = img.shape[0]
+    stride = -(-n // (budget // view_bytes))
+    arrays = dict(small, **{k: host(t[::stride]) for k, t in per_view.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    sys.stderr.write(f"--dump-outputs: {', '.join(arrays)} -> {out_dir} (views 0, {stride}, {2 * stride}, ... of {n})\n")
+
+
 # ---------------------------------------------------------------------------------------------------
 def make_inputs(s, rank):
     """Seeded synthetic inputs of one workload (SURVEY 8d "Synthetic inputs"); different objects on every rank."""
@@ -240,6 +287,7 @@ class Workload:
         self.obj = torch.tensor([0.99999] * 3, device=dev)
         self.light = torch.tensor([[0.0, 1.0, 0.0]], device=dev)
         self.graphed = None
+        self.keep_outputs, self.last_outputs = False, None      # --dump-outputs: step_resident keeps what its caller receives
         if s["kind"] == "mesh":
             self.nv = [v.shape[0] for v, _ in inp["meshes"]]
             self.nf = [f.shape[0] for _, f in inp["meshes"]]
@@ -282,15 +330,19 @@ class Workload:
         from mvtn_b200 import ops
         s, M, S = self.s, self.M, self.S
         az, el, di = (t.detach().requires_grad_() for t in self.views_d)
+        cams = frag = None
         if self.graphed is not None and not eager:
             img = self.graphed(az, el, di)
         elif s["kind"] == "mesh":
             geom = ops.PackedMeshes.from_packed(self.verts_d, self.faces_d, self.nv, self.nf)
-            img, _cams, _frag = ops.render_meshes_from_angles(geom, M, az, el, di, self.light, self.obj, self.bg, S)
+            img, cams, frag = ops.render_meshes_from_angles(geom, M, az, el, di, self.light, self.obj, self.bg, S)
         else:
-            img, _cams, self.last_frag = ops.render_points_from_angles(self.pts_d, self.obj, M, az, el, di, self.renderer.points_radius,
-                                                                       self.bg_black, S, points_per_pixel=s["K"], compositor=s["compositor"])
+            img, cams, frag = ops.render_points_from_angles(self.pts_d, self.obj, M, az, el, di, self.renderer.points_radius,
+                                                            self.bg_black, S, points_per_pixel=s["K"], compositor=s["compositor"])
+            self.last_frag = frag
         img.backward(self.cot)
+        if self.keep_outputs:
+            self.last_outputs = (img, cams, frag, az.grad, el.grad, di.grad)
         return az.grad, el.grad, di.grad
 
     def step_forward_only(self):
@@ -396,8 +448,8 @@ class Timer:
         return {"ms": ms, "per_step": per, "launches": lib.mvr_launch_count() - l0, "prof": prof, "wall": (w0, w1)}
 
 
-def measure(s, a, rank, world, dev, lib, parallel, with_cpu, clock_sampler=None):
-    """All numbers of one workload -> (record dict, wall-clock window)."""
+def measure(s, a, rank, world, dev, lib, parallel, with_cpu, clock_sampler=None, dump_dir=None):
+    """All numbers of one workload -> (record dict, wall-clock window).  dump_dir: see dump_outputs."""
     w = Workload(s, a, rank, dev)
     B, M, S, N = w.B, w.M, w.S, w.N
     tm = Timer(lib, parallel, dev, flush_l2=bool(s.get("flush_l2")))
@@ -422,7 +474,12 @@ def measure(s, a, rank, world, dev, lib, parallel, with_cpu, clock_sampler=None)
         if r["prof"][1] > 0:
             shares[k] = r["prof"][0] / 2      # ms per STEP spent in kernels of this name
     top = max(shares, key=shares.get)
+    w.keep_outputs = dump_dir is not None
     res = tm.bracket(w.step_resident, a.steps, profile=None if graphed else top)
+    if dump_dir is not None:      # before any later step can overwrite the buffers the last timed step returned
+        w.keep_outputs = False
+        dump_outputs(dump_dir, *w.last_outputs)
+        w.last_outputs = None
     if graphed:      # a replay re-issues no launches: kernel times and the launch count come from eager steps of the same work
         rk = tm.bracket(eager_step, 4, profile=top)
         res["prof"] = (rk["prof"][0] * a.steps / 4, rk["prof"][1] * a.steps // 4)
@@ -530,7 +587,7 @@ def measure_train(a, rank, world, dev, parallel, render_ms):
         import train_step as T
     except Exception as e:      # pragma: no cover
         return {"unavailable": f"{type(e).__name__}: {e}"}
-    steps = max(3, min(a.steps, 10))
+    steps = a.steps
     out = {"unit": "ms/step", "n_gpus": world, "steps": steps,
            "config": {"workload": "MVTN selector + MVCNN ResNet-18 training step, 32 objects/GPU x 12 views, 224x224, ~10k-face meshes, "
                                   "fp32 (torch defaults), AdamW x 2 (BASELINE configs[3])"}}
@@ -584,7 +641,7 @@ def run_ours(a):
     sampler = ClockSampler(local_rank)
     sampler.start()
     time.sleep(0.25)
-    out, wall = measure(spec, a, rank, world, dev, lib, parallel, with_cpu)
+    out, wall = measure(spec, a, rank, world, dev, lib, parallel, with_cpu, dump_dir=a.dump_outputs if rank == 0 else None)
     out["clocks"] = sampler.stop(*wall)
 
     mode = a.extras
@@ -771,7 +828,7 @@ def run_reference(a):
     n = max(1, min(len(inp["views"][0]), int(3.0 / max(t1, 1e-3))))      # ~3 s of CPU work per step
     for _ in range(min(a.warmup, 1)):
         oracle_step(s, inp, n)
-    steps = max(1, min(a.steps, 5))
+    steps = a.steps
     t0 = time.time()
     for _ in range(steps):
         oracle_step(s, inp, n)

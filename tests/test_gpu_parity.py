@@ -1284,15 +1284,16 @@ def test_points_normalized_and_bf16_output_matches_oracle(oracle, cuda_device):
 
 
 @pytest.mark.parametrize("workload", ["mesh", "points"])
-def test_bench_line_carries_the_contract_keys_and_parity(cuda_device, workload):
+def test_bench_line_carries_the_contract_keys_and_parity(cuda_device, workload, tmp_path):
     """One tiny `bench.py` run per workload: ONE JSON line with the contract's keys, and the parity object (SURVEY 8d)
-    says what the parity tests say -- bit-exact fragment indices, images / gradients within the stated tolerances."""
+    says what the parity tests say -- bit-exact fragment indices, images / gradients within the stated tolerances.
+    --dump-outputs writes what the last timed step returned (6 views: all of them fit the dump)."""
     import json
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     cmd = [sys.executable, os.path.join(root, "bench.py"), "--workload", workload, "--batch", "2", "--views", "3", "--image-size", "64",
-           "--faces", "600", "--points", "512", "--steps", "2", "--warmup", "1", "--cpu-sample-objects", "2"]
+           "--faces", "600", "--points", "512", "--steps", "2", "--warmup", "1", "--cpu-sample-objects", "2", "--dump-outputs", str(tmp_path)]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stderr[-3000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
@@ -1309,6 +1310,17 @@ def test_bench_line_carries_the_contract_keys_and_parity(cuda_device, workload):
     assert par["grad_camera_max_rel_err"] <= par["tolerance"]["gradients_rel"]
     assert par["look_at_max_abs_err"] <= par["tolerance"]["look_at_abs"]
     assert par["look_at_backward_max_rel_err"] <= 1e-4 and par["pass"]
+    assert d["steps"] == 2
+    index, K = ("pix_to_face", 1) if workload == "mesh" else ("idx", 4)
+    want = {"images": ((6, 3, 64, 64), np.float32), index: ((6, 64, 64, K), np.float64), "R": ((6, 3, 3), np.float32),
+            "T": ((6, 3), np.float32), "C": ((6, 3), np.float32), "grad_azim": ((2, 3), np.float32),
+            "grad_elev": ((2, 3), np.float32), "grad_dist": ((2, 3), np.float32)}
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(k + ".npy" for k in want)
+    got = {k: np.load(tmp_path / (k + ".npy")) for k in want}
+    for k, (shape, dtype) in want.items():
+        assert got[k].shape == shape and got[k].dtype == dtype and np.isfinite(got[k]).all(), k
+    assert (got[index] >= -1).all() and (got[index] == np.round(got[index])).all() and (got[index] >= 0).any()
+    assert np.abs(got["images"]).max() > 0 and np.abs(got["grad_azim"]).max() > 0
 
 
 def test_bench_extra_records_carry_parity_baseline_and_roofline(cuda_device):
