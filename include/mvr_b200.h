@@ -272,7 +272,9 @@ size_t mvr_points_hit_mask_words(int B, int M, int H, int W);
  * the IEEE reciprocal torch's `1.0 / dist` takes, and the backward returns d/d dist in g_inv_dist); radius in NDC; K = points_per_pixel; out_mean_std / MVR_IMAGES_BF16 as in mvr_mesh_forward.
  * outputs: images (n,3,H,W); idx (n,H,W,K) cloud-local point ids (-1 empty); optional zbuf,
  * dists2 (n,H,W,K); optional hit_mask (mvr_points_hit_mask_words words), which lets the backward pass skip
- * the ~90 % background pixels without reading idx. */
+ * the ~90 % background pixels without reading idx.
+ * For K = 2 and K = 4, idx must be aligned to 4*K bytes (a pixel's ids are stored as one vector): a misaligned idx, e.g. a
+ * slice of a larger int32 buffer, is rejected with status -10 before any launch.  mvr_points_backward takes any idx. */
 int mvr_points_forward(const float* points, const float* rgb, int B, int Np, int M, const float* R,
                        const float* T, const float* inv_dist, double radius, const float* bg_rgb,
                        int H, int W, int K, int flags, const float* out_mean_std, void* images, int* idx,

@@ -1067,6 +1067,8 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
   const int64_t N = (int64_t)B * M;
   if (N == 0) return 0;
   if ((Np > 0 && !points) || !rgb || !R || !T || !inv_dist || !bg_rgb || !images || !idx || !workspace) { set_error("mvr_points_forward: null pointer"); return -6; }
+  // K = 2 / 4: the kernels store a pixel's K ids as one int2 / int4 (a slice of a larger int32 buffer may not be aligned for that)
+  if ((K == 2 || K == 4) && ((uintptr_t)idx & (uintptr_t)(4 * K - 1))) { set_error("mvr_points_forward: idx must be aligned to 4*K = %d bytes", 4 * K); return -10; }
   if (!out_norm_valid(out_mean_std)) { set_error("mvr_points_forward: out_mean_std needs std > 0"); return -9; }
   const PointsWs w = points_ws(B, Np, M, H, W, K, radius);
   const size_t HW = (size_t)H * W;

@@ -98,6 +98,22 @@ def test_argument_validation_returns_status_not_crash():
     assert lib.mvr_look_at_forward(None, None, None, 0, None, None, None, None, None) == 0
 
 
+@pytest.mark.skipif(torch.cuda.is_available(), reason="the pointers are fake: they must never reach a device")
+def test_points_forward_rejects_misaligned_idx_before_any_launch():
+    """K = 2 / 4: the forward stores a pixel's ids as one int2 / int4, so an idx not aligned to 4 K bytes is refused on the host
+    (status -10, a message naming the alignment) before any CUDA call -- here with fake, otherwise valid, pointers."""
+    lib = _lib.load()
+    fake = 1 << 20
+    for K in (2, 4):
+        for off in range(4, 4 * K, 4):
+            n0 = lib.mvr_launch_count()
+            rc = lib.mvr_points_forward(fake, fake, 1, 16, 1, fake, fake, fake, 0.01, fake, 64, 64, K, 0, None, fake, fake + off, None, None,
+                                        None, fake, 1 << 30, None)
+            assert rc == -10, (K, off, rc)
+            assert b"idx must be aligned to 4*K = %d bytes" % (4 * K) in lib.mvr_last_error_string()
+            assert lib.mvr_launch_count() == n0
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")
 def test_no_cpu_fallback():
     r = MVRenderer(nb_views=2, image_size=32)
