@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MVR_ABI_VERSION 9
+#define MVR_ABI_VERSION 10
 
 /* flags */
 #define MVR_PERSPECTIVE_CORRECT 1  /* [upstream] RasterizationSettings.perspective_correct (FoV persp.: True) */
@@ -48,10 +48,6 @@ extern "C" {
                                       point image) are not stored; mvr_points_backward never reads them */
 #define MVR_FACES_U16 8192         /* mvr_mesh_prepare: faces given as uint16 (F,3) -- every mesh of the batch has at most 65536 vertices; half
                                       the bytes of int32 on the host-to-device copy (mvtn_b200.collate_meshes narrows when it can) */
-#define MVR_FORWARD_TILED 2048     /* mvr_mesh_forward, K == 1: the tile-binned rasterizer + shader (coarse binning pass, per-tile face
-                                      lists staged by TMA bulk copies, depth keys in shared memory, shading in the same CTA) instead of
-                                      the default bin-free scatter + shade pair.  Same fragments bit for bit; slower on B200 at the
-                                      BASELINE sizes (DESIGN.md section 4), kept selectable for A/B measurements */
 #define MVR_CLIP_BARYCENTRIC 4096  /* [upstream] RasterizationSettings.clip_barycentric_coords (default: True iff blur_radius > 0): the
                                       fragment's barycentrics are clamped below at 0 and renormalised (BarycentricClipForward) */
 #define MVR_TEST_TINY_QUEUES 0x40000000 /* tests only: shrink the scatter kernel's work queues to force their fallbacks */
@@ -161,16 +157,6 @@ int mvr_mesh_prepare(const float* verts, const void* faces, const int* vert_off,
                      int B, int64_t total_verts, int64_t total_faces, int max_faces,
                      const float* vert_rgb, int flags, void* geometry, size_t geometry_bytes,
                      void* stream);
-/* The same for objects [obj_begin, obj_end) only, whose vertices are the packed rows [vert_begin, vert_end) (all other
- * arguments describe the WHOLE batch, as above).  Every kernel of the mesh path indexes the packed arrays absolutely, so a
- * batch can be prepared -- and then rendered: mvr_mesh_forward / mvr_mesh_backward with vert_off + obj_begin,
- * face_off + obj_begin, B = obj_end - obj_begin and the per-view arrays offset by obj_begin * M views -- piece by piece
- * while the rest of it is still on its way to the device (MVRenderer(h2d_chunks=...): the H2D copy of chunk c + 1 overlaps
- * the kernels of chunk c inside ONE step; SURVEY 8f N1, renderer.py:67-77). */
-int mvr_mesh_prepare_range(const float* verts, const void* faces, const int* vert_off, const int* face_off,
-                           int B, int64_t total_verts, int64_t total_faces, int max_faces,
-                           const float* vert_rgb, int flags, void* geometry, size_t geometry_bytes,
-                           int obj_begin, int obj_end, int64_t vert_begin, int64_t vert_end, void* stream);
 /* copy of the per-vertex unit normals (Vtot,3) out of a prepared geometry (tests / callers) */
 int mvr_mesh_get_normals(const void* geometry, int64_t total_verts, int64_t total_faces,
                          float* normals, void* stream);
@@ -184,8 +170,7 @@ int mvr_mesh_normals_backward(const void* geometry, const int* vert_off, const i
                               float* grad_verts, void* stream);
 
 /* scratch for one forward or backward call: projected vertices of every view (16 B * M * total_verts), the
- * pixel-centre table, the 64-bit key plane(s) / backward partial sums and, for K == 1, the per-(view, tile) face lists of the
- * binned rasterizer (<= 24 B * M * total_faces) */
+ * pixel-centre table, the 64-bit key plane(s) (one for K == 1, two for K > 1) and the backward partial sums */
 size_t mvr_mesh_workspace_bytes(int B, int M, int H, int W, int K, int64_t total_verts, int64_t total_faces);
 /* MeshRenderer(MeshRasterizer, HardPhongShader)(meshes.extend(M), cameras, lights)
  * (renderer.py:89-113; [upstream] _C.rasterize_meshes + interp_face_attrs + phong_shading +

@@ -5,7 +5,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvr_b200.so")
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 PERSPECTIVE_CORRECT = 1
 CULL_BACKFACES = 2
 COMPOSITE_ALPHA = 4
@@ -19,7 +19,6 @@ WS_PROJECTED = 512
 IDX_SPARSE = 1024
 CLIP_BARYCENTRIC = 4096   # [upstream] clip_barycentric_coords
 FACES_U16 = 8192         # faces as uint16 (meshes of at most 65536 vertices): collate_meshes narrows when it can
-FORWARD_TILED = 2048     # mesh forward, K == 1: tile-binned rasterizer + shader (opt-in A/B alternative)
 TEST_TINY_QUEUES = 0x40000000   # tests only: shrink the scatter kernel's work queues to force their fallbacks
 CNT_STRADDLE, CNT_BIG_FACES, NUM_COUNTERS = 0, 1, 4
 
@@ -50,7 +49,6 @@ SIGNATURES = {
     "mvr_images_regularize_forward": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _vp, _vp]),
     "mvr_images_regularize_backward": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _vp, _vp]),
     "mvr_mesh_prepare": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _i64, _i, _vp, _i, _vp, _sz, _vp]),
-    "mvr_mesh_prepare_range": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _i64, _i, _vp, _i, _vp, _sz, _i, _i, _i64, _i64, _vp]),
     "mvr_mesh_get_normals": (_i, [_vp, _i64, _i64, _vp, _vp]),
     "mvr_mesh_normals_backward": (_i, [_vp, _vp, _vp, _i, _i64, _i64, _i, _vp, _vp, _vp]),
     "mvr_mesh_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i64, _i64]),

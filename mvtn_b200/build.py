@@ -15,7 +15,7 @@ LIB = os.path.join(HERE, "libmvr_b200.so")
 # source -> allow FMA contraction?  The forward units decide fragments and keep the written IEEE operation order
 # (-fmad=false); mvr_mesh_bwd.cu only produces tolerance-compared gradients from inputs that are exact by construction
 # (intrinsics in mvr_common.cuh / mvr_mesh.cuh) and is compiled with contraction.
-SOURCES = {"mvr_util.cu": False, "mvr_camera.cu": False, "mvr_mesh.cu": False, "mvr_mesh_clip.cu": False, "mvr_mesh_tile.cu": False, "mvr_mesh_soft.cu": False, "mvr_mesh_bwd.cu": True,
+SOURCES = {"mvr_util.cu": False, "mvr_camera.cu": False, "mvr_mesh.cu": False, "mvr_mesh_clip.cu": False, "mvr_mesh_soft.cu": False, "mvr_mesh_bwd.cu": True,
            "mvr_points.cu": False, "mvr_augment.cu": False}
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

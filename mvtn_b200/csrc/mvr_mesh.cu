@@ -467,21 +467,15 @@ extern "C" size_t mvr_mesh_geometry_bytes(int64_t total_verts, int64_t total_fac
   return geom_layout(total_verts, total_faces).total;
 }
 
-// objects [obj_begin, obj_end) of the batch, whose vertices are the packed rows [vert_begin, vert_end): every kernel indexes the
-// packed arrays absolutely, so a batch may be prepared piecewise (and rendered piecewise through vert_off + obj_begin) while the
-// rest of it is still on its way to the device
-extern "C" int mvr_mesh_prepare_range(const float* verts, const void* faces, const int* vert_off, const int* face_off,
-                                      int B, int64_t total_verts, int64_t total_faces, int max_faces,
-                                      const float* vert_rgb, int flags, void* geometry, size_t geometry_bytes,
-                                      int obj_begin, int obj_end, int64_t vert_begin, int64_t vert_end, void* stream) {
+extern "C" int mvr_mesh_prepare(const float* verts, const void* faces, const int* vert_off, const int* face_off,
+                                int B, int64_t total_verts, int64_t total_faces, int max_faces,
+                                const float* vert_rgb, int flags, void* geometry, size_t geometry_bytes,
+                                void* stream) {
   if (B < 0 || total_verts < 0 || total_faces < 0 || max_faces < 0) { set_error("mvr_mesh_prepare: negative size"); return -1; }
   if (total_verts > 0x7fffffffLL || total_faces > 0x7fffffffLL) { set_error("mvr_mesh_prepare: more than 2^31-1 packed verts/faces"); return -2; }
-  if (obj_begin < 0 || obj_end > B || obj_begin > obj_end || vert_begin < 0 || vert_end > total_verts || vert_begin > vert_end) {
-    set_error("mvr_mesh_prepare_range: objects [%d, %d) / vertices [%lld, %lld) outside the batch", obj_begin, obj_end, (long long)vert_begin, (long long)vert_end); return -6;
-  }
   const GeomLayout g = geom_layout(total_verts, total_faces);
   if (geometry_bytes < g.total) { set_error("mvr_mesh_prepare: geometry buffer too small (%zu < %zu)", geometry_bytes, g.total); return -3; }
-  if (obj_begin == obj_end || vert_begin == vert_end) return 0;
+  if (B == 0 || total_verts == 0) return 0;
   if (!verts || !vert_off || !face_off || !geometry || (total_faces > 0 && !faces)) { set_error("mvr_mesh_prepare: null pointer"); return -4; }
   if ((flags & MVR_RGB_PER_ELEMENT) && !vert_rgb) { set_error("mvr_mesh_prepare: MVR_RGB_PER_ELEMENT without vert_rgb"); return -5; }
   if ((flags & MVR_FACES_I64) && (flags & MVR_FACES_U16)) { set_error("mvr_mesh_prepare: MVR_FACES_I64 and MVR_FACES_U16 are exclusive"); return -7; }
@@ -493,26 +487,17 @@ extern "C" int mvr_mesh_prepare_range(const float* verts, const void* faces, con
   int4* faces4 = (int4*)(base + g.faces4);
   double* nacc = (double*)(base + g.nacc);
   const int tb = 256;
-  const int64_t nv = vert_end - vert_begin;
-  MVR_LAUNCH(geom_pack_verts_kernel, (unsigned)((nv + tb - 1) / tb), tb, 0, st, verts + 3 * vert_begin,
-             (flags & MVR_RGB_PER_ELEMENT) ? vert_rgb + 3 * vert_begin : nullptr, nv, verts4 + vert_begin, rgb4 + vert_begin, nacc + 3 * vert_begin);
+  MVR_LAUNCH(geom_pack_verts_kernel, (unsigned)((total_verts + tb - 1) / tb), tb, 0, st, verts,
+             (flags & MVR_RGB_PER_ELEMENT) ? vert_rgb : nullptr, total_verts, verts4, rgb4, nacc);
   if (total_faces > 0 && max_faces > 0) {
-    dim3 grid((max_faces + tb - 1) / tb, obj_end - obj_begin);
-    if (flags & MVR_FACES_I64) MVR_LAUNCH_PDL(geom_pack_faces_kernel<long long>, grid, tb, 0, st, (const long long*)faces, vert_off + obj_begin, face_off + obj_begin, verts4, faces4, nacc);
-    else if (flags & MVR_FACES_U16) MVR_LAUNCH_PDL(geom_pack_faces_kernel<unsigned short>, grid, tb, 0, st, (const unsigned short*)faces, vert_off + obj_begin, face_off + obj_begin, verts4, faces4, nacc);
-    else MVR_LAUNCH_PDL(geom_pack_faces_kernel<int>, grid, tb, 0, st, (const int*)faces, vert_off + obj_begin, face_off + obj_begin, verts4, faces4, nacc);
+    dim3 grid((max_faces + tb - 1) / tb, B);
+    if (flags & MVR_FACES_I64) MVR_LAUNCH_PDL(geom_pack_faces_kernel<long long>, grid, tb, 0, st, (const long long*)faces, vert_off, face_off, verts4, faces4, nacc);
+    else if (flags & MVR_FACES_U16) MVR_LAUNCH_PDL(geom_pack_faces_kernel<unsigned short>, grid, tb, 0, st, (const unsigned short*)faces, vert_off, face_off, verts4, faces4, nacc);
+    else MVR_LAUNCH_PDL(geom_pack_faces_kernel<int>, grid, tb, 0, st, (const int*)faces, vert_off, face_off, verts4, faces4, nacc);
   }
-  MVR_LAUNCH_PDL(geom_finish_normals_kernel, (unsigned)((nv + tb - 1) / tb), tb, 0, st, nacc + 3 * vert_begin, nv, verts4 + vert_begin, normals4 + vert_begin,
-             (float4*)(base + g.xn8) + 2 * vert_begin);
+  MVR_LAUNCH_PDL(geom_finish_normals_kernel, (unsigned)((total_verts + tb - 1) / tb), tb, 0, st, nacc, total_verts, verts4, normals4,
+                 (float4*)(base + g.xn8));
   return check_launch("mvr_mesh_prepare");
-}
-
-extern "C" int mvr_mesh_prepare(const float* verts, const void* faces, const int* vert_off, const int* face_off,
-                                int B, int64_t total_verts, int64_t total_faces, int max_faces,
-                                const float* vert_rgb, int flags, void* geometry, size_t geometry_bytes,
-                                void* stream) {
-  return mvr_mesh_prepare_range(verts, faces, vert_off, face_off, B, total_verts, total_faces, max_faces, vert_rgb, flags, geometry,
-                                geometry_bytes, 0, B > 0 ? B : 0, 0, total_verts > 0 ? total_verts : 0, stream);
 }
 
 extern "C" int mvr_mesh_get_normals(const void* geometry, int64_t total_verts, int64_t total_faces, float* normals, void* stream) {
@@ -633,7 +618,6 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
     p.jx_scale = (float)W / rx; p.jx_off = (0.5f * rx * (float)W - 0.5f * rx) / rx;
     p.jy_scale = (float)H / ry; p.jy_off = (0.5f * ry * (float)H - 0.5f * ry) / ry;
   }
-  p.item_cap = (flags & MVR_TEST_TINY_QUEUES) ? 24 : ITEM_CAP;
   p.wcap = (flags & MVR_TEST_TINY_QUEUES) ? 40 : SC_QCAP;      // candidate queue of a round (scatter kernel)
   p.pv = (float4*)(wb + w.pv); p.tab = (float*)(wb + w.tab);
   p.keys = (unsigned long long*)(wb + w.keys); p.prev = (unsigned long long*)(wb + w.prev);
@@ -643,18 +627,6 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
   p.wsflags = (int*)(wb + w.flags);
   const size_t HW = (size_t)H * W;
   const bool soft_raster = p.blur_radius > 0.f || (flags & MVR_CLIP_BARYCENTRIC);
-  if (K == 1 && !soft_raster && ((flags & MVR_FORWARD_TILED) || mesh_tiled_enabled())) {
-    // tile-binned path (mvr_mesh_tile.cu): keys live in shared memory -- no key plane, no memset of it, no separate shade pass
-    p.flags &= ~(MVR_WS_KEYS_ARMED | MVR_WS_REARM_KEYS);
-    cudaError_t e = cudaMemsetAsync(wb + w.flags, 0xFF, 4 * sizeof(int), st);      // arms WSF_CLIP
-    if (e != cudaSuccess) { set_error("mvr_mesh_forward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return (int)e; }
-    rc = launch_project("mesh_project_kernel", g, w, geometry, vert_off, R, T, B, M, H, W, max_verts, k00, k11, z_clip, false, workspace, st, (long long*)counters);
-    if (rc) return rc;
-    rc = launch_mesh_forward_tiled(p, w, workspace, B, M, max_faces, zbuf || bary || dists, st);
-    if (rc) return rc;
-    if (z_clip >= 0.f) rc = launch_mesh_shade_clipped(p, (int)N, st);
-    return rc;
-  }
   // every key = EMPTY, and the workspace flags right in front of the plane armed (WSF_CLIP)
   const size_t plane_bytes = (flags & MVR_WS_KEYS_ARMED) ? 0 : (size_t)N * HW * 8;
   cudaError_t e = cudaMemsetAsync(wb + w.flags, 0xFF, (w.keys - w.flags) + plane_bytes, st);

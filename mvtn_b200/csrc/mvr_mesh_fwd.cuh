@@ -1,7 +1,6 @@
-// mvr_mesh_fwd.cuh -- device code shared by the two forward rasterizers of the mesh path: the bin-free scatter onto a
-// global key plane (mvr_mesh.cu: faces_per_pixel > 1) and the tile-binned fused rasterizer + shader (mvr_mesh_tile.cu:
-// faces_per_pixel == 1).  Both translation units are compiled with -fmad=false: everything here that decides a fragment
-// is IEEE fp32 in the written order.
+// mvr_mesh_fwd.cuh -- device code of the mesh path's forward rasterizer, the bin-free scatter onto a global key plane
+// (mvr_mesh.cu): face setup, the scanline candidate spans and the exact per-(face, pixel) test.  mvr_mesh.cu is compiled
+// with -fmad=false: everything here that decides a fragment is IEEE fp32 in the written order.
 #pragma once
 #include "mvr_mesh.cuh"
 
@@ -62,16 +61,6 @@ __device__ __forceinline__ unsigned int smem_addr_pinned(const void* ptr) {
   asm volatile("{ .reg .u64 t; cvta.to.shared.u64 t, %1; cvt.u32.u64 %0, t; }" : "=r"(a) : "l"(ptr));
   return a;
 }
-__device__ __forceinline__ unsigned int lanemask_lt() {
-  unsigned int m;
-  asm volatile("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
-  return m;
-}
-__device__ __forceinline__ float lds_f32(unsigned int a) {
-  float v;
-  asm("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
 __device__ __forceinline__ void sts_u32(unsigned int a, unsigned int v) {
   asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
 }
@@ -131,65 +120,17 @@ __device__ __forceinline__ void resolve_pixel_with(const Face& fc, const FaceEdg
   atomicMin(key_ptr, key);      // result unused: RED.MIN.64 resolved in L2
 }
 
-// Phase B's pixel filter in FMA form.  Edge function i of the oracle, e_i = (px - xa) A - (py - ya) B (five IEEE
+// The pixel filter in FMA form.  Edge function i of the oracle, e_i = (px - xa) A - (py - ya) B (five IEEE
 // operations), is evaluated as fma(px, A, fma(-py, B, C)) with C = ya B - xa A: two instructions.  The two differ by
 // rounding only: with u = 2^-24, |px|, |py| <= pmax (1, or the aspect ratio of a non-square image) and
 // S = (pmax + |xa|) |A| + (pmax + |ya|) |B|, the IEEE sequence is within
 // 3 u S of the real value and the FMA form within 4 u S, so adding 16 u S to C makes "fma form > 0" a NECESSARY condition
-// for "IEEE form > 0": the filter never drops a pixel the exact test of phase C would accept, it only lets a few pixels
-// within 2^-20 S of an edge through to be rejected there.  The sign of the area is folded into (A, B, C) first (negation
-// is exact).  Record words 12..20 of the face: (A0, B0, C0', A1, B1, C1', A2, B2, C2').
-__device__ __forceinline__ void store_filter_edges(const Face& f, float pmax, float* rec) {
-  float A[3] = {f.y2 - f.y1, f.y0 - f.y2, f.y1 - f.y0};
-  float B[3] = {f.x2 - f.x1, f.x0 - f.x2, f.x1 - f.x0};
-  const float xa[3] = {f.x1, f.x2, f.x0}, ya[3] = {f.y1, f.y2, f.y0};
-  const float area_p = ((f.x2 - f.x0) * A[2] - (f.y2 - f.y0) * B[2]) + MVR_K_EPS;
-  const bool flip = !(area_p > 0.f);
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    if (flip) { A[i] = -A[i]; B[i] = -B[i]; }
-    const float C = ya[i] * B[i] - xa[i] * A[i];
-    const float S = (pmax + fabsf(xa[i])) * fabsf(A[i]) + (pmax + fabsf(ya[i])) * fabsf(B[i]);
-    rec[(3 * i + 0) * MVR_THREADS] = A[i];
-    rec[(3 * i + 1) * MVR_THREADS] = B[i];
-    rec[(3 * i + 2) * MVR_THREADS] = C + 9.5367431640625e-07f * S;      // 2^-20
-  }
-}
-
-// Phase B as a SCANLINE: the pixels of one bbox row that can pass the edge filter form an interval, and its end points come
-// from the three filter inequalities  fma(xf, A_i, t_i) > 0,  t_i = fma(-yf, B_i, C_i)  (store_filter_edges) solved for xf:
-// xf > -t_i / A_i where A_i > 0, xf < -t_i / A_i where A_i < 0 (fma(xf, A, t) > 0 implies xf A + t > 0 in the reals: rounding
-// to nearest never changes the sign of a non-zero value, and a real value <= 0 never rounds above 0).  The bounds are
-// evaluated with an SFU reciprocal (<= 2 ulp on -t / A) and mapped to pixel columns through the inverse pixel map widened by
-// 8e-3 pixel -- an order of magnitude above the accumulated rounding (bound, map, pixel-centre table: ~1e-3 pixel at 4096
-// columns) -- so the interval is a SUPERSET of the filter's pixels, themselves a superset of the oracle's.  Which of them are
-// fragments is phase C's exact test.  A face of 17 bbox pixels has ~4.6 inside (C2): the per-pixel filter loop of earlier
-// versions spent 3/4 of its lanes on pixels a closed form can exclude.
-// Returns the number of candidate columns; xs = the first one (pixel index, xl <= xs, xs + count - 1 <= xl + bw - 1).
-__device__ __forceinline__ int row_span(const float* __restrict__ rec /* &s_rec[12][slot] */, int stride, float yf, int xl, int bw, int W,
-                                        float jx_scale, float jx_off, int& xs) {
-  float lo = -3.0e38f, hi = 3.0e38f;
-  bool empty = false;
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    const float A = rec[(3 * i + 0) * stride], B = rec[(3 * i + 1) * stride], Cc = rec[(3 * i + 2) * stride];
-    const float t = fmaf(-yf, B, Cc);
-    if (fabsf(A) < 1e-30f) { empty = empty || !(t > 0.f); }      // no x dependence: the row passes or fails as a whole
-    else {
-      const float bnd = -t * rcp_fast(A);
-      if (A > 0.f) lo = fmaxf(lo, bnd); else hi = fminf(hi, bnd);
-    }
-  }
-  // flipped column j grows with x; pixel index i = W - 1 - j
-  float jlo = ceilf(fmaf(lo, jx_scale, jx_off) - 8e-3f), jhi = floorf(fmaf(hi, jx_scale, jx_off) + 8e-3f);
-  jlo = fminf(fmaxf(jlo, -1.0f), (float)W); jhi = fminf(fmaxf(jhi, -1.0f), (float)W);      // (NaN -> -1)
-  const int i_lo = max(W - 1 - (int)jhi, xl), i_hi = min(W - 1 - (int)jlo, xl + bw - 1);
-  xs = i_lo;
-  return empty ? 0 : max(i_hi - i_lo + 1, 0);
-}
-
-// register-resident variant for the scatter kernel, where the thread that set a face up also walks its rows: per edge the
-// coefficients (B, C') of t(y) = fma(-y, B, C'), the reciprocal of A, and its class (flat / lower bound / upper bound)
+// for "IEEE form > 0": the filter never drops a pixel the exact test (resolve_pixel_with) would accept, it only lets a few
+// pixels within 2^-20 S of an edge through to be rejected there.  The sign of the area is folded into (A, B, C) first
+// (negation is exact).
+// span_edges keeps the filter in registers -- the thread that set a face up also walks its rows: per edge the
+// coefficients (B, C' = C + 2^-20 S) of t(y) = fma(-y, B, C'), the reciprocal of A, and its class (flat / lower bound /
+// upper bound)
 struct SpanEdges {
   float B[3], C[3], rA[3];
   int cls;      // 2 bits per edge: 0 = no x dependence, 1 = lower bound on x (A > 0), 2 = upper bound (A < 0)
@@ -203,18 +144,30 @@ __device__ __forceinline__ SpanEdges span_edges(const Face& f, float pmax) {
   const bool flip = !(area_p > 0.f);
   se.cls = 0;
 #pragma unroll
-  for (int i = 0; i < 3; ++i) {      // same (A, B, C + 2^-20 S) as store_filter_edges
+  for (int i = 0; i < 3; ++i) {
     if (flip) { A[i] = -A[i]; B[i] = -B[i]; }
     const float C = ya[i] * B[i] - xa[i] * A[i];
     const float S = (pmax + fabsf(xa[i])) * fabsf(A[i]) + (pmax + fabsf(ya[i])) * fabsf(B[i]);
     se.B[i] = B[i];
-    se.C[i] = C + 9.5367431640625e-07f * S;
+    se.C[i] = C + 9.5367431640625e-07f * S;      // 2^-20
     const bool flat = fabsf(A[i]) < 1e-30f;
     se.rA[i] = flat ? 0.f : rcp_fast(A[i]);
     se.cls |= (flat ? 0 : (A[i] > 0.f ? 1 : 2)) << (2 * i);
   }
   return se;
 }
+
+// The filter as a SCANLINE: the pixels of one bbox row that can pass it form an interval, and its end points come from the
+// three filter inequalities  fma(xf, A_i, t_i) > 0,  t_i = fma(-yf, B_i, C_i')  (span_edges) solved for xf:
+// xf > -t_i / A_i where A_i > 0, xf < -t_i / A_i where A_i < 0 (fma(xf, A, t) > 0 implies xf A + t > 0 in the reals: rounding
+// to nearest never changes the sign of a non-zero value, and a real value <= 0 never rounds above 0).  An edge with no x
+// dependence passes or fails the row as a whole.  The bounds are evaluated with an SFU reciprocal (<= 2 ulp on -t / A) and
+// mapped to pixel columns (flipped column j grows with x; pixel index i = W - 1 - j) through the inverse pixel map widened
+// by 8e-3 pixel -- an order of magnitude above the accumulated rounding (bound, map, pixel-centre table: ~1e-3 pixel at
+// 4096 columns) -- so the interval is a SUPERSET of the filter's pixels, themselves a superset of the oracle's.  Which of
+// them are fragments is the exact test's decision.  A face of 17 bbox pixels has ~4.6 inside (C2): a per-pixel filter loop
+// spends 3/4 of its lanes on pixels this closed form excludes.
+// Returns the number of candidate columns; xs = the first one (pixel index, xl <= xs, xs + count - 1 <= xl + bw - 1).
 __device__ __forceinline__ int row_span_regs(const SpanEdges& se, float yf, int xl, int bw, int W, float jx_scale, float jx_off, int& xs) {
   float lo = -3.0e38f, hi = 3.0e38f;
   bool empty = false;

@@ -555,14 +555,10 @@ class PackedMeshes:
                                           overlap, offs_h, offs)
         return (v_dev, f_dev, nv, nf, device, vert_rgb, job, keep, offs)
 
-    def finish(self, lazy_chunks: bool = False):
+    def finish(self):
         """Stage (if deferred) or join the staging job (if overlapped), then build the packed device geometry
-        (mvr_mesh_prepare).  Idempotent.  lazy_chunks=True leaves the groups of a chunked batch (from_host_packed(chunks=k))
-        to the render launches, which prepare each one just before they render it."""
+        (mvr_mesh_prepare).  Idempotent."""
         if self._pending is None:
-            if self._chunks and not lazy_chunks:
-                for i in range(len(self._chunks)):
-                    self.finish_chunk(i)
             return self
         pending, self._pending = self._pending, None
         if PackedMeshes._inflight is self:
@@ -587,16 +583,11 @@ class PackedMeshes:
         return self
 
     @classmethod
-    def from_host_packed(cls, hp: "HostPackedMeshes", device, vert_rgb: Optional[torch.Tensor] = None, copy_stream: bool = False,
-                         chunks: int = 1):
+    def from_host_packed(cls, hp: "HostPackedMeshes", device, vert_rgb: Optional[torch.Tensor] = None, copy_stream: bool = False):
         """Two async H2D copies of an already packed (ideally pinned) host batch + mvr_mesh_prepare.
         copy_stream=True: the copies go through a dedicated stream (the compute stream waits on an event), so that in a
         loop that does not synchronise every step they overlap with the previous step's kernels instead of queueing
-        behind them (5.8 MB = 0.11 ms per step at C2).
-        chunks=k > 1: the batch travels as k groups of objects on that stream, an event behind each; the geometry of group c
-        is prepared (mvr_mesh_prepare_range) and rendered as soon as ITS event has fired, while group c + 1 is still on
-        the bus -- the copy overlaps the kernels inside one step, also in a loop that synchronises every step.  The
-        groups are finished lazily by the render launches (finish_chunk); finish() completes them all."""
+        behind them (5.8 MB = 0.11 ms per step at C2)."""
         device = torch.device(device)
         if device.type != "cuda":
             raise L.MVRError("PackedMeshes needs a CUDA device: mvtn_b200 has no CPU path")
@@ -615,39 +606,6 @@ class PackedMeshes:
             staged = True
         else:
             staged = False
-        rgb = vert_rgb if vert_rgb is not None else hp.vert_rgb
-        B = len(hp)
-        chunks = max(1, min(int(chunks), B))
-        if rgb is not None or hp.verts.shape[0] == 0:
-            chunks = 1
-        if chunks > 1:
-            cur = torch.cuda.current_stream(device)
-            cs = _copy_streams.get(device.index)
-            if cs is None:
-                cs = _copy_streams[device.index] = torch.cuda.Stream(device)
-            bounds = [(B * c) // chunks for c in range(chunks + 1)]
-            plan = []
-            with torch.cuda.stream(cs):
-                offs = hp.offs.to(device, non_blocking=True)
-                v_dev = torch.empty((hp.verts.shape[0], 3), dtype=torch.float32, device=device)
-                f_dev = torch.empty((hp.faces.shape[0], 3), dtype=hp.faces.dtype, device=device)
-                for c in range(chunks):
-                    b0, b1 = bounds[c], bounds[c + 1]
-                    v0, v1 = hp.vert_off_host[b0], hp.vert_off_host[b1]
-                    f0, f1 = hp.face_off_host[b0], hp.face_off_host[b1]
-                    v_dev[v0:v1].copy_(hp.verts[v0:v1], non_blocking=True)
-                    f_dev[f0:f1].copy_(hp.faces[f0:f1], non_blocking=True)
-                    ev = torch.cuda.Event()
-                    ev.record(cs)
-                    plan.append([b0, b1, v0, v1, ev])
-            for t in (v_dev, f_dev, offs):
-                t.record_stream(cur)
-            if staged:
-                _staging_done(device)
-            self._init_packed(v_dev, f_dev, hp.num_verts, hp.num_faces, device, None,
-                              offsets=(hp.vert_off_host, hp.face_off_host, offs), prepare=False)
-            self._chunks = plan
-            return self
         if copy_stream:
             cur = torch.cuda.current_stream(device)
             cs = _copy_streams.get(device.index)
@@ -666,34 +624,10 @@ class PackedMeshes:
             offs = hp.offs.to(device, non_blocking=True)
         if staged:
             _staging_done(device)
-        self._init_packed(v_dev, f_dev, hp.num_verts, hp.num_faces, device, rgb,
+        self._init_packed(v_dev, f_dev, hp.num_verts, hp.num_faces, device,
+                          vert_rgb if vert_rgb is not None else hp.vert_rgb,
                           offsets=(hp.vert_off_host, hp.face_off_host, offs))
         return self
-
-    # -- chunked staging (from_host_packed(chunks=k)) --
-    _chunks = None
-
-    def chunk_ranges(self):
-        """[(obj_begin, obj_end)] the render launches walk: the staging groups, or the whole batch."""
-        if self._chunks:
-            return [(c[0], c[1]) for c in self._chunks]
-        return [(0, self.B)]
-
-    def finish_chunk(self, i: int):
-        """The compute stream waits for group i's copy, then prepares its objects.  Idempotent; no-op without chunks."""
-        if not self._chunks:
-            return
-        c = self._chunks[i]
-        if c[4] is None:
-            return
-        b0, b1, v0, v1, ev = c
-        c[4] = None
-        torch.cuda.current_stream(self.device).wait_event(ev)
-        with _on(self.device):
-            L.check(L.load().mvr_mesh_prepare_range(_ptr(self.verts), _ptr(self.faces), _ptr(self.vert_off), _ptr(self.face_off),
-                                                    self.B, self.total_verts, self.total_faces, self.max_faces, None,
-                                                    self._prep_flags, _ptr(self.geometry), self.geometry.numel(),
-                                                    b0, b1, v0, v1, _stream(self.device)), "mvr_mesh_prepare_range")
 
     @classmethod
     def from_packed(cls, verts: torch.Tensor, faces: torch.Tensor, num_verts: Sequence[int], num_faces: Sequence[int],
@@ -754,11 +688,6 @@ class PackedMeshes:
         (mvr_mesh_prepare): call it after updating self.verts in place.  Pure device work on the current stream."""
         if self.B == 0:
             return self
-        if self._chunks:      # every group must have arrived; they are all rebuilt below
-            for c in self._chunks:
-                if c[4] is not None:
-                    torch.cuda.current_stream(self.device).wait_event(c[4])
-                    c[4] = None
         with _on(self.device):
             L.check(L.load().mvr_mesh_prepare(_ptr(self.verts), _ptr(self.faces), _ptr(self.vert_off), _ptr(self.face_off),
                                               self.B, self.total_verts, self.total_faces, self.max_faces, _ptr(self._rgb),
@@ -815,38 +744,18 @@ def _mesh_forward_launch(geom: "PackedMeshes", M, R, T, Cc, light, obj_rgb, bg_r
         zbuf = torch.empty((N, H, W, K), dtype=torch.float32, device=dev)
         bary = torch.empty((N, H, W, K, 3), dtype=torch.float32, device=dev)
         dists = torch.empty((N, H, W, K), dtype=torch.float32, device=dev)
-    # One launch for the whole batch -- or one per staging group of a chunked batch (PackedMeshes.from_host_packed(chunks=k)):
-    # objects [b0, b1) are addressed through vert_off + b0 / face_off + b0 (every kernel indexes the packed arrays
-    # absolutely) and views [b0 M, b1 M) through offset views of the per-view tensors; group c is prepared right before it
-    # is rendered, while group c + 1 is still being copied.
-    ranges = geom.chunk_ranges() if (blur_radius == 0.0 and not want_fragments) else [(0, geom.B)]
-    if len(ranges) == 1:
-        geom.finish()
-    counters = torch.empty((len(ranges), L.NUM_COUNTERS), dtype=torch.int64, device=dev)      # zeroed by mvr_mesh_forward
-    tokens = []
-    for ci, (b0, b1) in enumerate(ranges):
-        if len(ranges) > 1:
-            geom.finish_chunk(ci)
-        Bc, n0, n1 = b1 - b0, b0 * M, b1 * M
-        ws_bytes = lib.mvr_mesh_workspace_bytes(Bc, M, H, W, K, geom.total_verts, geom.total_faces)
-        ws = workspace(dev, ws_bytes, _mesh_owner=True)
-        ws_flags, ws_commit = _ws_mesh_flags_forward(dev, ws, (Bc, M, H, W, K, geom.total_verts))
-        if len(ranges) == 1:      # (no views of views on the one-launch path: host microseconds in front of this call are step time)
-            sl = lambda t: t
-            voff, foff, lt, cnt = geom.vert_off, geom.face_off, light, counters
-        else:
-            sl = lambda t: None if t is None else t[n0:n1]
-            voff, foff, lt, cnt = geom.vert_off[b0:], geom.face_off[b0:], (light if light_stride == 0 else light[n0:n1]), counters[ci]
-        with _on(dev):
-            L.check(lib.mvr_mesh_forward(_ptr(geom.geometry), _ptr(voff), _ptr(foff), Bc, M,
-                                         geom.total_verts, geom.total_faces, geom.max_verts, geom.max_faces, _ptr(sl(R)), _ptr(sl(T)),
-                                         _ptr(sl(Cc)), _ptr(lt), light_stride, _ptr(obj_rgb),
-                                         _ptr(bg_rgb), k00, k11, z_clip, float(blur_radius), H, W,
-                                         K, flags | ws_flags, out_norm, _ptr(sl(images)), _ptr(sl(p2f)), _ptr(sl(zbuf)), _ptr(sl(bary)),
-                                         _ptr(sl(dists)), _ptr(cnt), _ptr(ws), ws.numel(), _stream(dev)), "mvr_mesh_forward")
-        tokens.append(ws_commit())
-    counters = counters.view(-1) if len(ranges) == 1 else counters.sum(0)
-    cfg = (k00, k11, H, W, K, flags, out_norm, light_stride, z_clip, (ranges, tokens))
+    geom.finish()
+    counters = torch.empty(L.NUM_COUNTERS, dtype=torch.int64, device=dev)      # zeroed by mvr_mesh_forward
+    ws_bytes = lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, K, geom.total_verts, geom.total_faces)
+    ws = workspace(dev, ws_bytes, _mesh_owner=True)
+    ws_flags, ws_commit = _ws_mesh_flags_forward(dev, ws, (geom.B, M, H, W, K, geom.total_verts))
+    with _on(dev):
+        L.check(lib.mvr_mesh_forward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                     geom.total_verts, geom.total_faces, geom.max_verts, geom.max_faces, _ptr(R), _ptr(T), _ptr(Cc),
+                                     _ptr(light), light_stride, _ptr(obj_rgb), _ptr(bg_rgb), k00, k11, z_clip, float(blur_radius), H, W,
+                                     K, flags | ws_flags, out_norm, _ptr(images), _ptr(p2f), _ptr(zbuf), _ptr(bary), _ptr(dists),
+                                     _ptr(counters), _ptr(ws), ws.numel(), _stream(dev)), "mvr_mesh_forward")
+    cfg = (k00, k11, H, W, K, flags, out_norm, light_stride, z_clip, ws_commit())
     saved = (R, T, Cc, light, obj_rgb if obj_rgb is not None else bg_rgb, p2f)
     extras = [p2f, counters]
     if want_fragments:
@@ -855,16 +764,15 @@ def _mesh_forward_launch(geom: "PackedMeshes", M, R, T, Cc, light, obj_rgb, bg_r
 
 
 def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_verts, angles=None):
-    """mvr_mesh_backward (one call per staging group of the forward) -> (gR, gT, gC, gV | None) (gV includes the chain through
-    the vertex normals).  angles = (azim, elev, dist) flat fp32: mvr_mesh_backward_angles instead, whose last kernel also applies
-    the camera backward -> (g_azim, g_elev, g_dist, gV | None)."""
+    """ONE mvr_mesh_backward call -> (gR, gT, gC, gV | None) (gV includes the chain through the vertex normals).  angles =
+    (azim, elev, dist) flat fp32: mvr_mesh_backward_angles instead, whose last kernel also applies the camera backward ->
+    (g_azim, g_elev, g_dist, gV | None)."""
     lib = L.load()
     R, T, Cc, light, obj_rgb, p2f = saved
-    k00, k11, H, W, K, flags, out_norm, light_stride, z_clip, (ranges, tokens) = cfg
+    k00, k11, H, W, K, flags, out_norm, light_stride, z_clip, ws_token = cfg
     dev = geom.device
     N = geom.B * M
     g_images = _grad_like_images(g_images, flags)
-    # three separate (N, .) blocks, so that a group's views are a contiguous slice of each
     if angles is None:
         g = torch.empty(15 * N, dtype=torch.float32, device=dev)
         gR, gT, gC = g[: 9 * N].view(N, 3, 3), g[9 * N: 12 * N].view(N, 3), g[12 * N:].view(N, 3)
@@ -875,33 +783,24 @@ def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_ve
     if want_verts:
         gV = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
         gN = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
-    for ci in reversed(range(len(ranges))):      # last group first: its projected vertices may still be in the workspace
-        b0, b1 = ranges[ci]
-        Bc, n0, n1 = b1 - b0, b0 * M, b1 * M
-        ws_bytes = lib.mvr_mesh_workspace_bytes(Bc, M, H, W, K, geom.total_verts, geom.total_faces)
-        ws = workspace(dev, ws_bytes, _mesh_owner=True)
-        fl = flags | _ws_mesh_flags_backward(dev, ws, tokens[ci])
-        if len(ranges) == 1:
-            sl = lambda t: t
-            voff, foff, lt = geom.vert_off, geom.face_off, light
-        else:
-            sl = lambda t: t[n0:n1]
-            voff, foff, lt = geom.vert_off[b0:], geom.face_off[b0:], (light if light_stride == 0 else light[n0:n1])
-        if angles is not None:
-            az, el, di = angles
-            with _on(dev):
-                L.check(lib.mvr_mesh_backward_angles(_ptr(geom.geometry), _ptr(voff), _ptr(foff), Bc, M, geom.total_verts, geom.total_faces,
-                                                     geom.max_verts, _ptr(sl(R)), _ptr(sl(T)), _ptr(sl(Cc)), _ptr(lt), light_stride,
-                                                     _ptr(obj_rgb), k00, k11, z_clip, H, W, K, fl, out_norm, _ptr(sl(p2f)),
-                                                     _ptr(sl(g_images)), _ptr(sl(az)), _ptr(sl(el)), _ptr(sl(di)), _ptr(sl(ga)), _ptr(sl(ge)),
-                                                     _ptr(sl(gd)), None, None, None, _ptr(gV), _ptr(gN), _ptr(ws), ws.numel(),
-                                                     _stream(dev)), "mvr_mesh_backward_angles")
-            continue
+    ws_bytes = lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, K, geom.total_verts, geom.total_faces)
+    ws = workspace(dev, ws_bytes, _mesh_owner=True)
+    flags = flags | _ws_mesh_flags_backward(dev, ws, ws_token)
+    if angles is not None:
+        az, el, di = angles
         with _on(dev):
-            L.check(lib.mvr_mesh_backward(_ptr(geom.geometry), _ptr(voff), _ptr(foff), Bc, M,
-                                          geom.total_verts, geom.total_faces, geom.max_verts, _ptr(sl(R)), _ptr(sl(T)), _ptr(sl(Cc)), _ptr(lt),
-                                          light_stride, _ptr(obj_rgb), k00, k11, z_clip, H, W, K, fl, out_norm, _ptr(sl(p2f)),
-                                          _ptr(sl(g_images)), _ptr(sl(gR)), _ptr(sl(gT)), _ptr(sl(gC)), _ptr(gV), _ptr(gN), _ptr(ws),
+            L.check(lib.mvr_mesh_backward_angles(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                                 geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc),
+                                                 _ptr(light), light_stride, _ptr(obj_rgb), k00, k11, z_clip, H, W, K, flags, out_norm,
+                                                 _ptr(p2f), _ptr(g_images), _ptr(az), _ptr(el), _ptr(di), _ptr(ga), _ptr(ge), _ptr(gd),
+                                                 None, None, None, _ptr(gV), _ptr(gN), _ptr(ws), ws.numel(),
+                                                 _stream(dev)), "mvr_mesh_backward_angles")
+    else:
+        with _on(dev):
+            L.check(lib.mvr_mesh_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                          geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc), _ptr(light),
+                                          light_stride, _ptr(obj_rgb), k00, k11, z_clip, H, W, K, flags, out_norm, _ptr(p2f),
+                                          _ptr(g_images), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(gV), _ptr(gN), _ptr(ws),
                                           ws.numel(), _stream(dev)), "mvr_mesh_backward")
     if gV is not None:
         # the kernel returned d/d verts through projection + interpolated position, and d/d unit normals; the
@@ -953,7 +852,7 @@ class _MeshRenderFromAngles(torch.autograd.Function):
         a, e, d, R, T, Cc, bad = _look_at_launch(azim, elev, dist, sink)
         if after_cameras is not None and sink is None:
             after_cameras(bad)
-        geom.finish(lazy_chunks=True)      # a deferred / worker-thread staging (PackedMeshes.begin) ends here, behind the camera launch
+        geom.finish()      # a deferred / worker-thread staging (PackedMeshes.begin) ends here, behind the camera launch
         cfg, saved, images, extras = _mesh_forward_launch(geom, M, R, T, Cc, Cc if light is None else light, obj_rgb, bg_rgb,
                                                           k00, k11, z_clip, H, W, K, flags, False, out_norm, out_dtype)
         ctx.set_materialize_grads(False)

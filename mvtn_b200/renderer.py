@@ -107,12 +107,6 @@ class MVRenderer(nn.Module):
             calling thread's OpenMP team would have to be woken for every batch), 1.27 vs 1.28 with the policy unset (the team is still
             spinning from the previous batch: no gain, no loss); with OMP_WAIT_POLICY=active every core is taken by a spinning OpenMP
             worker and the staging threads queue behind them (1.26 ... 1.45 ms vs 1.29) -- pass False there.
-        h2d_chunks: how many groups of objects a collated host batch (collate_meshes) travels in (default 1).  With k > 1 group c
-            is prepared and rendered as soon as its own copy has landed, while group c + 1 is still on the bus (one forward and
-            one backward launch per group, same images / fragments / gradients bit for bit).  Measured on B200 it does NOT pay at
-            MVTN's sizes: the step's first 0.3 ms are bound by the host reaching the rasterizer launch, not by the 0.18 ms copy,
-            and every group adds launches (1.09 -> 1.27 ms per end-to-end step at 32 x 12 views with k = 2;
-            profiles/r3y_h2d_chunks.txt) -- kept for batches whose copy does dominate (large meshes, slow links).
         cuda_graph (mesh path): only when True, and only for collated host batches (collate_meshes) rendered with the hard Phong
             shader: the device part of the forward and of the backward -- mvr_mesh_prepare, look_at, rasterizer, shader -- is captured
             once per batch SHAPE (the per-mesh vertex / face counts, views-require-grad) and replayed; a batch of another shape is
@@ -147,9 +141,8 @@ class MVRenderer(nn.Module):
                  faces_per_pixel=1, points_radius=0.006, points_per_pixel=1, light_direction="random",
                  cull_backfaces=False, *, compositor="norm", perspective_correct=True, cache_geometry=False,
                  normalize=None, out_dtype=None, copy_stream=False, cuda_graph=None, shader="hard_phong", blur_radius=0.0,
-                 blend_sigma=1e-4, blend_gamma=1e-4, keep_alpha=False, h2d_chunks=1, stage_overlap=True):
+                 blend_sigma=1e-4, blend_gamma=1e-4, keep_alpha=False, stage_overlap=True):
         super().__init__()
-        self.h2d_chunks = h2d_chunks
         self.stage_overlap = bool(stage_overlap)
         self.shader, self.blur_radius, self.blend_sigma, self.blend_gamma, self.keep_alpha = shader, blur_radius, blend_sigma, blend_gamma, keep_alpha
         self.copy_stream = copy_stream
@@ -250,7 +243,7 @@ class MVRenderer(nn.Module):
         soft = self.shader != "hard_phong"
 
         def render(R, T, C, dist_, C_light):
-            geom.finish(lazy_chunks=not soft)      # (the groups of a chunked batch are finished by the render launches)
+            geom.finish()
             light = C_light if fixed_light is None else fixed_light
             if soft:
                 return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
@@ -481,8 +474,7 @@ class MVRenderer(nn.Module):
             if color_t.numel() != 3:
                 color_t = color_t.reshape(len(meshes), -1, 3)
                 vert_rgb = torch.cat([color_t[b, :n] for b, n in enumerate(meshes.num_verts)], 0)
-            chunks = self.h2d_chunks if self.shader == "hard_phong" else 1
-            return ops.PackedMeshes.from_host_packed(meshes, device, vert_rgb=vert_rgb, copy_stream=self.copy_stream, chunks=chunks)
+            return ops.PackedMeshes.from_host_packed(meshes, device, vert_rgb=vert_rgb, copy_stream=self.copy_stream)
         if meshes is None:
             raise ValueError("mesh rendering (pc_rendering=False) needs `meshes`")
         if self.cache_geometry and self._geom_cache[0] is meshes:

@@ -30,7 +30,7 @@ def wrap(name):
         return rc
     setattr(lib, name, w)
 
-for n in ("mvr_host_stage_meshes_packed", "mvr_host_stage_meshes_packed_begin", "mvr_host_stage_meshes_end", "mvr_look_at_forward", "mvr_look_at_forward_flagged", "mvr_mesh_prepare", "mvr_mesh_prepare_range", "mvr_mesh_forward", "mvr_mesh_backward", "mvr_mesh_backward_angles", "mvr_look_at_backward"):
+for n in ("mvr_host_stage_meshes_packed", "mvr_host_stage_meshes_packed_begin", "mvr_host_stage_meshes_end", "mvr_look_at_forward", "mvr_look_at_forward_flagged", "mvr_mesh_prepare", "mvr_mesh_forward", "mvr_mesh_backward", "mvr_mesh_backward_angles", "mvr_look_at_backward"):
     wrap(n)
 
 def step(rec):

@@ -14,7 +14,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import test_gpu_parity as T
 from mvtn_b200 import synth
-from mvtn_b200 import _lib as L
 from oracle import oracle as orc
 
 orc.build()
@@ -105,7 +104,7 @@ def views(rng, B, M, near):
 
 
 def mesh_case(rng, kind):
-    """One random mesh configuration -> (cfg for run_mesh, forward flags, near, any_soup)."""
+    """One random mesh configuration -> (cfg for run_mesh, near, any_soup)."""
     B, M = int(rng.integers(1, 4)), int(rng.integers(1, 4))
     H = int(rng.choice([8, 17, 31, 32, 33, 48, 50, 64, 97, 128]))
     K = int(rng.choice([1, 1, 1, 2, 3]))
@@ -124,8 +123,7 @@ def mesh_case(rng, kind):
         cfg["light"] = "relative"      # lit from the camera: the visible faces are lit, the gradients are not ~0
     else:
         cfg["light_dir"] = [float(x) for x in rng.normal(size=3)]
-    flags = L.FORWARD_TILED if (K == 1 and rng.integers(0, 3) == 0) else 0
-    return cfg, flags, near, any_soup
+    return cfg, near, any_soup
 
 
 fails, n_highlight = [], 0
@@ -133,9 +131,9 @@ for case in (range(seed0, seed0 + n_cases) if __name__ == "__main__" else ()):
     rng = np.random.default_rng(10_000 + case)
     try:
         if case % 3 != 2:
-            cfg, flags, near, any_soup = mesh_case(rng, kind_of_mesh)
+            cfg, near, any_soup = mesh_case(rng, kind_of_mesh)
             meshes, B, M, H, K = cfg["meshes"], len(cfg["meshes"]), cfg["M"], cfg["H"], cfg["K"]
-            res = T.run_mesh(orc, dev, cfg, backward=True, extra_flags=flags)
+            res = T.run_mesh(orc, dev, cfg, backward=True)
             d = np.abs(res["img"].detach().cpu().numpy() - res["o"]["images"])
             hl = ""
             if 1e-5 < d.max() <= 1.5e-5 and int((d > 1e-5).sum()) <= 6 and res["o"]["images"][d > 1e-5].min() > 0.9:
@@ -146,7 +144,7 @@ for case in (range(seed0, seed0 + n_cases) if __name__ == "__main__" else ()):
                 n, c, y, x = np.unravel_index(d.argmax(), d.shape)
                 raise AssertionError(f"image error {d.max():.3e} at view {n} channel {c} pixel ({y}, {x}): got {float(res['img'][n, c, y, x]):.7f} "
                                      f"want {res['o']['images'][n, c, y, x]:.7f}, face {int(res['p2f'][n, y, x, 0])}, {int((d > 1e-5).sum())} values over 1e-5")
-            what = f"mesh soup={any_soup} light={cfg.get('light', 'fixed')} B={B} M={M} H={H} K={K} near={near} persp={cfg['persp']} cull={cfg['cull']} tiled={bool(flags)} F={[int(f.shape[0]) for _, f in meshes]}"
+            what = f"mesh soup={any_soup} light={cfg.get('light', 'fixed')} B={B} M={M} H={H} K={K} near={near} persp={cfg['persp']} cull={cfg['cull']} F={[int(f.shape[0]) for _, f in meshes]}"
         else:
             B, M = int(rng.integers(1, 3)), int(rng.integers(1, 4))
             Np = int(rng.choice([2, 7, 100, 900, 3000, 5000]))

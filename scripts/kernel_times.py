@@ -29,7 +29,7 @@ for _ in range(5):
     step()
 torch.cuda.synchronize()
 names = ["look_at_forward_one_cta_kernel", "geom_pack_verts_kernel", "geom_pack_faces_kernel", "geom_finish_normals_kernel", "mesh_project_kernel",
-         "mesh_bin_kernel", "mesh_bin_scan_kernel", "mesh_tile_kernel", "mesh_scatter_kernel", "mesh_shade_kernel", "mesh_shade_clipped_kernel", "mesh_backward_kernel", "mesh_backward_finish_kernel", "look_at_backward_kernel"]
+         "mesh_scatter_kernel", "mesh_shade_kernel", "mesh_shade_clipped_kernel", "mesh_backward_kernel", "mesh_backward_finish_kernel", "look_at_backward_kernel"]
 tot_all = 0.0
 for nm in names:
     lib.mvr_profile_enable(nm.encode())

@@ -1,8 +1,7 @@
-"""Tiny forward + backward of both paths (mesh: scatter + shade, strip and tile backward, K = 1 and 2, a clipped view, the
-tile-binned forward with its TMA bulk copies, vertex gradients with the warp-aggregated scatter, the soft shaders, a collated batch
-rendered in h2d_chunks groups; points: tiled and generic K, the clustered binning (> 4096 points: DSMEM counters), point / colour
-gradients; the view regulariser; the one-node mesh path from a python list of host meshes -- camera kernel that stores its flag into
-the pinned word, staging threads, backward ending in the angle gradients; the multi-CTA camera kernel) for compute-sanitizer:   compute-sanitizer --tool memcheck|racecheck python scripts/sanitize_small.py"""
+"""Tiny forward + backward of both paths (mesh: scatter + shade, strip and tile backward, K = 1 and 2, a clipped view, vertex
+gradients with the warp-aggregated scatter, the soft shaders, a collated batch with uint16 faces; points: tiled and generic K,
+the clustered binning (> 4096 points: DSMEM counters), point / colour gradients; the view regulariser; the one-node mesh path
+from a python list of host meshes -- camera kernel that stores its flag into the pinned word, staging threads, backward ending in the angle gradients; the multi-CTA camera kernel) for compute-sanitizer:   compute-sanitizer --tool memcheck|racecheck python scripts/sanitize_small.py"""
 import os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -22,14 +21,6 @@ for H, K, vs in ((64, 1, views), (50, 1, views), (40, 2, views), (64, 1, near), 
     img.backward(torch.ones_like(img))
     torch.cuda.synchronize()
     print("mesh", H, K, float(img.sum()), float(a.grad.abs().sum()))
-from mvtn_b200 import _lib as L
-for H, vs, flags in ((64, views, L.FORWARD_TILED), (50, near, L.FORWARD_TILED)):      # tile-binned forward (+ clipped faces)
-    a, e, d = (t.to(dev).reshape(-1).requires_grad_() for t in vs)
-    R, T, C, _ = ops._LookAt.apply(a, e, d)
-    img, fr = ops.render_meshes(geom, 3, R, T, C, light, col, bg, H, _extra_flags=flags)
-    img.backward(torch.ones_like(img))
-    torch.cuda.synchronize()
-    print("mesh tiled", H, float(img.detach().sum()), float(a.grad.abs().sum()))
 v = geom.verts.detach().clone().requires_grad_()                      # vertex gradients: warp-aggregated atomic scatter + normals backward
 a, e, d = (t.to(dev).reshape(-1) for t in views)
 R, T, C, _ = ops._LookAt.apply(a, e, d)
@@ -61,12 +52,12 @@ for K, mode in ((4, "alpha"), (1, "norm")):
     print("points clustered", K, float(img.sum()), float(pg.grad.abs().sum()), float(cg.grad.abs().sum()))
 from mvtn_b200 import MVRenderer, Meshes, collate_meshes
 ml = [Meshes([v], [f]) for v, f in synth.make_meshes(4, 500, 21)]
-r = MVRenderer(3, image_size=48, pc_rendering=False, light_direction="fixed", h2d_chunks=2).to(dev)
+r = MVRenderer(3, image_size=48, pc_rendering=False, light_direction="fixed").to(dev)
 a, e, d = (t.to(dev).requires_grad_() for t in synth.learned_spherical_views(4, 3, 8))
 img, _ = r(collate_meshes(ml), None, a, e, d)
 img.backward(torch.ones_like(img))
 torch.cuda.synchronize()
-print("mesh h2d_chunks=2 (uint16 faces)", float(img.detach().sum()), float(a.grad.abs().sum()), collate_meshes(ml).faces.dtype)
+print("mesh collated (uint16 faces)", float(img.detach().sum()), float(a.grad.abs().sum()), collate_meshes(ml).faces.dtype)
 from mvtn_b200 import regularize_rendered_views
 for dt, S in ((torch.float32, 48), (torch.bfloat16, 48), (torch.float32, 30)):      # the view regulariser: gather + adjoint (quads / scalar rows)
     x = torch.rand(2, 3, 3, S, S, device=dev).to(dt).requires_grad_()

@@ -5,7 +5,7 @@ import os, re, subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "mvtn_b200", "libmvr_b200.so")
-KERNELS = ("mesh_shade_kernelILb0ELi4ELi4ELb0", "mesh_scatter_kernelILi4ELb0ELi256", "mesh_scatter_kernelILi8ELb0ELi128", "mesh_tile_kernelILb0ELi4ELb0", "mesh_bin_kernelILb0",
+KERNELS = ("mesh_shade_kernelILb0ELi4ELi4ELb0", "mesh_scatter_kernelILi4ELb0ELi256", "mesh_scatter_kernelILi8ELb0ELi128",
            "mesh_backward_kernel_stripILi3ELb0ELb0", "mesh_backward_kernel_stripILi2ELb0ELb1", "points_tile_kernelILi4E",
            "points_bin_kernel_fused", "points_backward_kernelILi4ELb0ELb0", "images_regularize_kernelILb1", "images_regularize_backward_rows_kernelILb1",
            "mesh_soft_blend_kernel", "mesh_soft_backward_kernel", "mesh_backward_finish_kernel", "look_at_forward_one_cta_kernel", "geom_pack_faces_kernelIt")
@@ -25,7 +25,7 @@ for line in sass.splitlines():
 
 print("SASS mnemonic counts of the shipped libmvr_b200.so (cuobjdump -sass mvtn_b200/libmvr_b200.so; full listings: profiles/sass_*.txt;")
 print("regenerate: python scripts/sass_summary.py)")
-print("UBLKCP / SYNCS = 1-D TMA bulk copy + mbarrier (scatter kernel: face records; point tile kernel: point lists; mesh tile kernel: face lists);")
+print("UBLKCP / SYNCS = 1-D TMA bulk copy + mbarrier (scatter kernel: face records; point tile kernel: point lists);")
 print("LDGSTS = cp.async (strip backward); UCGABAR = thread-block-cluster barrier (clustered point binning, counters read through distributed")
 print("shared memory); MATCH = __match_any_sync (warp-aggregated atomics); ATOMS = shared-memory atomics; RED/ATOMG = global atomics;")
 print("FCHK = range check of an IEEE division's fast path; ACQBULK / PREEXIT = griddepcontrol.wait / .launch_dependents (programmatic dependent launch)")

@@ -1,5 +1,5 @@
-"""GPU (CUDA events) and host (perf_counter) timeline of the C-ABI calls of one end-to-end mesh step, for h2d_chunks = 1 and 2
-(profiles/r3y_h2d_chunks.txt).  usage: python scripts/trace_e2e_timeline.py"""
+"""GPU (CUDA events) and host (perf_counter) timeline of the C-ABI calls of one end-to-end mesh step from a collated batch.
+usage: python scripts/trace_e2e_timeline.py"""
 import os, sys, time
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -24,28 +24,25 @@ def wrap(name):
     def w(*a):
         mark(name + " >"); rc = fn(*a); mark(name + " <"); return rc
     setattr(lib, name, w)
-for n in ("mvr_mesh_prepare_range", "mvr_mesh_prepare", "mvr_mesh_forward", "mvr_mesh_backward", "mvr_look_at_forward", "mvr_look_at_backward"):
+for n in ("mvr_mesh_prepare", "mvr_mesh_forward", "mvr_mesh_backward", "mvr_look_at_forward", "mvr_look_at_backward"):
     wrap(n)
-for k in (1, 2):
-    r = MVRenderer(M, image_size=S, pc_rendering=False, light_direction="fixed", h2d_chunks=k).to(dev).train()
-    def step(trace):
-        T0[0] = time.perf_counter()
-        if trace: mark("start")
-        a = az.to(dev, non_blocking=True).requires_grad_(); e = el.to(dev, non_blocking=True).requires_grad_(); d = di.to(dev, non_blocking=True).requires_grad_()
-        img, _ = r(host, None, a, e, d)
-        if trace: mark("forward returned")
-        img.backward(cot)
-        if trace: mark("backward returned")
-        g_host[0].copy_(a.grad, non_blocking=True); g_host[1].copy_(e.grad, non_blocking=True); g_host[2].copy_(d.grad, non_blocking=True)
-        if trace: mark("end")
-        st.synchronize()
-    for _ in range(10): step(False)
-    marks.clear()
-    torch.cuda.synchronize()
-    step(True)
-    torch.cuda.synchronize()
-    print("== h2d_chunks", k)
-    e0 = marks[0][1]
-    for label, ev, host_us in marks:
-        print("  %-28s gpu %8.1f us   host %8.1f us" % (label, 1e3 * e0.elapsed_time(ev), host_us))
-    marks.clear()
+r = MVRenderer(M, image_size=S, pc_rendering=False, light_direction="fixed").to(dev).train()
+def step(trace):
+    T0[0] = time.perf_counter()
+    if trace: mark("start")
+    a = az.to(dev, non_blocking=True).requires_grad_(); e = el.to(dev, non_blocking=True).requires_grad_(); d = di.to(dev, non_blocking=True).requires_grad_()
+    img, _ = r(host, None, a, e, d)
+    if trace: mark("forward returned")
+    img.backward(cot)
+    if trace: mark("backward returned")
+    g_host[0].copy_(a.grad, non_blocking=True); g_host[1].copy_(e.grad, non_blocking=True); g_host[2].copy_(d.grad, non_blocking=True)
+    if trace: mark("end")
+    st.synchronize()
+for _ in range(10): step(False)
+marks.clear()
+torch.cuda.synchronize()
+step(True)
+torch.cuda.synchronize()
+e0 = marks[0][1]
+for label, ev, host_us in marks:
+    print("  %-28s gpu %8.1f us   host %8.1f us" % (label, 1e3 * e0.elapsed_time(ev), host_us))

@@ -221,34 +221,20 @@ def test_mesh_queue_overflow_fallbacks_are_exact(oracle, cuda_device):
         run_mesh(oracle, cuda_device, mesh_case(name), backward=False, extra_flags=L.TEST_TINY_QUEUES)
 
 
-@pytest.mark.parametrize("name", [n for n in MESH_CASES if mesh_case(n)["K"] == 1] if False else
-                         ["small", "spherical", "cull_noperspective", "vertex_rgb", "relative_light", "c2_slice", "dense_subpixel", "odd_width_k1"])
-def test_mesh_tile_binned_forward_is_exact(oracle, cuda_device, name):
-    """MVR_FORWARD_TILED (K = 1): coarse tile binning + one fine kernel with the depth keys in shared memory and the face lists
-    staged by TMA bulk copies -- the opt-in alternative of the scatter + shade pair.  Same bars: fragments bit-exact."""
-    res = run_mesh(oracle, cuda_device, mesh_case(name), extra_flags=L.FORWARD_TILED)
-    assert (res["p2f"][..., 0] >= 0).mean() > 0.05
-
-
-def test_mesh_tile_binned_forward_edge_paths(oracle, cuda_device):
-    """Tile path: tiny queues (in-place fallbacks), a cube of faces spanning many tiles (per-view big list), near-plane clipping."""
-    run_mesh(oracle, cuda_device, mesh_case("spherical"), backward=False, extra_flags=L.FORWARD_TILED | L.TEST_TINY_QUEUES)
+def test_mesh_forward_edge_cases_k1(oracle, cuda_device):
+    """K = 1: a cube of faces spanning many pixels (walked by a whole CTA), near-plane clipping, a single triangle, a ragged batch
+    and a non-square image.  (An object behind the camera at K = 1: test_mesh_edge_cases.)"""
     cube = dict(mesh_case("cube_big_faces"), K=1)
-    res = run_mesh(oracle, cuda_device, cube, backward=False, extra_flags=L.FORWARD_TILED)
+    res = run_mesh(oracle, cuda_device, cube, backward=False)
     assert int(res["frag"]["counters"][L.CNT_BIG_FACES]) > 0
     close = dict(mesh_case("close_camera_400"), K=1)
-    res = run_mesh(oracle, cuda_device, close, extra_flags=L.FORWARD_TILED)
+    res = run_mesh(oracle, cuda_device, close)
     assert res["o"]["straddle"] > 0
-    # a single triangle, an object behind the camera (every list empty), a ragged batch with per-vertex colours
     tri_v = torch.tensor([[-0.5, -0.5, 0.0], [0.5, -0.5, 0.0], [0.0, 0.6, 0.0]]); tri_f = torch.tensor([[0, 1, 2]])
     run_mesh(oracle, cuda_device, dict(meshes=[(tri_v, tri_f)], M=2, H=33, K=1, views=(torch.tensor([[0.0, 40.0]]), torch.tensor([[10.0, 30.0]]),
-                                       torch.tensor([[2.2, 2.0]])), light_dir=[0.3, 0.5, 0.8]), backward=False, extra_flags=L.FORWARD_TILED)
-    far = tri_v + torch.tensor([0.0, 0.0, 50.0])
-    res = run_mesh(oracle, cuda_device, dict(meshes=[(far, tri_f)], M=1, H=16, K=1, views=(torch.tensor([[0.0]]), torch.tensor([[0.0]]), torch.tensor([[2.0]]))),
-                   backward=False, extra_flags=L.FORWARD_TILED)
-    assert (res["p2f"] == -1).all()
-    run_mesh(oracle, cuda_device, dict(mesh_case("ragged_k3"), K=1), extra_flags=L.FORWARD_TILED)
-    # non-square image (both rasterizers, K = 1)
+                                       torch.tensor([[2.2, 2.0]])), light_dir=[0.3, 0.5, 0.8]), backward=False)
+    run_mesh(oracle, cuda_device, dict(mesh_case("ragged_k3"), K=1))
+    # non-square image
     dev = cuda_device
     H, W, M = 40, 104, 2
     meshes = synth.make_meshes(1, 700, 79)
@@ -259,10 +245,9 @@ def test_mesh_tile_binned_forward_edge_paths(oracle, cuda_device):
     o = oracle.mesh_forward(vp, fp, voff, foff, oracle.vertex_normals(vp, fp), np.full(3, 0.99999, np.float32), M, R, T, C,
                             np.array([[0.2, 1.0, 0.3]], np.float32), np.full(3, 0.499995, np.float32), K00, K11, 0.5, H, W, 1,
                             oracle.PERSPECTIVE_CORRECT)
-    for fl in (0, L.FORWARD_TILED):
-        img, frag = ops.render_meshes(geom, M, Rd, Td, Cd, light, col, col * 0.5, (H, W), fragments=True, _extra_flags=fl)
-        assert (frag["pix_to_face"].cpu().numpy() == o["pix_to_face"]).all() and (frag["zbuf"].cpu().numpy() == o["zbuf"]).all()
-        assert np.abs(img.cpu().numpy() - o["images"]).max() <= IMG_ATOL
+    img, frag = ops.render_meshes(geom, M, Rd, Td, Cd, light, col, col * 0.5, (H, W), fragments=True)
+    assert (frag["pix_to_face"].cpu().numpy() == o["pix_to_face"]).all() and (frag["zbuf"].cpu().numpy() == o["zbuf"]).all()
+    assert np.abs(img.cpu().numpy() - o["images"]).max() <= IMG_ATOL
 
 
 # ------------------------------------------------------------------------------------------------ soft shaders (8f N3)
@@ -699,9 +684,8 @@ def test_points_golden(cuda_device):
 def test_mesh_full_size_c5_properties(oracle, cuda_device):
     """BASELINE configs[4] at full size (8 meshes x 20 views, ~100k faces, 400^2): properties that need no O(H W F) oracle pass --
     run-to-run determinism, object independence (an object rendered alone gives the slice of the batch: no cross-object term),
-    invariance of the image under a permutation of the faces (ids map through the permutation), agreement of the two forward
-    rasterizers (scatter + shade vs the tile-binned one), determinism of the backward.  The oracle itself is run at this shape
-    by test_mesh_parity[c5_mesh_100k_400] (two views) and by bench.py's parity gate."""
+    invariance of the image under a permutation of the faces (ids map through the permutation), determinism of the backward.
+    The oracle itself is run at this shape by test_mesh_parity[c5_mesh_100k_400] (two views) and by bench.py's parity gate."""
     dev = cuda_device
     B, M, H = 8, 20, 400
     meshes = synth.make_meshes(B, 100000, 1290)
@@ -714,8 +698,6 @@ def test_mesh_full_size_c5_properties(oracle, cuda_device):
     assert torch.equal(f1["pix_to_face"], f2["pix_to_face"]) and torch.equal(img1, img2)
     cov = float((f1["pix_to_face"] >= 0).float().mean())
     assert 0.2 < cov < 0.8
-    img3, f3 = ops.render_meshes(geom, M, Rd, Td, Cd, light, col, col, H, _extra_flags=L.FORWARD_TILED)
-    assert torch.equal(f3["pix_to_face"], f1["pix_to_face"]) and torch.equal(img3, img1)
     b = 5
     s = slice(b * M, (b + 1) * M)
     gb = ops.PackedMeshes([meshes[b][0]], [meshes[b][1]], dev)
@@ -953,11 +935,11 @@ def test_mvrenderer_accepts_collated_host_batch(cuda_device):
     assert g_big.faces.dtype == torch.int32 and torch.equal(shot(g_big), shot(g_big_dev))
 
 
-@pytest.mark.parametrize("chunks,K", [(2, 1), (3, 1), (4, 2), (64, 1)])
-def test_mvrenderer_h2d_chunks_match_single_copy(cuda_device, chunks, K):
-    """h2d_chunks: a collated batch copied / prepared / rendered in groups of objects (mvr_mesh_prepare_range + offset
-    vert_off / per-view pointers, one forward and one backward launch per group) gives the images, fragments and gradients
-    of the single-copy path bit for bit -- uneven groups, more groups than objects, K > 1, pinned or pageable source."""
+@pytest.mark.parametrize("K", [1, 2])
+def test_mvrenderer_pageable_collated_batch_matches_pinned(cuda_device, K):
+    """A collated batch in pageable host memory (a DataLoader without pin_memory=True) is re-staged through pinned buffers by
+    PackedMeshes.from_host_packed: a ragged batch gives the images, fragments and azim / elev / dist gradients of the pinned
+    batch bit for bit."""
     from mvtn_b200 import collate_meshes
     dev = cuda_device
     meshes = [synth.make_mesh(nf, 70 + i) for i, nf in enumerate((700, 90, 2500, 300, 1200, 40))]
@@ -966,19 +948,19 @@ def test_mvrenderer_h2d_chunks_match_single_copy(cuda_device, chunks, K):
     views = [t.to(dev) for t in synth.learned_spherical_views(B, M, 23)]
     cot = torch.randn(B, M, 3, 56, 56, device=dev)
 
-    def run(nch, pin):
-        r = MVRenderer(M, image_size=56, pc_rendering=False, light_direction="relative", faces_per_pixel=K, h2d_chunks=nch).to(dev).eval()
+    def run(pin):
+        r = MVRenderer(M, image_size=56, pc_rendering=False, light_direction="relative", faces_per_pixel=K).to(dev).eval()
         a, e, d = (t.detach().clone().requires_grad_() for t in views)
-        img, cams = r(collate_meshes(ml, pin_memory=pin), None, a, e, d)
+        hp = collate_meshes(ml, pin_memory=pin)
+        assert hp.is_pinned() == pin
+        img, cams = r(hp, None, a, e, d)
         p2f = r.last_fragments["pix_to_face"].clone()
         img.backward(cot)
         return img.detach().clone(), p2f, a.grad.clone(), e.grad.clone(), d.grad.clone()
 
-    ref = run(1, True)
-    for pin in (True, False):
-        out = run(chunks, pin)
-        for x, y in zip(ref, out):
-            assert torch.equal(x, y)
+    ref, out = run(True), run(False)
+    for x, y in zip(ref, out):
+        assert torch.equal(x, y)
     assert int((ref[1] >= 0).sum()) > 0
 
 
@@ -1495,7 +1477,7 @@ def test_points_from_angles_fused_backward_equals_the_two_node_chain(cuda_device
 def test_mesh_from_angles_fused_backward_equals_the_two_node_chain(cuda_device):
     """ops.render_meshes_from_angles ends its backward in mvr_mesh_backward_angles (rasterizer/shader backward + per-view sums + camera
     backward in one call); ops._LookAt + ops.render_meshes runs the same chain as two autograd nodes (mvr_mesh_backward,
-    mvr_look_at_backward): same gradients bit for bit, fixed and relative light, with a staged batch (h2d_chunks-style groups) too;
+    mvr_look_at_backward): same gradients bit for bit, fixed and relative light;
     gradients sent through the cameras take the unfused path and add up."""
     dev = cuda_device
     B, M, S = 3, 4, 64

@@ -395,7 +395,7 @@ def test_flag_constants_match_the_header():
     assert defs["ABI_VERSION"] == _lib.ABI_VERSION
     mirrored = [n for n in defs if hasattr(_lib, n) and n != "ABI_VERSION"]
     assert {"PERSPECTIVE_CORRECT", "CULL_BACKFACES", "COMPOSITE_ALPHA", "RGB_PER_ELEMENT", "FACES_I64", "IMAGES_BF16", "SCALE_IS_DIST",
-            "WS_KEYS_ARMED", "WS_REARM_KEYS", "WS_PROJECTED", "IDX_SPARSE", "FORWARD_TILED", "FACES_U16", "CLIP_BARYCENTRIC", "TEST_TINY_QUEUES", "NUM_COUNTERS"} <= set(mirrored)
+            "WS_KEYS_ARMED", "WS_REARM_KEYS", "WS_PROJECTED", "IDX_SPARSE", "FACES_U16", "CLIP_BARYCENTRIC", "TEST_TINY_QUEUES", "NUM_COUNTERS"} <= set(mirrored)
     for n in mirrored:
         assert getattr(_lib, n) == defs[n], n
     flags = [defs[n] for n in mirrored if n not in ("NUM_COUNTERS", "CNT_STRADDLE", "CNT_BIG_FACES")]
