@@ -658,7 +658,7 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
     rc = check_launch("mesh_shade_kernel");
     if (rc) return rc;
     if (z_clip >= 0.f) {      // pixels won by a face crossing the near plane (none in MVTN's default configurations: the kernel exits at once)
-      rc = launch_mesh_shade_clipped(p, (int)N, st);
+      rc = launch_mesh_shade_clipped(p, (int)N, soft_raster, st);
       if (rc) return rc;
     }
   }

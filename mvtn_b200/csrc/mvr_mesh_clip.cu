@@ -13,16 +13,6 @@
 
 namespace mvr {
 
-// sub-triangle level rejection of the rasterizer (the tests of face_pixel_bbox that do not involve the pixel)
-__device__ __forceinline__ bool sub_face_ok(const Face& f, int flags) {
-  const float zmin = fminf(fminf(f.z0, f.z1), f.z2);
-  if (zmin < MVR_K_EPS) return false;
-  const float face_area = (f.x0 - f.x1) * (f.y2 - f.y1) - (f.y0 - f.y1) * (f.x2 - f.x1);
-  if ((flags & MVR_CULL_BACKFACES) && face_area < 0.f) return false;
-  if (face_area <= MVR_K_EPS && face_area >= -1.0f * MVR_K_EPS) return false;
-  return true;
-}
-
 // The sub-triangle the rasterizer kept for pixel (xf, yf): inside, smallest (pz, index).  want_z_bits != 0: the one
 // whose depth is the recorded key (forward); bcl = its barycentrics, pz its depth.  Returns -1 if none.
 __device__ __forceinline__ int pick_sub(const ClipSub& cs, int flags, bool persp, float xf, float yf, unsigned int want_z_bits,
@@ -41,6 +31,9 @@ __device__ __forceinline__ int pick_sub(const ClipSub& cs, int flags, bool persp
   return best;
 }
 
+// SOFT: the blurred rasterizer (blur_radius > 0 / clipped barycentrics) -- the sub-triangle is picked by its soft test
+// (pick_sub_soft), the fragment carries its (clipped) barycentrics converted to the original face and its SIGNED edge distance
+template <bool SOFT>
 __device__ __forceinline__ void shade_clipped_pixel(const MeshParams& p, int b, int m, int n, int pix) {
   const int HW = p.H * p.W;
   const int yi = pix / p.W, xi = pix - yi * p.W;
@@ -60,17 +53,26 @@ __device__ __forceinline__ void shade_clipped_pixel(const MeshParams& p, int b, 
   clip_face(fc, p.z_clip, persp, cs);
   const float xf = __ldg(p.tab + xi), yf = __ldg(p.tab + p.W + yi);
   float bcl[3], pz;
-  int s = pick_sub(cs, p.flags, persp, xf, yf, (unsigned int)(key >> 32), bcl, pz);
-  if (s < 0) s = pick_sub(cs, p.flags, persp, xf, yf, 0u, bcl, pz);
   float bb[3] = {-1.f, -1.f, -1.f}, dd = -1.f;
+  int s;
+  if (SOFT) {
+    SoftHit h;
+    s = pick_sub_soft(cs, p.flags, persp, p.flags & MVR_CLIP_BARYCENTRIC, p.blur_radius, p.blur_r, xf, yf, (unsigned int)(key >> 32), 0, h);
+    if (s >= 0) { bcl[0] = h.bc[0]; bcl[1] = h.bc[1]; bcl[2] = h.bc[2]; dd = h.sd; }
+  } else {
+    s = pick_sub(cs, p.flags, persp, xf, yf, (unsigned int)(key >> 32), bcl, pz);
+    if (s < 0) s = pick_sub(cs, p.flags, persp, xf, yf, 0u, bcl, pz);
+  }
   float out[3] = {__ldg(p.bg_rgb), __ldg(p.bg_rgb + 1), __ldg(p.bg_rgb + 2)};
   if (s >= 0) {
     conv_bary(cs.conv[s], bcl, bb);
-    const Face sf = cs.f[s];
-    const float e01 = point_line_dist2(xf, yf, sf.x0, sf.y0, sf.x1, sf.y1);
-    const float e02 = point_line_dist2(xf, yf, sf.x0, sf.y0, sf.x2, sf.y2);
-    const float e12 = point_line_dist2(xf, yf, sf.x1, sf.y1, sf.x2, sf.y2);
-    dd = -fminf(fminf(e01, e02), e12);
+    if (!SOFT) {
+      const Face sf = cs.f[s];
+      const float e01 = point_line_dist2(xf, yf, sf.x0, sf.y0, sf.x1, sf.y1);
+      const float e02 = point_line_dist2(xf, yf, sf.x0, sf.y0, sf.x2, sf.y2);
+      const float e12 = point_line_dist2(xf, yf, sf.x1, sf.y1, sf.x2, sf.y2);
+      dd = -fminf(fminf(e01, e02), e12);
+    }
     if (k == 0) {
       const float4 X0 = __ldg(p.verts4 + voff + fi.x), X1 = __ldg(p.verts4 + voff + fi.y), X2 = __ldg(p.verts4 + voff + fi.z);
       const float4 N0 = __ldg(p.normals4 + voff + fi.x), N1 = __ldg(p.normals4 + voff + fi.y), N2 = __ldg(p.normals4 + voff + fi.z);
@@ -91,72 +93,21 @@ __device__ __forceinline__ void shade_clipped_pixel(const MeshParams& p, int b, 
 
 // grid: one CTA per view, striding over its pixels (the common case is "flag down": N tiny CTAs that exit at once).
 // Writes EVERY output of a pixel whose winning face straddles the plane (mesh_shade_kernel left it untouched).
+template <bool SOFT>
 __global__ void __launch_bounds__(MVR_THREADS) mesh_shade_clipped_kernel(const MeshParams p) {
   pdl_enter();
   if (!may_clip(p.wsflags)) return;
   const int n = blockIdx.x, b = n / p.M, m = n - b * p.M;
   const int HW = p.H * p.W;
-  for (int pix = threadIdx.x; pix < HW; pix += MVR_THREADS) shade_clipped_pixel(p, b, m, n, pix);
+  for (int pix = threadIdx.x; pix < HW; pix += MVR_THREADS) shade_clipped_pixel<SOFT>(p, b, m, n, pix);
 }
 
 
 // ------------------------------------------------------------------------------------------------
 // backward of one clipped pixel: d image -> Phong -> unclipped barycentrics -> (conversion, clipped barycentrics) ->
-// clipped triangle -> original (x_ndc, y_ndc, z_view) (autograd of [upstream] clip.py), then the projection as usual.
+// clipped triangle -> original (x_ndc, y_ndc, z_view) (clip_face_backward, mvr_mesh.cuh), then the projection as usual.
 // Same derivation as oracle/mvr_oracle.c clip_face_bwd / raster_bwd_one / phong_pixel_bwd, in fp32.
 // ------------------------------------------------------------------------------------------------
-// backward of clip_face + conv_bary for one pixel of sub-triangle s: gq (3,3) w.r.t. the clipped triangle, gb (3)
-// w.r.t. the UNCLIPPED barycentrics, bcl the clipped barycentrics -> gfv (3,3) w.r.t. the original (x_ndc, y_ndc, z_view)
-static __device__ __noinline__ void clip_face_backward(const Face& f, float c, bool persp, int info, int s, const float gq[9],
-                                                       const float gb[3], const float bcl[3], float gfv[9]) {
-  const float v[9] = {f.x0, f.y0, f.z0, f.x1, f.y1, f.z1, f.x2, f.y2, f.z2};
-  const int i1 = info & 3, case4 = (info >> 2) & 1;
-  const int i2 = (i1 + 1) % 3, i3 = (i1 + 2) % 3;
-  const float p1[3] = {v[3 * i1], v[3 * i1 + 1], v[3 * i1 + 2]};
-  const float p2[3] = {v[3 * i2], v[3 * i2 + 1], v[3 * i2 + 2]};
-  const float p3[3] = {v[3 * i3], v[3 * i3 + 1], v[3 * i3 + 2]};
-  const float w2 = (p1[2] - c) / (p1[2] - p2[2]), w3 = (p1[2] - c) / (p1[2] - p3[2]);
-  int pick[3];
-  if (!case4) { pick[0] = 3; pick[1] = 4; pick[2] = 0; }
-  else if (s == 0) { pick[0] = 3; pick[1] = 1; pick[2] = 4; }
-  else { pick[0] = 4; pick[1] = 1; pick[2] = 2; }
-  float gP[5][3];
-  for (int q = 0; q < 5; ++q) { gP[q][0] = 0.f; gP[q][1] = 0.f; gP[q][2] = 0.f; }
-  float gw2 = 0.f, gw3 = 0.f;
-  for (int k = 0; k < 3; ++k) {
-    for (int d = 0; d < 3; ++d) gP[pick[k]][d] += gq[3 * k + d];
-    if (pick[k] == 3) gw2 += bcl[k] * (gb[i2] - gb[i1]);
-    if (pick[k] == 4) gw3 += bcl[k] * (gb[i3] - gb[i1]);
-  }
-  float g1[3] = {gP[0][0], gP[0][1], gP[0][2]}, g2[3] = {gP[1][0], gP[1][1], gP[1][2]}, g3[3] = {gP[2][0], gP[2][1], gP[2][2]};
-  for (int q = 0; q < 2; ++q) {
-    const float* gp = q == 0 ? gP[3] : gP[4];
-    const float* po = q == 0 ? p2 : p3;
-    float* go = q == 0 ? g2 : g3;
-    const float w = q == 0 ? w2 : w3;
-    float gw = 0.f;
-    for (int d = 0; d < 2; ++d) {
-      if (persp) {     // p.xy = ((p1.xy p1.z)(1 - w) + (po.xy po.z) w) / c
-        const float A = p1[d] * p1[2], Bq = po[d] * po[2];
-        const float gA = gp[d] * (1.f - w) / c, gB = gp[d] * w / c;
-        gw += gp[d] * (Bq - A) / c;
-        g1[d] += gA * p1[2]; g1[2] += gA * p1[d];
-        go[d] += gB * po[2]; go[2] += gB * po[d];
-      } else {
-        g1[d] += gp[d] * (1.f - w); go[d] += gp[d] * w; gw += gp[d] * (po[d] - p1[d]);
-      }
-    }
-    g1[2] += gp[2] * (1.f - w); go[2] += gp[2] * w; gw += gp[2] * (po[2] - p1[2]);
-    if (q == 0) gw2 += gw; else gw3 += gw;
-  }
-  {   // w2 = (z1 - c) / (z1 - z2), w3 = (z1 - c) / (z1 - z3)
-    const float d2 = p1[2] - p2[2], d3 = p1[2] - p3[2];
-    g1[2] += gw2 * (c - p2[2]) / (d2 * d2); g2[2] += gw2 * (p1[2] - c) / (d2 * d2);
-    g1[2] += gw3 * (c - p3[2]) / (d3 * d3); g3[2] += gw3 * (p1[2] - c) / (d3 * d3);
-  }
-  for (int d = 0; d < 3; ++d) { gfv[3 * i1 + d] = g1[d]; gfv[3 * i2 + d] = g2[d]; gfv[3 * i3 + d] = g3[d]; }
-}
-
 // The clipped-face pixels of view n (those mesh_backward_kernel skipped), accumulated by the whole CTA into acc (per thread).
 __device__ __forceinline__ void backward_clipped_view(const MeshBwdParams& p, int n, float (&acc)[16]) {
   const int tid = threadIdx.x;
@@ -274,8 +225,9 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_backward_finish_kernel(const
 
 using namespace mvr;
 
-int launch_mesh_shade_clipped(const MeshParams& p, int N, cudaStream_t st) {
-  MVR_LAUNCH_PDL(mesh_shade_clipped_kernel, (unsigned)N, MVR_THREADS, 0, st, p);
+int launch_mesh_shade_clipped(const MeshParams& p, int N, bool soft, cudaStream_t st) {
+  if (soft) MVR_LAUNCH_PDL(mesh_shade_clipped_kernel<true>, (unsigned)N, MVR_THREADS, 0, st, p);
+  else MVR_LAUNCH_PDL(mesh_shade_clipped_kernel<false>, (unsigned)N, MVR_THREADS, 0, st, p);
   return check_launch("mesh_shade_clipped_kernel");
 }
 

@@ -93,31 +93,68 @@ __device__ __forceinline__ void point_line_dist2_bwd(float px, float py, float a
   gax = (1.f - tt) * ex; gay = (1.f - tt) * ey; gbx = tt * ex; gby = tt * ey;
 }
 
-// One fragment: recompute, and push (g_colour, g_zbuf, g_sdist) back to the camera accumulators acc[15].
-__device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, int voff, const float4* __restrict__ pvn, const int4 fi,
-                                                       bool persp, bool clipb, float xf, float yf, const ShadeCtx& sc, const float gcol[3],
-                                                       float gz, float gsd, bool with_colour, float acc[16]) {
-  const Face fc = gather_face(pvn, fi);
-  const FaceEdges fe = face_edges(fc);
-  float bu[3], bc[3], pz, sd;
-  bool inside;
-  raster_soft(fc, fe, persp, clipb, xf, yf, bu, bc, pz, sd, inside);
+// One fragment of a pixel, recomputed from the projected vertices: raster_soft on its face, or -- a face crossing the near
+// plane (p.z_clip, while the projection has found a vertex behind it) -- on the sub-triangle the forward's scatter kept
+// (pick_sub_soft), with the barycentrics mapped back to the face (conv_bary) as mvr_mesh_shade_clipped_kernel writes them.
+struct SoftFrag {
+  Face g;            // the triangle rasterized: the face, or sub-triangle s of its clipping
+  int s;             // -1: not clipped
+  SoftHit h;         // barycentrics (raw, carried), depth and signed distance on g
+  float bb[3];       // barycentrics on the original face (colour)
+};
+// rank: how many entries of the same face precede this one in the pixel's K-list (a clipped face may hold two)
+__device__ __forceinline__ bool soft_fragment(const MeshParams& p, const Face& fc, bool persp, bool clipb, bool clip_on, float xf,
+                                              float yf, int rank, ClipSub& cs, SoftFrag& fr) {
+  fr.s = -1;
+  if (clip_on && face_straddles(fc, p.z_clip)) {
+    clip_face(fc, p.z_clip, persp, cs);
+    fr.s = pick_sub_soft(cs, p.flags, persp, clipb, p.blur_radius, p.blur_r, xf, yf, 0u, rank, fr.h);
+    if (fr.s < 0) return false;
+    fr.g = cs.f[fr.s];
+    conv_bary(cs.conv[fr.s], fr.h.bc, fr.bb);
+    return true;
+  }
+  fr.g = fc;
+  raster_soft(fc, face_edges(fc), persp, clipb, xf, yf, fr.h.bu, fr.h.bc, fr.h.pz, fr.h.sd, fr.h.inside);
+  fr.bb[0] = fr.h.bc[0]; fr.bb[1] = fr.h.bc[1]; fr.bb[2] = fr.h.bc[2];
+  return true;
+}
+
+__device__ __forceinline__ int rank_in_list(const int* list, int k, int fid) {
+  int r = 0;
+  for (int j = 0; j < k; ++j) r += list[j] == fid;
+  return r;
+}
+
+// One fragment: push (g_colour, g_zbuf, g_sdist) back to the camera accumulators acc[15].
+__device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, int voff, const int4 fi, const Face& fc, const SoftFrag& fr,
+                                                       const ClipSub& cs, bool persp, bool clipb, float xf, float yf, const ShadeCtx& sc,
+                                                       const float gcol[3], float gz, float gsd, bool with_colour, float acc[16]) {
+  const Face& g = fr.g;
   float4 X0, X1, X2, N0, N1, N2;
   gather_xn(p.xn8, voff + fi.x, X0, N0); gather_xn(p.xn8, voff + fi.y, X1, N1); gather_xn(p.xn8, voff + fi.z, X2, N2);
-  float gbc[3] = {0.f, 0.f, 0.f};
+  float gbb[3] = {0.f, 0.f, 0.f};      // w.r.t. the barycentrics on the original face
   if (with_colour) {
     float4 c0, c1, c2;
     if (p.flags & MVR_RGB_PER_ELEMENT) { c0 = __ldg(p.rgb4 + voff + fi.x); c1 = __ldg(p.rgb4 + voff + fi.y); c2 = __ldg(p.rgb4 + voff + fi.z); }
     else { c0 = c1 = c2 = make_float4(__ldg(p.obj_rgb), __ldg(p.obj_rgb + 1), __ldg(p.obj_rgb + 2), 0.f); }
     float gv[3], gN[3];
-    phong_backward(bc, X0, X1, X2, N0, N1, N2, c0, c1, c2, sc, gcol[0], gcol[1], gcol[2], gbc, gv, gN);
+    phong_backward(fr.bb, X0, X1, X2, N0, N1, N2, c0, c1, c2, sc, gcol[0], gcol[1], gcol[2], gbb, gv, gN);
     acc[12] += gv[0]; acc[13] += gv[1]; acc[14] += gv[2];      // dC
+  }
+  // w.r.t. the barycentrics carried on g: through the conversion bb_j = sum_k conv[3 j + k] bc_k for a sub-triangle
+  float gbc[3] = {gbb[0], gbb[1], gbb[2]};
+  if (fr.s >= 0) {
+    const float* cv = cs.conv[fr.s];
+    for (int k = 0; k < 3; ++k) gbc[k] = cv[k] * gbb[0] + cv[3 + k] * gbb[1] + cv[6 + k] * gbb[2];
   }
   // zbuf = bc . z
   float gq[9];
-  gbc[0] += gz * fc.z0; gbc[1] += gz * fc.z1; gbc[2] += gz * fc.z2;
+  gbc[0] += gz * g.z0; gbc[1] += gz * g.z1; gbc[2] += gz * g.z2;
   float gb[3] = {gbc[0], gbc[1], gbc[2]};
   bool orth = false;
+  const float* bu = fr.h.bu;
+  const float* bc = fr.h.bc;
   if (clipb) {      // [upstream] BarycentricClipBackward: bc = w / s, w = max(b, 0), s = max(sum w, 1e-5)
     const float w0 = fmaxf(bu[0], 0.f), w1 = fmaxf(bu[1], 0.f), w2 = fmaxf(bu[2], 0.f);
     const float ssum = (w0 + w1) + w2;
@@ -128,18 +165,23 @@ __device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, int 
     gb[2] = bu[2] > 0.f ? (gbc[2] - dot) * is : 0.f;
     orth = ssum > 1e-5f;      // sum_i bu_i gb_i = dot - dot sum(bc) = 0
   }
-  raster_backward(fc, persp, xf, yf, gb, gq, orth);
+  raster_backward(g, persp, xf, yf, gb, gq, orth);
   gq[2] += gz * bc[0]; gq[5] += gz * bc[1]; gq[8] += gz * bc[2];
   // signed distance: sd = inside ? -d : d over the nearest edge ([upstream] PointTriangleDistanceBackward)
   if (gsd != 0.f) {
-    const float g = inside ? -gsd : gsd;
-    const float e01 = point_line_dist2(xf, yf, fc.x0, fc.y0, fc.x1, fc.y1);
-    const float e02 = point_line_dist2(xf, yf, fc.x0, fc.y0, fc.x2, fc.y2);
-    const float e12 = point_line_dist2(xf, yf, fc.x1, fc.y1, fc.x2, fc.y2);
+    const float gs = fr.h.inside ? -gsd : gsd;
+    const float e01 = point_line_dist2(xf, yf, g.x0, g.y0, g.x1, g.y1);
+    const float e02 = point_line_dist2(xf, yf, g.x0, g.y0, g.x2, g.y2);
+    const float e12 = point_line_dist2(xf, yf, g.x1, g.y1, g.x2, g.y2);
     float ax, ay, bx, by;
-    if (e01 <= e02 && e01 <= e12) { point_line_dist2_bwd(xf, yf, fc.x0, fc.y0, fc.x1, fc.y1, g, ax, ay, bx, by); gq[0] += ax; gq[1] += ay; gq[3] += bx; gq[4] += by; }
-    else if (e02 <= e01 && e02 <= e12) { point_line_dist2_bwd(xf, yf, fc.x0, fc.y0, fc.x2, fc.y2, g, ax, ay, bx, by); gq[0] += ax; gq[1] += ay; gq[6] += bx; gq[7] += by; }
-    else { point_line_dist2_bwd(xf, yf, fc.x1, fc.y1, fc.x2, fc.y2, g, ax, ay, bx, by); gq[3] += ax; gq[4] += ay; gq[6] += bx; gq[7] += by; }
+    if (e01 <= e02 && e01 <= e12) { point_line_dist2_bwd(xf, yf, g.x0, g.y0, g.x1, g.y1, gs, ax, ay, bx, by); gq[0] += ax; gq[1] += ay; gq[3] += bx; gq[4] += by; }
+    else if (e02 <= e01 && e02 <= e12) { point_line_dist2_bwd(xf, yf, g.x0, g.y0, g.x2, g.y2, gs, ax, ay, bx, by); gq[0] += ax; gq[1] += ay; gq[6] += bx; gq[7] += by; }
+    else { point_line_dist2_bwd(xf, yf, g.x1, g.y1, g.x2, g.y2, gs, ax, ay, bx, by); gq[3] += ax; gq[4] += ay; gq[6] += bx; gq[7] += by; }
+  }
+  if (fr.s >= 0) {      // sub-triangle -> original face ([upstream] clip.py under autograd), as the hard path's clipped pixels
+    float gfv[9];
+    clip_face_backward(fc, p.z_clip, persp, cs.info, fr.s, gq, gbb, bc, gfv);
+    for (int i = 0; i < 9; ++i) gq[i] = gfv[i];
   }
   // projection backward + X R + T backward
   const float xn[3] = {fc.x0, fc.x1, fc.x2}, yn[3] = {fc.y0, fc.y1, fc.y2}, zv[3] = {fc.z0, fc.z1, fc.z2};
@@ -169,6 +211,7 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
   const int f0 = p.face_off[b], voff = p.vert_off[b], V = p.vert_off[b + 1] - voff;
   const float4* pvn = p.pv + (size_t)p.M * voff + (size_t)m * V;
   const bool persp = p.flags & MVR_PERSPECTIVE_CORRECT, clipb = p.flags & MVR_CLIP_BARYCENTRIC;
+  const bool clip_on = may_clip(p.wsflags);      // some vertex lies behind the near plane: faces may straddle it
   const ShadeCtx sc = load_shade_ctx(p.light, p.light_stride, p.Cc, n);
   const float zscale = 1.0f / (sp.zfar - sp.znear);
   float acc[16];
@@ -180,22 +223,23 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
     const int pix = yi * p.W + xi;
     const float xf = __ldg(p.tab + xi), yf = __ldg(p.tab + p.W + yi);
     const size_t fo = ((size_t)n * HW + pix) * K;
+    const int* list = p.pix_to_face + fo;
     const float* g = sp.grad_rgba + (size_t)n * 4 * HW + pix;
     const float g0 = g[0], g1 = g[(size_t)HW], g2 = g[2 * (size_t)HW], ga = g[3 * (size_t)HW];
     if (g0 == 0.f && g1 == 0.f && g2 == 0.f && ga == 0.f) continue;
-    if (p.pix_to_face[fo] < 0) continue;      // fragments are sorted: no first fragment, no fragment
+    // every loop below skips -1 entries, as mesh_soft_blend_kernel does
     // pass 1: z_inv_max (and which fragment holds it), the product of (1 - prob) with its zeros counted
     float zmax = 0.f, keep_nz = 1.0f;
     int kmax = -1, nzero = 0, kzero = -1;
     for (int k = 0; k < K; ++k) {
-      const int fid = p.pix_to_face[fo + k];
-      if (fid < 0) break;
+      const int fid = list[k];
+      if (fid < 0) continue;
       const Face fc = gather_face(pvn, __ldg(p.faces4 + f0 + fid));
-      float bu[3], bc[3], pz, sd; bool inside;
-      raster_soft(fc, face_edges(fc), persp, clipb, xf, yf, bu, bc, pz, sd, inside);
-      const float zi = (sp.zfar - pz) * zscale;
+      ClipSub cs; SoftFrag fr;
+      if (!soft_fragment(p, fc, persp, clipb, clip_on, xf, yf, clip_on ? rank_in_list(list, k, fid) : 0, cs, fr)) continue;
+      const float zi = (sp.zfar - fr.h.pz) * zscale;
       if (zi > zmax) { zmax = zi; kmax = k; }
-      const float q = 1.0f - sigmoidf_(-sd / sp.sigma);
+      const float q = 1.0f - sigmoidf_(-fr.h.sd / sp.sigma);
       if (q == 0.f) { ++nzero; kzero = k; } else keep_nz *= q;
     }
     const bool zmax_live = zmax >= SOFT_EPS;
@@ -205,15 +249,15 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
     bool delta_live = false;
     if (sp.mode == 0) {
       for (int k = 0; k < K; ++k) {
-        const int fid = p.pix_to_face[fo + k];
-        if (fid < 0) break;
+        const int fid = list[k];
+        if (fid < 0) continue;
         const int4 fi = __ldg(p.faces4 + f0 + fid);
         const Face fc = gather_face(pvn, fi);
-        float bu[3], bc[3], pz, sd; bool inside;
-        raster_soft(fc, face_edges(fc), persp, clipb, xf, yf, bu, bc, pz, sd, inside);
+        ClipSub cs; SoftFrag fr;
+        if (!soft_fragment(p, fc, persp, clipb, clip_on, xf, yf, clip_on ? rank_in_list(list, k, fid) : 0, cs, fr)) continue;
         float col[3];
-        fragment_colour(p, voff, fi, bc, sc, col);
-        const float w = sigmoidf_(-sd / sp.sigma) * expf(((sp.zfar - pz) * zscale - zmax) / sp.gamma);
+        fragment_colour(p, voff, fi, fr.bb, sc, col);
+        const float w = sigmoidf_(-fr.h.sd / sp.sigma) * expf(((sp.zfar - fr.h.pz) * zscale - zmax) / sp.gamma);
         num[0] += w * col[0]; num[1] += w * col[1]; num[2] += w * col[2]; den += w;
       }
       const float dr = expf((SOFT_EPS - zmax) / sp.gamma);
@@ -228,21 +272,21 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
       gzmax -= (g0 * (__ldg(p.bg_rgb) - rgb[0]) + g1 * (__ldg(p.bg_rgb + 1) - rgb[1]) + g2 * (__ldg(p.bg_rgb + 2) - rgb[2])) * inv * delta / sp.gamma;
     for (int pass = 0; pass < 2; ++pass) {      // pass 0: every fragment (its own terms); pass 1: fragment kmax gets g_zmax
       for (int k = 0; k < K; ++k) {
-        const int fid = p.pix_to_face[fo + k];
-        if (fid < 0) break;
+        const int fid = list[k];
+        if (fid < 0) continue;
         if (pass == 1 && k != kmax) continue;
         const int4 fi = __ldg(p.faces4 + f0 + fid);
         const Face fc = gather_face(pvn, fi);
-        float bu[3], bc[3], pz, sd; bool inside;
-        raster_soft(fc, face_edges(fc), persp, clipb, xf, yf, bu, bc, pz, sd, inside);
+        ClipSub cs; SoftFrag fr;
+        if (!soft_fragment(p, fc, persp, clipb, clip_on, xf, yf, clip_on ? rank_in_list(list, k, fid) : 0, cs, fr)) continue;
         if (pass == 1) {      // z_inv_max = z_inv of this fragment
           if (zmax_live && gzmax != 0.f) {
             const float gcz[3] = {0.f, 0.f, 0.f};
-            soft_fragment_backward(p, voff, pvn, fi, persp, clipb, xf, yf, sc, gcz, -gzmax * zscale, 0.f, false, acc);
+            soft_fragment_backward(p, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, -gzmax * zscale, 0.f, false, acc);
           }
           continue;
         }
-        const float prob = sigmoidf_(-sd / sp.sigma);
+        const float prob = sigmoidf_(-fr.h.sd / sp.sigma);
         float gprob = 0.f, gzi = 0.f, gcol[3] = {0.f, 0.f, 0.f};
         // alpha = 1 - prod(1 - prob): d alpha / d prob_k = prod over the others
         {
@@ -255,8 +299,8 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
         }
         if (sp.mode == 0) {
           float col[3];
-          fragment_colour(p, voff, fi, bc, sc, col);
-          const float E = expf(((sp.zfar - pz) * zscale - zmax) / sp.gamma);
+          fragment_colour(p, voff, fi, fr.bb, sc, col);
+          const float E = expf(((sp.zfar - fr.h.pz) * zscale - zmax) / sp.gamma);
           const float w = prob * E;
           gcol[0] = g0 * w * inv; gcol[1] = g1 * w * inv; gcol[2] = g2 * w * inv;
           const float gw = (g0 * (col[0] - rgb[0]) + g1 * (col[1] - rgb[1]) + g2 * (col[2] - rgb[2])) * inv;
@@ -266,7 +310,7 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
           gzmax -= gzi;
         }
         const float gsd = gprob * (-1.0f / sp.sigma) * prob * (1.0f - prob);
-        soft_fragment_backward(p, voff, pvn, fi, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc);
+        soft_fragment_backward(p, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc);
       }
     }
   }
@@ -317,8 +361,9 @@ extern "C" int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert
 
 extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M, int64_t total_verts,
                                       int64_t total_faces, int max_verts, const float* R, const float* T, const float* Cc, const float* light,
-                                      int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, int H, int W, int K,
-                                      int flags, int mode, float sigma, float gamma, float znear, float zfar, const int* pix_to_face,
+                                      int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, float z_clip,
+                                      float blur_radius, int H, int W, int K, int flags, int mode, float sigma, float gamma, float znear,
+                                      float zfar, const int* pix_to_face,
                                       const float* grad_rgba, float* gR, float* gT, float* gC, void* workspace, size_t workspace_bytes,
                                       void* stream) {
   int rc = check_mesh_common("mvr_mesh_soft_backward", B, M, H, W, K, total_verts, total_faces, max_verts);
@@ -328,17 +373,21 @@ extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off,
   if (!geometry || !vert_off || !face_off || !R || !T || !Cc || !light || !bg_rgb || !pix_to_face || !grad_rgba || !gR || !gT || !gC || !workspace) { set_error("mvr_mesh_soft_backward: null pointer"); return -5; }
   if (!(flags & MVR_RGB_PER_ELEMENT) && !obj_rgb) { set_error("mvr_mesh_soft_backward: obj_rgb is NULL"); return -6; }
   if (mode < 0 || mode > 1 || !(sigma > 0.f) || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_backward: bad mode / sigma / gamma / z range"); return -7; }
+  if (!(blur_radius >= 0.f)) { set_error("mvr_mesh_soft_backward: blur_radius must be >= 0"); return -9; }
   const WsLayout w = ws_layout(B, M, H, W, K, total_verts, total_faces);
   if (workspace_bytes < w.total) { set_error("mvr_mesh_soft_backward: workspace too small (%zu < %zu)", workspace_bytes, w.total); return -8; }
   const GeomLayout g = geom_layout(total_verts, total_faces);
   cudaStream_t st = (cudaStream_t)stream;
   char* wb = (char*)workspace;
-  // project again (z_clip off: near-plane straddlers are not special-cased in the soft modes)
-  rc = launch_project("mesh_project_kernel", g, w, geometry, vert_off, R, T, B, M, H, W, max_verts, k00, k11, -1.f, true, workspace, st);
+  // project again, with the forward's z_clip: the projection clears the workspace flag WSF_CLIP when a vertex lies behind the
+  // plane, and the fragments of faces crossing it are then recomputed on their clipped sub-triangles (soft_fragment)
+  rc = launch_project("mesh_project_kernel", g, w, geometry, vert_off, R, T, B, M, H, W, max_verts, k00, k11, z_clip, true, workspace, st);
   if (rc) return rc;
   MeshParams p;
   fill_params(p, geometry, vert_off, face_off, B, M, total_verts, total_faces, R, T, Cc, light, light_stride, obj_rgb, bg_rgb, k00, k11, H, W, K, flags, pix_to_face);
   p.pv = (float4*)(wb + w.pv); p.tab = (float*)(wb + w.tab); p.wsflags = (int*)(wb + w.flags);
+  p.z_clip = z_clip;
+  p.blur_radius = blur_radius > 0.f ? blur_radius : 0.f; p.blur_r = sqrtf(p.blur_radius);      // as mvr_mesh_forward
   SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, nullptr, nullptr, nullptr, nullptr, grad_rgba};
   const int tiles_x = (W + 31) / 32;
   const dim3 grid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
@@ -347,7 +396,9 @@ extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off,
   if (rc) return rc;
   MeshBwdParams q;
   q.azim = q.elev = q.dist = nullptr; q.g_azim = q.g_elev = q.g_dist = nullptr;
-  q.partials = (float*)(wb + w.partials); q.parts_per_view = w.bwd_parts_per_view; q.wsflags = (int*)(wb + w.flags);
+  // the finish kernel only sums the partials here: its hard clipped-pixel pass is kept off by pointing its flag at a word of the
+  // armed flag block that the projection never clears (word WSF_CLIP may be cleared above)
+  q.partials = (float*)(wb + w.partials); q.parts_per_view = w.bwd_parts_per_view; q.wsflags = (int*)(wb + w.flags) + WSF_CLIP + 1;
   q.B = B; q.M = M; q.H = H; q.W = W; q.K = K; q.flags = flags; q.z_clip = -1.f; q.grad_verts = nullptr; q.grad_normals = nullptr;
   return launch_mesh_backward_finish(q, (int)N, gR, gT, gC, st);
 }

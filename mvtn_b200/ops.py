@@ -918,7 +918,7 @@ class _MeshRenderSoft(torch.autograd.Function):
                     "mvr_mesh_soft_blend_forward")
         ctx.set_materialize_grads(False)
         ctx.geom, ctx.M = geom, M
-        ctx.cfg = (k00, k11, H, W, K, fl, light_stride, mode, sigma, gamma, znear, zfar)
+        ctx.cfg = (k00, k11, z_clip, blur_radius, H, W, K, fl, light_stride, mode, sigma, gamma, znear, zfar)
         ctx.save_for_backward(Rs, Ts, Cs, lt, col, bg, p2f)
         ctx.mark_non_differentiable(p2f, counters, zbuf, bary, dists)
         return rgba, p2f, counters, zbuf, bary, dists
@@ -930,7 +930,7 @@ class _MeshRenderSoft(torch.autograd.Function):
         lib = L.load()
         geom, M = ctx.geom, ctx.M
         R, T, Cc, light, col, bg, p2f = ctx.saved_tensors
-        k00, k11, H, W, K, fl, light_stride, mode, sigma, gamma, znear, zfar = ctx.cfg
+        k00, k11, z_clip, blur_radius, H, W, K, fl, light_stride, mode, sigma, gamma, znear, zfar = ctx.cfg
         dev = geom.device
         N = geom.B * M
         g_rgba = _f32c(g_rgba)
@@ -940,7 +940,8 @@ class _MeshRenderSoft(torch.autograd.Function):
         with _on(dev):
             L.check(lib.mvr_mesh_soft_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
                                                geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc),
-                                               _ptr(light), light_stride, _ptr(col), _ptr(bg), k00, k11, H, W, K, fl, mode, sigma,
+                                               _ptr(light), light_stride, _ptr(col), _ptr(bg), k00, k11, z_clip, blur_radius, H, W, K,
+                                               fl, mode, sigma,
                                                gamma, znear, zfar, _ptr(p2f), _ptr(g_rgba), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(ws),
                                                ws.numel(), _stream(dev)), "mvr_mesh_soft_backward")
         return (gR, gT, gC) + (None,) * 18

@@ -17,10 +17,14 @@ import torch.nn.functional as F
 K_EPS = 1e-8
 
 
-def pix_centers(S, dtype=torch.float32):
-    """NDC coordinate of pixel index i (0 = top row / left column): +Y up, +X left."""
+def pix_centers(S, dtype=torch.float32, other=None):
+    """NDC coordinate of pixel index i (0 = top row / left column): +Y up, +X left.  other: the image's other side -- the
+    longer side of a non-square image spans 2 * (S // other) NDC units ([upstream] PixToNonSquareNdc)."""
     i = torch.arange(S, dtype=dtype)
-    return -1.0 + (2.0 * (S - 1 - i) + 1.0) / S
+    if other is None or S <= other:
+        return -1.0 + (2.0 * (S - 1 - i) + 1.0) / S
+    rng = 2.0 * (S // other)
+    return -rng / 2 + (rng * (S - 1 - i) + rng / 2) / S
 
 
 def look_at_view_transform(dist, elev, azim):
@@ -310,15 +314,27 @@ def soft_fragments(px, py, fv, perspective_correct, clip_bary):
     return b, bc, pz, torch.where(inside, -d, d), inside
 
 
-def rasterize_meshes_soft(face_verts, H, W, K, blur_radius, perspective_correct=True, clip_bary=None, cull_backfaces=False):
+def rasterize_meshes_soft(face_verts, H, W, K, blur_radius, perspective_correct=True, clip_bary=None, cull_backfaces=False,
+                          z_clip=None, return_sub=False):
     """One view, blur_radius >= 0 (squared NDC units, as upstream).  -> p2f (H,W,K) long, zbuf, bary (H,W,K,3), dists (signed),
     all -1 padded.  A face is a fragment of a pixel when the pixel lies in its bbox grown by sqrt(blur_radius) and is inside it
-    or closer than blur_radius (squared) to an edge; the K lexicographically smallest (z, face) win."""
+    or closer than blur_radius (squared) to an edge; the K lexicographically smallest (z, face) win.
+    z_clip: faces crossing the plane z = z_clip are clipped first (clip_faces, as the hard path) and their sub-triangles are
+    rasterized with blur; bary is then converted back to the original face (after the clip of the sub-triangle's barycentrics),
+    zbuf and the signed dists are the sub-triangle's.  A sub-triangle competes under its ORIGINAL face id by the same (z, id)
+    rule as any candidate, so a pixel near the cut between the two halves of a quad may hold the face twice, nearer half first.
+    That is the CUDA rasterizer's rule; upstream's rasterizer merges the two halves instead (clipped_faces_neighbor_idx),
+    which is not reproduced.  return_sub: also -> p2c (H,W,K), the fragment's index in clip_faces' list (-1 padded)."""
     if clip_bary is None:
         clip_bary = blur_radius > 0
     dt = face_verts.dtype
-    yf = pix_centers(H, dt)[:, None, None]
-    xf = pix_centers(W, dt)[None, :, None]
+    yf = pix_centers(H, dt, W)[:, None, None]
+    xf = pix_centers(W, dt, H)[None, :, None]
+    Fn0 = face_verts.shape[0]
+    if z_clip is not None:
+        face_verts, c2u, conv = clip_faces(face_verts, z_clip, perspective_correct)
+    else:
+        c2u, conv = torch.arange(Fn0), None
     fv = face_verts[None, None]
     b, bc, pz, sd, inside = soft_fragments(xf, yf, fv, perspective_correct, clip_bary)
     x, y, z = face_verts[..., 0], face_verts[..., 1], face_verts[..., 2]
@@ -331,7 +347,17 @@ def rasterize_meshes_soft(face_verts, H, W, K, blur_radius, perspective_correct=
     inbox = (xf <= x.max(1).values + r) & (xf >= x.min(1).values - r) & (yf <= y.max(1).values + r) & (yf >= y.min(1).values - r)
     hit = ok[None, None] & inbox & ~(pz < 0) & (inside | (sd < blur_radius))
     key = torch.where(hit, pz, torch.full_like(pz, float("inf")))
+    # stable sort by z: ties in clip_faces' order, i.e. by original face id (c2u is non-decreasing)
     order = torch.sort(key, dim=-1, stable=True)
+    if z_clip is not None and order.values.shape[-1] > 1:
+        # two sub-triangles of one face with the same depth make the same (z, id) key: one fragment
+        oid = c2u[order.indices]
+        dup = (order.values[..., 1:] == order.values[..., :-1]) & (oid[..., 1:] == oid[..., :-1]) & torch.isfinite(order.values[..., 1:])
+        if dup.any():
+            vals = order.values.clone()
+            vals[..., 1:][dup] = float("inf")
+            o2 = torch.sort(vals, dim=-1, stable=True)
+            order = torch.return_types.sort((o2.values, torch.gather(order.indices, -1, o2.indices)))
     Fn = face_verts.shape[0]
     idx, zs = order.indices[..., :K], order.values[..., :K]
     if Fn < K:
@@ -339,10 +365,15 @@ def rasterize_meshes_soft(face_verts, H, W, K, blur_radius, perspective_correct=
         zs = torch.cat([zs, zs.new_full((H, W, K - Fn), float("inf"))], -1)
     valid = torch.isfinite(zs)
     g = idx.clamp(0, max(Fn - 1, 0))
-    p2f = torch.where(valid, idx, torch.full_like(idx, -1))
+    p2f = torch.where(valid, c2u[g] if Fn else g, torch.full_like(idx, -1))
     zbuf = torch.where(valid, zs, torch.full_like(zs, -1.0))
-    bary = torch.where(valid[..., None], torch.gather(bc, 2, g[..., None].expand(H, W, K, 3)), torch.full((H, W, K, 3), -1.0, dtype=dt))
-    dists = torch.where(valid, torch.gather(sd, 2, g), torch.full_like(zs, -1.0))
+    bsel = torch.gather(bc, 2, g[..., None].expand(H, W, K, 3)) if Fn else torch.zeros((H, W, K, 3), dtype=dt)
+    if conv is not None and Fn:
+        bsel = (conv[g] * bsel[..., None, :]).sum(-1)      # convert_clipped_rasterization_to_original_faces
+    bary = torch.where(valid[..., None], bsel, torch.full((H, W, K, 3), -1.0, dtype=dt))
+    dists = torch.where(valid, torch.gather(sd, 2, g), torch.full_like(zs, -1.0)) if Fn else torch.full_like(zs, -1.0)
+    if return_sub:
+        return p2f, zbuf, bary, dists, torch.where(valid, idx, torch.full_like(idx, -1))
     return p2f, zbuf, bary, dists
 
 
@@ -389,22 +420,40 @@ def sigmoid_alpha_blend(colors, p2f, dists, sigma=1e-4):
 
 
 def render_mesh_view_soft(verts, faces, normals, vert_rgb, R, T, Cc, light_dir, bg, k00, k11, H, W, K, blur_radius, shader,
-                          sigma=1e-4, gamma=1e-4, perspective_correct=True, clip_bary=None, p2f=None):
+                          sigma=1e-4, gamma=1e-4, perspective_correct=True, clip_bary=None, p2f=None, cull_backfaces=False,
+                          z_clip=None, p2c=None):
     """Differentiable single-view soft render -> (4,H,W) RGBA + fragments.  shader: "soft_phong" | "soft_silhouette".
     The raster step (which face is fragment k of a pixel) is not differentiated; barycentrics, depth and signed distances are
-    recomputed differentiably from the face ids (what autograd does through _RasterizeFaceVerts)."""
+    recomputed differentiably from the face ids (what autograd does through _RasterizeFaceVerts).
+    z_clip: near-plane clipping as rasterize_meshes_soft(z_clip=...); the fragments are then given (or found) as p2c, indices
+    into clip_faces' list, and everything is recomputed on the sub-triangles and chained through the clipping ([upstream]
+    clip.py under autograd); p2f must be None."""
     if clip_bary is None:
         clip_bary = blur_radius > 0
     ndc = project_perspective(verts, R, T, k00, k11)
     fv = ndc[faces]
-    if p2f is None:
-        with torch.no_grad():
-            p2f, _, _, _ = rasterize_meshes_soft(fv, H, W, K, blur_radius, perspective_correct, clip_bary)
-    yf = pix_centers(H, verts.dtype)[:, None, None].expand(H, W, K)
-    xf = pix_centers(W, verts.dtype)[None, :, None].expand(H, W, K)
-    valid = p2f >= 0
-    _, bc, pz, sd, _ = soft_fragments(xf, yf, fv[p2f.clamp_min(0)], perspective_correct, clip_bary)
+    yf = pix_centers(H, verts.dtype, W)[:, None, None].expand(H, W, K)
+    xf = pix_centers(W, verts.dtype, H)[None, :, None].expand(H, W, K)
     m1 = torch.full((), -1.0, dtype=verts.dtype)
+    if z_clip is not None:
+        assert p2f is None
+        fvc, c2u, conv = clip_faces(fv, z_clip, perspective_correct)
+        if p2c is None:
+            with torch.no_grad():
+                p2c = rasterize_meshes_soft(fv, H, W, K, blur_radius, perspective_correct, clip_bary, cull_backfaces, z_clip,
+                                            return_sub=True)[4]
+        assert int(p2c.max()) < fvc.shape[0]
+        valid = p2c >= 0
+        sel = p2c.clamp_min(0)
+        _, bcs, pz, sd, _ = soft_fragments(xf, yf, fvc[sel], perspective_correct, clip_bary)
+        bc = (conv[sel] * bcs[..., None, :]).sum(-1)
+        p2f = torch.where(valid, c2u[sel], torch.full_like(p2c, -1))
+    else:
+        if p2f is None:
+            with torch.no_grad():
+                p2f, _, _, _ = rasterize_meshes_soft(fv, H, W, K, blur_radius, perspective_correct, clip_bary, cull_backfaces)
+        valid = p2f >= 0
+        _, bc, pz, sd, _ = soft_fragments(xf, yf, fv[p2f.clamp_min(0)], perspective_correct, clip_bary)
     bary = torch.where(valid[..., None], bc, m1); zbuf = torch.where(valid, pz, m1); dists = torch.where(valid, sd, m1)
     if shader == "soft_silhouette":
         img = sigmoid_alpha_blend(torch.ones_like(bary), p2f, dists, sigma)
