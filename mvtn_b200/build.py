@@ -42,7 +42,7 @@ def needs_build():
 def build(force=False, verbose=False):
     if not force and not needs_build():
         return LIB
-    base = [_nvcc()] + NVCC_FLAGS + os.environ.get("MVR_NVCC_DEFINES", "").split()      # e.g. -DMVR_SHADE_HOIST_FACES for an A/B build
+    base = [_nvcc()] + NVCC_FLAGS
     if os.path.exists("/usr/bin/g++"):
         base += ["-ccbin", "/usr/bin/g++"]
     if verbose:
@@ -54,7 +54,6 @@ def build(force=False, verbose=False):
     def compile_one(item):
         src, fmad = item
         obj = os.path.join(objdir, src.replace(".cu", ".o"))
-        fmad = fmad and not os.environ.get("MVR_NO_FMAD")      # A/B builds: every file without contraction
         cmd = base + ["-fmad=true" if fmad else "-fmad=false", "-c", os.path.join(CSRC, src), "-o", obj]
         return obj, subprocess.run(cmd, capture_output=True, text=True)
 

@@ -163,7 +163,7 @@ __global__ void __launch_bounds__(NT, MINB) mesh_scatter_kernel(const MeshParams
   // grid: x = chunk of faces, y = view m, z = object b (no integer divisions in the prologue)
   const int chunk = blockIdx.x, m = blockIdx.y, b = blockIdx.z, n = b * p.M + m;
   const int f0 = p.face_off[b], F = p.face_off[b + 1] - f0;
-  const int fbeg = chunk * p.faces_per_cta, fend = min(F, fbeg + p.faces_per_cta);
+  const int fbeg = chunk * FACES_PER_CTA, fend = min(F, fbeg + FACES_PER_CTA);
   if (fbeg >= fend) return;
   const int voff = p.vert_off[b], V = p.vert_off[b + 1] - voff;
   const float4* pvn = p.pv + (size_t)p.M * voff + (size_t)m * V;     // this view's projected vertices
@@ -531,46 +531,11 @@ extern "C" size_t mvr_mesh_workspace_bytes(int B, int M, int H, int W, int K, in
   return ws_layout(B, M, H, W, K, total_verts, total_faces).total;
 }
 
-// tuning knob (profiling only): MVR_SCATTER_MINB=3 trades occupancy (3 CTAs/SM, 85 registers) for fewer
-// rematerialised instructions in the scatter kernel's inner loops; default 4 CTAs/SM
-static int scatter_minb() {
-  static const int v = [] { const char* e = getenv("MVR_SCATTER_MINB"); return (e && atoi(e) == 3) ? 3 : 4; }();
-  return v;
-}
-
 // Threads (= faces per round) of a scatter CTA: 256 (4 CTAs per SM), or 128 (8 per SM) for large meshes -- twice as many
 // independent CTAs to cover each other's two barriers per round: 706 -> 663 us at 100 k faces x 160 views (r3z), but 340 -> 358 us at
-// 10 k faces x 384 views, where the rounds are too few to fill.  MVR_SCATTER_NT=128|256 overrides (profiling).
-static int scatter_nt(int max_faces) {
-  static const int v = [] { const char* e = getenv("MVR_SCATTER_NT"); const int x = e ? atoi(e) : 0; return (x == 128 || x == 256) ? x : 0; }();
-  return v ? v : (max_faces > 32768 ? 128 : 256);
-}
+// 10 k faces x 384 views, where the rounds are too few to fill.
+static int scatter_nt(int max_faces) { return max_faces > 32768 ? 128 : 256; }
 
-static int shade_minb() {
-  static const int v = [] { const char* e = getenv("MVR_SHADE_MINB"); const int x = e ? atoi(e) : 4; return x == 3 ? 3 : 4; }();
-  return v;
-}
-// pixels per thread of the image-only shade kernel (profiling knob; default MVR_SHADE_PPT_DEFAULT)
-#ifndef MVR_SHADE_PPT_DEFAULT
-#define MVR_SHADE_PPT_DEFAULT 4
-#endif
-static int shade_ppt() {
-  static const int v = [] { const char* e = getenv("MVR_SHADE_PPT"); const int x = e ? atoi(e) : MVR_SHADE_PPT_DEFAULT; return (x == 1 || x == 2 || x == 4) ? x : MVR_SHADE_PPT_DEFAULT; }();
-  return v;
-}
-// scatter: faces per CTA (profiling knob: 256 / 512 / 1024 / 2048; 512 = 13 waves of CTAs at C2 instead of 6.5 -> shorter tail)
-static int scatter_fpc() {
-  static const int v = [] { const char* e = getenv("MVR_SCATTER_FPC"); const int x = e ? atoi(e) : FACES_PER_CTA; return (x == 256 || x == 512 || x == 1024 || x == 2048) ? x : FACES_PER_CTA; }();
-  return v;
-}
-template <int PPT, bool VRGB>
-static void launch_shade_fast(const MeshParams& p, int B, int M, int H, int W, cudaStream_t st) {
-  const int tiles_x = (W + 31) / 32, tiles_y = (H + 8 * PPT - 1) / (8 * PPT);
-  const dim3 grid((unsigned)(tiles_x * tiles_y), (unsigned)M, (unsigned)B);
-  const int mb = shade_minb();
-  if (mb == 3) MVR_LAUNCH_PDL((mesh_shade_kernel<false, 3, PPT, VRGB>), grid, MVR_THREADS, 0, st, p, tiles_x);
-  else MVR_LAUNCH_PDL((mesh_shade_kernel<false, 4, PPT, VRGB>), grid, MVR_THREADS, 0, st, p, tiles_x);
-}
 extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
                                 int64_t total_verts, int64_t total_faces, int max_verts, int max_faces,
                                 const float* R, const float* T, const float* Cc, const float* light,
@@ -594,8 +559,7 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
   if (!(blur_radius >= 0.f)) { set_error("mvr_mesh_forward: blur_radius must be >= 0"); return -10; }
   const WsLayout w = ws_layout(B, M, H, W, K, total_verts, total_faces);
   if (workspace_bytes < w.total) { set_error("mvr_mesh_forward: workspace too small (%zu < %zu)", workspace_bytes, w.total); return -7; }
-  const int fpc = scatter_fpc();
-  const int chunks_per_view = max_faces > 0 ? (max_faces + fpc - 1) / fpc : 0;
+  const int chunks_per_view = max_faces > 0 ? (max_faces + FACES_PER_CTA - 1) / FACES_PER_CTA : 0;
   if (N * (int64_t)(chunks_per_view + 1) > 0x7fffffffLL) { set_error("mvr_mesh_forward: too many face chunks"); return -8; }
   const GeomLayout g = geom_layout(total_verts, total_faces);
   const char* gb = (const char*)geometry;
@@ -610,7 +574,7 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
   p.k00 = k00; p.k11 = k11; p.z_clip = z_clip;
   p.blur_radius = blur_radius > 0.f ? blur_radius : 0.f; p.blur_r = sqrtf(p.blur_radius);
   p.B = B; p.M = M; p.H = H; p.W = W; p.K = K; p.flags = flags;
-  p.chunks_per_view = chunks_per_view; p.layer = 0; p.faces_per_cta = fpc;
+  p.chunks_per_view = chunks_per_view; p.layer = 0;
   p.ndc_max = W > H ? (float)((W + H - 1) / H) : (float)((H + W - 1) / W);      // bound on |pixel-centre NDC| (>= aspect ratio)
   {
     const float rx = W > H ? 2.0f * (float)(W / H) : 2.0f;
@@ -634,15 +598,15 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
   rc = launch_project("mesh_project_kernel", g, w, geometry, vert_off, R, T, B, M, H, W, max_verts, k00, k11, z_clip, false, workspace, st, (long long*)counters);
   if (rc) return rc;
   const size_t tab_smem = ((size_t)W + H) * sizeof(float);
-  const int tiles_x = (W + 31) / 32, tiles_y = (H + 7) / 8;
-  const dim3 shade_grid((unsigned)(tiles_x * tiles_y), (unsigned)M, (unsigned)B);
+  const int tiles_x = (W + 31) / 32;
+  const dim3 shade_grid((unsigned)(tiles_x * ((H + 7) / 8)), (unsigned)M, (unsigned)B);           // 1 pixel per thread
+  const dim3 shade_fast_grid((unsigned)(tiles_x * ((H + 31) / 32)), (unsigned)M, (unsigned)B);     // 4 pixels per thread
   for (int k = 0; k < K; ++k) {
     p.layer = k;
     if (chunks_per_view > 0) {
       const dim3 scatter_grid((unsigned)chunks_per_view, (unsigned)M, (unsigned)B);
       if (soft_raster) MVR_LAUNCH_PDL((mesh_scatter_kernel<3, true>), scatter_grid, MVR_THREADS, tab_smem, st, p);
       else if (scatter_nt(max_faces) == 128) { MeshParams q = p; q.wcap = p.wcap < SC_QCAP ? p.wcap : SC_QCAP / 2; MVR_LAUNCH_PDL((mesh_scatter_kernel<8, false, 128>), scatter_grid, 128, tab_smem, st, q); }
-      else if (scatter_minb() == 3) MVR_LAUNCH_PDL((mesh_scatter_kernel<3, false>), scatter_grid, MVR_THREADS, tab_smem, st, p);
       else MVR_LAUNCH_PDL((mesh_scatter_kernel<4, false>), scatter_grid, MVR_THREADS, tab_smem, st, p);
       rc = check_launch("mesh_scatter_kernel");
       if (rc) return rc;
@@ -651,10 +615,8 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
     if (zbuf || bary || dists) {
       if (vrgb) MVR_LAUNCH_PDL((mesh_shade_kernel<true, 3, 1, true>), shade_grid, MVR_THREADS, 0, st, p, tiles_x);
       else MVR_LAUNCH_PDL((mesh_shade_kernel<true, 3, 1, false>), shade_grid, MVR_THREADS, 0, st, p, tiles_x);
-    } else if (vrgb) launch_shade_fast<4, true>(p, B, M, H, W, st);
-    else if (shade_ppt() == 4) launch_shade_fast<4, false>(p, B, M, H, W, st);
-    else if (shade_ppt() == 2) launch_shade_fast<2, false>(p, B, M, H, W, st);
-    else launch_shade_fast<1, false>(p, B, M, H, W, st);
+    } else if (vrgb) MVR_LAUNCH_PDL((mesh_shade_kernel<false, 4, 4, true>), shade_fast_grid, MVR_THREADS, 0, st, p, tiles_x);
+    else MVR_LAUNCH_PDL((mesh_shade_kernel<false, 4, 4, false>), shade_fast_grid, MVR_THREADS, 0, st, p, tiles_x);
     rc = check_launch("mesh_shade_kernel");
     if (rc) return rc;
     if (z_clip >= 0.f) {      // pixels won by a face crossing the near plane (none in MVTN's default configurations: the kernel exits at once)

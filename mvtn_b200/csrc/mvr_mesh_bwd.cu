@@ -177,16 +177,6 @@ __device__ __forceinline__ bool mesh_backward_pixel(const MeshBwdParams& p, int 
 __device__ __forceinline__ void scatter_vertex_grads(const MeshBwdParams& p, int voff, int fid, const float gvn[18], const int vids[3]) {
   const unsigned int full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
-  if (p.gv_plain) {      // A/B baseline: every lane scatters its own 18 values
-    if (fid >= 0) {
-#pragma unroll
-      for (int i = 0; i < 3; ++i) {
-        if (p.grad_verts) { float* o = p.grad_verts + 3 * (size_t)(voff + vids[i]); atomicAdd(o, gvn[6 * i]); atomicAdd(o + 1, gvn[6 * i + 1]); atomicAdd(o + 2, gvn[6 * i + 2]); }
-        if (p.grad_normals) { float* o = p.grad_normals + 3 * (size_t)(voff + vids[i]); atomicAdd(o, gvn[6 * i + 3]); atomicAdd(o + 1, gvn[6 * i + 4]); atomicAdd(o + 2, gvn[6 * i + 5]); }
-      }
-    }
-    return;
-  }
   const unsigned int grp = __match_any_sync(full, fid);
   unsigned int peers = fid >= 0 ? grp : 0u;
   const bool leader = fid >= 0 && (int)(__ffs(grp) - 1) == lane;
@@ -410,17 +400,6 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel_strip(
 
 using namespace mvr;
 
-static int backward_minb() {
-  static const int v = [] { const char* e = getenv("MVR_BWD_MINB"); const int x = e ? atoi(e) : 3; return (x == 2 || x == 4) ? x : 3; }();
-  return v;
-}
-
-// profiling knob: MVR_BWD_STRIP=0 falls back to the tile-per-CTA kernel everywhere
-static bool backward_strip() {
-  static const bool v = [] { const char* e = getenv("MVR_BWD_STRIP"); return !(e && atoi(e) == 0); }();
-  return v;
-}
-
 static int mesh_backward_impl(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
                               int64_t total_verts, int64_t total_faces, int max_verts, const float* R,
                               const float* T, const float* Cc, const float* light, int light_stride,
@@ -462,10 +441,9 @@ static int mesh_backward_impl(const void* geometry, const int* vert_off, const i
   p.onorm = make_out_norm(out_mean_std);
   p.z_clip = z_clip; p.wsflags = (int*)(wb + w.flags); p.parts_per_view = w.bwd_parts_per_view;
   p.azim = azim; p.elev = elev; p.dist = dist; p.g_azim = g_azim; p.g_elev = g_elev; p.g_dist = g_dist;
-  { static const int plain = [] { const char* e = getenv("MVR_BWD_GV_AGG"); return (e && atoi(e) == 0) ? 1 : 0; }(); p.gv_plain = plain; }
   const dim3 bgrid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
   const bool vrgb = flags & MVR_RGB_PER_ELEMENT;
-  const bool strip = backward_strip() && K == 1 && !(flags & MVR_IMAGES_BF16) && W % 4 == 0 &&
+  const bool strip = K == 1 && !(flags & MVR_IMAGES_BF16) && W % 4 == 0 &&
                      ((uintptr_t)pix_to_face % 16 == 0) && ((uintptr_t)grad_images % 16 == 0);
   const bool gv = grad_verts || grad_normals;
   if (strip) {
@@ -476,13 +454,9 @@ static int mesh_backward_impl(const void* geometry, const int* vert_off, const i
       else MVR_LAUNCH_PDL((mesh_backward_kernel_strip<2, false, true>), sgrid, MVR_THREADS, 0, st, p);
     }
     else if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel_strip<3, true, false>), sgrid, MVR_THREADS, 0, st, p);
-    else if (backward_minb() == 4) MVR_LAUNCH_PDL((mesh_backward_kernel_strip<4, false, false>), sgrid, MVR_THREADS, 0, st, p);      // profiling knobs
-    else if (backward_minb() == 2) MVR_LAUNCH_PDL((mesh_backward_kernel_strip<2, false, false>), sgrid, MVR_THREADS, 0, st, p);
     else MVR_LAUNCH_PDL((mesh_backward_kernel_strip<3, false, false>), sgrid, MVR_THREADS, 0, st, p);
   }
   else if (gv) { if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel<2, true, true>), bgrid, MVR_THREADS, 0, st, p); else MVR_LAUNCH_PDL((mesh_backward_kernel<2, false, true>), bgrid, MVR_THREADS, 0, st, p); }
-  else if (backward_minb() == 2) { if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel<2, true, false>), bgrid, MVR_THREADS, 0, st, p); else MVR_LAUNCH_PDL((mesh_backward_kernel<2, false, false>), bgrid, MVR_THREADS, 0, st, p); }
-  else if (backward_minb() == 4) { if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel<4, true, false>), bgrid, MVR_THREADS, 0, st, p); else MVR_LAUNCH_PDL((mesh_backward_kernel<4, false, false>), bgrid, MVR_THREADS, 0, st, p); }
   else if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel<3, true, false>), bgrid, MVR_THREADS, 0, st, p);
   else MVR_LAUNCH_PDL((mesh_backward_kernel<3, false, false>), bgrid, MVR_THREADS, 0, st, p);
   rc = check_launch("mesh_backward_kernel");

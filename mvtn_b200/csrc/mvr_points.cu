@@ -724,7 +724,7 @@ __global__ void __launch_bounds__(MVR_THREADS) points_backward_kernel(const Poin
   __shared__ float s_part[8][16];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int b = blockIdx.z, n = b * p.M + blockIdx.y;
-  const int nw = blockDim.x >> 5;                    // warps (= tiles) per CTA (8; MVR_PBWD_WPC for profiling)
+  const int nw = blockDim.x >> 5;                    // warps (= tiles) per CTA (8)
   const int tgy = blockIdx.x / p.tiles_x, txb = blockIdx.x - tgy * p.tiles_x;
   const int tyb = tgy * nw + warp;                   // the tile row this warp compacts
   const bool alpha_mode = p.flags & MVR_COMPOSITE_ALPHA;
@@ -989,10 +989,7 @@ struct PointsWs {
   int tiles_x, tiles_y, ntiles, list_cap, ctas_per_view, mask_words;
   bool tiled;
 };
-static bool points_use_tiles(int K) {
-  static const bool off = [] { const char* e = getenv("MVR_POINTS_TILED"); return e && atoi(e) == 0; }();   // profiling knob
-  return !off && (K == 1 || K == 2 || K == 4 || K == 8);
-}
+static bool points_use_tiles(int K) { return K == 1 || K == 2 || K == 4 || K == 8; }
 static PointsWs points_ws(int B, int Np, int M, int H, int W, int K, double radius) {
   auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
   PointsWs w;
@@ -1042,21 +1039,6 @@ extern "C" size_t mvr_points_hit_mask_words(int B, int M, int H, int W) {
   return (size_t)B * M * H * ((W + 31) / 32);
 }
 
-static int points_tile_minb_k1() {
-  static const int v = [] { const char* e = getenv("MVR_TILE_MINB_K1"); return (e && atoi(e) == 5) ? 5 : 4; }();
-  return v;
-}
-// profiling knob: MVR_TILE_MINB=4 asks for four instead of five tile CTAs per SM at K = 4
-static int points_tile_minb() {
-  static const int v = [] { const char* e = getenv("MVR_TILE_MINB"); return (e && atoi(e) == 4) ? 4 : 5; }();
-  return v;
-}
-// profiling knob: MVR_POINTS_BIN_FUSED=0 keeps the three-launch binning everywhere
-static bool points_bin_fused() {
-  static const bool v = [] { const char* e = getenv("MVR_POINTS_BIN_FUSED"); return !(e && atoi(e) == 0); }();
-  return v;
-}
-
 extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, int Np, int M, const float* R,
                                   const float* T, const float* inv_dist, double radius, const float* bg_rgb,
                                   int H, int W, int K, int flags, const float* out_mean_std, void* images, int* idx,
@@ -1092,14 +1074,13 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
   p.onorm = make_out_norm(out_mean_std);
   cudaStream_t st = (cudaStream_t)stream;
   const dim3 point_grid((unsigned)((Np + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
-  const bool bin_fused = w.tiled && Np > 0 && Np <= BIN_FUSED_MAX_POINTS && w.ntiles <= BIN_FUSED_MAX_TILES && points_bin_fused();
+  const bool bin_fused = w.tiled && Np > 0 && Np <= BIN_FUSED_MAX_POINTS && w.ntiles <= BIN_FUSED_MAX_TILES;
   if (Np > 0 && !bin_fused) MVR_LAUNCH(pixel_table_kernel, 1, MVR_THREADS, 0, st, (float*)(wb + w.tab), H, W);
   if (w.tiled) {
     if (bin_fused) {
-      static const int cs_knob = [] { const char* e = getenv("MVR_BIN_CLUSTER"); return e ? atoi(e) : 0; }();      // profiling knob: 1 / 2 / 4 / 8
       // a cluster of 4 CTAs per view for large clouds, and whenever there are fewer views than SMs (configs[0]: 12 views -- one CTA per
       // view leaves 136 SMs idle while 12 CTAs walk 2048 points each: 24 -> 16 us, a fifth of that graph-replayed step)
-      const int cs = (cs_knob == 1 || cs_knob == 2 || cs_knob == 4 || cs_knob == 8) ? cs_knob : ((Np > 4096 || (N < 148 && Np >= 512)) ? 4 : 1);
+      const int cs = (Np > 4096 || (N < 148 && Np >= 512)) ? 4 : 1;
       if (cs == 1) {
         MVR_LAUNCH(points_bin_kernel_fused, dim3((unsigned)M, (unsigned)B), MVR_THREADS, ((size_t)W + H) * sizeof(float), st, p, (float*)(wb + w.tab), 1);
       } else {      // thread-block cluster of cs CTAs per view (distributed shared memory)
@@ -1134,15 +1115,9 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
       // 0.094 ms, 47 registers / 5 CTAs 0.102 ms, 55 registers / 4 CTAs 0.110 ms): K = 1 / 2 compile to 40 / 46 registers when
       // left alone (MINB = 0), K = 4 is held to five CTAs per SM (48 registers instead of 56, no spills: 0.131 vs 0.133 ms),
       // K = 8 to three (74 KB of shared memory per CTA).
-      case 1:
-        if (points_tile_minb_k1() == 5) MVR_LAUNCH_PDL((points_tile_kernel<1, 5>), tile_grid, MVR_THREADS, smem, st, p);
-        else MVR_LAUNCH_PDL((points_tile_kernel<1, 0>), tile_grid, MVR_THREADS, smem, st, p);
-        break;
+      case 1: MVR_LAUNCH_PDL((points_tile_kernel<1, 0>), tile_grid, MVR_THREADS, smem, st, p); break;
       case 2: MVR_LAUNCH_PDL((points_tile_kernel<2, 0>), tile_grid, MVR_THREADS, smem, st, p); break;
-      case 4:
-        if (points_tile_minb() == 4) MVR_LAUNCH_PDL((points_tile_kernel<4, 0>), tile_grid, MVR_THREADS, smem, st, p);
-        else MVR_LAUNCH_PDL((points_tile_kernel<4, 5>), tile_grid, MVR_THREADS, smem, st, p);
-        break;
+      case 4: MVR_LAUNCH_PDL((points_tile_kernel<4, 5>), tile_grid, MVR_THREADS, smem, st, p); break;
       default: {
         // 64 KB of dynamic shared memory needs the opt-in (per device; the call is a few hundred nanoseconds)
         e = cudaFuncSetAttribute(points_tile_kernel<8, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1163,13 +1138,7 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
     rc = check_launch("points_scatter_kernel");
     if (rc) return rc;
   }
-  switch (K) {
-    case 1: MVR_LAUNCH(points_resolve_kernel<1>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x); break;
-    case 2: MVR_LAUNCH(points_resolve_kernel<2>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x); break;
-    case 4: MVR_LAUNCH(points_resolve_kernel<4>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x); break;
-    case 8: MVR_LAUNCH(points_resolve_kernel<8>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x); break;
-    default: MVR_LAUNCH(points_resolve_kernel<0>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x); break;
-  }
+  MVR_LAUNCH(points_resolve_kernel<0>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x);
   return check_launch("points_resolve_kernel");
 }
 
@@ -1204,7 +1173,7 @@ static int points_backward_impl(const float* points, const float* rgb, int B, in
   p.grad_points = grad_points; p.grad_rgb = grad_rgb;
   p.onorm = make_out_norm(out_mean_std);
   cudaStream_t st = (cudaStream_t)stream;
-  static const int wpc = [] { const char* e = getenv("MVR_PBWD_WPC"); const int x = e ? atoi(e) : 8; return (x == 1 || x == 2 || x == 4 || x == 8) ? x : 8; }();      // profiling knob
+  const int wpc = 8;      // warps (= tiles of a column) per CTA
   const int groups_y = (p.tiles_y + wpc - 1) / wpc;
   p.ctas_per_view = w.tiles_x * groups_y;             // one partial per CTA (<= one per tile: the workspace is sized for that)
   const dim3 grid((unsigned)p.ctas_per_view, (unsigned)M, (unsigned)B);

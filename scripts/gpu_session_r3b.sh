@@ -1,7 +1,7 @@
 #!/bin/bash
 TAG=${1:-r3x}; OUT=gpurun_out; mkdir -p $OUT
 timeout 1800 python -m pytest tests -m gpu -q -x --durations=5 > $OUT/${TAG}_pytest.log 2>&1; tail -9 $OUT/${TAG}_pytest.log | cut -c1-220
-for v in 1 0; do MVR_BWD_GV_AGG=$v python scripts/time_vertex_grads.py 2>&1 | grep -v Warning | tail -3; done | tee $OUT/${TAG}_vertex_grads.txt
+python scripts/time_vertex_grads.py 2>&1 | grep -v Warning | tail -3 | tee $OUT/${TAG}_vertex_grads.txt
 ( time python bench.py ) > $OUT/${TAG}_bench.json 2> $OUT/${TAG}_bench.err; tail -4 $OUT/${TAG}_bench.err
 python - <<PY
 import json

@@ -1,5 +1,5 @@
 """Backward of the C2 mesh workload WITH vertex gradients (d/d verts through projection, interpolated position and vertex
-normals): per-kernel device time of the backward kernel.  MVR_BWD_GV_AGG=0 switches the warp-aggregated scatter off (A/B)."""
+normals): per-kernel device time of the backward kernel."""
 import ctypes, os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,5 +34,5 @@ for nm in ("mesh_backward_kernel", "geom_normals_bwd"):
         step()
     t, n = ctypes.c_double(0), ctypes.c_int(0)
     lib.mvr_profile_collect(ctypes.byref(t), ctypes.byref(n))
-    print("%-28s %8.1f us per step (%d launches/step)   MVR_BWD_GV_AGG=%s" % (nm, 1e3 * t.value / 5, n.value // 5, os.environ.get("MVR_BWD_GV_AGG", "1")))
+    print("%-28s %8.1f us per step (%d launches/step)" % (nm, 1e3 * t.value / 5, n.value // 5))
 print("|grad_verts| sum %.6e" % float(g.abs().sum()))
