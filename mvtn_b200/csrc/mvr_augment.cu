@@ -174,7 +174,7 @@ __global__ void __launch_bounds__(MVR_THREADS) images_regularize_backward_rows_k
 using namespace mvr;
 
 static int check_aug(const char* who, const void* in, const void* out, int N, int C, int H, int W, int sy, int sx) {
-  if (N < 0 || C <= 0 || H <= 0 || W <= 0 || H > 65535 || W > 65535 || (int64_t)N * C > 0x7fffffffLL) { set_error("%s: bad shape (%d, %d, %d, %d)", who, N, C, H, W); return -1; }
+  if (N < 0 || C <= 0 || C > 65535 || H <= 0 || W <= 0 || H > 65535 || W > 65535 || (int64_t)N * C > 0x7fffffffLL) { set_error("%s: bad shape (%d, %d, %d, %d)", who, N, C, H, W); return -1; }
   if (N == 0) return 0;
   if (!in || !out) { set_error("%s: null pointer", who); return -2; }
   if (in == out) { set_error("%s: in-place is not supported (the gather reads what another thread writes)", who); return -3; }
@@ -190,14 +190,13 @@ extern "C" int mvr_images_regularize_forward(const void* images, int N, int C, i
   const int64_t planes = (int64_t)N * C;
   const bool vec = W % 4 == 0 && ((uintptr_t)out % 16 == 0);
   const unsigned gx = (unsigned)(((int64_t)H * ((W + 3) / 4) + MVR_THREADS - 1) / MVR_THREADS);
-  for (int64_t z0 = 0; z0 < planes; z0 += 65535) {      // grid.y limit
-    const int nz = (int)((planes - z0) < 65535 ? (planes - z0) : 65535);
+  const int64_t chunk = (int64_t)(65535 / C) * C;      // grid.y limit, in whole views: a chunk's planes start at view z0 / C
+  for (int64_t z0 = 0; z0 < planes; z0 += chunk) {
+    const int nz = (int)((planes - z0) < chunk ? (planes - z0) : chunk);
     AugParams q = p;
     const size_t off = (size_t)z0 * H * W * (p.bf16 ? 2 : 4);
     q.in = (const char*)images + off; q.out = (char*)out + off;
-    // planes of a chunk start at view z0 / C: the chunk boundary must fall between views for the per-view factor
     q.scale = view_scale ? view_scale + z0 / C : nullptr;
-    if (z0 % C) { set_error("mvr_images_regularize_forward: more than 65535 planes needs C to divide 65535"); return -5; }
     if (vec) MVR_LAUNCH(images_regularize_kernel<true>, dim3(gx, (unsigned)nz), MVR_THREADS, 0, (cudaStream_t)stream, q);
     else MVR_LAUNCH(images_regularize_kernel<false>, dim3(gx, (unsigned)nz), MVR_THREADS, 0, (cudaStream_t)stream, q);
   }
@@ -211,13 +210,13 @@ extern "C" int mvr_images_regularize_backward(const void* grad_out, int N, int C
   if ((size_t)W * sizeof(float) > 48 * 1024) { set_error("mvr_images_regularize_backward: W > 12288"); return -6; }
   AugParams p{grad_out, grad_in, view_scale, N, C, H, W, flip ? 1 : 0, shift_y, shift_x, (flags & MVR_IMAGES_BF16) ? 1 : 0};
   const int64_t planes = (int64_t)N * C;
-  for (int64_t z0 = 0; z0 < planes; z0 += 65535) {      // grid.y limit
-    const int nz = (int)((planes - z0) < 65535 ? (planes - z0) : 65535);
+  const int64_t chunk = (int64_t)(65535 / C) * C;      // grid.y limit, in whole views
+  for (int64_t z0 = 0; z0 < planes; z0 += chunk) {
+    const int nz = (int)((planes - z0) < chunk ? (planes - z0) : chunk);
     AugParams q = p;
     const size_t off = (size_t)z0 * H * W * (p.bf16 ? 2 : 4);
     q.in = (const char*)grad_out + off; q.out = (char*)grad_in + off;
     q.scale = view_scale ? view_scale + z0 / C : nullptr;
-    if (z0 % C) { set_error("mvr_images_regularize_backward: more than 65535 planes needs C to divide 65535"); return -5; }
     const bool vec = W % 4 == 0 && ((uintptr_t)grad_out % 16 == 0) && ((uintptr_t)grad_in % 16 == 0);
     if (W <= 1024 && vec) MVR_LAUNCH(images_regularize_backward_rows_kernel<true>, dim3((unsigned)((H + 7) / 8), (unsigned)nz), MVR_THREADS, (size_t)8 * W * sizeof(float), (cudaStream_t)stream, q);
     else if (W <= 1024) MVR_LAUNCH(images_regularize_backward_rows_kernel<false>, dim3((unsigned)((H + 7) / 8), (unsigned)nz), MVR_THREADS, (size_t)8 * W * sizeof(float), (cudaStream_t)stream, q);

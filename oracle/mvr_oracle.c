@@ -76,11 +76,12 @@ static inline float pix_to_ndc(int i, int S1, int S2) {
 /* Cameras: [upstream] renderer/cameras.py camera_position_from_spherical_angles,              */
 /* look_at_rotation, look_at_view_transform (called at renderer.py:79,122,168; ops.py:160)     */
 /* ------------------------------------------------------------------------------------------ */
-static inline void normalize3(const float v[3], float eps, float out[3]) {
-  /* F.normalize: v / max(||v||_2, eps) */
+/* F.normalize: v / max(||v||_2, eps).  Returns whether the norm, not eps, divided. */
+static inline int normalize3(const float v[3], float eps, float out[3]) {
   float n = sqrtf((v[0] * v[0] + v[1] * v[1]) + v[2] * v[2]);
   float d = n > eps ? n : eps;
   out[0] = v[0] / d; out[1] = v[1] / d; out[2] = v[2] / d;
+  return n > eps;
 }
 static inline void cross3(const float a[3], const float b[3], float o[3]) {
   o[0] = a[1] * b[2] - a[2] * b[1];
@@ -88,30 +89,43 @@ static inline void cross3(const float a[3], const float b[3], float o[3]) {
   o[2] = a[0] * b[1] - a[1] * b[0];
 }
 
+/* The branch decisions of one view's fp32 forward: which of F.normalize's eps clamps bound and whether the x axis was
+ * replaced.  orc_look_at_backward differentiates the branches these name, so that near the poles, where the fp32 and the
+ * double forward part ways, it differentiates the function the fp32 forward computed. */
+typedef struct { int z_norm, x_norm, y_norm, xr_norm, replaced; } LookAtBranches;
+
+static void look_at_view(float azim, float elev, float dist, float R[9], float T[3], float C[3], LookAtBranches* b) {
+  const float deg = (float)(M_PI / 180.0);
+  const float e = deg * elev, a = deg * azim, d = dist;
+  float c[3];
+  c[0] = (d * cosf(e)) * sinf(a);
+  c[1] = d * sinf(e);
+  c[2] = (d * cosf(e)) * cosf(a);
+  const float up[3] = {0.f, 1.f, 0.f};
+  float mz[3] = {0.f - c[0], 0.f - c[1], 0.f - c[2]}; /* at - camera_position */
+  float x[3], y[3], z[3], t[3];
+  b->z_norm = normalize3(mz, 1e-5f, z);
+  cross3(up, z, t); b->x_norm = normalize3(t, 1e-5f, x);
+  cross3(z, x, t); b->y_norm = normalize3(t, 1e-5f, y);
+  /* isclose(x_axis, 0, atol=5e-3).all() -> x = normalize(cross(y, z)) */
+  b->replaced = fabsf(x[0]) <= 5e-3f && fabsf(x[1]) <= 5e-3f && fabsf(x[2]) <= 5e-3f;
+  b->xr_norm = 1;
+  if (b->replaced) {
+    cross3(y, z, t); b->xr_norm = normalize3(t, 1e-5f, x);
+  }
+  for (int r = 0; r < 3; ++r) { R[3 * r + 0] = x[r]; R[3 * r + 1] = y[r]; R[3 * r + 2] = z[r]; }
+  /* T = -bmm(R^T, C) */
+  for (int j = 0; j < 3; ++j)
+    T[j] = -((R[0 + j] * c[0] + R[3 + j] * c[1]) + R[6 + j] * c[2]);
+  C[0] = c[0]; C[1] = c[1]; C[2] = c[2];
+}
+
 void orc_look_at(const float* azim, const float* elev, const float* dist, int n,
                  float* R, float* T, float* C) {
-  const float deg = (float)(M_PI / 180.0);
   for (int i = 0; i < n; ++i) {
-    const float e = deg * elev[i], a = deg * azim[i], d = dist[i];
     float c[3];
-    c[0] = (d * cosf(e)) * sinf(a);
-    c[1] = d * sinf(e);
-    c[2] = (d * cosf(e)) * cosf(a);
-    const float up[3] = {0.f, 1.f, 0.f};
-    float mz[3] = {0.f - c[0], 0.f - c[1], 0.f - c[2]}; /* at - camera_position */
-    float x[3], y[3], z[3], t[3];
-    normalize3(mz, 1e-5f, z);
-    cross3(up, z, t); normalize3(t, 1e-5f, x);
-    cross3(z, x, t); normalize3(t, 1e-5f, y);
-    /* isclose(x_axis, 0, atol=5e-3).all() -> x = normalize(cross(y, z)) */
-    if (fabsf(x[0]) <= 5e-3f && fabsf(x[1]) <= 5e-3f && fabsf(x[2]) <= 5e-3f) {
-      cross3(y, z, t); normalize3(t, 1e-5f, x);
-    }
-    float* Ri = R + 9 * i;
-    for (int r = 0; r < 3; ++r) { Ri[3 * r + 0] = x[r]; Ri[3 * r + 1] = y[r]; Ri[3 * r + 2] = z[r]; }
-    /* T = -bmm(R^T, C) */
-    for (int j = 0; j < 3; ++j)
-      T[3 * i + j] = -((Ri[0 + j] * c[0] + Ri[3 + j] * c[1]) + Ri[6 + j] * c[2]);
+    LookAtBranches b;
+    look_at_view(azim[i], elev[i], dist[i], R + 9 * i, T + 3 * i, c, &b);
     if (C) { C[3 * i] = c[0]; C[3 * i + 1] = c[1]; C[3 * i + 2] = c[2]; }
   }
 }
@@ -137,10 +151,12 @@ int orc_count_invalid_rotations(const float* R, int n) {
   return bad;
 }
 
-/* Backward of orc_look_at in double: (gR, gT, gC) -> (g_azim, g_elev, g_dist) per view. */
-static void normalize_bwd_d(const double v[3], double eps, const double g[3], double gv[3]) {
+/* Backward of orc_look_at in double: (gR, gT, gC) -> (g_azim, g_elev, g_dist) per view.  Every branch (the eps clamps of the
+ * four normalisations, the x-axis replacement) is the one the fp32 forward took (LookAtBranches): at elevation +-90 the fp32
+ * cos is -4.4e-8 where the double one is 6e-17, and only the fp32 branches give fp32 PyTorch3D's gradient (DESIGN.md 2). */
+static void normalize_bwd_d(const double v[3], double eps, int above, const double g[3], double gv[3]) {
   double n = sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
-  if (n > eps) {
+  if (above) {
     double u[3] = {v[0] / n, v[1] / n, v[2] / n};
     double d = u[0] * g[0] + u[1] * g[1] + u[2] * g[2];
     for (int i = 0; i < 3; ++i) gv[i] = (g[i] - u[i] * d) / n;
@@ -157,29 +173,39 @@ void orc_look_at_backward(const float* azim, const float* elev, const float* dis
                           const float* gR, const float* gT, const float* gC,
                           float* g_azim, float* g_elev, float* g_dist) {
   const double deg = M_PI / 180.0;
+  const float degf = (float)(M_PI / 180.0);
   for (int i = 0; i < n; ++i) {
-    const double e = deg * elev[i], a = deg * azim[i], d = dist[i];
+    float Rf[9], Tf[3], Cf[3];
+    LookAtBranches b;
+    look_at_view(azim[i], elev[i], dist[i], Rf, Tf, Cf, &b);
+    /* Where the fp32 x axis is clamped (within 6e-4 deg of a pole) x = (up x z) / 1e-5 depends on cos(elev) itself, which the
+     * fp32 rounding of the angle sets: fp32(pi/180) 90 lies 4.4e-8 rad past the pole, so there the camera sits on the other
+     * side of it.  There the angles are taken as the fp32 forward rounds them; elsewhere that rounding is a 6e-8 relative
+     * perturbation like any other and the exact angles are kept. */
+    const double e = b.x_norm ? deg * elev[i] : (double)(degf * elev[i]);
+    const double a = b.x_norm ? deg * azim[i] : (double)(degf * azim[i]);
+    const double d = dist[i];
     const double ce = cos(e), se = sin(e), ca = cos(a), sa = sin(a);
     double c[3] = {d * ce * sa, d * se, d * ce * ca};
     double up[3] = {0, 1, 0}, mz[3] = {-c[0], -c[1], -c[2]};
     double nz = sqrt(mz[0] * mz[0] + mz[1] * mz[1] + mz[2] * mz[2]);
-    double dz = nz > 1e-5 ? nz : 1e-5;
+    double dz = b.z_norm ? nz : 1e-5;
     double z[3] = {mz[0] / dz, mz[1] / dz, mz[2] / dz};
     double tx[3]; cross_d(up, z, tx);
     double nx = sqrt(tx[0] * tx[0] + tx[1] * tx[1] + tx[2] * tx[2]);
-    double dx = nx > 1e-5 ? nx : 1e-5;
+    double dx = b.x_norm ? nx : 1e-5;
     double x[3] = {tx[0] / dx, tx[1] / dx, tx[2] / dx};
     double ty[3]; cross_d(z, x, ty);
     double ny = sqrt(ty[0] * ty[0] + ty[1] * ty[1] + ty[2] * ty[2]);
-    double dy = ny > 1e-5 ? ny : 1e-5;
+    double dy = b.y_norm ? ny : 1e-5;
     double y[3] = {ty[0] / dy, ty[1] / dy, ty[2] / dy};
-    int replaced = fabs(x[0]) <= 5e-3 && fabs(x[1]) <= 5e-3 && fabs(x[2]) <= 5e-3;
+    const int replaced = b.replaced;
     double x0[3] = {x[0], x[1], x[2]}; /* x before replacement: y depends on this one */
     double txr[3];
     if (replaced) {
       cross_d(y, z, txr);
       double nr = sqrt(txr[0] * txr[0] + txr[1] * txr[1] + txr[2] * txr[2]);
-      double dr = nr > 1e-5 ? nr : 1e-5;
+      double dr = b.xr_norm ? nr : 1e-5;
       for (int k = 0; k < 3; ++k) x[k] = txr[k] / dr;
     }
     /* upstream grads: R[r][0]=x[r], R[r][1]=y[r], R[r][2]=z[r];  T_j = -sum_r R[r][j] c_r */
@@ -196,20 +222,20 @@ void orc_look_at_backward(const float* azim, const float* elev, const float* dis
     }
     double gt[3], tmp[3];
     if (replaced) { /* x = normalize(cross(y, z)) */
-      normalize_bwd_d(txr, 1e-5, gx, gt);
+      normalize_bwd_d(txr, 1e-5, b.xr_norm, gx, gt);
       cross_d(z, gt, tmp); for (int k = 0; k < 3; ++k) gy[k] += tmp[k];  /* d cross(y,z)/dy */
       cross_d(gt, y, tmp); for (int k = 0; k < 3; ++k) gz[k] += tmp[k];  /* d cross(y,z)/dz */
       gx[0] = gx[1] = gx[2] = 0;
     }
     /* y = normalize(cross(z, x0)) */
-    normalize_bwd_d(ty, 1e-5, gy, gt);
+    normalize_bwd_d(ty, 1e-5, b.y_norm, gy, gt);
     cross_d(x0, gt, tmp); for (int k = 0; k < 3; ++k) gz[k] += tmp[k];
     cross_d(gt, z, tmp);  for (int k = 0; k < 3; ++k) gx[k] += tmp[k];
     /* x0 = normalize(cross(up, z)) */
-    normalize_bwd_d(tx, 1e-5, gx, gt);
+    normalize_bwd_d(tx, 1e-5, b.x_norm, gx, gt);
     cross_d(gt, up, tmp); for (int k = 0; k < 3; ++k) gz[k] += tmp[k];
     /* z = normalize(-c) */
-    normalize_bwd_d(mz, 1e-5, gz, gt);
+    normalize_bwd_d(mz, 1e-5, b.z_norm, gz, gt);
     for (int k = 0; k < 3; ++k) gc[k] -= gt[k];
     /* c(d, e, a) */
     double gd = gc[0] * ce * sa + gc[1] * se + gc[2] * ce * ca;

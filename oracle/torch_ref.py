@@ -44,6 +44,34 @@ def look_at_view_transform(dist, elev, azim):
     return R, T, C
 
 
+def look_at_backward_fp32(dist, elev, azim, gR, gT, gC):
+    """fp32 autograd of look_at_view_transform under the cotangents (gR, gT, gC) -> (g_azim, g_elev, g_dist, cot), all (n,).
+    cot[i] is the largest |cotangent| any node of view i's graph receives or passes on.  Near the poles the chain through
+    the normalisations builds cotangents of 1e7 that cancel to an O(1) d elev, so an fp32 evaluation of it (this one, or the
+    CUDA kernel) carries an absolute error of a few eps_fp32 * cot[i]: the conditioning bar of DESIGN.md 2."""
+    n = dist.shape[0]
+    d, e, a = (t.detach().float().clone().requires_grad_() for t in (dist, elev, azim))
+    R, T, C = look_at_view_transform(d, e, a)
+    loss = (R * gR.float()).sum() + (T * gT.float()).sum() + (C * gC.float()).sum()
+    cot = torch.zeros(n)
+
+    def hook(grad_inputs, grad_outputs):
+        for g in grad_inputs + grad_outputs:
+            if g is not None and g.dim() >= 1 and g.shape[0] == n:
+                cot.copy_(torch.maximum(cot, g.detach().abs().reshape(n, -1).amax(1)))
+
+    seen, todo = set(), [loss.grad_fn]
+    while todo:
+        node = todo.pop()
+        if node is None or node in seen:
+            continue
+        seen.add(node)
+        node.register_hook(hook)
+        todo.extend(nx for nx, _ in node.next_functions)
+    loss.backward()
+    return a.grad, e.grad, d.grad, cot
+
+
 def fov_k(fov_deg=60.0, znear=1.0, dtype=torch.float32):
     """[upstream] FoVPerspectiveCameras.compute_projection_matrix K00 = K11 (aspect 1), as fp32 ops."""
     fov = torch.tensor(fov_deg, dtype=dtype) * (math.pi / 180.0)

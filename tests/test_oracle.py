@@ -99,6 +99,49 @@ def test_look_at_backward_matches_autograd(oracle):
     assert rel(gd, di.grad.numpy()) < 1e-5
 
 
+POLE_COT_K = 64      # conditioning bar: |a - b| <= POLE_COT_K * eps_fp32 * (largest intermediate cotangent of the view)
+
+
+def pole_views(n_az=9):
+    """Elevations at and next to the poles, each at n_az azimuths: exactly +-90 and +-270 (the fp32 x axis is clamped and
+    replaced), a few fp32 ulps either side of 90 (clamped, not replaced: the guard must flag them), 89.999 and 89.99 (ill
+    conditioned, not clamped) and 89 / 0 as controls."""
+    f = np.float32
+    ulp = np.spacing(f(90))
+    els = [90.0, -90.0, 270.0, -270.0, 89.999, -89.999, 89.99, -89.99, 89.0, 0.0] + \
+          [float(f(90) + k * ulp) for k in (-3, -1, 1, 3)]
+    az = np.linspace(-180, 180, n_az, endpoint=False).astype(f) + f(7.5)
+    return (np.repeat(az[None], len(els), 0).ravel(), np.repeat(np.array(els, f), n_az), np.full(len(els) * n_az, 2.2, f))
+
+
+def test_look_at_backward_at_the_poles_matches_fp32_autograd(oracle):
+    """At elevation +-90 the fp32 forward and a double one take different branches (fp32 cos(fp32(pi/2)) = -4.4e-8, double
+    6e-17: the y normalisation is clamped in double only), and the fp32 angle lies on the other side of the pole.  The
+    oracle's double backward follows the fp32 forward's branches and there its rounded angles, so it differentiates what
+    fp32 PyTorch3D computes.  The chain builds cotangents of 1e7 there that cancel to O(1): fp32 autograd is held to
+    POLE_COT_K eps_fp32 times the view's largest intermediate cotangent (fp32 autograd lands within 31 of them on the pole
+    views of these tests), which is tight for d azim and d dist (small cotangents reach them) and loose for d elev at the
+    pole, where the fp32 result is rounding noise of that size."""
+    az, el, di = pole_views()
+    n = az.size
+    g = torch.Generator().manual_seed(11)
+    gR, gT, gC = torch.randn(n, 3, 3, generator=g), torch.randn(n, 3, generator=g), torch.randn(n, 3, generator=g)
+    ta, te, td, cot = tr.look_at_backward_fp32(*(torch.from_numpy(t) for t in (di, el, az)), gR, gT, gC)
+    ga, ge, gd = oracle.look_at_backward(az, el, di, gR.numpy(), gT.numpy(), gC.numpy())
+    R, _, _ = oracle.look_at(az, el, di)
+    valid = np.array([oracle.count_invalid_rotations(R[i:i + 1]) == 0 for i in range(n)])
+    assert valid[np.isin(np.abs(el), [90.0, 270.0])].all()        # replaced x: a rotation, the guard lets it through
+    assert not valid[np.abs(np.abs(el) - 90) < 1e-5].all() and np.isfinite(np.r_[ga, ge, gd]).all()
+    bar = POLE_COT_K * np.finfo(np.float32).eps * cot.numpy().astype(np.float64)
+    deg = math.pi / 180
+    for mine, ref, scale in ((ta, ga, deg), (te, ge, deg), (td, gd, 1.0)):
+        assert (np.abs(mine.numpy().astype(np.float64) - ref) <= bar * scale + 1e-5 * np.abs(ref).max()).all()
+    # where the angles are well conditioned the plain 1e-5 bar holds
+    calm = np.abs(el) <= 89.0
+    for mine, ref in ((ta, ga), (te, ge), (td, gd)):
+        assert rel(mine.numpy()[calm], ref[calm]) < 1e-5
+
+
 def test_degenerate_elevation_is_flagged(oracle):
     # exactly-vertical view: up x z = 0 -> x axis collapses -> R is not a rotation (ops.py:156-165 guard)
     R = np.zeros((1, 3, 3), np.float32); R[0, :, 2] = [0, -1, 0]
