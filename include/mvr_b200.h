@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MVR_ABI_VERSION 11
+#define MVR_ABI_VERSION 12
 
 /* flags */
 #define MVR_PERSPECTIVE_CORRECT 1  /* [upstream] RasterizationSettings.perspective_correct (FoV persp.: True) */
@@ -235,17 +235,22 @@ int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert_off, const
                                 int mode, float sigma, float gamma, float znear, float zfar, const int* pix_to_face,
                                 const float* zbuf, const float* bary, const float* dists, float* rgba, void* stream);
 /* backward of rasterizer (incl. grad_zbuf, grad_dists, clipped barycentrics: [upstream] RasterizeMeshesBackward) + blend +
- * Phong + projection w.r.t. the cameras: grad_rgba (n,4,H,W) -> gR, gT, gC.  Fragments are recomputed from pix_to_face;
+ * Phong + projection: grad_rgba (n,4,H,W) -> gR, gT, gC (deterministic: fixed-order sums);
+ * optional grad_verts (Vtot,3) (projection + interpolated-position paths) and grad_normals (Vtot,3) (gradient w.r.t. the
+ * per-vertex unit normals, to be chained with mvr_mesh_normals_backward), both ACCUMULATED with atomics (caller zero-fills;
+ * the summation order is not fixed).  NULL for both: camera gradients only.  Mode 1 (silhouette) produces no normal gradient:
+ * grad_normals stays untouched.  Fragments are recomputed from pix_to_face;
  * z_clip and blur_radius must be those of the mvr_mesh_forward call that produced it: a fragment of a face crossing the
  * near plane z_clip is recomputed on the clipped sub-triangle the forward kept, and the chain runs through the clipping
- * ([upstream] clip.py).  -1 entries of a pixel's K-list are skipped, as mvr_mesh_soft_blend_forward does. */
+ * ([upstream] clip.py) to the vertices of the original face.  -1 entries of a pixel's K-list are skipped, as
+ * mvr_mesh_soft_blend_forward does. */
 int mvr_mesh_soft_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
                            int64_t total_verts, int64_t total_faces, int max_verts, const float* R, const float* T,
                            const float* Cc, const float* light, int light_stride, const float* obj_rgb,
                            const float* bg_rgb, float k00, float k11, float z_clip, float blur_radius, int H, int W, int K,
                            int flags, int mode, float sigma, float gamma, float znear, float zfar, const int* pix_to_face,
-                           const float* grad_rgba, float* gR, float* gT, float* gC, void* workspace, size_t workspace_bytes,
-                           void* stream);
+                           const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
+                           void* workspace, size_t workspace_bytes, void* stream);
 
 /* -- point clouds --------------------------------------------------------------------------- */
 /* scratch for one forward or backward call (forward: pixel table + per-view projected points, tile lists, or for K not

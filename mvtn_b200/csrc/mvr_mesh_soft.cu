@@ -8,9 +8,13 @@
 //   backward: mesh_soft_backward_kernel -- per pixel, per fragment: recompute (barycentrics, depth, signed edge distance,
 //             colour) from the projected vertices, then d RGBA -> blend weights -> (colour, zbuf, dists) -> Phong /
 //             [upstream] RasterizeMeshesBackward (BarycentricClipBackward, perspective correction, edge functions,
-//             PointTriangleDistanceBackward) -> NDC vertices -> (dR, dT, dC); per-warp partials, fixed-order sum.
-// Tolerance-compared against the torch restatement (oracle/torch_ref.py render_mesh_view_soft, autograd): not on MVTN's default
-// path, written for clarity rather than tuned.
+//             PointTriangleDistanceBackward) -> NDC vertices -> (dR, dT, dC); per-warp partials, fixed-order sum (deterministic).
+//             <GV = true> also returns, per fragment, d/d position of the three vertices of its ORIGINAL face (projection
+//             chain through R, plus Phong's interpolated-position term) and d/d their unit normals (Phong, soft_phong only),
+//             scattered with one plain atomicAdd per value (as [upstream] RasterizeMeshesBackward): the vertex gradients are
+//             tolerance-level, their summation order is not fixed.  The camera arithmetic is the same in both instances.
+// Tolerance-compared against the torch restatement (oracle/torch_ref.py render_mesh_view_soft + vertex_normals, autograd): not
+// on MVTN's default path, written for clarity rather than tuned.
 #include "mvr_mesh.cuh"
 
 namespace mvr {
@@ -21,6 +25,7 @@ struct SoftParams {
   const float* zbuf; const float* bary; const float* dists;      // forward: the rasterizer's fragments (n, H, W, K[, 3])
   float* rgba;             // forward out: (n, 4, H, W)
   const float* grad_rgba;  // backward in
+  float* grad_verts; float* grad_normals;      // backward out (GV): (Vtot,3) accumulated, either may be NULL
 };
 
 constexpr float SOFT_EPS = 1e-10f;
@@ -126,14 +131,19 @@ __device__ __forceinline__ int rank_in_list(const int* list, int k, int fid) {
   return r;
 }
 
-// One fragment: push (g_colour, g_zbuf, g_sdist) back to the camera accumulators acc[15].
-__device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, int voff, const int4 fi, const Face& fc, const SoftFrag& fr,
-                                                       const ClipSub& cs, bool persp, bool clipb, float xf, float yf, const ShadeCtx& sc,
-                                                       const float gcol[3], float gz, float gsd, bool with_colour, float acc[16]) {
+// One fragment of view n: push (g_colour, g_zbuf, g_sdist) back to the camera accumulators acc[15]; GV: also to the vertices
+// of the original face (sp.grad_verts: projection chain + Phong's interpolated position; sp.grad_normals: Phong's normal term).
+template <bool GV>
+__device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, const SoftParams& sp, int n, int voff, const int4 fi, const Face& fc,
+                                                       const SoftFrag& fr, const ClipSub& cs, bool persp, bool clipb, float xf, float yf,
+                                                       const ShadeCtx& sc, const float gcol[3], float gz, float gsd, bool with_colour,
+                                                       float acc[16]) {
   const Face& g = fr.g;
   float4 X0, X1, X2, N0, N1, N2;
   gather_xn(p.xn8, voff + fi.x, X0, N0); gather_xn(p.xn8, voff + fi.y, X1, N1); gather_xn(p.xn8, voff + fi.z, X2, N2);
+  const int vid[3] = {fi.x, fi.y, fi.z};
   float gbb[3] = {0.f, 0.f, 0.f};      // w.r.t. the barycentrics on the original face
+  float gP[3] = {0.f, 0.f, 0.f};       // GV: w.r.t. the interpolated position P = sum_i bb_i X_i (= -d/d camera centre)
   if (with_colour) {
     float4 c0, c1, c2;
     if (p.flags & MVR_RGB_PER_ELEMENT) { c0 = __ldg(p.rgb4 + voff + fi.x); c1 = __ldg(p.rgb4 + voff + fi.y); c2 = __ldg(p.rgb4 + voff + fi.z); }
@@ -141,6 +151,14 @@ __device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, int 
     float gv[3], gN[3];
     phong_backward(fr.bb, X0, X1, X2, N0, N1, N2, c0, c1, c2, sc, gcol[0], gcol[1], gcol[2], gbb, gv, gN);
     acc[12] += gv[0]; acc[13] += gv[1]; acc[14] += gv[2];      // dC
+    if (GV) {
+      gP[0] = -gv[0]; gP[1] = -gv[1]; gP[2] = -gv[2];
+      if (sp.grad_normals)      // Nn = sum_i bb_i N_i
+        for (int i = 0; i < 3; ++i) {
+          float* o = sp.grad_normals + 3 * (size_t)(voff + vid[i]);
+          atomicAdd(o + 0, fr.bb[i] * gN[0]); atomicAdd(o + 1, fr.bb[i] * gN[1]); atomicAdd(o + 2, fr.bb[i] * gN[2]);
+        }
+    }
   }
   // w.r.t. the barycentrics carried on g: through the conversion bb_j = sum_k conv[3 j + k] bc_k for a sub-triangle
   float gbc[3] = {gbb[0], gbb[1], gbb[2]};
@@ -195,11 +213,20 @@ __device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, int 
     acc[3] += Xs[i].y * gpx; acc[4] += Xs[i].y * gpy; acc[5] += Xs[i].y * gpz;
     acc[6] += Xs[i].z * gpx; acc[7] += Xs[i].z * gpy; acc[8] += Xs[i].z * gpz;
     acc[9] += gpx; acc[10] += gpy; acc[11] += gpz;
+    if (GV && sp.grad_verts) {      // X_view = X R + T: d/d X = R (gpx, gpy, gpz); P = sum_i bb_i X_i
+      const float* r = p.R + 9 * (size_t)n;
+      float* o = sp.grad_verts + 3 * (size_t)(voff + vid[i]);
+      atomicAdd(o + 0, (__ldg(r + 0) * gpx + __ldg(r + 1) * gpy + __ldg(r + 2) * gpz) + fr.bb[i] * gP[0]);
+      atomicAdd(o + 1, (__ldg(r + 3) * gpx + __ldg(r + 4) * gpy + __ldg(r + 5) * gpz) + fr.bb[i] * gP[1]);
+      atomicAdd(o + 2, (__ldg(r + 6) * gpx + __ldg(r + 7) * gpy + __ldg(r + 8) * gpz) + fr.bb[i] * gP[2]);
+    }
   }
 }
 
 // grid: x = 32x32-pixel tiles, y = view m, z = object b; thread (lane, warp) owns pixels (x0 + lane, y0 + warp + 8 j); one
 // 16-float partial per warp at partials[(n * parts_per_view + tile * NWARPS + warp) * 16] (mesh_backward_finish_kernel sums them)
+// GV: vertex gradients too (soft_fragment_backward<true>)
+template <bool GV>
 __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const MeshParams p, const SoftParams sp, float* __restrict__ partials,
                                                                          int parts_per_view, int tiles_x) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -282,7 +309,7 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
         if (pass == 1) {      // z_inv_max = z_inv of this fragment
           if (zmax_live && gzmax != 0.f) {
             const float gcz[3] = {0.f, 0.f, 0.f};
-            soft_fragment_backward(p, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, -gzmax * zscale, 0.f, false, acc);
+            soft_fragment_backward<GV>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, -gzmax * zscale, 0.f, false, acc);
           }
           continue;
         }
@@ -310,7 +337,7 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
           gzmax -= gzi;
         }
         const float gsd = gprob * (-1.0f / sp.sigma) * prob * (1.0f - prob);
-        soft_fragment_backward(p, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc);
+        soft_fragment_backward<GV>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc);
       }
     }
   }
@@ -353,7 +380,7 @@ extern "C" int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert
   if (mode < 0 || mode > 1 || !(sigma > 0.f) || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_blend_forward: bad mode / sigma / gamma / z range"); return -7; }
   MeshParams p;
   fill_params(p, geometry, vert_off, face_off, B, M, total_verts, total_faces, nullptr, nullptr, Cc, light, light_stride, obj_rgb, bg_rgb, 0.f, 0.f, H, W, K, flags, pix_to_face);
-  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, zbuf, bary, dists, rgba, nullptr};
+  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, zbuf, bary, dists, rgba, nullptr, nullptr, nullptr};
   const dim3 grid((unsigned)(((size_t)H * W + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
   MVR_LAUNCH(mesh_soft_blend_kernel, grid, MVR_THREADS, 0, (cudaStream_t)stream, p, sp);
   return check_launch("mesh_soft_blend_kernel");
@@ -364,8 +391,8 @@ extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off,
                                       int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, float z_clip,
                                       float blur_radius, int H, int W, int K, int flags, int mode, float sigma, float gamma, float znear,
                                       float zfar, const int* pix_to_face,
-                                      const float* grad_rgba, float* gR, float* gT, float* gC, void* workspace, size_t workspace_bytes,
-                                      void* stream) {
+                                      const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
   int rc = check_mesh_common("mvr_mesh_soft_backward", B, M, H, W, K, total_verts, total_faces, max_verts);
   if (rc) return rc;
   const int64_t N = (int64_t)B * M;
@@ -388,10 +415,13 @@ extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off,
   p.pv = (float4*)(wb + w.pv); p.tab = (float*)(wb + w.tab); p.wsflags = (int*)(wb + w.flags);
   p.z_clip = z_clip;
   p.blur_radius = blur_radius > 0.f ? blur_radius : 0.f; p.blur_r = sqrtf(p.blur_radius);      // as mvr_mesh_forward
-  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, nullptr, nullptr, nullptr, nullptr, grad_rgba};
+  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, nullptr, nullptr, nullptr, nullptr, grad_rgba, grad_verts, grad_normals};
   const int tiles_x = (W + 31) / 32;
   const dim3 grid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
-  MVR_LAUNCH(mesh_soft_backward_kernel, grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
+  if (grad_verts || grad_normals)
+    MVR_LAUNCH((mesh_soft_backward_kernel<true>), grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
+  else
+    MVR_LAUNCH((mesh_soft_backward_kernel<false>), grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
   rc = check_launch("mesh_soft_backward_kernel");
   if (rc) return rc;
   MeshBwdParams q;

@@ -763,6 +763,17 @@ def _mesh_forward_launch(geom: "PackedMeshes", M, R, T, Cc, light, obj_rgb, bg_r
     return cfg, saved, images, extras
 
 
+def _normals_backward_launch(geom: "PackedMeshes", gN, gV):
+    """A backward kernel returned d/d verts through projection + interpolated position (gV) and d/d unit normals (gN); the
+    normals -> verts chain ([upstream] Meshes._compute_vertex_normals) is mvr_mesh_normals_backward: gN is consumed, gV
+    accumulated."""
+    dev = geom.device
+    with _on(dev):
+        L.check(L.load().mvr_mesh_normals_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B,
+                                                   geom.total_verts, geom.total_faces, geom.max_faces, _ptr(gN), _ptr(gV),
+                                                   _stream(dev)), "mvr_mesh_normals_backward")
+
+
 def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_verts, angles=None):
     """ONE mvr_mesh_backward call -> (gR, gT, gC, gV | None) (gV includes the chain through the vertex normals).  angles =
     (azim, elev, dist) flat fp32: mvr_mesh_backward_angles instead, whose last kernel also applies the camera backward ->
@@ -803,12 +814,7 @@ def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_ve
                                           _ptr(g_images), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(gV), _ptr(gN), _ptr(ws),
                                           ws.numel(), _stream(dev)), "mvr_mesh_backward")
     if gV is not None:
-        # the kernel returned d/d verts through projection + interpolated position, and d/d unit normals; the
-        # normals -> verts chain ([upstream] Meshes._compute_vertex_normals) is mvr_mesh_normals_backward
-        with _on(dev):
-            L.check(lib.mvr_mesh_normals_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B,
-                                                  geom.total_verts, geom.total_faces, geom.max_faces, _ptr(gN), _ptr(gV),
-                                                  _stream(dev)), "mvr_mesh_normals_backward")
+        _normals_backward_launch(geom, gN, gV)
     if angles is not None:
         return ga, ge, gd, gV
     return gR, gT, gC, gV
@@ -893,12 +899,13 @@ SOFT_SHADERS = {"soft_phong": 0, "soft_silhouette": 1}
 
 class _MeshRenderSoft(torch.autograd.Function):
     """Blurred rasterizer (K fragments per pixel, signed edge distances, clipped barycentrics) + soft blend as one autograd
-    node: (R, T, C) -> RGBA (n,4,H,W).  [upstream] MeshRasterizer(blur_radius, faces_per_pixel) + SoftPhongShader
+    node: (R, T, C, verts) -> RGBA (n,4,H,W).  [upstream] MeshRasterizer(blur_radius, faces_per_pixel) + SoftPhongShader
     (softmax_rgb_blend) / SoftSilhouetteShader (sigmoid_alpha_blend); renderer.py:4-6, :91-92 (SURVEY 8f N3)."""
 
     @staticmethod
-    def forward(ctx, R, T, Cc, geom: PackedMeshes, M, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags, blur_radius,
+    def forward(ctx, R, T, Cc, verts, geom: PackedMeshes, M, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags, blur_radius,
                 mode, sigma, gamma, znear, zfar):
+        # `verts` (packed (Vtot,3), same values as geom.verts) only carries autograd history for vertex gradients
         lib = L.load()
         cfg, saved, _hard, extras = _mesh_forward_launch(geom, M, R, T, Cc, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags,
                                                          True, None, None, blur_radius=blur_radius)
@@ -926,7 +933,7 @@ class _MeshRenderSoft(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_rgba, *_unused):
         if g_rgba is None:
-            return (None,) * 21
+            return (None,) * 22
         lib = L.load()
         geom, M = ctx.geom, ctx.M
         R, T, Cc, light, col, bg, p2f = ctx.saved_tensors
@@ -936,15 +943,22 @@ class _MeshRenderSoft(torch.autograd.Function):
         g_rgba = _f32c(g_rgba)
         g = torch.empty(15 * N, dtype=torch.float32, device=dev)
         gR, gT, gC = g[: 9 * N].view(N, 3, 3), g[9 * N: 12 * N].view(N, 3), g[12 * N:].view(N, 3)
+        gV = gN = None
+        if ctx.needs_input_grad[3]:
+            gV = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
+            if mode == SOFT_SHADERS["soft_phong"]:      # the silhouette does not depend on the normals
+                gN = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
         ws = workspace(dev, lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, K, geom.total_verts, geom.total_faces))
         with _on(dev):
             L.check(lib.mvr_mesh_soft_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
                                                geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc),
                                                _ptr(light), light_stride, _ptr(col), _ptr(bg), k00, k11, z_clip, blur_radius, H, W, K,
                                                fl, mode, sigma,
-                                               gamma, znear, zfar, _ptr(p2f), _ptr(g_rgba), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(ws),
-                                               ws.numel(), _stream(dev)), "mvr_mesh_soft_backward")
-        return (gR, gT, gC) + (None,) * 18
+                                               gamma, znear, zfar, _ptr(p2f), _ptr(g_rgba), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(gV),
+                                               _ptr(gN), _ptr(ws), ws.numel(), _stream(dev)), "mvr_mesh_soft_backward")
+        if gN is not None:
+            _normals_backward_launch(geom, gN, gV)
+        return (gR, gT, gC, gV) + (None,) * 18
 
 
 def render_meshes_from_angles(geom: PackedMeshes, M: int, azim, elev, dist, light, obj_rgb, bg_rgb, image_size,
@@ -971,8 +985,9 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
     shader="soft_phong" / "soft_silhouette" (SURVEY 8f N3) -- RGBA (B*M,4,H,W) from the K = faces_per_pixel fragments of the
     BLURRED rasterizer ([upstream] blur_radius in squared NDC units, clip_barycentric_coords default True iff blur_radius > 0)
     blended by softmax_rgb_blend over per-fragment Phong colours / sigmoid_alpha_blend (sigma, gamma = BlendParams);
-    differentiable w.r.t. R, T, C through colours, depths and the signed edge distances (grad_dists).
-    `verts`: pass the packed (Vtot,3) vertex tensor the geometry was built from to get gradients w.r.t. it.
+    differentiable w.r.t. R, T, C (and `verts`) through colours, depths and the signed edge distances (grad_dists).
+    `verts`: pass the packed (Vtot,3) vertex tensor the geometry was built from to get gradients w.r.t. it (any shader; the
+    vertex gradients are accumulated with float atomics: tolerance-level, not bit-reproducible run to run).
     `normalize=(mean, std)` / `out_dtype=torch.bfloat16`: consumer-side fusion (SURVEY 8f N2) -- the kernel writes
     (x - mean) / std (Trainer_mvt.py:41-49) in the dtype the CNN consumes; gradients flow through both."""
     H_, W_ = _hw(image_size)
@@ -986,10 +1001,10 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
     if shader != "hard_phong":
         if shader not in SOFT_SHADERS:
             raise ValueError("shader must be 'hard_phong', 'soft_phong' or 'soft_silhouette'")
-        if verts is not None or normalize is not None or out_dtype not in (None, torch.float32):
-            raise ValueError("the soft shaders return fp32 RGBA and gradients w.r.t. the cameras only")
+        if normalize is not None or out_dtype not in (None, torch.float32):
+            raise ValueError("the soft shaders return fp32 RGBA: normalize / out_dtype are not supported with them")
         flags |= L.CLIP_BARYCENTRIC if clip_barycentric_coords else 0
-        out = _MeshRenderSoft.apply(R, T, Cc, geom, M, light, obj_rgb, bg_rgb, k00, k11, float(z_clip), H, W, int(faces_per_pixel),
+        out = _MeshRenderSoft.apply(R, T, Cc, verts, geom, M, light, obj_rgb, bg_rgb, k00, k11, float(z_clip), H, W, int(faces_per_pixel),
                                     flags, float(blur_radius), SOFT_SHADERS[shader], float(sigma), float(gamma), float(znear), float(zfar))
         return out[0], {"pix_to_face": out[1], "counters": out[2], "zbuf": out[3], "bary_coords": out[4], "dists": out[5]}
     if blur_radius > 0 or clip_barycentric_coords:

@@ -131,6 +131,8 @@ class MVRenderer(nn.Module):
         shader / blur_radius / blend_sigma / blend_gamma / keep_alpha: mesh path -- "soft_phong" (SoftPhongShader) or
             "soft_silhouette" (SoftSilhouetteShader) blend the faces_per_pixel fragments of the blurred rasterizer (the
             shaders renderer.py:4-6 imports; SURVEY 8f N3); images keep 3 channels as renderer.py:112 unless keep_alpha.
+            Gradients reach the cameras and, when the meshes' vertex tensors require grad, the vertices (through colours,
+            depths and edge distances; tolerance-level: accumulated with float atomics), as with the hard shader.
         normalize: None or (mean, std) (3-vectors or scalars): the kernels write (image - mean) / std, the
             normalisation viewGCN/tools/Trainer_mvt.py:41-49 applies before the CNN (SURVEY 8f N2).
         out_dtype: torch.float32 (default) or torch.bfloat16 -- the dtype the images are written in (a bf16 backbone
@@ -248,8 +250,9 @@ class MVRenderer(nn.Module):
             if soft:
                 return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
                                          faces_per_pixel=self.faces_per_pixel, cull_backfaces=self.cull_backfaces,
-                                         perspective_correct=self.perspective_correct, shader=self.shader,
-                                         blur_radius=self.blur_radius, sigma=self.blend_sigma, gamma=self.blend_gamma)
+                                         perspective_correct=self.perspective_correct, verts=getattr(geom, "grad_verts", None),
+                                         shader=self.shader, blur_radius=self.blur_radius, sigma=self.blend_sigma,
+                                         gamma=self.blend_gamma)
             return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
                                      faces_per_pixel=self.faces_per_pixel, cull_backfaces=self.cull_backfaces,
                                      perspective_correct=self.perspective_correct, verts=getattr(geom, "grad_verts", None),
