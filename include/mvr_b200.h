@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MVR_ABI_VERSION 12
+#define MVR_ABI_VERSION 13
 
 /* flags */
 #define MVR_PERSPECTIVE_CORRECT 1  /* [upstream] RasterizationSettings.perspective_correct (FoV persp.: True) */
@@ -223,6 +223,18 @@ int mvr_mesh_backward_angles(const void* geometry, const int* vert_off, const in
                              const float* dist, float* g_azim, float* g_elev, float* g_dist, float* gR, float* gT,
                              float* gC, float* grad_verts, float* grad_normals, void* workspace, size_t workspace_bytes,
                              void* stream);
+/* mvr_mesh_backward that also returns the gradient w.r.t. the colours (texture fitting, colour attacks).  grad_rgb: with
+ * per-vertex colours (MVR_RGB_PER_ELEMENT) (Vtot,3), ACCUMULATED with atomics (caller zero-fills); with one object colour (3),
+ * WRITTEN by a fixed-order sum (per-warp partials, fp64 per view, fixed order over the views: bit-reproducible).  NULL: exactly
+ * mvr_mesh_backward.  The camera gradients are the same, bit for bit, with and without it. */
+int mvr_mesh_backward_rgb(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                          int64_t total_verts, int64_t total_faces, int max_verts, const float* R,
+                          const float* T, const float* Cc, const float* light, int light_stride,
+                          const float* obj_rgb, float k00, float k11, float z_clip, int H, int W, int K, int flags,
+                          const float* out_mean_std, const int* pix_to_face, const void* grad_images, float* gR,
+                          float* gT, float* gC,
+                          float* grad_verts, float* grad_normals, void* workspace, size_t workspace_bytes,
+                          void* stream, float* grad_rgb);
 
 /* -- soft shading of K fragments per pixel (SURVEY 8f N3; renderer.py:4-6 SoftPhongShader / SoftSilhouetteShader) -------- */
 /* mode 0: [upstream] blending.softmax_rgb_blend over per-fragment Phong colours (SoftPhongShader; sigma, gamma = BlendParams,
@@ -251,6 +263,15 @@ int mvr_mesh_soft_backward(const void* geometry, const int* vert_off, const int*
                            int flags, int mode, float sigma, float gamma, float znear, float zfar, const int* pix_to_face,
                            const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
                            void* workspace, size_t workspace_bytes, void* stream);
+/* mvr_mesh_soft_backward that also returns the colour gradient, grad_rgb as in mvr_mesh_backward_rgb.  Mode 1 (silhouette)
+ * does not depend on the colours: a (3) grad_rgb is written with zeros, a (Vtot,3) one stays untouched. */
+int mvr_mesh_soft_backward_rgb(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                               int64_t total_verts, int64_t total_faces, int max_verts, const float* R, const float* T,
+                               const float* Cc, const float* light, int light_stride, const float* obj_rgb,
+                               const float* bg_rgb, float k00, float k11, float z_clip, float blur_radius, int H, int W, int K,
+                               int flags, int mode, float sigma, float gamma, float znear, float zfar, const int* pix_to_face,
+                               const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
+                               void* workspace, size_t workspace_bytes, void* stream, float* grad_rgb);
 
 /* -- point clouds --------------------------------------------------------------------------- */
 /* scratch for one forward or backward call (forward: pixel table + per-view projected points, tile lists, or for K not

@@ -18,10 +18,13 @@ namespace mvr {
 // GV (vertex gradients wanted): the contributions to d/d verts and d/d normals of the pixel's three vertices are returned
 // in gvn[18] (vertex i: gvn[6 i .. 6 i + 2] = d/d position, gvn[6 i + 3 .. 6 i + 5] = d/d unit normal) and vids, and the
 // caller scatters them with warp-aggregated atomics (scatter_vertex_grads); returns false when nothing was produced.
-template <bool VRGB, bool GV>
+// GC (colour gradient wanted): with VRGB, gcol[3 i .. 3 i + 2] = d/d colour of vertex i (= bb_i d/d texel; vids set as for GV,
+// scattered by scatter_rgb_grads); with one object colour, gcol[0..2] += sum(bb) d/d texel (the thread's running sum).
+template <bool VRGB, bool GV, bool GC = false>
 __device__ __forceinline__ bool mesh_backward_pixel(const MeshBwdParams& p, int n, int f0, int voff, const float4* __restrict__ pvn,
                                                     bool persp, const ShadeCtx& sc, const float4 ucol, int fid, float g0, float g1,
-                                                    float g2, float xf, int yi, float acc[16], float* gvn = nullptr, int* vids = nullptr) {
+                                                    float g2, float xf, int yi, float acc[16], float* gvn = nullptr, int* vids = nullptr,
+                                                    float* gcol = nullptr) {
   const int4 fi = __ldg(p.faces4 + f0 + fid);
   // ---- forward recompute from the projected vertices (exact IEEE projection, done once per view by
   // mesh_project_kernel: for small faces the barycentrics amplify a 1-ulp change of a vertex by |xy| / area);
@@ -58,8 +61,9 @@ __device__ __forceinline__ bool mesh_backward_pixel(const MeshBwdParams& p, int 
   const float3 P = interp(bb, X0, X1, X2);
   const float3 Nn = interp(bb, N0, N1, N2);
   float3 tex;
+  float sb = 0.f;
   if (VRGB) tex = interp(bb, c0, c1, c2);
-  else { const float sb = bb[0] + bb[1] + bb[2]; tex = make_float3(ucol.x * sb, ucol.y * sb, ucol.z * sb); }
+  else { sb = bb[0] + bb[1] + bb[2]; tex = make_float3(ucol.x * sb, ucol.y * sb, ucol.z * sb); }
   const float in = inv_norm_clamped(Nn.x, Nn.y, Nn.z, 1e-6f);
   const float nx = Nn.x * in, ny = Nn.y * in, nz = Nn.z * in;
   const float cosang = fmaf(nx, sc.lx, fmaf(ny, sc.ly, nz * sc.lz));
@@ -73,6 +77,15 @@ __device__ __forceinline__ bool mesh_backward_pixel(const MeshBwdParams& p, int 
   const float alpha = (dt > 0.f && lit) ? dt : 0.f;
   const float kd = fmaf(MVR_DIFFUSE, diff, MVR_AMBIENT);
   const float gtx = g0 * kd, gty = g1 * kd, gtz = g2 * kd;
+  if (GC) {      // the texel is linear in the colours: d colour = bb_i d texel (per vertex) / sum(bb) d texel (one colour)
+    if (VRGB) {
+#pragma unroll
+      for (int i = 0; i < 3; ++i) { gcol[3 * i] = bb[i] * gtx; gcol[3 * i + 1] = bb[i] * gty; gcol[3 * i + 2] = bb[i] * gtz; }
+      vids[0] = fi.x; vids[1] = fi.y; vids[2] = fi.z;
+    } else {
+      gcol[0] = fmaf(sb, gtx, gcol[0]); gcol[1] = fmaf(sb, gty, gcol[1]); gcol[2] = fmaf(sb, gtz, gcol[2]);
+    }
+  }
   const float gdiff = MVR_DIFFUSE * fmaf(g0, tex.x, fmaf(g1, tex.y, g2 * tex.z));
   const float gs = MVR_SPECULAR * (g0 + g1 + g2);
   const float a2 = alpha * alpha, a4 = a2 * a2, a8 = a4 * a4, a16 = a8 * a8, a32 = a16 * a16;
@@ -207,9 +220,47 @@ __device__ __forceinline__ void scatter_vertex_grads(const MeshBwdParams& p, int
   }
 }
 
+// scatter_vertex_grads for the 9 per-vertex colour gradients of a pixel (gcol of mesh_backward_pixel<true, GV, true>): lanes that
+// hold the same face sum first, one lane per face issues the atomics.  Must be called by all 32 lanes (fid < 0: nothing to add).
+__device__ __forceinline__ void scatter_rgb_grads(const MeshBwdParams& p, int voff, int fid, const float gcol[9], const int vids[3]) {
+  const unsigned int full = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const unsigned int grp = __match_any_sync(full, fid);
+  unsigned int peers = fid >= 0 ? grp : 0u;
+  const bool leader = fid >= 0 && (int)(__ffs(grp) - 1) == lane;
+  float sum[9];
+#pragma unroll
+  for (int i = 0; i < 9; ++i) sum[i] = 0.f;
+  while (__any_sync(full, peers != 0u)) {
+    const int src = peers ? __ffs(peers) - 1 : lane;
+#pragma unroll
+    for (int i = 0; i < 9; ++i) {
+      const float t = __shfl_sync(full, gcol[i], src);
+      if (peers) sum[i] += t;
+    }
+    peers &= peers - 1u;
+  }
+  if (leader) {
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      float* o = p.grad_rgb + 3 * (size_t)(voff + vids[i]);
+      atomicAdd(o + 0, sum[3 * i + 0]); atomicAdd(o + 1, sum[3 * i + 1]); atomicAdd(o + 2, sum[3 * i + 2]);
+    }
+  }
+}
+
+// GC && !VRGB: the warp's colour partial (d r, d g, d b, 0) next to its camera partial (fixed-order sum in the finish kernel).
+// Must be called by all 32 lanes.
+__device__ __forceinline__ void store_rgb_partial(const MeshBwdParams& p, size_t part, const float gcol[3]) {
+  const float r = warp_sum(gcol[0]), g = warp_sum(gcol[1]), b = warp_sum(gcol[2]);
+  if ((threadIdx.x & 31) == 0) *reinterpret_cast<float4*>(p.rgb_partials + 4 * part) = make_float4(r, g, b, 0.f);
+}
+
 // VRGB: per-vertex colours (object_color == "custom"); otherwise ONE object colour: the texel is c * sum(b) and its
 // cotangent one dot product -- six registers and ~13 floating-point instructions less per covered pixel.
-template <int MINB, bool VRGB, bool GV>
+// GC: colour gradients too (mesh_backward_pixel's gcol): per vertex through scatter_rgb_grads, one object colour through the
+// per-warp partials rgb_partials.
+template <int MINB, bool VRGB, bool GV, bool GC = false>
 __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel(const MeshBwdParams p) {
   pdl_enter();
   const int tid = threadIdx.x;
@@ -247,26 +298,31 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel(const 
   const float xf = xi < p.W ? __ldg(p.tab + xi) : 0.f;
   float4 ucol = make_float4(0.f, 0.f, 0.f, 0.f);
   if (!VRGB) ucol = make_float4(__ldg(p.obj_rgb), __ldg(p.obj_rgb + 1), __ldg(p.obj_rgb + 2), 0.f);
+  constexpr bool SCAT = GV || (GC && VRGB);      // a warp-aggregated scatter follows every pixel
+  float gcol[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};      // GC: per-vertex (VRGB) or the running sum (one colour)
 #pragma unroll 1
   for (int j = 0; j < BWD_PIX_PER_THREAD; ++j) {
     const int fid = fids[j];
     const float g0 = gin[j][0], g1 = gin[j][1], g2 = gin[j][2];
     const bool live = !(fid < 0 || (g0 == 0.f && g1 == 0.f && g2 == 0.f));
     const int yi = yi0 + 8 * j;
-    if (GV) {      // all lanes stay together for the warp-aggregated scatter
+    if (SCAT) {      // all lanes stay together for the warp-aggregated scatter
       float gvn[18];
       int vids[3] = {0, 0, 0};
       bool done = false;
-      if (live) { any = true; done = mesh_backward_pixel<VRGB, true>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, yi, acc, gvn, vids); }
-      scatter_vertex_grads(p, voff, done ? fid : -1, gvn, vids);
+      if (live) { any = true; done = mesh_backward_pixel<VRGB, GV, GC>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, yi, acc, gvn, vids, gcol); }
+      if (GV) scatter_vertex_grads(p, voff, done ? fid : -1, gvn, vids);
+      if (GC && VRGB) scatter_rgb_grads(p, voff, done ? fid : -1, gcol, vids);
       continue;
     }
     if (!live) continue;
     any = true;
-    mesh_backward_pixel<VRGB, false>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, yi, acc);
+    mesh_backward_pixel<VRGB, false, GC>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, yi, acc, nullptr, nullptr, gcol);
   }
   // one partial per WARP, no block barrier: a warp retires as soon as its own pixels are done
-  float* out = p.partials + ((size_t)n * p.parts_per_view + (size_t)cta * NWARPS + (tid >> 5)) * 16;
+  const size_t part = (size_t)n * p.parts_per_view + (size_t)cta * NWARPS + (tid >> 5);
+  if (GC && !VRGB) store_rgb_partial(p, part, gcol);
+  float* out = p.partials + part * 16;
   const int lane = tid & 31;
   if (!__any_sync(0xffffffffu, any)) {   // background-only warp
     if (lane < 16) out[lane] = 0.f;
@@ -290,7 +346,7 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-template <int MINB, bool VRGB, bool GV>
+template <int MINB, bool VRGB, bool GV, bool GC = false>
 __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel_strip(const MeshBwdParams p) {
   pdl_enter();
   // Every WARP stages its own pixels: the four 8x4-pixel blocks it owns in a 32x32 tile (128 pixels x 4 planes = 2 KB per
@@ -338,6 +394,8 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel_strip(
   const ShadeCtx sc = load_shade_ctx(p.light, p.light_stride, p.Cc, n);
   float4 ucol = make_float4(0.f, 0.f, 0.f, 0.f);
   if (!VRGB) ucol = make_float4(__ldg(p.obj_rgb), __ldg(p.obj_rgb + 1), __ldg(p.obj_rgb + 2), 0.f);
+  constexpr bool SCAT = GV || (GC && VRGB);      // as mesh_backward_kernel
+  float gcol[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   // Pixels -> lanes: a warp takes 8x4-pixel BLOCKS (lane = 8 r + c) instead of 32x1 rows.  A face covers ~2.5 x 2.5 pixels
   // at C2: a block touches ~5 faces where a row touches ~13, and every gather instruction of the warp (face record, 3 + 6
   // vertex records) splits into that many fewer L1 wavefronts.
@@ -361,32 +419,35 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel_strip(
 #pragma unroll 1
     for (int base = 0; base < cnt; base += 32) {
       const bool has = base + lane < cnt;
-      if (!GV && !has) continue;
+      if (!SCAT && !has) continue;
       const int o = has ? s_list[warp][base + lane] : 0;          // = 32 j + 8 r + c: the pixel's offset in the stage
       const int x = bx0 + (o & 7), y = by0 + ((o >> 5) << 3) + ((o >> 3) & 3);
       const int fid = s_fid[warp][buf][o];
       float g0 = s_g[warp][buf][0][o], g1 = s_g[warp][buf][1][o], g2 = s_g[warp][buf][2][o];
       const bool live = has && !(g0 == 0.f && g1 == 0.f && g2 == 0.f);
-      if (!GV && !live) continue;
+      if (!SCAT && !live) continue;
       if (p.onorm.on) { g0 *= p.onorm.s0; g1 *= p.onorm.s1; g2 *= p.onorm.s2; }
-      if (GV) {      // all lanes stay together for the warp-aggregated scatter
+      if (SCAT) {      // all lanes stay together for the warp-aggregated scatter
         float gvn[18];
         int vids[3] = {0, 0, 0};
         bool done = false;
         if (live) {
           any = true;
-          done = mesh_backward_pixel<VRGB, true>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, __ldg(p.tab + t * 32 + x), tyb * 32 + y, acc, gvn, vids);
+          done = mesh_backward_pixel<VRGB, GV, GC>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, __ldg(p.tab + t * 32 + x), tyb * 32 + y, acc, gvn, vids, gcol);
         }
-        scatter_vertex_grads(p, voff, done ? fid : -1, gvn, vids);
+        if (GV) scatter_vertex_grads(p, voff, done ? fid : -1, gvn, vids);
+        if (GC && VRGB) scatter_rgb_grads(p, voff, done ? fid : -1, gcol, vids);
         continue;
       }
       any = true;
       const float xf = __ldg(p.tab + t * 32 + x);      // covered => inside the image
-      mesh_backward_pixel<VRGB, false>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, tyb * 32 + y, acc);
+      mesh_backward_pixel<VRGB, false, GC>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, tyb * 32 + y, acc, nullptr, nullptr, gcol);
     }
     __syncwarp();                                      // the list and stage `buf` are free again (tile t + 2 overwrites it)
   }
-  float* out = p.partials + ((size_t)n * p.parts_per_view + (size_t)tyb * NWARPS + warp) * 16;
+  const size_t part = (size_t)n * p.parts_per_view + (size_t)tyb * NWARPS + warp;
+  if (GC && !VRGB) store_rgb_partial(p, part, gcol);
+  float* out = p.partials + part * 16;
   if (!__any_sync(0xffffffffu, any)) {
     if (lane < 16) out[lane] = 0.f;
     return;
@@ -407,7 +468,7 @@ static int mesh_backward_impl(const void* geometry, const int* vert_off, const i
                               const float* out_mean_std, const int* pix_to_face, const void* grad_images, float* gR, float* gT, float* gC,
                               float* grad_verts, float* grad_normals, void* workspace, size_t workspace_bytes,
                               void* stream, const float* azim, const float* elev, const float* dist, float* g_azim, float* g_elev,
-                              float* g_dist) {
+                              float* g_dist, float* grad_rgb) {
   int rc = check_mesh_common("mvr_mesh_backward", B, M, H, W, K, total_verts, total_faces, max_verts);
   if (rc) return rc;
   const int64_t N = (int64_t)B * M;
@@ -441,12 +502,28 @@ static int mesh_backward_impl(const void* geometry, const int* vert_off, const i
   p.onorm = make_out_norm(out_mean_std);
   p.z_clip = z_clip; p.wsflags = (int*)(wb + w.flags); p.parts_per_view = w.bwd_parts_per_view;
   p.azim = azim; p.elev = elev; p.dist = dist; p.g_azim = g_azim; p.g_elev = g_elev; p.g_dist = g_dist;
+  p.grad_rgb = grad_rgb; p.rgb_partials = (float*)(wb + w.rgb_partials); p.rgb_views = (double*)(wb + w.rgb_views);
   const dim3 bgrid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
   const bool vrgb = flags & MVR_RGB_PER_ELEMENT;
   const bool strip = K == 1 && !(flags & MVR_IMAGES_BF16) && W % 4 == 0 &&
                      ((uintptr_t)pix_to_face % 16 == 0) && ((uintptr_t)grad_images % 16 == 0);
   const bool gv = grad_verts || grad_normals;
-  if (strip) {
+  if (grad_rgb) {      // colour gradients: instances of their own (GC), so that the ones above stay as they are
+    if (strip) {
+      p.parts_per_view = ((H + 31) / 32) * NWARPS;
+      const dim3 sgrid((unsigned)((H + 31) / 32), (unsigned)M, (unsigned)B);
+      if (gv) {
+        if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel_strip<2, true, true, true>), sgrid, MVR_THREADS, 0, st, p);
+        else MVR_LAUNCH_PDL((mesh_backward_kernel_strip<2, false, true, true>), sgrid, MVR_THREADS, 0, st, p);
+      }
+      else if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel_strip<2, true, false, true>), sgrid, MVR_THREADS, 0, st, p);
+      else MVR_LAUNCH_PDL((mesh_backward_kernel_strip<3, false, false, true>), sgrid, MVR_THREADS, 0, st, p);
+    }
+    else if (gv) { if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel<2, true, true, true>), bgrid, MVR_THREADS, 0, st, p); else MVR_LAUNCH_PDL((mesh_backward_kernel<2, false, true, true>), bgrid, MVR_THREADS, 0, st, p); }
+    else if (vrgb) MVR_LAUNCH_PDL((mesh_backward_kernel<2, true, false, true>), bgrid, MVR_THREADS, 0, st, p);
+    else MVR_LAUNCH_PDL((mesh_backward_kernel<3, false, false, true>), bgrid, MVR_THREADS, 0, st, p);
+  }
+  else if (strip) {
     p.parts_per_view = ((H + 31) / 32) * NWARPS;      // one partial per warp of every tile ROW
     const dim3 sgrid((unsigned)((H + 31) / 32), (unsigned)M, (unsigned)B);
     if (gv) {      // vertex gradients: the variant with the warp-aggregated atomic scatter (its 18 extra live values cost occupancy)
@@ -461,7 +538,7 @@ static int mesh_backward_impl(const void* geometry, const int* vert_off, const i
   else MVR_LAUNCH_PDL((mesh_backward_kernel<3, false, false>), bgrid, MVR_THREADS, 0, st, p);
   rc = check_launch("mesh_backward_kernel");
   if (rc) return rc;
-  // clipped-face pixels (if any) + the fixed-order sum of the per-warp partials -> gR, gT, gC
+  // clipped-face pixels (if any) + the fixed-order sum of the per-warp partials -> gR, gT, gC (and the colour gradient)
   return launch_mesh_backward_finish(p, (int)N, gR, gT, gC, st);
 }
 
@@ -474,7 +551,21 @@ extern "C" int mvr_mesh_backward(const void* geometry, const int* vert_off, cons
                                  void* stream) {
   return mesh_backward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, R, T, Cc, light, light_stride, obj_rgb,
                             k00, k11, z_clip, H, W, K, flags, out_mean_std, pix_to_face, grad_images, gR, gT, gC, grad_verts, grad_normals,
-                            workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
+                            workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
+}
+
+// mvr_mesh_backward that also returns the colour gradient: grad_rgb (Vtot, 3), accumulated, for per-vertex colours
+// (MVR_RGB_PER_ELEMENT), else (3) for the one object colour, written (fixed-order sum, bit-reproducible).
+extern "C" int mvr_mesh_backward_rgb(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                                     int64_t total_verts, int64_t total_faces, int max_verts, const float* R,
+                                     const float* T, const float* Cc, const float* light, int light_stride,
+                                     const float* obj_rgb, float k00, float k11, float z_clip, int H, int W, int K, int flags,
+                                     const float* out_mean_std, const int* pix_to_face, const void* grad_images, float* gR, float* gT, float* gC,
+                                     float* grad_verts, float* grad_normals, void* workspace, size_t workspace_bytes,
+                                     void* stream, float* grad_rgb) {
+  return mesh_backward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, R, T, Cc, light, light_stride, obj_rgb,
+                            k00, k11, z_clip, H, W, K, flags, out_mean_std, pix_to_face, grad_images, gR, gT, gC, grad_verts, grad_normals,
+                            workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, grad_rgb);
 }
 
 // mvr_mesh_backward for cameras that came from mvr_look_at_forward(azim, elev, dist): the kernel that sums the per-warp partials of a
@@ -490,5 +581,5 @@ extern "C" int mvr_mesh_backward_angles(const void* geometry, const int* vert_of
   if (!azim) { set_error("mvr_mesh_backward_angles: null pointer"); return -5; }
   return mesh_backward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, R, T, Cc, light, light_stride, obj_rgb,
                             k00, k11, z_clip, H, W, K, flags, out_mean_std, pix_to_face, grad_images, gR, gT, gC, grad_verts, grad_normals,
-                            workspace, workspace_bytes, stream, azim, elev, dist, g_azim, g_elev, g_dist);
+                            workspace, workspace_bytes, stream, azim, elev, dist, g_azim, g_elev, g_dist, nullptr);
 }

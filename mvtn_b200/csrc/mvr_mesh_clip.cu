@@ -109,7 +109,9 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_shade_clipped_kernel(const M
 // Same derivation as oracle/mvr_oracle.c clip_face_bwd / raster_bwd_one / phong_pixel_bwd, in fp32.
 // ------------------------------------------------------------------------------------------------
 // The clipped-face pixels of view n (those mesh_backward_kernel skipped), accumulated by the whole CTA into acc (per thread).
-__device__ __forceinline__ void backward_clipped_view(const MeshBwdParams& p, int n, float (&acc)[16]) {
+// GC: colour gradients too -- per-vertex colours into p.grad_rgb (atomics), one object colour into gcol (per thread).
+template <bool GC>
+__device__ __forceinline__ void backward_clipped_view(const MeshBwdParams& p, int n, float (&acc)[16], float (&gcol)[3]) {
   const int tid = threadIdx.x;
   const int b = n / p.M, m = n - b * p.M;
   const int HW = p.H * p.W;
@@ -142,9 +144,20 @@ __device__ __forceinline__ void backward_clipped_view(const MeshBwdParams& p, in
     const float4 N0 = __ldg(p.normals4 + voff + fi.x), N1 = __ldg(p.normals4 + voff + fi.y), N2 = __ldg(p.normals4 + voff + fi.z);
     float4 c0 = ucol, c1 = ucol, c2 = ucol;
     if (per_vertex_rgb) { c0 = __ldg(p.rgb4 + voff + fi.x); c1 = __ldg(p.rgb4 + voff + fi.y); c2 = __ldg(p.rgb4 + voff + fi.z); }
-    float gb[3], gv[3], gN[3];
-    phong_backward(bb, X[0], X[1], X[2], N0, N1, N2, c0, c1, c2, sc, g0, g1, g2, gb, gv, gN);
+    float gb[3], gv[3], gN[3], gt[3];
+    phong_backward(bb, X[0], X[1], X[2], N0, N1, N2, c0, c1, c2, sc, g0, g1, g2, gb, gv, gN, GC ? gt : nullptr);
     acc[12] += gv[0]; acc[13] += gv[1]; acc[14] += gv[2];      // dC
+    if (GC) {      // texel = sum_i bb_i c_i
+      if (per_vertex_rgb) {
+        for (int i = 0; i < 3; ++i) {
+          float* o = p.grad_rgb + 3 * (size_t)(voff + (i == 0 ? fi.x : i == 1 ? fi.y : fi.z));
+          atomicAdd(o + 0, bb[i] * gt[0]); atomicAdd(o + 1, bb[i] * gt[1]); atomicAdd(o + 2, bb[i] * gt[2]);
+        }
+      } else {
+        const float sb = bb[0] + bb[1] + bb[2];
+        gcol[0] += sb * gt[0]; gcol[1] += sb * gt[1]; gcol[2] += sb * gt[2];
+      }
+    }
     float gbeta[3], gq[9], gfv[9];
     for (int k = 0; k < 3; ++k) gbeta[k] = cs.conv[s][k] * gb[0] + cs.conv[s][3 + k] * gb[1] + cs.conv[s][6 + k] * gb[2];
     raster_backward(cs.f[s], persp, xf, yf, gbeta, gq);
@@ -180,19 +193,25 @@ __device__ __forceinline__ void backward_clipped_view(const MeshBwdParams& p, in
 // straddling faces, which mesh_backward_kernel skipped, are redone with the clipped geometry; (2) fixed-order sum of the
 // per-warp partials of mesh_backward_kernel: thread t owns value t & 15 of the parts congruent to t >> 4 modulo 16
 // (coalesced 64-byte rows), then 16 threads add the 16 group sums (and the clipped part) in a fixed order.
+// GC (p.grad_rgb set): also the colour gradient -- the clipped pixels' share and, for one object colour, the view's total of
+// the colour partials in fp64 (rgb_views; mesh_rgb_grad_sum_kernel adds the views).
+template <bool GC>
 __global__ void __launch_bounds__(MVR_THREADS) mesh_backward_finish_kernel(const MeshBwdParams p, float* __restrict__ gR,
                                                                            float* __restrict__ gT, float* __restrict__ gC) {
   __shared__ double s_sum[MVR_THREADS];
   __shared__ float s_red[(MVR_THREADS / 32) * 16];
+  __shared__ float s_cred[GC ? (MVR_THREADS / 32) * 3 : 1];
   pdl_enter();
   const int n = blockIdx.x, tid = threadIdx.x;
   const bool clip = may_clip(p.wsflags);      // block-uniform
+  const bool one_rgb = GC && !(p.flags & MVR_RGB_PER_ELEMENT);
   if (clip) {
-    float acc[16];
+    float acc[16], gcol[3] = {0.f, 0.f, 0.f};
 #pragma unroll
     for (int i = 0; i < 16; ++i) acc[i] = 0.f;
-    backward_clipped_view(p, n, acc);
+    backward_clipped_view<GC>(p, n, acc, gcol);
     block_sum<16>(acc, s_red);                // s_red[0..15] = the clipped pixels' totals
+    if (one_rgb) block_sum<3>(gcol, s_cred);  // s_cred[0..2]: their colour gradient
   }
   // the per-warp partials (tens to hundreds per view, of mixed sign) are summed in fp64: free here, and it removes the
   // one accumulation level whose operands are large next to the result
@@ -211,6 +230,20 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_backward_finish_kernel(const
     else if (tid < 15) { if (gC) gC[3 * (size_t)n + tid - 12] = out; }
     s_red[tid] = out;
   }
+  if (one_rgb) {      // block-uniform: the view's colour partials, value tid & 3 of the parts congruent to tid >> 2 modulo 64
+    __syncthreads();
+    const int c = tid & 3, cg = tid >> 2;
+    double t = 0.0;
+    if (c < 3)
+      for (int q = cg; q < p.parts_per_view; q += MVR_THREADS / 4) t += (double)p.rgb_partials[((size_t)n * p.parts_per_view + q) * 4 + c];
+    s_sum[tid] = t;
+    __syncthreads();
+    if (tid < 3) {
+      double tot = clip ? (double)s_cred[tid] : 0.0;
+      for (int g = 0; g < MVR_THREADS / 4; ++g) tot += s_sum[g * 4 + tid];
+      p.rgb_views[3 * (size_t)n + tid] = tot;
+    }
+  }
   if (p.azim) {      // mvr_mesh_backward_angles: (dR, dT, dC) -> (d azim, d elev, d dist) of this view, same launch (block-uniform)
     __syncthreads();
     if (tid == 0) {
@@ -218,6 +251,24 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_backward_finish_kernel(const
       look_at_backward_view(__ldg(p.azim + n), __ldg(p.elev + n), __ldg(p.dist + n), s_red, s_red + 9, s_red + 12, ga, ge, gd);
       p.g_azim[n] = ga; p.g_elev[n] = ge; p.g_dist[n] = gd;
     }
+  }
+}
+
+// One object colour: grad_rgb[c] = the sum of the N per-view fp64 totals in a fixed order (thread t: views congruent to t >> 2
+// modulo 64, then thread c adds the 64 group sums in order) -- bit-reproducible, as the camera gradients are.
+__global__ void __launch_bounds__(MVR_THREADS) mesh_rgb_grad_sum_kernel(const double* __restrict__ views, int N, float* __restrict__ grad_rgb) {
+  __shared__ double s_sum[MVR_THREADS];
+  pdl_enter();
+  const int tid = threadIdx.x, c = tid & 3, g = tid >> 2;
+  double t = 0.0;
+  if (c < 3)
+    for (int n = g; n < N; n += MVR_THREADS / 4) t += views[3 * (size_t)n + c];
+  s_sum[tid] = t;
+  __syncthreads();
+  if (tid < 3) {
+    double tot = 0.0;
+    for (int q = 0; q < MVR_THREADS / 4; ++q) tot += s_sum[q * 4 + tid];
+    grad_rgb[tid] = (float)tot;
   }
 }
 
@@ -232,6 +283,13 @@ int launch_mesh_shade_clipped(const MeshParams& p, int N, bool soft, cudaStream_
 }
 
 int launch_mesh_backward_finish(const MeshBwdParams& p, int N, float* gR, float* gT, float* gC, cudaStream_t st) {
-  MVR_LAUNCH_PDL(mesh_backward_finish_kernel, (unsigned)N, MVR_THREADS, 0, st, p, gR, gT, gC);
-  return check_launch("mesh_backward_finish_kernel");
+  if (!p.grad_rgb) {
+    MVR_LAUNCH_PDL(mesh_backward_finish_kernel<false>, (unsigned)N, MVR_THREADS, 0, st, p, gR, gT, gC);
+    return check_launch("mesh_backward_finish_kernel");
+  }
+  MVR_LAUNCH_PDL(mesh_backward_finish_kernel<true>, (unsigned)N, MVR_THREADS, 0, st, p, gR, gT, gC);
+  int rc = check_launch("mesh_backward_finish_kernel");
+  if (rc || (p.flags & MVR_RGB_PER_ELEMENT)) return rc;
+  MVR_LAUNCH_PDL(mesh_rgb_grad_sum_kernel, 1u, MVR_THREADS, 0, st, p.rgb_views, N, p.grad_rgb);
+  return check_launch("mesh_rgb_grad_sum_kernel");
 }

@@ -26,6 +26,9 @@ struct SoftParams {
   float* rgba;             // forward out: (n, 4, H, W)
   const float* grad_rgba;  // backward in
   float* grad_verts; float* grad_normals;      // backward out (GV): (Vtot,3) accumulated, either may be NULL
+  // backward out (GC): per-vertex colours -> grad_rgb (Vtot,3) accumulated; one object colour -> per-warp partials rgb_partials
+  // (4 floats each, summed in fixed order by mesh_backward_finish_kernel<true>)
+  float* grad_rgb; float* rgb_partials;
 };
 
 constexpr float SOFT_EPS = 1e-10f;
@@ -133,11 +136,13 @@ __device__ __forceinline__ int rank_in_list(const int* list, int k, int fid) {
 
 // One fragment of view n: push (g_colour, g_zbuf, g_sdist) back to the camera accumulators acc[15]; GV: also to the vertices
 // of the original face (sp.grad_verts: projection chain + Phong's interpolated position; sp.grad_normals: Phong's normal term).
-template <bool GV>
+// GC: also to the colours -- d texel = kd g_colour, then bb_i per vertex (sp.grad_rgb, atomics) or sum(bb) for one object
+// colour (rgbacc, the thread's running sum).
+template <bool GV, bool GC = false>
 __device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, const SoftParams& sp, int n, int voff, const int4 fi, const Face& fc,
                                                        const SoftFrag& fr, const ClipSub& cs, bool persp, bool clipb, float xf, float yf,
                                                        const ShadeCtx& sc, const float gcol[3], float gz, float gsd, bool with_colour,
-                                                       float acc[16]) {
+                                                       float acc[16], float* rgbacc = nullptr) {
   const Face& g = fr.g;
   float4 X0, X1, X2, N0, N1, N2;
   gather_xn(p.xn8, voff + fi.x, X0, N0); gather_xn(p.xn8, voff + fi.y, X1, N1); gather_xn(p.xn8, voff + fi.z, X2, N2);
@@ -148,9 +153,20 @@ __device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, cons
     float4 c0, c1, c2;
     if (p.flags & MVR_RGB_PER_ELEMENT) { c0 = __ldg(p.rgb4 + voff + fi.x); c1 = __ldg(p.rgb4 + voff + fi.y); c2 = __ldg(p.rgb4 + voff + fi.z); }
     else { c0 = c1 = c2 = make_float4(__ldg(p.obj_rgb), __ldg(p.obj_rgb + 1), __ldg(p.obj_rgb + 2), 0.f); }
-    float gv[3], gN[3];
-    phong_backward(fr.bb, X0, X1, X2, N0, N1, N2, c0, c1, c2, sc, gcol[0], gcol[1], gcol[2], gbb, gv, gN);
+    float gv[3], gN[3], gt[3];
+    phong_backward(fr.bb, X0, X1, X2, N0, N1, N2, c0, c1, c2, sc, gcol[0], gcol[1], gcol[2], gbb, gv, gN, GC ? gt : nullptr);
     acc[12] += gv[0]; acc[13] += gv[1]; acc[14] += gv[2];      // dC
+    if (GC) {
+      if (p.flags & MVR_RGB_PER_ELEMENT) {
+        for (int i = 0; i < 3; ++i) {
+          float* o = sp.grad_rgb + 3 * (size_t)(voff + vid[i]);
+          atomicAdd(o + 0, fr.bb[i] * gt[0]); atomicAdd(o + 1, fr.bb[i] * gt[1]); atomicAdd(o + 2, fr.bb[i] * gt[2]);
+        }
+      } else {
+        const float sb = fr.bb[0] + fr.bb[1] + fr.bb[2];
+        rgbacc[0] += sb * gt[0]; rgbacc[1] += sb * gt[1]; rgbacc[2] += sb * gt[2];
+      }
+    }
     if (GV) {
       gP[0] = -gv[0]; gP[1] = -gv[1]; gP[2] = -gv[2];
       if (sp.grad_normals)      // Nn = sum_i bb_i N_i
@@ -225,8 +241,8 @@ __device__ __forceinline__ void soft_fragment_backward(const MeshParams& p, cons
 
 // grid: x = 32x32-pixel tiles, y = view m, z = object b; thread (lane, warp) owns pixels (x0 + lane, y0 + warp + 8 j); one
 // 16-float partial per warp at partials[(n * parts_per_view + tile * NWARPS + warp) * 16] (mesh_backward_finish_kernel sums them)
-// GV: vertex gradients too (soft_fragment_backward<true>)
-template <bool GV>
+// GV: vertex gradients too (soft_fragment_backward<true>); GC: colour gradients too
+template <bool GV, bool GC = false>
 __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const MeshParams p, const SoftParams sp, float* __restrict__ partials,
                                                                          int parts_per_view, int tiles_x) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -241,7 +257,7 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
   const bool clip_on = may_clip(p.wsflags);      // some vertex lies behind the near plane: faces may straddle it
   const ShadeCtx sc = load_shade_ctx(p.light, p.light_stride, p.Cc, n);
   const float zscale = 1.0f / (sp.zfar - sp.znear);
-  float acc[16];
+  float acc[16], rgbacc[3] = {0.f, 0.f, 0.f};
 #pragma unroll
   for (int i = 0; i < 16; ++i) acc[i] = 0.f;
   for (int j = 0; j < 4; ++j) {
@@ -309,7 +325,7 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
         if (pass == 1) {      // z_inv_max = z_inv of this fragment
           if (zmax_live && gzmax != 0.f) {
             const float gcz[3] = {0.f, 0.f, 0.f};
-            soft_fragment_backward<GV>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, -gzmax * zscale, 0.f, false, acc);
+            soft_fragment_backward<GV, GC>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, -gzmax * zscale, 0.f, false, acc, rgbacc);
           }
           continue;
         }
@@ -337,11 +353,16 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
           gzmax -= gzi;
         }
         const float gsd = gprob * (-1.0f / sp.sigma) * prob * (1.0f - prob);
-        soft_fragment_backward<GV>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc);
+        soft_fragment_backward<GV, GC>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc, rgbacc);
       }
     }
   }
-  float* out = partials + ((size_t)n * parts_per_view + (size_t)cta * NWARPS + warp) * 16;
+  const size_t part = (size_t)n * parts_per_view + (size_t)cta * NWARPS + warp;
+  if (GC && !(p.flags & MVR_RGB_PER_ELEMENT)) {      // block-uniform
+    const float r = warp_sum(rgbacc[0]), g = warp_sum(rgbacc[1]), b = warp_sum(rgbacc[2]);
+    if (lane == 0) *reinterpret_cast<float4*>(sp.rgb_partials + 4 * part) = make_float4(r, g, b, 0.f);
+  }
+  float* out = partials + part * 16;
   const float mine = warp_sum16_transposed(acc);
   if (!(lane & 1)) out[lane >> 1] = mine;
 }
@@ -380,19 +401,19 @@ extern "C" int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert
   if (mode < 0 || mode > 1 || !(sigma > 0.f) || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_blend_forward: bad mode / sigma / gamma / z range"); return -7; }
   MeshParams p;
   fill_params(p, geometry, vert_off, face_off, B, M, total_verts, total_faces, nullptr, nullptr, Cc, light, light_stride, obj_rgb, bg_rgb, 0.f, 0.f, H, W, K, flags, pix_to_face);
-  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, zbuf, bary, dists, rgba, nullptr, nullptr, nullptr};
+  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, zbuf, bary, dists, rgba, nullptr, nullptr, nullptr, nullptr, nullptr};
   const dim3 grid((unsigned)(((size_t)H * W + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
   MVR_LAUNCH(mesh_soft_blend_kernel, grid, MVR_THREADS, 0, (cudaStream_t)stream, p, sp);
   return check_launch("mesh_soft_blend_kernel");
 }
 
-extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M, int64_t total_verts,
-                                      int64_t total_faces, int max_verts, const float* R, const float* T, const float* Cc, const float* light,
-                                      int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, float z_clip,
-                                      float blur_radius, int H, int W, int K, int flags, int mode, float sigma, float gamma, float znear,
-                                      float zfar, const int* pix_to_face,
-                                      const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
-                                      void* workspace, size_t workspace_bytes, void* stream) {
+static int mesh_soft_backward_impl(const void* geometry, const int* vert_off, const int* face_off, int B, int M, int64_t total_verts,
+                                   int64_t total_faces, int max_verts, const float* R, const float* T, const float* Cc, const float* light,
+                                   int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, float z_clip,
+                                   float blur_radius, int H, int W, int K, int flags, int mode, float sigma, float gamma, float znear,
+                                   float zfar, const int* pix_to_face,
+                                   const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
+                                   void* workspace, size_t workspace_bytes, void* stream, float* grad_rgb) {
   int rc = check_mesh_common("mvr_mesh_soft_backward", B, M, H, W, K, total_verts, total_faces, max_verts);
   if (rc) return rc;
   const int64_t N = (int64_t)B * M;
@@ -415,10 +436,17 @@ extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off,
   p.pv = (float4*)(wb + w.pv); p.tab = (float*)(wb + w.tab); p.wsflags = (int*)(wb + w.flags);
   p.z_clip = z_clip;
   p.blur_radius = blur_radius > 0.f ? blur_radius : 0.f; p.blur_r = sqrtf(p.blur_radius);      // as mvr_mesh_forward
-  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, nullptr, nullptr, nullptr, nullptr, grad_rgba, grad_verts, grad_normals};
+  SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, nullptr, nullptr, nullptr, nullptr, grad_rgba, grad_verts, grad_normals,
+                   grad_rgb, (float*)(wb + w.rgb_partials)};
   const int tiles_x = (W + 31) / 32;
   const dim3 grid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
-  if (grad_verts || grad_normals)
+  if (grad_rgb) {      // colour gradients: instances of their own, the two below stay as they are
+    if (grad_verts || grad_normals)
+      MVR_LAUNCH((mesh_soft_backward_kernel<true, true>), grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
+    else
+      MVR_LAUNCH((mesh_soft_backward_kernel<false, true>), grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
+  }
+  else if (grad_verts || grad_normals)
     MVR_LAUNCH((mesh_soft_backward_kernel<true>), grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
   else
     MVR_LAUNCH((mesh_soft_backward_kernel<false>), grid, MVR_THREADS, 0, st, p, sp, (float*)(wb + w.partials), w.bwd_parts_per_view, tiles_x);
@@ -430,5 +458,34 @@ extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off,
   // armed flag block that the projection never clears (word WSF_CLIP may be cleared above)
   q.partials = (float*)(wb + w.partials); q.parts_per_view = w.bwd_parts_per_view; q.wsflags = (int*)(wb + w.flags) + WSF_CLIP + 1;
   q.B = B; q.M = M; q.H = H; q.W = W; q.K = K; q.flags = flags; q.z_clip = -1.f; q.grad_verts = nullptr; q.grad_normals = nullptr;
+  // per-vertex colours are complete after the kernel; one object colour is summed from its partials by the finish kernel
+  q.grad_rgb = (flags & MVR_RGB_PER_ELEMENT) ? nullptr : grad_rgb;
+  q.rgb_partials = (float*)(wb + w.rgb_partials); q.rgb_views = (double*)(wb + w.rgb_views);
   return launch_mesh_backward_finish(q, (int)N, gR, gT, gC, st);
+}
+
+extern "C" int mvr_mesh_soft_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M, int64_t total_verts,
+                                      int64_t total_faces, int max_verts, const float* R, const float* T, const float* Cc, const float* light,
+                                      int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, float z_clip,
+                                      float blur_radius, int H, int W, int K, int flags, int mode, float sigma, float gamma, float znear,
+                                      float zfar, const int* pix_to_face,
+                                      const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
+  return mesh_soft_backward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, R, T, Cc, light, light_stride,
+                                 obj_rgb, bg_rgb, k00, k11, z_clip, blur_radius, H, W, K, flags, mode, sigma, gamma, znear, zfar,
+                                 pix_to_face, grad_rgba, gR, gT, gC, grad_verts, grad_normals, workspace, workspace_bytes, stream, nullptr);
+}
+
+// mvr_mesh_soft_backward that also returns the colour gradient (semantics of grad_rgb as mvr_mesh_backward_rgb); the silhouette
+// does not depend on the colours: zero.
+extern "C" int mvr_mesh_soft_backward_rgb(const void* geometry, const int* vert_off, const int* face_off, int B, int M, int64_t total_verts,
+                                          int64_t total_faces, int max_verts, const float* R, const float* T, const float* Cc, const float* light,
+                                          int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11, float z_clip,
+                                          float blur_radius, int H, int W, int K, int flags, int mode, float sigma, float gamma, float znear,
+                                          float zfar, const int* pix_to_face,
+                                          const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
+                                          void* workspace, size_t workspace_bytes, void* stream, float* grad_rgb) {
+  return mesh_soft_backward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, R, T, Cc, light, light_stride,
+                                 obj_rgb, bg_rgb, k00, k11, z_clip, blur_radius, H, W, K, flags, mode, sigma, gamma, znear, zfar,
+                                 pix_to_face, grad_rgba, gR, gT, gC, grad_verts, grad_normals, workspace, workspace_bytes, stream, grad_rgb);
 }

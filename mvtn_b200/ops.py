@@ -774,10 +774,19 @@ def _normals_backward_launch(geom: "PackedMeshes", gN, gV):
                                                    _stream(dev)), "mvr_mesh_normals_backward")
 
 
-def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_verts, angles=None):
+def _rgb_grad_buffer(geom: "PackedMeshes", dev):
+    """The colour gradient the _rgb entry points fill: (Vtot,3) zero-filled (accumulated) for per-vertex colours, else (3)
+    (written)."""
+    if geom.per_vertex_rgb:
+        return torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
+    return torch.empty(3, dtype=torch.float32, device=dev)
+
+
+def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_verts, angles=None, want_rgb=False):
     """ONE mvr_mesh_backward call -> (gR, gT, gC, gV | None) (gV includes the chain through the vertex normals).  angles =
     (azim, elev, dist) flat fp32: mvr_mesh_backward_angles instead, whose last kernel also applies the camera backward ->
-    (g_azim, g_elev, g_dist, gV | None)."""
+    (g_azim, g_elev, g_dist, gV | None).  want_rgb (not with angles): mvr_mesh_backward_rgb, and the colour gradient
+    ((Vtot,3) per-vertex colours, else (3)) is appended to the tuple."""
     lib = L.load()
     R, T, Cc, light, obj_rgb, p2f = saved
     k00, k11, H, W, K, flags, out_norm, light_stride, z_clip, ws_token = cfg
@@ -794,10 +803,20 @@ def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_ve
     if want_verts:
         gV = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
         gN = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
+    gRGB = _rgb_grad_buffer(geom, dev) if want_rgb else None
     ws_bytes = lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, K, geom.total_verts, geom.total_faces)
     ws = workspace(dev, ws_bytes, _mesh_owner=True)
     flags = flags | _ws_mesh_flags_backward(dev, ws, ws_token)
-    if angles is not None:
+    if want_rgb:
+        if angles is not None:
+            raise ValueError("the colour gradient is not fused with the angle backward")
+        with _on(dev):
+            L.check(lib.mvr_mesh_backward_rgb(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                              geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc), _ptr(light),
+                                              light_stride, _ptr(obj_rgb), k00, k11, z_clip, H, W, K, flags, out_norm, _ptr(p2f),
+                                              _ptr(g_images), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(gV), _ptr(gN), _ptr(ws),
+                                              ws.numel(), _stream(dev), _ptr(gRGB)), "mvr_mesh_backward_rgb")
+    elif angles is not None:
         az, el, di = angles
         with _on(dev):
             L.check(lib.mvr_mesh_backward_angles(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
@@ -817,18 +836,33 @@ def _mesh_backward_launch(geom: "PackedMeshes", M, cfg, saved, g_images, want_ve
         _normals_backward_launch(geom, gN, gV)
     if angles is not None:
         return ga, ge, gd, gV
+    if want_rgb:
+        return gR, gT, gC, gV, gRGB
     return gR, gT, gC, gV
+
+
+def _rgb_grads_wanted(ctx, geom, obj_idx, rgb_idx):
+    """(obj_rgb gets a gradient, the per-vertex colours get one) from needs_input_grad: obj_rgb only counts without
+    per-vertex colours (the kernels ignore it then), `rgb` only with them."""
+    return (ctx.needs_input_grad[obj_idx] and not geom.per_vertex_rgb), (ctx.needs_input_grad[rgb_idx] and geom.per_vertex_rgb)
+
+
+def _split_rgb_grad(g, want_obj, want_vert, obj_shape):
+    """The colour gradient of a backward launch -> (gradient of obj_rgb, gradient of the per-vertex colours)."""
+    return (g.reshape(obj_shape) if want_obj else None), (g if want_vert else None)
 
 
 class _MeshRender(torch.autograd.Function):
     @staticmethod
     def forward(ctx, R, T, Cc, verts, geom: PackedMeshes, M, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags,
-                want_fragments, out_norm=None, out_dtype=None):
-        # `verts` (packed (Vtot,3), same values as geom.verts) only carries autograd history for vertex gradients
+                want_fragments, out_norm=None, out_dtype=None, rgb=None):
+        # `verts` / `rgb` (packed (Vtot,3), same values as geom's vertices / per-vertex colours) only carry autograd history for
+        # vertex / colour gradients
         cfg, saved, images, extras = _mesh_forward_launch(geom, M, R, T, Cc, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K,
                                                           flags, want_fragments, out_norm, out_dtype)
         ctx.set_materialize_grads(False)      # no zero-filled "gradients" for pix_to_face & co (77 MB at C2)
         ctx.geom, ctx.M, ctx.cfg = geom, M, cfg
+        ctx.obj_shape = None if obj_rgb is None else obj_rgb.shape
         ctx.save_for_backward(*saved)
         ctx.mark_non_differentiable(*extras)
         return (images, *extras)
@@ -836,9 +870,12 @@ class _MeshRender(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_images, *_unused):
         if g_images is None:
-            return (None,) * 19
-        gR, gT, gC, gV = _mesh_backward_launch(ctx.geom, ctx.M, ctx.cfg, ctx.saved_tensors, g_images, ctx.needs_input_grad[3])
-        return (gR, gT, gC, gV) + (None,) * 15
+            return (None,) * 20
+        want_obj, want_vert = _rgb_grads_wanted(ctx, ctx.geom, 7, 19)
+        out = _mesh_backward_launch(ctx.geom, ctx.M, ctx.cfg, ctx.saved_tensors, g_images, ctx.needs_input_grad[3],
+                                    want_rgb=want_obj or want_vert)
+        g_obj, g_rgb = _split_rgb_grad(out[4], want_obj, want_vert, ctx.obj_shape) if len(out) == 5 else (None, None)
+        return out[:4] + (None,) * 3 + (g_obj,) + (None,) * 11 + (g_rgb,)
 
 
 class _MeshRenderFromAngles(torch.autograd.Function):
@@ -864,6 +901,7 @@ class _MeshRenderFromAngles(torch.autograd.Function):
         ctx.set_materialize_grads(False)
         ctx.geom, ctx.M, ctx.cfg = geom, M, cfg
         ctx.shapes = (azim.shape, elev.shape, dist.shape)
+        ctx.obj_shape = None if obj_rgb is None else obj_rgb.shape
         ctx.save_for_backward(a, e, d, *saved)
         ctx.mark_non_differentiable(bad, *extras)
         return (images, R, T, Cc, bad, *extras)
@@ -873,15 +911,20 @@ class _MeshRenderFromAngles(torch.autograd.Function):
         if g_images is None and gR_ext is None and gT_ext is None and gC_ext is None:
             return (None,) * 18
         a, e, d = ctx.saved_tensors[:3]
-        if g_images is not None and gR_ext is None and gT_ext is None and gC_ext is None:
+        want_obj = ctx.needs_input_grad[6] and not ctx.geom.per_vertex_rgb
+        if g_images is not None and gR_ext is None and gT_ext is None and gC_ext is None and not want_obj:
             # nothing arrives through the cameras object (the usual case): rasterizer backward, reduction and camera backward in
             # ONE call ending in (d azim, d elev, d dist) -- mvr_mesh_backward_angles
             ga, ge, gd, _ = _mesh_backward_launch(ctx.geom, ctx.M, ctx.cfg, ctx.saved_tensors[3:], g_images, False, (a, e, d))
             sa, se, sd = ctx.shapes
             return (ga.reshape(sa), ge.reshape(se), gd.reshape(sd)) + (None,) * 15
-        gR = gT = gC = None
+        gR = gT = gC = g_obj = None
         if g_images is not None:
-            gR, gT, gC, _ = _mesh_backward_launch(ctx.geom, ctx.M, ctx.cfg, ctx.saved_tensors[3:], g_images, False)
+            # (an object colour that requires grad takes this two-call route too: the colour gradient is not fused with the angles)
+            out = _mesh_backward_launch(ctx.geom, ctx.M, ctx.cfg, ctx.saved_tensors[3:], g_images, False, want_rgb=want_obj)
+            gR, gT, gC = out[:3]
+            if want_obj:
+                g_obj = out[4].reshape(ctx.obj_shape)
         # R, T, C are outputs too (the cameras object): gradients a caller sends through them join the renderer's
         if gR_ext is not None:
             gR = gR_ext if gR is None else gR + gR_ext
@@ -891,7 +934,7 @@ class _MeshRenderFromAngles(torch.autograd.Function):
             gC = gC_ext if gC is None else gC + gC_ext
         ga, ge, gd = _look_at_backward_launch(a, e, d, gR, gT, gC)
         sa, se, sd = ctx.shapes
-        return (ga.reshape(sa), ge.reshape(se), gd.reshape(sd)) + (None,) * 15
+        return (ga.reshape(sa), ge.reshape(se), gd.reshape(sd)) + (None,) * 3 + (g_obj,) + (None,) * 11
 
 
 SOFT_SHADERS = {"soft_phong": 0, "soft_silhouette": 1}
@@ -904,8 +947,9 @@ class _MeshRenderSoft(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, R, T, Cc, verts, geom: PackedMeshes, M, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags, blur_radius,
-                mode, sigma, gamma, znear, zfar):
-        # `verts` (packed (Vtot,3), same values as geom.verts) only carries autograd history for vertex gradients
+                mode, sigma, gamma, znear, zfar, rgb=None):
+        # `verts` / `rgb` (packed (Vtot,3), same values as geom's vertices / per-vertex colours) only carry autograd history for
+        # vertex / colour gradients
         lib = L.load()
         cfg, saved, _hard, extras = _mesh_forward_launch(geom, M, R, T, Cc, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags,
                                                          True, None, None, blur_radius=blur_radius)
@@ -925,6 +969,7 @@ class _MeshRenderSoft(torch.autograd.Function):
                     "mvr_mesh_soft_blend_forward")
         ctx.set_materialize_grads(False)
         ctx.geom, ctx.M = geom, M
+        ctx.obj_shape = None if obj_rgb is None else obj_rgb.shape
         ctx.cfg = (k00, k11, z_clip, blur_radius, H, W, K, fl, light_stride, mode, sigma, gamma, znear, zfar)
         ctx.save_for_backward(Rs, Ts, Cs, lt, col, bg, p2f)
         ctx.mark_non_differentiable(p2f, counters, zbuf, bary, dists)
@@ -933,7 +978,7 @@ class _MeshRenderSoft(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_rgba, *_unused):
         if g_rgba is None:
-            return (None,) * 22
+            return (None,) * 23
         lib = L.load()
         geom, M = ctx.geom, ctx.M
         R, T, Cc, light, col, bg, p2f = ctx.saved_tensors
@@ -948,17 +993,23 @@ class _MeshRenderSoft(torch.autograd.Function):
             gV = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
             if mode == SOFT_SHADERS["soft_phong"]:      # the silhouette does not depend on the normals
                 gN = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev)
+        # the silhouette does not depend on the colours: no colour gradient (None)
+        want_obj, want_vert = _rgb_grads_wanted(ctx, geom, 7, 22) if mode == SOFT_SHADERS["soft_phong"] else (False, False)
+        gRGB = _rgb_grad_buffer(geom, dev) if want_obj or want_vert else None
         ws = workspace(dev, lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, K, geom.total_verts, geom.total_faces))
+        args = (_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M, geom.total_verts, geom.total_faces,
+                geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc), _ptr(light), light_stride, _ptr(col), _ptr(bg), k00, k11, z_clip,
+                blur_radius, H, W, K, fl, mode, sigma, gamma, znear, zfar, _ptr(p2f), _ptr(g_rgba), _ptr(gR), _ptr(gT), _ptr(gC),
+                _ptr(gV), _ptr(gN), _ptr(ws), ws.numel(), _stream(dev))
         with _on(dev):
-            L.check(lib.mvr_mesh_soft_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
-                                               geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), _ptr(Cc),
-                                               _ptr(light), light_stride, _ptr(col), _ptr(bg), k00, k11, z_clip, blur_radius, H, W, K,
-                                               fl, mode, sigma,
-                                               gamma, znear, zfar, _ptr(p2f), _ptr(g_rgba), _ptr(gR), _ptr(gT), _ptr(gC), _ptr(gV),
-                                               _ptr(gN), _ptr(ws), ws.numel(), _stream(dev)), "mvr_mesh_soft_backward")
+            if gRGB is None:
+                L.check(lib.mvr_mesh_soft_backward(*args), "mvr_mesh_soft_backward")
+            else:
+                L.check(lib.mvr_mesh_soft_backward_rgb(*args, _ptr(gRGB)), "mvr_mesh_soft_backward_rgb")
         if gN is not None:
             _normals_backward_launch(geom, gN, gV)
-        return (gR, gT, gC, gV) + (None,) * 18
+        g_obj, g_rgb = _split_rgb_grad(gRGB, want_obj, want_vert, ctx.obj_shape) if gRGB is not None else (None, None)
+        return (gR, gT, gC, gV) + (None,) * 3 + (g_obj,) + (None,) * 14 + (g_rgb,)
 
 
 def render_meshes_from_angles(geom: PackedMeshes, M: int, azim, elev, dist, light, obj_rgb, bg_rgb, image_size,
@@ -980,7 +1031,8 @@ def render_meshes_from_angles(geom: PackedMeshes, M: int, azim, elev, dist, ligh
 def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, image_size: int, faces_per_pixel=1,
                   cull_backfaces=False, perspective_correct=True, fov=60.0, znear=1.0, z_clip: Optional[float] = None,
                   fragments=False, verts: Optional[torch.Tensor] = None, _extra_flags=0, normalize=None, out_dtype=None,
-                  shader="hard_phong", blur_radius=0.0, clip_barycentric_coords=None, sigma=1e-4, gamma=1e-4, zfar=100.0):
+                  shader="hard_phong", blur_radius=0.0, clip_barycentric_coords=None, sigma=1e-4, gamma=1e-4, zfar=100.0,
+                  rgb: Optional[torch.Tensor] = None):
     """images (B*M,3,H,W) [+ dict of fragments].  HardPhong + hard blend, blur_radius 0 (MVTN's configuration), or --
     shader="soft_phong" / "soft_silhouette" (SURVEY 8f N3) -- RGBA (B*M,4,H,W) from the K = faces_per_pixel fragments of the
     BLURRED rasterizer ([upstream] blur_radius in squared NDC units, clip_barycentric_coords default True iff blur_radius > 0)
@@ -988,6 +1040,9 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
     differentiable w.r.t. R, T, C (and `verts`) through colours, depths and the signed edge distances (grad_dists).
     `verts`: pass the packed (Vtot,3) vertex tensor the geometry was built from to get gradients w.r.t. it (any shader; the
     vertex gradients are accumulated with float atomics: tolerance-level, not bit-reproducible run to run).
+    Colour gradients: `rgb` -- pass the packed (Vtot,3) per-vertex colour tensor the geometry was built from (vert_rgb) to get
+    gradients w.r.t. it (float atomics, as the vertices); an `obj_rgb` that requires grad gets its gradient when the geometry
+    has no per-vertex colours (a fixed-order sum: bit-reproducible).  Hard and soft Phong; the silhouette gives none.
     `normalize=(mean, std)` / `out_dtype=torch.bfloat16`: consumer-side fusion (SURVEY 8f N2) -- the kernel writes
     (x - mean) / std (Trainer_mvt.py:41-49) in the dtype the CNN consumes; gradients flow through both."""
     H_, W_ = _hw(image_size)
@@ -1005,12 +1060,13 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
             raise ValueError("the soft shaders return fp32 RGBA: normalize / out_dtype are not supported with them")
         flags |= L.CLIP_BARYCENTRIC if clip_barycentric_coords else 0
         out = _MeshRenderSoft.apply(R, T, Cc, verts, geom, M, light, obj_rgb, bg_rgb, k00, k11, float(z_clip), H, W, int(faces_per_pixel),
-                                    flags, float(blur_radius), SOFT_SHADERS[shader], float(sigma), float(gamma), float(znear), float(zfar))
+                                    flags, float(blur_radius), SOFT_SHADERS[shader], float(sigma), float(gamma), float(znear), float(zfar),
+                                    rgb)
         return out[0], {"pix_to_face": out[1], "counters": out[2], "zbuf": out[3], "bary_coords": out[4], "dists": out[5]}
     if blur_radius > 0 or clip_barycentric_coords:
         raise ValueError("blur_radius > 0 / clipped barycentrics need shader='soft_phong' or 'soft_silhouette'")
     out = _MeshRender.apply(R, T, Cc, verts, geom, M, light, obj_rgb, bg_rgb, k00, k11, float(z_clip), H, W,
-                            int(faces_per_pixel), flags, bool(fragments), _out_norm(normalize), out_dtype)
+                            int(faces_per_pixel), flags, bool(fragments), _out_norm(normalize), out_dtype, rgb)
     images, p2f, counters = out[0], out[1], out[2]
     frag = {"pix_to_face": p2f, "counters": counters}
     if fragments:

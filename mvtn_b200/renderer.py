@@ -60,6 +60,22 @@ def _device_vec(values, device):
     return hit
 
 
+def _requires_grad(color):
+    return isinstance(color, torch.Tensor) and color.requires_grad
+
+
+def _vertex_colours(color_t, nv):
+    """Per-vertex colours packed as the vertices, (sum nv, 3), from a colour broadcast against (B, maxV, 3) as the
+    reference's color * ones((B, maxV, 3)) (renderer.py:76-77): (B, maxV, 3), per object (B, 1, 3), or any layout of B x V x 3
+    values with V >= maxV.  Differentiable: a colour that requires grad keeps its history."""
+    B, maxV = len(nv), max(nv, default=0)
+    if color_t.numel() % (3 * max(B, 1)) == 0 and color_t.numel() // (3 * max(B, 1)) >= maxV:
+        c = color_t.reshape(B, -1, 3)
+    else:
+        c = torch.broadcast_to(color_t, (B, maxV, 3))
+    return torch.cat([c[b, :n] for b, n in enumerate(nv)], 0)
+
+
 _flag_bufs = {}
 
 
@@ -229,9 +245,10 @@ class MVRenderer(nn.Module):
         # deferred: the meshes are staged (gather + H2D + mvr_mesh_prepare) inside render(), AFTER the camera kernel and
         # the constants below have been enqueued, so that the rasterizer launch follows the geometry with as little host
         # work in between as possible (the GPU would idle through it)
+        # (a colour that requires grad runs eagerly: the captured step has no colour gradient)
         if (self.cuda_graph is True and isinstance(meshes, ops.HostPackedMeshes) and self.shader == "hard_phong" and torch.is_grad_enabled()
-                and meshes.vert_rgb is None and torch.as_tensor(color).numel() == 3 and len(meshes) == azim.shape[0] and len(meshes) > 0
-                and not torch.cuda.is_current_stream_capturing()):
+                and meshes.vert_rgb is None and torch.as_tensor(color).numel() == 3 and not _requires_grad(color)
+                and len(meshes) == azim.shape[0] and len(meshes) > 0 and not torch.cuda.is_current_stream_capturing()):
             out = self._render_meshes_graphed(meshes, color, azim, elev, dist, lights, background_color, device)
             if out is not None:
                 return out
@@ -239,7 +256,13 @@ class MVRenderer(nn.Module):
         if geom.B != azim.shape[0]:
             raise ValueError(f"{geom.B} meshes but azim has batch {azim.shape[0]}")
         bg = _device_vec(background_color, device)
-        obj = None if geom.per_vertex_rgb else _device_vec(color, device)
+        if geom.per_vertex_rgb:
+            obj = None
+        elif _requires_grad(color):      # with its history, not through _device_vec's cache of constants
+            obj = color.to(device=device, dtype=torch.float32).reshape(3)
+        else:
+            obj = _device_vec(color, device)
+        grad_rgb = getattr(geom, "grad_rgb", None)
         fixed_light = None if lights is None else _device_vec(lights, device)
 
         soft = self.shader != "hard_phong"
@@ -252,16 +275,16 @@ class MVRenderer(nn.Module):
                                          faces_per_pixel=self.faces_per_pixel, cull_backfaces=self.cull_backfaces,
                                          perspective_correct=self.perspective_correct, verts=getattr(geom, "grad_verts", None),
                                          shader=self.shader, blur_radius=self.blur_radius, sigma=self.blend_sigma,
-                                         gamma=self.blend_gamma)
+                                         gamma=self.blend_gamma, rgb=grad_rgb)
             return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
                                      faces_per_pixel=self.faces_per_pixel, cull_backfaces=self.cull_backfaces,
                                      perspective_correct=self.perspective_correct, verts=getattr(geom, "grad_verts", None),
-                                     normalize=self.normalize, out_dtype=self.out_dtype)
+                                     normalize=self.normalize, out_dtype=self.out_dtype, rgb=grad_rgb)
 
         try:
             out = None
             flag = None
-            if getattr(geom, "grad_verts", None) is None and not soft:
+            if getattr(geom, "grad_verts", None) is None and grad_rgb is None and not soft:
                 # fast path: cameras + rasterizer as ONE autograd node (ops.render_meshes_from_angles); the validity flag
                 # is still awaited through an event recorded between the camera kernel and the rasterizer
                 az, el, di = self._views(azim, elev, dist, device)
@@ -277,7 +300,7 @@ class MVRenderer(nn.Module):
                     after_cameras=flag)
                 if flag.read() == 0:
                     out = (images, frag)
-            if out is None:      # vertex gradients wanted, or invalid rotations: the general path with the redraw loop
+            if out is None:      # vertex / per-vertex colour gradients wanted, or invalid rotations: the general path with the redraw loop
                 out, R, T, C = self._render_with_guard(azim, elev, dist, device, render, known_invalid=flag is not None)
             images, frag = out
         finally:
@@ -299,17 +322,19 @@ class MVRenderer(nn.Module):
             raise ValueError(f"{points.shape[0]} clouds but azim has batch {azim.shape[0]}")
         bg = _device_vec(background_color, device)
         rgb = torch.as_tensor(color, dtype=torch.float32)
+        rgb_grad = _requires_grad(rgb)
         use_graph = self.cuda_graph
         if use_graph is None:      # auto: only where the step is launch-bound (DESIGN.md section 5)
             use_graph = (points.shape[0] * self.nb_views <= GRAPH_AUTO_MAX_VIEWS and not torch.cuda.is_current_stream_capturing())
-        if use_graph and rgb.numel() == 3 and torch.is_grad_enabled():      # under no_grad the eager path runs
+        # under no_grad, and for a colour that requires grad (the captured step has no colour gradient), the eager path runs
+        if use_graph and rgb.numel() == 3 and torch.is_grad_enabled() and not rgb_grad:
             az, el, di = self._views(azim, elev, dist, device)
             out = self._render_points_graphed(points, _device_vec(rgb, device), az, el, di, bg, device)
             if out is not None:
                 return out
         pts = points.to(device=device, dtype=torch.float32, non_blocking=True)
         if rgb.numel() == 3:
-            rgb = _device_vec(rgb, device)
+            rgb = rgb.to(device) if rgb_grad else _device_vec(rgb, device)
         else:
             rgb = rgb.to(device) * torch.ones_like(pts)          # renderer.py:119-120 features = color * ones_like(points)
 
@@ -471,30 +496,35 @@ class MVRenderer(nn.Module):
     def _packed(self, meshes, color, device):
         if isinstance(meshes, ops.PackedMeshes):
             return meshes
+        color_t = torch.as_tensor(color, dtype=torch.float32)
         if isinstance(meshes, ops.HostPackedMeshes):     # collated by the data loader: two H2D copies, no gather
-            color_t = torch.as_tensor(color, dtype=torch.float32)
             vert_rgb = None
             if color_t.numel() != 3:
-                color_t = color_t.reshape(len(meshes), -1, 3)
-                vert_rgb = torch.cat([color_t[b, :n] for b, n in enumerate(meshes.num_verts)], 0)
-            return ops.PackedMeshes.from_host_packed(meshes, device, vert_rgb=vert_rgb, copy_stream=self.copy_stream)
+                vert_rgb = _vertex_colours(color_t, meshes.num_verts)
+            geom = ops.PackedMeshes.from_host_packed(meshes, device, vert_rgb=None if vert_rgb is None else vert_rgb.detach(),
+                                                     copy_stream=self.copy_stream)
+            if vert_rgb is not None and vert_rgb.requires_grad:      # colour gradients: keep the history of the packing
+                geom.grad_rgb = vert_rgb.to(device)
+            return geom
         if meshes is None:
             raise ValueError("mesh rendering (pc_rendering=False) needs `meshes`")
-        if self.cache_geometry and self._geom_cache[0] is meshes:
+        # a colour that requires grad changes from step to step: the cached geometry's colours would be stale
+        cache = self.cache_geometry and not color_t.requires_grad
+        if cache and self._geom_cache[0] is meshes:
             return self._geom_cache[1]
         verts, faces = unpack_mesh_list(meshes)
         vert_rgb = None
-        color_t = torch.as_tensor(color, dtype=torch.float32)
         if color_t.numel() != 3:
-            # renderer.py:76-77 verts_rgb = color * ones((B, maxV, 3)): per-vertex colours (B, maxV, 3)
-            color_t = color_t.reshape(len(verts), -1, 3)
-            vert_rgb = torch.cat([color_t[b, : verts[b].shape[0]] for b in range(len(verts))], 0)
+            # renderer.py:76-77 verts_rgb = color * ones((B, maxV, 3)): per-vertex colours
+            vert_rgb = _vertex_colours(color_t, [v.shape[0] for v in verts])
         # (a capturing stream must only see calls from the capturing thread: no worker-thread copies then)
-        geom = ops.PackedMeshes.begin(verts, faces, device, vert_rgb=vert_rgb,
+        geom = ops.PackedMeshes.begin(verts, faces, device, vert_rgb=None if vert_rgb is None else vert_rgb.detach(),
                                       overlap=self.stage_overlap and not torch.cuda.is_current_stream_capturing())
         if any(v.requires_grad for v in verts):      # vertex gradients: keep the autograd history of the packing
             geom.grad_verts = torch.cat([v.to(device=device, dtype=torch.float32) for v in verts], 0)
-        if self.cache_geometry:
+        if vert_rgb is not None and vert_rgb.requires_grad:      # colour gradients: likewise
+            geom.grad_rgb = vert_rgb.to(device)
+        if cache:
             self._geom_cache = (meshes, geom)
         return geom
 
