@@ -143,7 +143,8 @@ class MVRenderer(nn.Module):
             captured buffer; the tensors the captured backward reads are static, so at most ONE forward may be outstanding
             per backward (two forwards of the same shapes before a backward would overwrite the first one's saved state).
         cache_geometry: keep the packed device geometry of the last mesh batch and reuse it when the
-            same list object is rendered again (SURVEY 8f N1).
+            same list object is rendered again (SURVEY 8f N1).  Not used when the colour or any vertex tensor requires grad:
+            a fitting loop updates those in place between steps, so a cached copy would be stale.
         shader / blur_radius / blend_sigma / blend_gamma / keep_alpha: mesh path -- "soft_phong" (SoftPhongShader) or
             "soft_silhouette" (SoftSilhouetteShader) blend the faces_per_pixel fragments of the blurred rasterizer (the
             shaders renderer.py:4-6 imports; SURVEY 8f N3); images keep 3 channels as renderer.py:112 unless keep_alpha.
@@ -508,11 +509,12 @@ class MVRenderer(nn.Module):
             return geom
         if meshes is None:
             raise ValueError("mesh rendering (pc_rendering=False) needs `meshes`")
-        # a colour that requires grad changes from step to step: the cached geometry's colours would be stale
-        cache = self.cache_geometry and not color_t.requires_grad
+        verts, faces = unpack_mesh_list(meshes)
+        # a colour or a vertex tensor that requires grad changes from step to step (an optimiser updates it in place): the cached
+        # geometry's colours / positions, and the autograd history of the packing, would be stale
+        cache = self.cache_geometry and not color_t.requires_grad and not any(v.requires_grad for v in verts)
         if cache and self._geom_cache[0] is meshes:
             return self._geom_cache[1]
-        verts, faces = unpack_mesh_list(meshes)
         vert_rgb = None
         if color_t.numel() != 3:
             # renderer.py:76-77 verts_rgb = color * ones((B, maxV, 3)): per-vertex colours
