@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MVR_ABI_VERSION 13
+#define MVR_ABI_VERSION 14
 
 /* flags */
 #define MVR_PERSPECTIVE_CORRECT 1  /* [upstream] RasterizationSettings.perspective_correct (FoV persp.: True) */
@@ -236,6 +236,26 @@ int mvr_mesh_backward_rgb(const void* geometry, const int* vert_off, const int* 
                           float* grad_verts, float* grad_normals, void* workspace, size_t workspace_bytes,
                           void* stream, float* grad_rgb);
 
+/* -- hard depth ([upstream] HardDepthShader: the nearest fragment's zbuf, zfar where no face covers the pixel) -------------- */
+/* The depth of the nearest fragment -- the (z, face) winner of the hard rasterizer of mvr_mesh_forward with K = 1, bit for bit its
+ * zbuf[..., 0] (near-plane clipping included) -- without shading: depth (n,1,H,W) fp32 = that z, depth_background where no face
+ * covers the pixel; pix_to_face (n,H,W) view-local face ids, -1 empty; counters as in mvr_mesh_forward (or NULL).  flags:
+ * MVR_PERSPECTIVE_CORRECT, MVR_CULL_BACKFACES and the workspace hints; MVR_IMAGES_BF16 / MVR_CLIP_BARYCENTRIC are rejected (-11).
+ * The workspace is mvr_mesh_workspace_bytes(B, M, H, W, 1, ...). */
+int mvr_mesh_depth_forward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                           int64_t total_verts, int64_t total_faces, int max_verts, int max_faces,
+                           const float* R, const float* T, float k00, float k11, float z_clip, float depth_background,
+                           int H, int W, int flags, float* depth, int* pix_to_face, int64_t* counters,
+                           void* workspace, size_t workspace_bytes, void* stream);
+/* its backward: grad_depth (n,1,H,W) -> gR (n,3,3), gT (n,3), WRITTEN (fixed-order sums: bit-reproducible, and the same with or
+ * without grad_verts); grad_verts (Vtot,3) or NULL, ACCUMULATED with atomics (caller zero-fills).  Background pixels and
+ * silhouette edges carry no gradient.  z_clip and flags: those of the forward. */
+int mvr_mesh_depth_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                            int64_t total_verts, int64_t total_faces, int max_verts, const float* R, const float* T,
+                            float k00, float k11, float z_clip, int H, int W, int flags, const int* pix_to_face,
+                            const float* grad_depth, float* gR, float* gT, float* grad_verts, void* workspace,
+                            size_t workspace_bytes, void* stream);
+
 /* -- soft shading of K fragments per pixel (SURVEY 8f N3; renderer.py:4-6 SoftPhongShader / SoftSilhouetteShader) -------- */
 /* mode 0: [upstream] blending.softmax_rgb_blend over per-fragment Phong colours (SoftPhongShader; sigma, gamma = BlendParams,
  * znear / zfar = the camera's 1 / 100); mode 1: blending.sigmoid_alpha_blend (SoftSilhouetteShader: RGB = 1, alpha = 1 -
@@ -314,6 +334,19 @@ int mvr_points_backward_angles(const float* points, const float* rgb, int B, int
                                const uint32_t* hit_mask, const void* grad_images, float* g_azim, float* g_elev,
                                float* g_dist, float* gR, float* gT, float* grad_points, float* grad_rgb, void* workspace,
                                size_t workspace_bytes, void* stream);
+/* Hard depth of a point cloud: the nearest point's view-space z (the (z, index) winner of mvr_points_forward, bit for bit its
+ * zbuf[..., 0]) -- independent of K and of the compositor --, depth_background where no point covers the pixel.  Outputs:
+ * depth (n,1,H,W) fp32, idx (n,H,W) (-1 empty), hit_mask (required: the backward reads it).  flags: MVR_SCALE_IS_DIST only;
+ * MVR_IMAGES_BF16 / MVR_IDX_SPARSE are rejected (-11).  The workspace is mvr_points_workspace_bytes(B, Np, M, H, W, 1, radius). */
+int mvr_points_depth_forward(const float* points, int B, int Np, int M, const float* R, const float* T, const float* inv_dist,
+                             double radius, float depth_background, int H, int W, int flags, float* depth, int* idx,
+                             uint32_t* hit_mask, void* workspace, size_t workspace_bytes, void* stream);
+/* its backward: grad_depth (n,1,H,W) -> gR (n,3,3) (only its third column is non-zero), gT (n,3) (only z), g_inv_dist (n) (d/d dist
+ * with MVR_SCALE_IS_DIST), WRITTEN (fixed-order sums); grad_points (B,Np,3) or NULL, ACCUMULATED with atomics (caller zero-fills). */
+int mvr_points_depth_backward(const float* points, int B, int Np, int M, const float* R, const float* T, const float* inv_dist,
+                              double radius, int H, int W, int flags, const int* idx, const uint32_t* hit_mask,
+                              const float* grad_depth, float* gR, float* gT, float* g_inv_dist, float* grad_points,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -5,7 +5,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvr_b200.so")
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 PERSPECTIVE_CORRECT = 1
 CULL_BACKFACES = 2
 COMPOSITE_ALPHA = 4
@@ -66,6 +66,10 @@ SIGNATURES = {
                                    _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp]),
     "mvr_mesh_backward_angles": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp, _vp, _vp, _vp, _i, _vp, _f, _f, _f, _i, _i, _i, _i,
                                       _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mvr_mesh_depth_forward": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _i, _vp, _vp, _f, _f, _f, _f, _i, _i, _i, _vp, _vp, _vp,
+                                    _vp, _sz, _vp]),
+    "mvr_mesh_depth_backward": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp, _vp, _f, _f, _f, _i, _i, _i, _vp, _vp, _vp, _vp,
+                                     _vp, _vp, _sz, _vp]),
     "mvr_points_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _d]),
     "mvr_points_hit_mask_words": (_sz, [_i, _i, _i, _i]),
     "mvr_points_forward": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _d, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp,
@@ -74,6 +78,9 @@ SIGNATURES = {
                                  _vp, _vp, _vp, _vp, _sz, _vp]),
     "mvr_points_backward_angles": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp,
                                         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mvr_points_depth_forward": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _d, _f, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mvr_points_depth_backward": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _d, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                       _sz, _vp]),
 }
 
 _lib = None

@@ -370,7 +370,9 @@ __global__ void __launch_bounds__(NT, MINB) mesh_scatter_kernel(const MeshParams
 // PPT pixels per thread (rows yi0 + 8 j): the keys -- the one operand that comes from DRAM -- of all of them are
 // loaded before the first is shaded, so a thread pays the DRAM trip once instead of once per pixel; the dependent L2
 // trips (face -> vertex records) of pixel j then overlap with those of the other warps only.
-template <bool EXACT, int MINB, int PPT, bool VRGB>
+// DEPTH (hard depth, K = 1): the winning key's z -- the nearest fragment's depth, bit for bit -- or p.depth_bg into the
+// (n,1,H,W) plane `images`, and pix_to_face; no vertex / normal / colour gathers, no shading, no 3-channel stores.
+template <bool EXACT, int MINB, int PPT, bool VRGB, bool DEPTH = false>
 __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_shade_kernel(const MeshParams p, int tiles_x) {
   pdl_enter();
   const int b = blockIdx.z, m = blockIdx.y, n = b * p.M + m;
@@ -389,13 +391,27 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_shade_kernel(const Mes
   const float4* pvn = p.pv + (size_t)p.M * voff + (size_t)m * V;
   const bool persp = p.flags & MVR_PERSPECTIVE_CORRECT;
   float bg[3] = {0.f, 0.f, 0.f};
-  if (k == 0) { bg[0] = __ldg(p.bg_rgb); bg[1] = __ldg(p.bg_rgb + 1); bg[2] = __ldg(p.bg_rgb + 2); }
+  if (k == 0 && !DEPTH) { bg[0] = __ldg(p.bg_rgb); bg[1] = __ldg(p.bg_rgb + 1); bg[2] = __ldg(p.bg_rgb + 2); }
 #pragma unroll
   for (int j = 0; j < PPT; ++j) {
     const int yi = yi0 + 8 * j;
     if (j > 0 && yi >= p.H) break;
     const int pix = yi * p.W + xi;
     const unsigned long long key = keys[j];
+    if (DEPTH) {
+      int fid = -1;
+      float z = p.depth_bg;
+      if (key != MVR_EMPTY_KEY) {
+        fid = (int)(unsigned int)(key & 0xffffffffull);
+        // a face crossing the near plane: mesh_shade_clipped_kernel<false, true> owns the pixel (the face is read only then)
+        if (may_clip(p.wsflags) && face_straddles(gather_face(pvn, __ldg(p.faces4 + f0 + fid)), p.z_clip)) continue;
+        if (p.flags & MVR_WS_REARM_KEYS) p.keys[(size_t)n * HW + pix] = MVR_EMPTY_KEY;
+        z = __uint_as_float((unsigned int)(key >> 32));
+      }
+      p.pix_to_face[(size_t)n * HW + pix] = fid;
+      reinterpret_cast<float*>(p.images)[(size_t)n * HW + pix] = z;
+      continue;
+    }
     if (k + 1 < p.K) {            // hand the layer to the next peeling pass
       p.prev[(size_t)n * HW + pix] = key;
       p.keys[(size_t)n * HW + pix] = MVR_EMPTY_KEY;
@@ -536,13 +552,14 @@ extern "C" size_t mvr_mesh_workspace_bytes(int B, int M, int H, int W, int K, in
 // 10 k faces x 384 views, where the rounds are too few to fill.
 static int scatter_nt(int max_faces) { return max_faces > 32768 ? 128 : 256; }
 
-extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
-                                int64_t total_verts, int64_t total_faces, int max_verts, int max_faces,
-                                const float* R, const float* T, const float* Cc, const float* light,
-                                int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11,
-                                float z_clip, float blur_radius, int H, int W, int K, int flags, const float* out_mean_std, void* images,
-                                int* pix_to_face, float* zbuf, float* bary, float* dists, int64_t* counters,
-                                void* workspace, size_t workspace_bytes, void* stream) {
+// depth: mvr_mesh_depth_forward -- `images` is the (n,1,H,W) depth plane, K = 1, no shading inputs, no optional fragments
+static int mesh_forward_impl(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                             int64_t total_verts, int64_t total_faces, int max_verts, int max_faces,
+                             const float* R, const float* T, const float* Cc, const float* light,
+                             int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11,
+                             float z_clip, float blur_radius, int H, int W, int K, int flags, const float* out_mean_std, void* images,
+                             int* pix_to_face, float* zbuf, float* bary, float* dists, int64_t* counters,
+                             void* workspace, size_t workspace_bytes, void* stream, bool depth, float depth_bg) {
   int rc = check_mesh_common("mvr_mesh_forward", B, M, H, W, K, total_verts, total_faces, max_verts);
   if (rc) return rc;
   const int64_t N = (int64_t)B * M;
@@ -551,10 +568,10 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
     if (ce != cudaSuccess) { set_error("mvr_mesh_forward: cudaMemsetAsync: %s", cudaGetErrorString(ce)); return (int)ce; }
   }
   if (N == 0) return 0;
-  if (!geometry || !vert_off || !face_off || !R || !T || !Cc || !light || !bg_rgb || !images || !pix_to_face || !workspace) {
+  if (!geometry || !vert_off || !face_off || !R || !T || (!depth && (!Cc || !light || !bg_rgb)) || !images || !pix_to_face || !workspace) {
     set_error("mvr_mesh_forward: null pointer"); return -5;
   }
-  if (!(flags & MVR_RGB_PER_ELEMENT) && !obj_rgb) { set_error("mvr_mesh_forward: obj_rgb is NULL and the geometry has no per-vertex colours"); return -6; }
+  if (!depth && !(flags & MVR_RGB_PER_ELEMENT) && !obj_rgb) { set_error("mvr_mesh_forward: obj_rgb is NULL and the geometry has no per-vertex colours"); return -6; }
   if (!out_norm_valid(out_mean_std)) { set_error("mvr_mesh_forward: out_mean_std needs std > 0"); return -9; }
   if (!(blur_radius >= 0.f)) { set_error("mvr_mesh_forward: blur_radius must be >= 0"); return -10; }
   const WsLayout w = ws_layout(B, M, H, W, K, total_verts, total_faces);
@@ -589,6 +606,7 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
   p.counters = (long long*)counters;
   p.onorm = make_out_norm(out_mean_std);
   p.wsflags = (int*)(wb + w.flags);
+  p.depth_bg = depth_bg;
   const size_t HW = (size_t)H * W;
   const bool soft_raster = p.blur_radius > 0.f || (flags & MVR_CLIP_BARYCENTRIC);
   // every key = EMPTY, and the workspace flags right in front of the plane armed (WSF_CLIP)
@@ -612,7 +630,8 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
       if (rc) return rc;
     }
     const bool vrgb = flags & MVR_RGB_PER_ELEMENT;
-    if (zbuf || bary || dists) {
+    if (depth) MVR_LAUNCH_PDL((mesh_shade_kernel<false, 4, 4, false, true>), shade_fast_grid, MVR_THREADS, 0, st, p, tiles_x);
+    else if (zbuf || bary || dists) {
       if (vrgb) MVR_LAUNCH_PDL((mesh_shade_kernel<true, 3, 1, true>), shade_grid, MVR_THREADS, 0, st, p, tiles_x);
       else MVR_LAUNCH_PDL((mesh_shade_kernel<true, 3, 1, false>), shade_grid, MVR_THREADS, 0, st, p, tiles_x);
     } else if (vrgb) MVR_LAUNCH_PDL((mesh_shade_kernel<false, 4, 4, true>), shade_fast_grid, MVR_THREADS, 0, st, p, tiles_x);
@@ -620,10 +639,33 @@ extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const
     rc = check_launch("mesh_shade_kernel");
     if (rc) return rc;
     if (z_clip >= 0.f) {      // pixels won by a face crossing the near plane (none in MVTN's default configurations: the kernel exits at once)
-      rc = launch_mesh_shade_clipped(p, (int)N, soft_raster, st);
+      rc = launch_mesh_shade_clipped(p, (int)N, soft_raster, st, depth);
       if (rc) return rc;
     }
   }
   return 0;
+}
+
+extern "C" int mvr_mesh_forward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                                int64_t total_verts, int64_t total_faces, int max_verts, int max_faces,
+                                const float* R, const float* T, const float* Cc, const float* light,
+                                int light_stride, const float* obj_rgb, const float* bg_rgb, float k00, float k11,
+                                float z_clip, float blur_radius, int H, int W, int K, int flags, const float* out_mean_std, void* images,
+                                int* pix_to_face, float* zbuf, float* bary, float* dists, int64_t* counters,
+                                void* workspace, size_t workspace_bytes, void* stream) {
+  return mesh_forward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, max_faces, R, T, Cc, light,
+                           light_stride, obj_rgb, bg_rgb, k00, k11, z_clip, blur_radius, H, W, K, flags, out_mean_std, images,
+                           pix_to_face, zbuf, bary, dists, counters, workspace, workspace_bytes, stream, false, 0.f);
+}
+
+extern "C" int mvr_mesh_depth_forward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                                      int64_t total_verts, int64_t total_faces, int max_verts, int max_faces,
+                                      const float* R, const float* T, float k00, float k11, float z_clip, float depth_background,
+                                      int H, int W, int flags, float* depth, int* pix_to_face, int64_t* counters,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
+  if (flags & (MVR_IMAGES_BF16 | MVR_CLIP_BARYCENTRIC)) { set_error("mvr_mesh_depth_forward: the depth is fp32 from the hard rasterizer"); return -11; }
+  return mesh_forward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, max_faces, R, T, nullptr, nullptr,
+                           0, nullptr, nullptr, k00, k11, z_clip, 0.f, H, W, 1, flags & ~MVR_RGB_PER_ELEMENT, nullptr, depth, pix_to_face,
+                           nullptr, nullptr, nullptr, counters, workspace, workspace_bytes, stream, true, depth_background);
 }
 

@@ -19,7 +19,7 @@ namespace mvr {
 // in gvn[18] (vertex i: gvn[6 i .. 6 i + 2] = d/d position, gvn[6 i + 3 .. 6 i + 5] = d/d unit normal) and vids, and the
 // caller scatters them with warp-aggregated atomics (scatter_vertex_grads); returns false when nothing was produced.
 // GC (colour gradient wanted): with VRGB, gcol[3 i .. 3 i + 2] = d/d colour of vertex i (= bb_i d/d texel; vids set as for GV,
-// scattered by scatter_rgb_grads); with one object colour, gcol[0..2] += sum(bb) d/d texel (the thread's running sum).
+// scattered by scatter_vertex9<true>); with one object colour, gcol[0..2] += sum(bb) d/d texel (the thread's running sum).
 template <bool VRGB, bool GV, bool GC = false>
 __device__ __forceinline__ bool mesh_backward_pixel(const MeshBwdParams& p, int n, int f0, int voff, const float4* __restrict__ pvn,
                                                     bool persp, const ShadeCtx& sc, const float4 ucol, int fid, float g0, float g1,
@@ -220,9 +220,11 @@ __device__ __forceinline__ void scatter_vertex_grads(const MeshBwdParams& p, int
   }
 }
 
-// scatter_vertex_grads for the 9 per-vertex colour gradients of a pixel (gcol of mesh_backward_pixel<true, GV, true>): lanes that
-// hold the same face sum first, one lane per face issues the atomics.  Must be called by all 32 lanes (fid < 0: nothing to add).
-__device__ __forceinline__ void scatter_rgb_grads(const MeshBwdParams& p, int voff, int fid, const float gcol[9], const int vids[3]) {
+// scatter_vertex_grads for 9 per-vertex values of a pixel: the colour gradients (RGB: gcol of mesh_backward_pixel<true, GV, true>, into
+// p.grad_rgb) or the hard depth's position gradients (into p.grad_verts): lanes that hold the same face sum first, one lane per face
+// issues the atomics.  Must be called by all 32 lanes (fid < 0: nothing to add).
+template <bool RGB>
+__device__ __forceinline__ void scatter_vertex9(const MeshBwdParams& p, int voff, int fid, const float gcol[9], const int vids[3]) {
   const unsigned int full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const unsigned int grp = __match_any_sync(full, fid);
@@ -243,7 +245,7 @@ __device__ __forceinline__ void scatter_rgb_grads(const MeshBwdParams& p, int vo
   if (leader) {
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
-      float* o = p.grad_rgb + 3 * (size_t)(voff + vids[i]);
+      float* o = (RGB ? p.grad_rgb : p.grad_verts) + 3 * (size_t)(voff + vids[i]);
       atomicAdd(o + 0, sum[3 * i + 0]); atomicAdd(o + 1, sum[3 * i + 1]); atomicAdd(o + 2, sum[3 * i + 2]);
     }
   }
@@ -258,7 +260,7 @@ __device__ __forceinline__ void store_rgb_partial(const MeshBwdParams& p, size_t
 
 // VRGB: per-vertex colours (object_color == "custom"); otherwise ONE object colour: the texel is c * sum(b) and its
 // cotangent one dot product -- six registers and ~13 floating-point instructions less per covered pixel.
-// GC: colour gradients too (mesh_backward_pixel's gcol): per vertex through scatter_rgb_grads, one object colour through the
+// GC: colour gradients too (mesh_backward_pixel's gcol): per vertex through scatter_vertex9<true>, one object colour through the
 // per-warp partials rgb_partials.
 template <int MINB, bool VRGB, bool GV, bool GC = false>
 __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel(const MeshBwdParams p) {
@@ -312,7 +314,7 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel(const 
       bool done = false;
       if (live) { any = true; done = mesh_backward_pixel<VRGB, GV, GC>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, xf, yi, acc, gvn, vids, gcol); }
       if (GV) scatter_vertex_grads(p, voff, done ? fid : -1, gvn, vids);
-      if (GC && VRGB) scatter_rgb_grads(p, voff, done ? fid : -1, gcol, vids);
+      if (GC && VRGB) scatter_vertex9<true>(p, voff, done ? fid : -1, gcol, vids);
       continue;
     }
     if (!live) continue;
@@ -436,7 +438,7 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel_strip(
           done = mesh_backward_pixel<VRGB, GV, GC>(p, n, f0, voff, pvn, persp, sc, ucol, fid, g0, g1, g2, __ldg(p.tab + t * 32 + x), tyb * 32 + y, acc, gvn, vids, gcol);
         }
         if (GV) scatter_vertex_grads(p, voff, done ? fid : -1, gvn, vids);
-        if (GC && VRGB) scatter_rgb_grads(p, voff, done ? fid : -1, gcol, vids);
+        if (GC && VRGB) scatter_vertex9<true>(p, voff, done ? fid : -1, gcol, vids);
         continue;
       }
       any = true;
@@ -456,10 +458,191 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) mesh_backward_kernel_strip(
   if (!(lane & 1)) out[lane >> 1] = mine;
 }
 
+// ---- hard depth: d depth -> barycentrics / z_i -> perspective correction -> edge functions -> NDC -> view space ----
+// One covered pixel of mesh_depth_backward_kernel, depth = sum_i b_i z_i (the key's z), cotangent g: acc += (dR 9, dT 3); GV: the
+// d/d position of its three vertices in gv[9] (R . d view position), vids set.  Returns false for a pixel of a face crossing the near
+// plane (mesh_backward_finish_kernel<false, true> owns it).
+// The per-vertex d/d b_i = g z_i are nearly equal (their common part g depth is ~1e3 times their differences on a 10 k-face mesh
+// at 224^2), and the Jacobian behind them is ~1/area: they are never formed.  With perspective correction b = t / sum(t) annihilates
+// a common shift, so only g (z_i - z_j) enters (the difference form of mesh_backward_pixel with z as the attribute); without it,
+// depth = z0 S + w1 (z1 - z0) + w2 (z2 - z0) with S = sum w = A / (A + eps) identically, whose only dependence on the vertices is
+// through the area, d S = eps / (A + eps)^2 d A.
+template <bool GV>
+__device__ __forceinline__ bool mesh_depth_backward_pixel(const MeshBwdParams& p, int n, int f0, int voff, const float4* __restrict__ pvn,
+                                                          bool persp, int fid, float g, float xf, int yi, float acc[16], float gv[9],
+                                                          int vids[3]) {
+  const int4 fi = __ldg(p.faces4 + f0 + fid);
+  const Face fc = gather_face(pvn, fi);
+  if (may_clip(p.wsflags) && face_straddles(fc, p.z_clip)) return false;
+  const FaceEdges fe = face_edges(fc);
+  const float yf = __ldg(p.tab + p.W + yi);
+  const float e0 = (xf - fc.x1) * fe.A0 - (yf - fc.y1) * fe.B0;
+  const float e1 = (xf - fc.x2) * fe.A1 - (yf - fc.y2) * fe.B1;
+  const float e2 = (xf - fc.x0) * fe.A2 - (yf - fc.y0) * fe.B2;
+  const float inv_area = rcp_fast(fe.area_p);
+  const float w0 = e0 * inv_area, w1 = e1 * inv_area, w2 = e2 * inv_area;
+  const float d10 = g * (fc.z1 - fc.z0), d20 = g * (fc.z2 - fc.z0);      // g (z_i - z_0)
+  float gb0, gb1, gb2, dz0, dz1, dz2, garea;
+  if (persp) {
+    const float t0 = w0 * fc.z1 * fc.z2, t1 = w1 * fc.z0 * fc.z2, t2 = w2 * fc.z0 * fc.z1;
+    const float st = t0 + t1 + t2;
+    const bool clamped = st < MVR_K_EPS;
+    const float id = rcp_fast(fmaxf(st, MVR_K_EPS));
+    const float b0 = t0 * id, b1 = t1 * id, b2 = t2 * id;
+    dz0 = g * b0; dz1 = g * b1; dz2 = g * b2;
+    float gden = 0.f;
+    if (!clamped) {      // gb_i - sum_j b_j gb_j = sum_j b_j g (z_i - z_j)
+      const float d01 = -d10, d02 = -d20, d12 = d02 - d01;
+      gb0 = fmaf(b1, d01, b2 * d02);
+      gb1 = fmaf(b2, d12, -b0 * d01);
+      gb2 = -fmaf(b0, d02, b1 * d12);
+    } else {
+      gb0 = g * fc.z0; gb1 = g * fc.z1; gb2 = g * fc.z2;
+      gden = -(gb0 * t0 + gb1 * t1 + gb2 * t2) * id * id;
+    }
+    const float gt0 = fmaf(gb0, id, gden), gt1 = fmaf(gb1, id, gden), gt2 = fmaf(gb2, id, gden);
+    gb0 = gt0 * fc.z1 * fc.z2; gb1 = gt1 * fc.z0 * fc.z2; gb2 = gt2 * fc.z0 * fc.z1;
+    dz0 += gt1 * w1 * fc.z2 + gt2 * w2 * fc.z1;
+    dz1 += gt0 * w0 * fc.z2 + gt2 * w2 * fc.z0;
+    dz2 += gt0 * w0 * fc.z1 + gt1 * w1 * fc.z0;
+    garea = clamped ? -(gb0 * e0 + gb1 * e1 + gb2 * e2) * inv_area * inv_area : 0.f;
+  } else {
+    gb0 = 0.f; gb1 = d10; gb2 = d20;
+    dz0 = g * w0; dz1 = g * w1; dz2 = g * w2;
+    garea = (g * fc.z0 * MVR_K_EPS - (d10 * e1 + d20 * e2)) * inv_area * inv_area;
+  }
+  const float ge0 = gb0 * inv_area, ge1 = gb1 * inv_area, ge2 = gb2 * inv_area;
+  float gx0, gy0, gx1, gy1, gx2, gy2;
+  gx1 = ge0 * (yf - fc.y2); gy1 = ge0 * (fc.x2 - xf); gx2 = ge0 * (fc.y1 - yf); gy2 = ge0 * (xf - fc.x1);          // e0 = E(p,v1,v2)
+  gx2 += ge1 * (yf - fc.y0); gy2 += ge1 * (fc.x0 - xf); gx0 = ge1 * (fc.y2 - yf); gy0 = ge1 * (xf - fc.x2);        // e1 = E(p,v2,v0)
+  gx0 += ge2 * (yf - fc.y1); gy0 += ge2 * (fc.x1 - xf); gx1 += ge2 * (fc.y0 - yf); gy1 += ge2 * (xf - fc.x0);      // e2 = E(p,v0,v1)
+  gx0 += garea * (fc.y2 - fc.y1); gy0 += garea * (fc.x1 - fc.x2);                                                  // area = E(v2,v0,v1)
+  gx1 += garea * (fc.y0 - fc.y2); gy1 += garea * (fc.x2 - fc.x0);
+  gx2 += garea * (fc.y1 - fc.y0); gy2 += garea * (fc.x0 - fc.x1);
+  const float gxn[3] = {gx0, gx1, gx2}, gyn[3] = {gy0, gy1, gy2}, gzn[3] = {dz0, dz1, dz2};
+  const float xn[3] = {fc.x0, fc.x1, fc.x2}, yn[3] = {fc.y0, fc.y1, fc.y2}, zv[3] = {fc.z0, fc.z1, fc.z2};
+  const int vid[3] = {fi.x, fi.y, fi.z};
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const float4 X = __ldg(p.verts4 + voff + vid[i]);
+    const float iz = rcp_fast(zv[i]);
+    const float gpx = gxn[i] * p.k00 * iz;
+    const float gpy = gyn[i] * p.k11 * iz;
+    const float gpz = gzn[i] - (gxn[i] * xn[i] + gyn[i] * yn[i]) * iz;
+    acc[0] = fmaf(X.x, gpx, acc[0]); acc[1] = fmaf(X.x, gpy, acc[1]); acc[2] = fmaf(X.x, gpz, acc[2]);
+    acc[3] = fmaf(X.y, gpx, acc[3]); acc[4] = fmaf(X.y, gpy, acc[4]); acc[5] = fmaf(X.y, gpz, acc[5]);
+    acc[6] = fmaf(X.z, gpx, acc[6]); acc[7] = fmaf(X.z, gpy, acc[7]); acc[8] = fmaf(X.z, gpz, acc[8]);
+    acc[9] += gpx; acc[10] += gpy; acc[11] += gpz;
+    if (GV) {
+      const float* r = p.R + 9 * (size_t)n;
+      gv[3 * i + 0] = fmaf(__ldg(r + 0), gpx, fmaf(__ldg(r + 1), gpy, __ldg(r + 2) * gpz));
+      gv[3 * i + 1] = fmaf(__ldg(r + 3), gpx, fmaf(__ldg(r + 4), gpy, __ldg(r + 5) * gpz));
+      gv[3 * i + 2] = fmaf(__ldg(r + 6), gpx, fmaf(__ldg(r + 7), gpy, __ldg(r + 8) * gpz));
+      vids[i] = vid[i];
+    }
+  }
+  return true;
+}
+
+// grid: x = 32x32-pixel tiles, y = view m, z = object b; thread (lane, warp) owns pixels (x0 + lane, y0 + warp + 8 j), as
+// mesh_backward_kernel.  grad_images = the cotangent of the (n,1,H,W) depth plane.  One 16-float camera partial per warp (dC = 0) in
+// the layout mesh_backward_finish_kernel sums in fixed order.  GV: d/d vertex positions into p.grad_verts (warp-aggregated atomics).
+template <bool GV>
+__global__ void __launch_bounds__(MVR_THREADS) mesh_depth_backward_kernel(const MeshBwdParams p) {
+  pdl_enter();
+  const int tid = threadIdx.x;
+  const int b = blockIdx.z, m = blockIdx.y, n = b * p.M + m, cta = blockIdx.x;
+  int tyb, txb;
+  tile_rc(cta, p.tiles_x, tyb, txb);
+  const int xi = txb * 32 + (tid & 31), yi0 = tyb * 32 + (tid >> 5);
+  const int HW = p.H * p.W;
+  const int f0 = p.face_off[b], voff = p.vert_off[b], V = p.vert_off[b + 1] - voff;
+  const float4* pvn = p.pv + (size_t)p.M * voff + (size_t)m * V;
+  const bool persp = p.flags & MVR_PERSPECTIVE_CORRECT;
+  const float* gd = reinterpret_cast<const float*>(p.grad_images) + (size_t)n * HW;
+  int fids[BWD_PIX_PER_THREAD];
+  float gin[BWD_PIX_PER_THREAD];
+#pragma unroll
+  for (int j = 0; j < BWD_PIX_PER_THREAD; ++j) {
+    const int yi = yi0 + 8 * j;
+    fids[j] = (xi < p.W && yi < p.H) ? __ldg(p.pix_to_face + (size_t)n * HW + (size_t)yi * p.W + xi) : -1;
+  }
+#pragma unroll
+  for (int j = 0; j < BWD_PIX_PER_THREAD; ++j) gin[j] = fids[j] >= 0 ? __ldg(gd + (size_t)(yi0 + 8 * j) * p.W + xi) : 0.f;
+  float acc[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  bool any = false;
+  const float xf = xi < p.W ? __ldg(p.tab + xi) : 0.f;
+#pragma unroll 1
+  for (int j = 0; j < BWD_PIX_PER_THREAD; ++j) {
+    const int fid = fids[j];
+    const bool live = fid >= 0 && gin[j] != 0.f;
+    if (GV) {      // all lanes stay together for the warp-aggregated scatter
+      float gv[9];
+      int vids[3] = {0, 0, 0};
+      bool done = false;
+      if (live) { any = true; done = mesh_depth_backward_pixel<true>(p, n, f0, voff, pvn, persp, fid, gin[j], xf, yi0 + 8 * j, acc, gv, vids); }
+      scatter_vertex9<false>(p, voff, done ? fid : -1, gv, vids);
+      continue;
+    }
+    if (!live) continue;
+    any = true;
+    mesh_depth_backward_pixel<false>(p, n, f0, voff, pvn, persp, fid, gin[j], xf, yi0 + 8 * j, acc, nullptr, nullptr);
+  }
+  float* out = p.partials + ((size_t)n * p.parts_per_view + (size_t)cta * NWARPS + (tid >> 5)) * 16;
+  const int lane = tid & 31;
+  if (!__any_sync(0xffffffffu, any)) {
+    if (lane < 16) out[lane] = 0.f;
+    return;
+  }
+  const float mine = warp_sum16_transposed(acc);
+  if (!(lane & 1)) out[lane >> 1] = mine;
+}
 
 }  // namespace mvr
 
 using namespace mvr;
+
+extern "C" int mvr_mesh_depth_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                                       int64_t total_verts, int64_t total_faces, int max_verts, const float* R, const float* T,
+                                       float k00, float k11, float z_clip, int H, int W, int flags, const int* pix_to_face,
+                                       const float* grad_depth, float* gR, float* gT, float* grad_verts, void* workspace,
+                                       size_t workspace_bytes, void* stream) {
+  int rc = check_mesh_common("mvr_mesh_depth_backward", B, M, H, W, 1, total_verts, total_faces, max_verts);
+  if (rc) return rc;
+  const int64_t N = (int64_t)B * M;
+  if (N == 0) return 0;
+  if (!geometry || !vert_off || !face_off || !R || !T || !pix_to_face || !grad_depth || !gR || !gT || !workspace) {
+    set_error("mvr_mesh_depth_backward: null pointer"); return -5;
+  }
+  const WsLayout w = ws_layout(B, M, H, W, 1, total_verts, total_faces);
+  if (workspace_bytes < w.total) { set_error("mvr_mesh_depth_backward: workspace too small (%zu < %zu)", workspace_bytes, w.total); return -7; }
+  const GeomLayout g = geom_layout(total_verts, total_faces);
+  const char* gb = (const char*)geometry;
+  char* wb = (char*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!(flags & MVR_WS_PROJECTED)) rc = launch_project("mesh_project_kernel", g, w, geometry, vert_off, R, T, B, M, H, W, max_verts, k00, k11, z_clip, true, workspace, st);
+  if (rc) return rc;
+  MeshBwdParams p = {};
+  p.verts4 = (const float4*)(gb + g.verts4); p.normals4 = (const float4*)(gb + g.normals4);
+  p.rgb4 = (const float4*)(gb + g.rgb4); p.faces4 = (const int4*)(gb + g.faces4); p.xn8 = (const float4*)(gb + g.xn8);
+  p.vert_off = vert_off; p.face_off = face_off;
+  p.R = R; p.T = T;
+  p.k00 = k00; p.k11 = k11;
+  p.B = B; p.M = M; p.H = H; p.W = W; p.K = 1; p.flags = flags; p.ctas_per_view = w.bwd_ctas_per_view; p.tiles_x = (W + 31) / 32;
+  p.pv = (const float4*)(wb + w.pv); p.tab = (const float*)(wb + w.tab);
+  p.pix_to_face = pix_to_face; p.grad_images = grad_depth;
+  p.partials = (float*)(wb + w.partials); p.grad_verts = grad_verts;
+  p.z_clip = z_clip; p.wsflags = (int*)(wb + w.flags); p.parts_per_view = w.bwd_parts_per_view;
+  const dim3 bgrid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
+  if (grad_verts) MVR_LAUNCH_PDL(mesh_depth_backward_kernel<true>, bgrid, MVR_THREADS, 0, st, p);
+  else MVR_LAUNCH_PDL(mesh_depth_backward_kernel<false>, bgrid, MVR_THREADS, 0, st, p);
+  rc = check_launch("mesh_depth_backward_kernel");
+  if (rc) return rc;
+  // clipped-face pixels (if any) + the fixed-order sum of the per-warp partials -> gR, gT
+  return launch_mesh_backward_finish(p, (int)N, gR, gT, nullptr, st, true);
+}
 
 static int mesh_backward_impl(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
                               int64_t total_verts, int64_t total_faces, int max_verts, const float* R,

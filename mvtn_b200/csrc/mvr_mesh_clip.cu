@@ -91,15 +91,42 @@ __device__ __forceinline__ void shade_clipped_pixel(const MeshParams& p, int b, 
   if (k == 0) store_rgb(p.images, p.flags & MVR_IMAGES_BF16, (size_t)n * 3 * HW + pix, (size_t)HW, out[0], out[1], out[2], p.onorm);
 }
 
+// Hard depth (K = 1) of a pixel won by a face crossing the near plane: the depth is the key's z -- the z of the sub-triangle
+// the scatter kept -- unless no sub-triangle passes the forward's own test at this pixel (then background, as shade_clipped_pixel).
+__device__ __forceinline__ void depth_clipped_pixel(const MeshParams& p, int b, int m, int n, int pix) {
+  const int HW = p.H * p.W;
+  const int yi = pix / p.W, xi = pix - yi * p.W;
+  const unsigned long long key = p.keys[(size_t)n * HW + pix];
+  if (key == MVR_EMPTY_KEY) return;
+  if (p.flags & MVR_WS_REARM_KEYS) p.keys[(size_t)n * HW + pix] = MVR_EMPTY_KEY;
+  const int f0 = p.face_off[b], voff = p.vert_off[b], V = p.vert_off[b + 1] - voff;
+  const bool persp = p.flags & MVR_PERSPECTIVE_CORRECT;
+  const int fid = (int)(unsigned int)(key & 0xffffffffull);
+  const Face fc = gather_face(p.pv + (size_t)p.M * voff + (size_t)m * V, __ldg(p.faces4 + f0 + fid));
+  if (!face_straddles(fc, p.z_clip)) return;
+  ClipSub cs;
+  clip_face(fc, p.z_clip, persp, cs);
+  const float xf = __ldg(p.tab + xi), yf = __ldg(p.tab + p.W + yi);
+  float bcl[3], pz;
+  int s = pick_sub(cs, p.flags, persp, xf, yf, (unsigned int)(key >> 32), bcl, pz);
+  if (s < 0) s = pick_sub(cs, p.flags, persp, xf, yf, 0u, bcl, pz);
+  p.pix_to_face[(size_t)n * HW + pix] = s >= 0 ? fid : -1;
+  reinterpret_cast<float*>(p.images)[(size_t)n * HW + pix] = s >= 0 ? __uint_as_float((unsigned int)(key >> 32)) : p.depth_bg;
+}
+
 // grid: one CTA per view, striding over its pixels (the common case is "flag down": N tiny CTAs that exit at once).
 // Writes EVERY output of a pixel whose winning face straddles the plane (mesh_shade_kernel left it untouched).
-template <bool SOFT>
+// DEPTH: the hard depth instance (depth_clipped_pixel).
+template <bool SOFT, bool DEPTH = false>
 __global__ void __launch_bounds__(MVR_THREADS) mesh_shade_clipped_kernel(const MeshParams p) {
   pdl_enter();
   if (!may_clip(p.wsflags)) return;
   const int n = blockIdx.x, b = n / p.M, m = n - b * p.M;
   const int HW = p.H * p.W;
-  for (int pix = threadIdx.x; pix < HW; pix += MVR_THREADS) shade_clipped_pixel<SOFT>(p, b, m, n, pix);
+  for (int pix = threadIdx.x; pix < HW; pix += MVR_THREADS) {
+    if (DEPTH) depth_clipped_pixel(p, b, m, n, pix);
+    else shade_clipped_pixel<SOFT>(p, b, m, n, pix);
+  }
 }
 
 
@@ -189,13 +216,68 @@ __device__ __forceinline__ void backward_clipped_view(const MeshBwdParams& p, in
   }
 }
 
+// Hard depth: the clipped-face pixels of view n (those mesh_depth_backward_kernel skipped) -> acc (dR, dT; dC stays 0).  The pixel's
+// depth is the sub-triangle's bcl . z_sub: d/d its barycentrics = g z_sub (raster_backward), d/d z_sub = g bcl, and nothing reaches
+// the converted (original-face) barycentrics; then clip_face_backward and the projection as backward_clipped_view.
+__device__ __forceinline__ void backward_clipped_view_depth(const MeshBwdParams& p, int n, float (&acc)[16]) {
+  const int b = n / p.M, m = n - b * p.M;
+  const int HW = p.H * p.W;
+  const int f0 = p.face_off[b], voff = p.vert_off[b], V = p.vert_off[b + 1] - voff;
+  const float4* pvn = p.pv + (size_t)p.M * voff + (size_t)m * V;
+  const bool persp = p.flags & MVR_PERSPECTIVE_CORRECT;
+  const float* gd = reinterpret_cast<const float*>(p.grad_images);
+  for (int pix = threadIdx.x; pix < HW; pix += MVR_THREADS) {
+    const int fid = __ldg(p.pix_to_face + (size_t)n * HW + pix);
+    if (fid < 0) continue;
+    const int4 fi = __ldg(p.faces4 + f0 + fid);
+    const Face fc = gather_face(pvn, fi);
+    if (!face_straddles(fc, p.z_clip)) continue;
+    const float g = __ldg(gd + (size_t)n * HW + pix);
+    if (g == 0.f) continue;
+    const int yi = pix / p.W, xi = pix - yi * p.W;
+    const float xf = __ldg(p.tab + xi), yf = __ldg(p.tab + p.W + yi);
+    ClipSub cs;
+    clip_face(fc, p.z_clip, persp, cs);
+    float bcl[3], pz;
+    const int s = pick_sub(cs, p.flags, persp, xf, yf, 0u, bcl, pz);
+    if (s < 0) continue;
+    const Face sf = cs.f[s];
+    const float gbeta[3] = {g * sf.z0, g * sf.z1, g * sf.z2}, gb0[3] = {0.f, 0.f, 0.f};
+    float gq[9], gfv[9];
+    raster_backward(sf, persp, xf, yf, gbeta, gq);
+    gq[2] += g * bcl[0]; gq[5] += g * bcl[1]; gq[8] += g * bcl[2];
+    clip_face_backward(fc, p.z_clip, persp, cs.info, s, gq, gb0, bcl, gfv);
+    const float4 X[3] = {__ldg(p.verts4 + voff + fi.x), __ldg(p.verts4 + voff + fi.y), __ldg(p.verts4 + voff + fi.z)};
+    const float xn[3] = {fc.x0, fc.x1, fc.x2}, yn[3] = {fc.y0, fc.y1, fc.y2}, zv[3] = {fc.z0, fc.z1, fc.z2};
+    const int vid[3] = {fi.x, fi.y, fi.z};
+    for (int i = 0; i < 3; ++i) {
+      const float iz = 1.0f / zv[i];
+      const float gpx = gfv[3 * i] * p.k00 * iz;
+      const float gpy = gfv[3 * i + 1] * p.k11 * iz;
+      const float gpz = gfv[3 * i + 2] - (gfv[3 * i] * xn[i] + gfv[3 * i + 1] * yn[i]) * iz;
+      acc[0] += X[i].x * gpx; acc[1] += X[i].x * gpy; acc[2] += X[i].x * gpz;
+      acc[3] += X[i].y * gpx; acc[4] += X[i].y * gpy; acc[5] += X[i].y * gpz;
+      acc[6] += X[i].z * gpx; acc[7] += X[i].z * gpy; acc[8] += X[i].z * gpz;
+      acc[9] += gpx; acc[10] += gpy; acc[11] += gpz;
+      if (p.grad_verts) {
+        const float* r = p.R + 9 * (size_t)n;
+        float* o = p.grad_verts + 3 * (size_t)(voff + vid[i]);
+        atomicAdd(o + 0, __ldg(r + 0) * gpx + __ldg(r + 1) * gpy + __ldg(r + 2) * gpz);
+        atomicAdd(o + 1, __ldg(r + 3) * gpx + __ldg(r + 4) * gpy + __ldg(r + 5) * gpz);
+        atomicAdd(o + 2, __ldg(r + 6) * gpx + __ldg(r + 7) * gpy + __ldg(r + 8) * gpz);
+      }
+    }
+  }
+}
+
 // grid: one CTA per view -> gR, gT, gC.  (1) when some vertex lies behind the near plane (WSF_CLIP), the pixels of
 // straddling faces, which mesh_backward_kernel skipped, are redone with the clipped geometry; (2) fixed-order sum of the
 // per-warp partials of mesh_backward_kernel: thread t owns value t & 15 of the parts congruent to t >> 4 modulo 16
 // (coalesced 64-byte rows), then 16 threads add the 16 group sums (and the clipped part) in a fixed order.
 // GC (p.grad_rgb set): also the colour gradient -- the clipped pixels' share and, for one object colour, the view's total of
 // the colour partials in fp64 (rgb_views; mesh_rgb_grad_sum_kernel adds the views).
-template <bool GC>
+// DEPTH: the partials are mesh_depth_backward_kernel's and the clipped pixels go through backward_clipped_view_depth.
+template <bool GC, bool DEPTH = false>
 __global__ void __launch_bounds__(MVR_THREADS) mesh_backward_finish_kernel(const MeshBwdParams p, float* __restrict__ gR,
                                                                            float* __restrict__ gT, float* __restrict__ gC) {
   __shared__ double s_sum[MVR_THREADS];
@@ -209,7 +291,8 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_backward_finish_kernel(const
     float acc[16], gcol[3] = {0.f, 0.f, 0.f};
 #pragma unroll
     for (int i = 0; i < 16; ++i) acc[i] = 0.f;
-    backward_clipped_view<GC>(p, n, acc, gcol);
+    if (DEPTH) backward_clipped_view_depth(p, n, acc);
+    else backward_clipped_view<GC>(p, n, acc, gcol);
     block_sum<16>(acc, s_red);                // s_red[0..15] = the clipped pixels' totals
     if (one_rgb) block_sum<3>(gcol, s_cred);  // s_cred[0..2]: their colour gradient
   }
@@ -276,13 +359,18 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_rgb_grad_sum_kernel(const do
 
 using namespace mvr;
 
-int launch_mesh_shade_clipped(const MeshParams& p, int N, bool soft, cudaStream_t st) {
-  if (soft) MVR_LAUNCH_PDL(mesh_shade_clipped_kernel<true>, (unsigned)N, MVR_THREADS, 0, st, p);
+int launch_mesh_shade_clipped(const MeshParams& p, int N, bool soft, cudaStream_t st, bool depth) {
+  if (depth) MVR_LAUNCH_PDL((mesh_shade_clipped_kernel<false, true>), (unsigned)N, MVR_THREADS, 0, st, p);
+  else if (soft) MVR_LAUNCH_PDL(mesh_shade_clipped_kernel<true>, (unsigned)N, MVR_THREADS, 0, st, p);
   else MVR_LAUNCH_PDL(mesh_shade_clipped_kernel<false>, (unsigned)N, MVR_THREADS, 0, st, p);
   return check_launch("mesh_shade_clipped_kernel");
 }
 
-int launch_mesh_backward_finish(const MeshBwdParams& p, int N, float* gR, float* gT, float* gC, cudaStream_t st) {
+int launch_mesh_backward_finish(const MeshBwdParams& p, int N, float* gR, float* gT, float* gC, cudaStream_t st, bool depth) {
+  if (depth) {
+    MVR_LAUNCH_PDL((mesh_backward_finish_kernel<false, true>), (unsigned)N, MVR_THREADS, 0, st, p, gR, gT, gC);
+    return check_launch("mesh_backward_finish_kernel");
+  }
   if (!p.grad_rgb) {
     MVR_LAUNCH_PDL(mesh_backward_finish_kernel<false>, (unsigned)N, MVR_THREADS, 0, st, p, gR, gT, gC);
     return check_launch("mesh_backward_finish_kernel");

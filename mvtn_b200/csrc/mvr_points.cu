@@ -38,6 +38,7 @@ struct PointsParams {
   int vec_bg;                    // W % 4 == 0 and 16-byte aligned images: the tile kernel paints the background 4 pixels per store
   void* images; int* idx; float* zbuf; float* dists2; unsigned int* hit_mask;
   OutNorm onorm;
+  float depth_bg;                // hard depth (mvr_points_depth_forward): the value of an uncovered pixel; `images` is (n,1,H,W) fp32
 };
 
 __device__ __forceinline__ void project_point(const float* __restrict__ pts, int pi, float s, const Camera& cam,
@@ -476,7 +477,9 @@ __device__ __forceinline__ void insert_key_smem(unsigned long long* s_keys, int 
 
 // grid: x = tile (ty * tiles_x + tx), y = view m, z = object b; dynamic shared memory: KT * 1024 keys
 // MINB: minimum CTAs per SM for the register allocator; 0 = unconstrained
-template <int KT, int MINB>
+// DEPTH (KT = 1, no zbuf / dists2): the nearest point's z -- the key's -- or p.depth_bg into the (n,1,H,W) plane `images`, idx and
+// the hit mask; no compositing.
+template <int KT, int MINB, bool DEPTH = false>
 __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const PointsParams p) {
   pdl_enter();
   extern __shared__ unsigned long long s_keys[];              // [KT][1024]
@@ -586,9 +589,9 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
     unsigned int* mask_v = p.hit_mask ? p.hit_mask + (size_t)n * p.H * p.mask_words + tx : nullptr;
     const bool bf16 = p.flags & MVR_IMAGES_BF16;
     const bool sparse_idx = (p.flags & MVR_IDX_SPARSE) && mask_v;
-    float* img_f = reinterpret_cast<float*>(p.images) + (size_t)n * 3 * HW;
+    float* img_f = reinterpret_cast<float*>(p.images) + (size_t)n * (DEPTH ? 1 : 3) * HW;
     __nv_bfloat16* img_h = reinterpret_cast<__nv_bfloat16*>(p.images) + (size_t)n * 3 * HW;
-    float g0 = __ldg(p.bg_rgb), g1 = __ldg(p.bg_rgb + 1), g2 = __ldg(p.bg_rgb + 2);
+    float g0 = DEPTH ? p.depth_bg : __ldg(p.bg_rgb), g1 = DEPTH ? 0.f : __ldg(p.bg_rgb + 1), g2 = DEPTH ? 0.f : __ldg(p.bg_rgb + 2);
     if (p.onorm.on) { g0 = (g0 - p.onorm.m0) * p.onorm.s0; g1 = (g1 - p.onorm.m1) * p.onorm.s1; g2 = (g2 - p.onorm.m2) * p.onorm.s2; }
     const __nv_bfloat16 h0 = __float2bfloat16_rn(g0), h1 = __float2bfloat16_rn(g1), h2 = __float2bfloat16_rn(g2);
     const int hw = (int)HW, xi = x0 + lane;
@@ -598,7 +601,9 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
       const int yv = y0 + (tid >> 3), xv = x0 + ((tid & 7) << 2);
       if (yv < p.H && xv < p.W) {
         const int pv = yv * p.W + xv;
-        if (bf16) {
+        if (DEPTH) {
+          *reinterpret_cast<float4*>(img_f + pv) = make_float4(g0, g0, g0, g0);
+        } else if (bf16) {
           const unsigned int u0 = __bfloat16_as_ushort(h0), u1 = __bfloat16_as_ushort(h1), u2 = __bfloat16_as_ushort(h2);
           *reinterpret_cast<uint2*>(img_h + pv) = make_uint2(u0 | (u0 << 16), u0 | (u0 << 16));
           *reinterpret_cast<uint2*>(img_h + pv + hw) = make_uint2(u1 | (u1 << 16), u1 | (u1 << 16));
@@ -644,7 +649,8 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
           for (int l = 0; l < KT; ++l) p.dists2[frag_o + KT * pix + l] = -1.f;
         }
         if (!p.vec_bg) {
-          if (bf16) { img_h[pix] = h0; img_h[pix + hw] = h1; img_h[pix + 2 * hw] = h2; }
+          if (DEPTH) img_f[pix] = g0;
+          else if (bf16) { img_h[pix] = h0; img_h[pix + hw] = h1; img_h[pix + 2 * hw] = h2; }
           else { img_f[pix] = g0; img_f[pix + hw] = g1; img_f[pix + 2 * hw] = g2; }
         }
       }
@@ -652,7 +658,17 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
   }
   __syncthreads();
   const int nhit = s_n;
-  if (nhit > 0) {
+  if (DEPTH) {
+    float* dep = reinterpret_cast<float*>(p.images) + (size_t)n * p.H * p.W;
+    int* idx_v = p.idx + (size_t)n * p.H * p.W;
+    for (int i = tid; i < nhit; i += MVR_THREADS) {
+      const int q = s_hits[i];
+      const unsigned long long key = s_keys[q];
+      const int pix = (y0 + (q >> 5)) * p.W + x0 + (q & 31);
+      idx_v[pix] = (int)(unsigned int)(key & 0xffffffffull);
+      dep[pix] = __uint_as_float((unsigned int)(key >> 32));
+    }
+  } else if (nhit > 0) {
     const Camera cam = load_camera(p.R, p.T, n);
     const float s = view_scale(p.inv_dist, p.flags, n);
     for (int i = tid; i < nhit; i += MVR_THREADS) {
@@ -916,6 +932,55 @@ __global__ void __launch_bounds__(MVR_THREADS) points_backward_kernel(const Poin
   }
 }
 
+// Hard depth backward: grid x = 32x32-pixel tile, y = view m, z = object b; thread (lane, warp) owns pixels (x0 + lane, y0 + warp + 8 j),
+// the covered ones read from the forward's hit mask (one word per tile row).  depth = s (X . R[:,2]) + T_z with s the cloud's scale:
+// (dR[:,2], dT_z, d s) into one 13-value partial per tile in the layout points_backward_reduce_kernel sums in fixed order;
+// grad_points (optional) accumulated with atomics.
+__global__ void __launch_bounds__(MVR_THREADS) points_depth_backward_kernel(const PointsBwdParams p) {
+  __shared__ float s_part[MVR_THREADS / 32][16];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.z, n = b * p.M + blockIdx.y, t = blockIdx.x;
+  const int ty = t / p.tiles_x, tx = t - ty * p.tiles_x;
+  const int xi = tx * 32 + lane;
+  const size_t plane = (size_t)p.H * p.W;
+  const float* pts = p.points + 3 * (size_t)b * p.Np;
+  const float* gd = reinterpret_cast<const float*>(p.grad_images) + (size_t)n * plane;
+  const Camera cam = load_camera(p.R, p.T, n);
+  const float s = view_scale(p.inv_dist, p.flags, n);
+  float acc[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int yi = ty * 32 + warp + 8 * j;
+    if (yi >= p.H) break;
+    const unsigned int word = __ldg(p.hit_mask + ((size_t)n * p.H + yi) * p.mask_words + tx);
+    if (!((word >> lane) & 1u)) continue;
+    const size_t pix = (size_t)yi * p.W + xi;
+    const float g = __ldg(gd + pix);
+    if (g == 0.f) continue;
+    const int q = __ldg(p.idx + (size_t)n * plane + pix);
+    const float X0 = __ldg(pts + 3 * (size_t)q), X1 = __ldg(pts + 3 * (size_t)q + 1), X2 = __ldg(pts + 3 * (size_t)q + 2);
+    const float gs = g * s;
+    acc[2] = fmaf(X0, gs, acc[2]); acc[5] = fmaf(X1, gs, acc[5]); acc[8] = fmaf(X2, gs, acc[8]);
+    acc[11] += g;
+    acc[12] = fmaf(g, cam.r[2] * X0 + cam.r[5] * X1 + cam.r[8] * X2, acc[12]);
+    if (p.grad_points) {
+      float* o = p.grad_points + 3 * ((size_t)b * p.Np + q);
+      atomicAdd(o, gs * cam.r[2]); atomicAdd(o + 1, gs * cam.r[5]); atomicAdd(o + 2, gs * cam.r[8]);
+    }
+  }
+  // one partial per tile: warp totals, then the warps in fixed order
+  const float mine = warp_sum16_transposed(acc);
+  if (!(lane & 1)) s_part[warp][lane >> 1] = mine;
+  __syncthreads();
+  if (tid < 16) {
+    float v = 0.f;
+    for (int w = 0; w < MVR_THREADS / 32; ++w) v += s_part[w][tid];
+    p.partials[((size_t)n * p.ctas_per_view + t) * 16 + tid] = v;
+  }
+}
+
 // grad_rgb_uniform: the (3,) gradient of the single point colour, or NULL (per-point colours / not wanted)
 __global__ void points_backward_reduce_kernel(const float* __restrict__ partials, int N, int n_parts,
                                               float* __restrict__ gR, float* __restrict__ gT, float* __restrict__ gs,
@@ -1039,6 +1104,46 @@ extern "C" size_t mvr_points_hit_mask_words(int B, int M, int H, int W) {
   return (size_t)B * M * H * ((W + 31) / 32);
 }
 
+// Binning of the tiled forward (K in {1, 2, 4, 8}): pixel table, per-(view, point) projection + pixel window, per-(view, tile) point
+// lists -- what points_tile_kernel reads.
+static int launch_points_binning(const PointsParams& p, const PointsWs& w, char* wb, cudaStream_t st) {
+  const int Np = p.Np, M = p.M, B = p.B, H = p.H, W = p.W;
+  const int64_t N = (int64_t)B * M;
+  const dim3 point_grid((unsigned)((Np + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
+  const bool bin_fused = Np > 0 && Np <= BIN_FUSED_MAX_POINTS && w.ntiles <= BIN_FUSED_MAX_TILES;
+  if (Np > 0 && !bin_fused) MVR_LAUNCH(pixel_table_kernel, 1, MVR_THREADS, 0, st, (float*)(wb + w.tab), H, W);
+  if (bin_fused) {
+    // a cluster of 4 CTAs per view for large clouds, and whenever there are fewer views than SMs (configs[0]: 12 views -- one CTA per
+    // view leaves 136 SMs idle while 12 CTAs walk 2048 points each: 24 -> 16 us, a fifth of that graph-replayed step)
+    const int cs = (Np > 4096 || (N < 148 && Np >= 512)) ? 4 : 1;
+    if (cs == 1) {
+      MVR_LAUNCH(points_bin_kernel_fused, dim3((unsigned)M, (unsigned)B), MVR_THREADS, ((size_t)W + H) * sizeof(float), st, p, (float*)(wb + w.tab), 1);
+    } else {      // thread-block cluster of cs CTAs per view (distributed shared memory)
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3((unsigned)(M * cs), (unsigned)B); cfg.blockDim = dim3(MVR_THREADS);
+      cfg.dynamicSmemBytes = ((size_t)W + H) * sizeof(float); cfg.stream = st;
+      cudaLaunchAttribute attr[1];
+      attr[0].id = cudaLaunchAttributeClusterDimension;
+      attr[0].val.clusterDim.x = (unsigned)cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+      cfg.attrs = attr; cfg.numAttrs = 1;
+      mvr::prof_begin("points_bin_kernel_fused", st);
+      cudaError_t le = cudaLaunchKernelEx(&cfg, points_bin_kernel_fused, p, (float*)(wb + w.tab), cs);
+      mvr::prof_end("points_bin_kernel_fused", st);
+      if (le != cudaSuccess) { set_error("points binning: cudaLaunchKernelEx: %s", cudaGetErrorString(le)); return (int)le; }
+    }
+    return check_launch("points_bin_kernel_fused");
+  }
+  if (Np > 0) {
+    cudaError_t e = cudaMemsetAsync(p.tile_cnt, 0, (size_t)N * w.ntiles * sizeof(int), st);
+    if (e != cudaSuccess) { set_error("points binning: cudaMemsetAsync: %s", cudaGetErrorString(e)); return (int)e; }
+    MVR_LAUNCH(points_bin_kernel<false>, point_grid, MVR_THREADS, 0, st, p);
+    MVR_LAUNCH(points_bin_scan_kernel, (unsigned)N, MVR_THREADS, 0, st, p);
+    MVR_LAUNCH(points_bin_kernel<true>, point_grid, MVR_THREADS, 0, st, p);
+    return check_launch("points_bin_kernel");
+  }
+  return 0;
+}
+
 extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, int Np, int M, const float* R,
                                   const float* T, const float* inv_dist, double radius, const float* bg_rgb,
                                   int H, int W, int K, int flags, const float* out_mean_std, void* images, int* idx,
@@ -1074,39 +1179,9 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
   p.onorm = make_out_norm(out_mean_std);
   cudaStream_t st = (cudaStream_t)stream;
   const dim3 point_grid((unsigned)((Np + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
-  const bool bin_fused = w.tiled && Np > 0 && Np <= BIN_FUSED_MAX_POINTS && w.ntiles <= BIN_FUSED_MAX_TILES;
-  if (Np > 0 && !bin_fused) MVR_LAUNCH(pixel_table_kernel, 1, MVR_THREADS, 0, st, (float*)(wb + w.tab), H, W);
   if (w.tiled) {
-    if (bin_fused) {
-      // a cluster of 4 CTAs per view for large clouds, and whenever there are fewer views than SMs (configs[0]: 12 views -- one CTA per
-      // view leaves 136 SMs idle while 12 CTAs walk 2048 points each: 24 -> 16 us, a fifth of that graph-replayed step)
-      const int cs = (Np > 4096 || (N < 148 && Np >= 512)) ? 4 : 1;
-      if (cs == 1) {
-        MVR_LAUNCH(points_bin_kernel_fused, dim3((unsigned)M, (unsigned)B), MVR_THREADS, ((size_t)W + H) * sizeof(float), st, p, (float*)(wb + w.tab), 1);
-      } else {      // thread-block cluster of cs CTAs per view (distributed shared memory)
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(M * cs), (unsigned)B); cfg.blockDim = dim3(MVR_THREADS);
-        cfg.dynamicSmemBytes = ((size_t)W + H) * sizeof(float); cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        mvr::prof_begin("points_bin_kernel_fused", st);
-        cudaError_t le = cudaLaunchKernelEx(&cfg, points_bin_kernel_fused, p, (float*)(wb + w.tab), cs);
-        mvr::prof_end("points_bin_kernel_fused", st);
-        if (le != cudaSuccess) { set_error("mvr_points_forward: cudaLaunchKernelEx: %s", cudaGetErrorString(le)); return (int)le; }
-      }
-      rc = check_launch("points_bin_kernel_fused");
-      if (rc) return rc;
-    } else if (Np > 0) {
-      cudaError_t e = cudaMemsetAsync(p.tile_cnt, 0, (size_t)N * w.ntiles * sizeof(int), st);
-      if (e != cudaSuccess) { set_error("mvr_points_forward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return (int)e; }
-      MVR_LAUNCH(points_bin_kernel<false>, point_grid, MVR_THREADS, 0, st, p);
-      MVR_LAUNCH(points_bin_scan_kernel, (unsigned)N, MVR_THREADS, 0, st, p);
-      MVR_LAUNCH(points_bin_kernel<true>, point_grid, MVR_THREADS, 0, st, p);
-      rc = check_launch("points_bin_kernel");
-      if (rc) return rc;
-    }
+    rc = launch_points_binning(p, w, wb, st);
+    if (rc) return rc;
     const dim3 tile_grid((unsigned)w.ntiles, (unsigned)M, (unsigned)B);
     const size_t smem = (size_t)K * 1024 * sizeof(unsigned long long);
     cudaError_t e = cudaSuccess;
@@ -1128,6 +1203,7 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
     return check_launch("points_tile_kernel");
   }
   // ---- generic K: global key plane (memset + scatter with global atomics + resolve) ----
+  if (Np > 0) MVR_LAUNCH(pixel_table_kernel, 1, MVR_THREADS, 0, st, (float*)(wb + w.tab), H, W);
   const size_t need = (size_t)N * HW * K * 8;
   cudaError_t e = cudaMemsetAsync(p.keys, 0xFF, need, st);      // every key = EMPTY
   if (e != cudaSuccess) { set_error("mvr_points_forward: cudaMemsetAsync: %s", cudaGetErrorString(e)); return (int)e; }
@@ -1140,6 +1216,73 @@ extern "C" int mvr_points_forward(const float* points, const float* rgb, int B, 
   }
   MVR_LAUNCH(points_resolve_kernel<0>, resolve_grid, MVR_THREADS, 0, st, p, tiles_x);
   return check_launch("points_resolve_kernel");
+}
+
+// hard depth: the K = 1 tile forward's DEPTH instance (binning as mvr_points_forward)
+extern "C" int mvr_points_depth_forward(const float* points, int B, int Np, int M, const float* R, const float* T, const float* inv_dist,
+                                        double radius, float depth_background, int H, int W, int flags, float* depth, int* idx,
+                                        uint32_t* hit_mask, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_points_common("mvr_points_depth_forward", B, Np, M, H, W, 1, radius);
+  if (rc) return rc;
+  const int64_t N = (int64_t)B * M;
+  if (N == 0) return 0;
+  if ((Np > 0 && !points) || !R || !T || !inv_dist || !depth || !idx || !hit_mask || !workspace) { set_error("mvr_points_depth_forward: null pointer"); return -6; }
+  if (flags & (MVR_IMAGES_BF16 | MVR_IDX_SPARSE)) { set_error("mvr_points_depth_forward: the depth is fp32 and idx dense"); return -11; }
+  const PointsWs w = points_ws(B, Np, M, H, W, 1, radius);
+  if (workspace_bytes < w.total) { set_error("mvr_points_depth_forward: workspace too small (%zu < %zu)", workspace_bytes, w.total); return -7; }
+  if (Np > 0 && (long long)w.list_cap >= 0x7fffffffLL) { set_error("mvr_points_depth_forward: point lists too large"); return -8; }
+  char* wb = (char*)workspace;
+  PointsParams p = {};
+  p.points = points; p.R = R; p.T = T; p.inv_dist = inv_dist;
+  p.radius = (float)radius;
+  p.r2_raster = p.radius * p.radius;
+  p.r2_weight = (float)(radius * radius);
+  p.B = B; p.Np = Np; p.M = M; p.H = H; p.W = W; p.K = 1; p.flags = flags & (MVR_SCALE_IS_DIST); p.mask_words = w.mask_words;
+  p.keys = (unsigned long long*)(wb + w.keys);
+  p.tab = (const float*)(wb + w.tab);
+  p.pp = (float4*)(wb + w.pp); p.pw = (int2*)(wb + w.pw);
+  p.tile_cnt = (int*)(wb + w.tile_cnt); p.tile_off = (int*)(wb + w.tile_off); p.tile_cur = (int*)(wb + w.tile_cur);
+  p.list = (int*)(wb + w.list);
+  p.tiles_x = w.tiles_x; p.tiles_y = w.tiles_y; p.ntiles = w.ntiles; p.list_cap = w.list_cap;
+  p.vec_bg = (W % 4 == 0) && ((uintptr_t)depth % 16 == 0);
+  p.images = depth; p.idx = idx; p.hit_mask = hit_mask;
+  p.depth_bg = depth_background;
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = launch_points_binning(p, w, wb, st);
+  const dim3 tile_grid((unsigned)w.ntiles, (unsigned)M, (unsigned)B);
+  MVR_LAUNCH_PDL((points_tile_kernel<1, 0, true>), tile_grid, MVR_THREADS, 1024 * sizeof(unsigned long long), st, p);
+  return check_launch("points_tile_kernel");
+}
+
+extern "C" int mvr_points_depth_backward(const float* points, int B, int Np, int M, const float* R, const float* T, const float* inv_dist,
+                                         double radius, int H, int W, int flags, const int* idx, const uint32_t* hit_mask,
+                                         const float* grad_depth, float* gR, float* gT, float* g_inv_dist, float* grad_points,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_points_common("mvr_points_depth_backward", B, Np, M, H, W, 1, radius);
+  if (rc) return rc;
+  const int64_t N = (int64_t)B * M;
+  if (N == 0) return 0;
+  if ((Np > 0 && !points) || !R || !T || !inv_dist || !idx || !hit_mask || !grad_depth || !gR || !gT || !g_inv_dist || !workspace) {
+    set_error("mvr_points_depth_backward: null pointer"); return -6;
+  }
+  const PointsWs w = points_ws(B, Np, M, H, W, 1, radius);
+  const size_t need = (size_t)N * w.ntiles * 16 * sizeof(float);
+  if (workspace_bytes < need) { set_error("mvr_points_depth_backward: workspace too small (%zu < %zu)", workspace_bytes, need); return -7; }
+  PointsBwdParams p = {};
+  p.points = points; p.R = R; p.T = T; p.inv_dist = inv_dist;
+  p.B = B; p.Np = Np; p.M = M; p.H = H; p.W = W; p.K = 1; p.flags = flags & MVR_SCALE_IS_DIST;
+  p.tiles_x = w.tiles_x; p.tiles_y = w.tiles_y; p.ctas_per_view = w.ntiles; p.mask_words = w.mask_words;
+  p.idx = idx; p.grad_images = grad_depth; p.hit_mask = hit_mask;
+  p.partials = (float*)((char*)workspace + w.partials);
+  p.grad_points = grad_points;
+  cudaStream_t st = (cudaStream_t)stream;
+  MVR_LAUNCH(points_depth_backward_kernel, dim3((unsigned)w.ntiles, (unsigned)M, (unsigned)B), MVR_THREADS, 0, st, p);
+  rc = check_launch("points_depth_backward_kernel");
+  if (rc) return rc;
+  const int wpb = 8;
+  MVR_LAUNCH_PDL(points_backward_reduce_kernel, (unsigned)((N + wpb - 1) / wpb), wpb * 32, 0, st, (const float*)p.partials, (int)N, w.ntiles,
+                 gR, gT, g_inv_dist, inv_dist, p.flags, (float*)nullptr);
+  return check_launch("points_backward_reduce_kernel");
 }
 
 static int points_backward_impl(const float* points, const float* rgb, int B, int Np, int M, const float* R,

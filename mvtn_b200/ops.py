@@ -1012,6 +1012,68 @@ class _MeshRenderSoft(torch.autograd.Function):
         return (gR, gT, gC, gV) + (None,) * 3 + (g_obj,) + (None,) * 14 + (g_rgb,)
 
 
+class _MeshDepth(torch.autograd.Function):
+    """Hard depth ([upstream] HardDepthShader) as one autograd node: (R, T, C, verts) -> depth (n,1,H,W) = the nearest fragment's
+    view-space z (the K = 1 rasterizer's zbuf[..., 0], bit for bit), depth_background where no face covers the pixel; + pix_to_face
+    (n,H,W,1), counters.  Differentiable w.r.t. R, T and `verts` (mvr_mesh_depth_backward); the depth does not depend on the camera
+    centres (their gradient is 0)."""
+
+    @staticmethod
+    def forward(ctx, R, T, Cc, verts, geom: PackedMeshes, M, k00, k11, z_clip, H, W, flags, depth_background):
+        lib = L.load()
+        dev = geom.device
+        R, T = _f32c(R), _f32c(T)
+        N = geom.B * M
+        if R.shape[0] != N:
+            raise ValueError(f"expected {N} cameras (B*M), got {R.shape[0]}")
+        depth = torch.empty((N, 1, H, W), dtype=torch.float32, device=dev)
+        p2f = torch.empty((N, H, W, 1), dtype=torch.int32, device=dev)
+        counters = torch.empty(L.NUM_COUNTERS, dtype=torch.int64, device=dev)
+        geom.finish()
+        ws = workspace(dev, lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, 1, geom.total_verts, geom.total_faces), _mesh_owner=True)
+        ws_flags, ws_commit = _ws_mesh_flags_forward(dev, ws, (geom.B, M, H, W, 1, geom.total_verts))
+        with _on(dev):
+            L.check(lib.mvr_mesh_depth_forward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                               geom.total_verts, geom.total_faces, geom.max_verts, geom.max_faces, _ptr(R), _ptr(T),
+                                               k00, k11, z_clip, depth_background, H, W, flags | ws_flags, _ptr(depth), _ptr(p2f),
+                                               _ptr(counters), _ptr(ws), ws.numel(), _stream(dev)), "mvr_mesh_depth_forward")
+        ctx.set_materialize_grads(False)
+        ctx.geom, ctx.M, ctx.cfg = geom, M, (k00, k11, z_clip, H, W, flags, ws_commit())
+        ctx.save_for_backward(R, T, p2f)
+        ctx.mark_non_differentiable(p2f, counters)
+        return depth, p2f, counters
+
+    @staticmethod
+    def backward(ctx, g_depth, *_unused):
+        if g_depth is None:
+            return (None,) * 13
+        lib = L.load()
+        geom, M = ctx.geom, ctx.M
+        R, T, p2f = ctx.saved_tensors
+        k00, k11, z_clip, H, W, flags, ws_token = ctx.cfg
+        dev = geom.device
+        N = geom.B * M
+        g_depth = _f32c(g_depth)
+        g = torch.empty(12 * N, dtype=torch.float32, device=dev)
+        gR, gT = g[: 9 * N].view(N, 3, 3), g[9 * N:].view(N, 3)
+        gV = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev) if ctx.needs_input_grad[3] else None
+        ws = workspace(dev, lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, 1, geom.total_verts, geom.total_faces), _mesh_owner=True)
+        flags = flags | _ws_mesh_flags_backward(dev, ws, ws_token)
+        with _on(dev):
+            L.check(lib.mvr_mesh_depth_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                                geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), k00, k11,
+                                                z_clip, H, W, flags, _ptr(p2f), _ptr(g_depth), _ptr(gR), _ptr(gT), _ptr(gV),
+                                                _ptr(ws), ws.numel(), _stream(dev)), "mvr_mesh_depth_backward")
+        gC = torch.zeros((N, 3), dtype=torch.float32, device=dev) if ctx.needs_input_grad[2] else None
+        return (gR, gT, gC, gV) + (None,) * 9
+
+
+def _check_depth_options(normalize, out_dtype, blur_radius=0.0):
+    if normalize is not None or out_dtype not in (None, torch.float32) or blur_radius > 0:
+        raise ValueError("shader='hard_depth' returns the fp32 depth of the hard rasterizer: normalize / out_dtype / blur_radius > 0 "
+                         "are not supported with it")
+
+
 def render_meshes_from_angles(geom: PackedMeshes, M: int, azim, elev, dist, light, obj_rgb, bg_rgb, image_size,
                               faces_per_pixel=1, cull_backfaces=False, perspective_correct=True, fov=60.0, znear=1.0,
                               z_clip: Optional[float] = None, normalize=None, out_dtype=None, after_cameras=None):
@@ -1032,7 +1094,7 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
                   cull_backfaces=False, perspective_correct=True, fov=60.0, znear=1.0, z_clip: Optional[float] = None,
                   fragments=False, verts: Optional[torch.Tensor] = None, _extra_flags=0, normalize=None, out_dtype=None,
                   shader="hard_phong", blur_radius=0.0, clip_barycentric_coords=None, sigma=1e-4, gamma=1e-4, zfar=100.0,
-                  rgb: Optional[torch.Tensor] = None):
+                  rgb: Optional[torch.Tensor] = None, depth_background=100.0):
     """images (B*M,3,H,W) [+ dict of fragments].  HardPhong + hard blend, blur_radius 0 (MVTN's configuration), or --
     shader="soft_phong" / "soft_silhouette" (SURVEY 8f N3) -- RGBA (B*M,4,H,W) from the K = faces_per_pixel fragments of the
     BLURRED rasterizer ([upstream] blur_radius in squared NDC units, clip_barycentric_coords default True iff blur_radius > 0)
@@ -1044,7 +1106,12 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
     gradients w.r.t. it (float atomics, as the vertices); an `obj_rgb` that requires grad gets its gradient when the geometry
     has no per-vertex colours (a fixed-order sum: bit-reproducible).  Hard and soft Phong; the silhouette gives none.
     `normalize=(mean, std)` / `out_dtype=torch.bfloat16`: consumer-side fusion (SURVEY 8f N2) -- the kernel writes
-    (x - mean) / std (Trainer_mvt.py:41-49) in the dtype the CNN consumes; gradients flow through both."""
+    (x - mean) / std (Trainer_mvt.py:41-49) in the dtype the CNN consumes; gradients flow through both.
+    shader="hard_depth" ([upstream] HardDepthShader): (B*M,1,H,W) fp32, the view-space depth of each pixel's nearest fragment
+    (bit for bit the rasterizer's zbuf[..., 0]) and `depth_background` (default 100, the cameras' zfar) where no face covers it.
+    The nearest fragment does not depend on K: the depth always rasterizes with K = 1 and faces_per_pixel is ignored.
+    Differentiable w.r.t. R, T and `verts` (not across silhouette edges; background pixels carry no gradient); it does not depend
+    on the colours or the light.  normalize / out_dtype / blur_radius > 0 raise."""
     H_, W_ = _hw(image_size)
     k00, k11 = fov_projection_scale(fov, znear, aspect=1.0)
     if z_clip is None:
@@ -1053,9 +1120,14 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
     H, W = _hw(image_size)
     if clip_barycentric_coords is None:
         clip_barycentric_coords = blur_radius > 0
+    if shader == "hard_depth":
+        _check_depth_options(normalize, out_dtype, blur_radius)
+        depth, p2f, counters = _MeshDepth.apply(R, T, Cc, verts, geom, M, k00, k11, float(z_clip), H, W, flags, float(depth_background))
+        frag = {"pix_to_face": p2f, "counters": counters}
+        return depth, frag
     if shader != "hard_phong":
         if shader not in SOFT_SHADERS:
-            raise ValueError("shader must be 'hard_phong', 'soft_phong' or 'soft_silhouette'")
+            raise ValueError("shader must be 'hard_phong', 'hard_depth', 'soft_phong' or 'soft_silhouette'")
         if normalize is not None or out_dtype not in (None, torch.float32):
             raise ValueError("the soft shaders return fp32 RGBA: normalize / out_dtype are not supported with them")
         flags |= L.CLIP_BARYCENTRIC if clip_barycentric_coords else 0
@@ -1241,6 +1313,59 @@ class _PointsRenderFromAngles(torch.autograd.Function):
         return (ga.reshape(sa), ge.reshape(se), gd.reshape(sd), gP, gF) + (None,) * 10
 
 
+class _PointsDepth(torch.autograd.Function):
+    """Hard depth of point clouds as one autograd node: (R, T, scale, points) -> depth (n,1,H,W) = the nearest point's view-space z
+    (bit for bit the rasterizer's zbuf[..., 0]), depth_background where no point covers the pixel; + idx (n,H,W,1).  The scale is
+    1 / dist, or dist itself under SCALE_IS_DIST (then its gradient is d/d dist)."""
+
+    @staticmethod
+    def forward(ctx, R, T, scale, points, M, radius, H, W, flags, depth_background):
+        lib = L.load()
+        _require_cuda(points, "points")
+        dev = points.device
+        pts = _f32c(points)
+        if pts.dim() != 3 or pts.shape[2] != 3:
+            raise ValueError("points must be (B,N,3)")
+        B, Np, _ = pts.shape
+        N = B * M
+        R, T, sc = _f32c(R), _f32c(T), _f32c(scale).reshape(-1)
+        if R.shape[0] != N or sc.numel() != N:
+            raise ValueError(f"expected {N} cameras (B*M)")
+        depth = torch.empty((N, 1, H, W), dtype=torch.float32, device=dev)
+        idx = torch.empty((N, H, W, 1), dtype=torch.int32, device=dev)
+        mask = torch.empty(max(lib.mvr_points_hit_mask_words(B, M, H, W), 1), dtype=torch.int32, device=dev)
+        ws = workspace(dev, lib.mvr_points_workspace_bytes(B, Np, M, H, W, 1, float(radius)))
+        with _on(dev):
+            L.check(lib.mvr_points_depth_forward(_ptr(pts), B, Np, M, _ptr(R), _ptr(T), _ptr(sc), float(radius), depth_background,
+                                                 H, W, flags, _ptr(depth), _ptr(idx), _ptr(mask), _ptr(ws), ws.numel(), _stream(dev)),
+                    "mvr_points_depth_forward")
+        ctx.set_materialize_grads(False)
+        ctx.cfg = (B, Np, M, float(radius), H, W, flags, scale.shape, points.shape)
+        ctx.save_for_backward(R, T, sc, pts, idx, mask)
+        ctx.mark_non_differentiable(idx)
+        return depth, idx
+
+    @staticmethod
+    def backward(ctx, g_depth, *_unused):
+        if g_depth is None:
+            return (None,) * 10
+        lib = L.load()
+        R, T, sc, pts, idx, mask = ctx.saved_tensors
+        B, Np, M, radius, H, W, flags, scale_shape, points_shape = ctx.cfg
+        dev = pts.device
+        N = B * M
+        g_depth = _f32c(g_depth)
+        g = torch.empty(13 * N, dtype=torch.float32, device=dev)
+        gR, gT, gs = g[: 9 * N].view(N, 3, 3), g[9 * N: 12 * N].view(N, 3), g[12 * N:]
+        gP = torch.zeros_like(pts) if ctx.needs_input_grad[3] else None
+        ws = workspace(dev, lib.mvr_points_workspace_bytes(B, Np, M, H, W, 1, radius))
+        with _on(dev):
+            L.check(lib.mvr_points_depth_backward(_ptr(pts), B, Np, M, _ptr(R), _ptr(T), _ptr(sc), radius, H, W, flags, _ptr(idx),
+                                                  _ptr(mask), _ptr(g_depth), _ptr(gR), _ptr(gT), _ptr(gs), _ptr(gP), _ptr(ws),
+                                                  ws.numel(), _stream(dev)), "mvr_points_depth_backward")
+        return (gR, gT, gs.reshape(scale_shape), None if gP is None else gP.reshape(points_shape)) + (None,) * 6
+
+
 def render_points_from_angles(points, rgb, M: int, azim, elev, dist, radius: float, bg_rgb, image_size, points_per_pixel=1,
                               compositor="norm", normalize=None, out_dtype=None, after_cameras=None):
     """look_at_view_transform + render_points(dist=...) in one autograd node (see _PointsRenderFromAngles).
@@ -1256,14 +1381,20 @@ def render_points_from_angles(points, rgb, M: int, azim, elev, dist, radius: flo
 
 
 def render_points(points, rgb, M: int, R, T, inv_dist, radius: float, bg_rgb, image_size: int, points_per_pixel=1,
-                  compositor="norm", fragments=False, normalize=None, out_dtype=None, dist=None):
+                  compositor="norm", fragments=False, normalize=None, out_dtype=None, dist=None, shader="composite",
+                  depth_background=100.0):
     """images (B*M,3,H,W) [+ fragments].  compositor: "norm" (NormWeightedCompositor) | "alpha".
     The clouds are scaled by inv_dist (renderer.py:142 scale_(1 / dist)); pass inv_dist=None and dist=(B*M,) or (B, M)
     to have the kernels take the reciprocal themselves (same IEEE division as torch's 1.0 / dist) and return the gradient
     w.r.t. dist directly -- no elementwise launches or autograd nodes around the renderer.
-    normalize / out_dtype: as in render_meshes (consumer-side fusion)."""
+    normalize / out_dtype: as in render_meshes (consumer-side fusion).
+    shader="hard_depth": (B*M,1,H,W) fp32, the view-space depth of each pixel's nearest point (bit for bit the rasterizer's
+    zbuf[..., 0]), `depth_background` (default 100) where no point covers it; rgb, points_per_pixel and compositor do not change it
+    (it always rasterizes with K = 1).  Differentiable w.r.t. R, T, the scale and `points`.  normalize / out_dtype raise."""
     if compositor not in ("norm", "alpha"):
         raise ValueError("compositor must be 'norm' or 'alpha'")
+    if shader not in ("composite", "hard_depth"):
+        raise ValueError("shader must be 'composite' or 'hard_depth'")
     flags = L.COMPOSITE_ALPHA if compositor == "alpha" else 0
     if (inv_dist is None) == (dist is None):
         raise ValueError("pass exactly one of inv_dist and dist")
@@ -1271,6 +1402,11 @@ def render_points(points, rgb, M: int, R, T, inv_dist, radius: float, bg_rgb, im
         inv_dist = dist
         flags |= L.SCALE_IS_DIST
     H, W = _hw(image_size)
+    if shader == "hard_depth":
+        _check_depth_options(normalize, out_dtype)
+        depth, idx = _PointsDepth.apply(R, T, inv_dist, points, M, radius, H, W, flags & L.SCALE_IS_DIST, float(depth_background))
+        frag = {"idx": idx}
+        return depth, frag
     out = _PointsRender.apply(R, T, inv_dist, points, rgb, M, radius, bg_rgb, H, W,
                               int(points_per_pixel), flags, bool(fragments), _out_norm(normalize), out_dtype)
     if fragments:

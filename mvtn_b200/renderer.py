@@ -145,6 +145,13 @@ class MVRenderer(nn.Module):
         cache_geometry: keep the packed device geometry of the last mesh batch and reuse it when the
             same list object is rendered again (SURVEY 8f N1).  Not used when the colour or any vertex tensor requires grad:
             a fitting loop updates those in place between steps, so a cached copy would be stale.
+        shader="hard_depth" / depth_background (both paths; [upstream] HardDepthShader): rendered_images is (B, M, 1, H, W) fp32, the
+            view-space depth of each pixel's nearest fragment (face or point; bit for bit the rasterizer's zbuf[..., 0]) and
+            depth_background (default 100, the cameras' zfar) where nothing covers it.  The nearest fragment does not depend on K:
+            faces_per_pixel, points_per_pixel and the compositor do not change the result.  Gradients reach the angles and, when they
+            require grad, the meshes' vertex tensors or the points (not across silhouette edges; background pixels carry none); the
+            depth does not depend on the colour.  normalize, out_dtype=torch.bfloat16 and blur_radius > 0 raise ValueError.  Depth
+            steps run eagerly (never from CUDA graphs).
         shader / blur_radius / blend_sigma / blend_gamma / keep_alpha: mesh path -- "soft_phong" (SoftPhongShader) or
             "soft_silhouette" (SoftSilhouetteShader) blend the faces_per_pixel fragments of the blurred rasterizer (the
             shaders renderer.py:4-6 imports; SURVEY 8f N3); images keep 3 channels as renderer.py:112 unless keep_alpha.
@@ -160,8 +167,11 @@ class MVRenderer(nn.Module):
                  faces_per_pixel=1, points_radius=0.006, points_per_pixel=1, light_direction="random",
                  cull_backfaces=False, *, compositor="norm", perspective_correct=True, cache_geometry=False,
                  normalize=None, out_dtype=None, copy_stream=False, cuda_graph=None, shader="hard_phong", blur_radius=0.0,
-                 blend_sigma=1e-4, blend_gamma=1e-4, keep_alpha=False, stage_overlap=True):
+                 blend_sigma=1e-4, blend_gamma=1e-4, keep_alpha=False, stage_overlap=True, depth_background=100.0):
         super().__init__()
+        if shader == "hard_depth":
+            ops._check_depth_options(normalize, out_dtype, blur_radius)
+        self.depth_background = float(depth_background)
         self.stage_overlap = bool(stage_overlap)
         self.shader, self.blur_radius, self.blend_sigma, self.blend_gamma, self.keep_alpha = shader, blur_radius, blend_sigma, blend_gamma, keep_alpha
         self.copy_stream = copy_stream
@@ -266,11 +276,17 @@ class MVRenderer(nn.Module):
         grad_rgb = getattr(geom, "grad_rgb", None)
         fixed_light = None if lights is None else _device_vec(lights, device)
 
-        soft = self.shader != "hard_phong"
+        depth = self.shader == "hard_depth"
+        soft = self.shader != "hard_phong" and not depth
 
         def render(R, T, C, dist_, C_light):
             geom.finish()
             light = C_light if fixed_light is None else fixed_light
+            if depth:
+                return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
+                                         cull_backfaces=self.cull_backfaces, perspective_correct=self.perspective_correct,
+                                         verts=getattr(geom, "grad_verts", None), shader="hard_depth",
+                                         depth_background=self.depth_background)
             if soft:
                 return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
                                          faces_per_pixel=self.faces_per_pixel, cull_backfaces=self.cull_backfaces,
@@ -285,7 +301,7 @@ class MVRenderer(nn.Module):
         try:
             out = None
             flag = None
-            if getattr(geom, "grad_verts", None) is None and grad_rgb is None and not soft:
+            if getattr(geom, "grad_verts", None) is None and grad_rgb is None and not soft and not depth:
                 # fast path: cameras + rasterizer as ONE autograd node (ops.render_meshes_from_angles); the validity flag
                 # is still awaited through an event recorded between the camera kernel and the rasterizer
                 az, el, di = self._views(azim, elev, dist, device)
@@ -309,7 +325,9 @@ class MVRenderer(nn.Module):
         self.last_fragments = frag
         B = geom.B
         H, W = ops._hw(self.image_size)
-        if soft:      # RGBA from the soft shaders; renderer.py:112 keeps [..., 0:3]
+        if depth:
+            rendered_images = images.view(B, self.nb_views, 1, H, W)
+        elif soft:      # RGBA from the soft shaders; renderer.py:112 keeps [..., 0:3]
             rendered_images = images.view(B, self.nb_views, 4, H, W)
             if not self.keep_alpha:
                 rendered_images = rendered_images[:, :, :3]
@@ -324,8 +342,9 @@ class MVRenderer(nn.Module):
         bg = _device_vec(background_color, device)
         rgb = torch.as_tensor(color, dtype=torch.float32)
         rgb_grad = _requires_grad(rgb)
-        use_graph = self.cuda_graph
-        if use_graph is None:      # auto: only where the step is launch-bound (DESIGN.md section 5)
+        depth = self.shader == "hard_depth"
+        use_graph = self.cuda_graph and not depth      # depth steps run eagerly
+        if use_graph is None and not depth:      # auto: only where the step is launch-bound (DESIGN.md section 5)
             use_graph = (points.shape[0] * self.nb_views <= GRAPH_AUTO_MAX_VIEWS and not torch.cuda.is_current_stream_capturing())
         # under no_grad, and for a colour that requires grad (the captured step has no colour gradient), the eager path runs
         if use_graph and rgb.numel() == 3 and torch.is_grad_enabled() and not rgb_grad:
@@ -341,10 +360,18 @@ class MVRenderer(nn.Module):
 
         def render(R, T, C, dist_, _C_light=None):
             # renderer.py:142 point_cloud.scale_(1/dist): the reciprocal is taken inside the kernels (dist=)
+            if depth:
+                return ops.render_points(pts, rgb, self.nb_views, R, T, None, self.points_radius, bg, self.image_size,
+                                         dist=dist_, shader="hard_depth", depth_background=self.depth_background)
             return ops.render_points(pts, rgb, self.nb_views, R, T, None, self.points_radius, bg, self.image_size,
                                      points_per_pixel=self.points_per_pixel, compositor=self.compositor,
                                      normalize=self.normalize, out_dtype=self.out_dtype, dist=dist_)
 
+        if depth:      # the general path: cameras (with the redraw loop) and the depth node
+            (images, frag), R, T, C = self._render_with_guard(azim, elev, dist, device, render)
+            self.last_fragments = frag
+            H, W = ops._hw(self.image_size)
+            return images.view(pts.shape[0], self.nb_views, 1, H, W), FoVOrthographicCameras(R, T, C, znear=0.01)
         az, el, di = self._views(azim, elev, dist, device)
         # fast path: cameras + rasterizer + compositor as ONE autograd node (ops.render_points_from_angles); the validity
         # flag is awaited through an event recorded between the camera kernel and the rasterizer
