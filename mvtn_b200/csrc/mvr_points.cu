@@ -1249,6 +1249,7 @@ extern "C" int mvr_points_depth_forward(const float* points, int B, int Np, int 
   p.depth_bg = depth_background;
   cudaStream_t st = (cudaStream_t)stream;
   rc = launch_points_binning(p, w, wb, st);
+  if (rc) return rc;
   const dim3 tile_grid((unsigned)w.ntiles, (unsigned)M, (unsigned)B);
   MVR_LAUNCH_PDL((points_tile_kernel<1, 0, true>), tile_grid, MVR_THREADS, 1024 * sizeof(unsigned long long), st, p);
   return check_launch("points_tile_kernel");
