@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MVR_ABI_VERSION 14
+#define MVR_ABI_VERSION 15
 
 /* flags */
 #define MVR_PERSPECTIVE_CORRECT 1  /* [upstream] RasterizationSettings.perspective_correct (FoV persp.: True) */
@@ -292,6 +292,23 @@ int mvr_mesh_soft_backward_rgb(const void* geometry, const int* vert_off, const 
                                int flags, int mode, float sigma, float gamma, float znear, float zfar, const int* pix_to_face,
                                const float* grad_rgba, float* gR, float* gT, float* gC, float* grad_verts, float* grad_normals,
                                void* workspace, size_t workspace_bytes, void* stream, float* grad_rgb);
+/* -- soft depth ([upstream] SoftDepthShader) ------------------------------------------------------------------------------ */
+/* The K fragments mvr_mesh_forward wrote with K = faces_per_pixel and blur_radius > 0 (pix_to_face, zbuf, dists: (n,H,W,K)),
+ * blended into depth (n,1,H,W) fp32: over the valid entries of a pixel in list order, p_k = sigmoid(-dists_k / sigma),
+ * c_k = sum_{j <= k} p_j, m_k = min(c_k, 1); depth = sum_k (m_k - m_prev) zbuf_k + (1 - m_last) depth_background.  A pixel with
+ * no fragment holds depth_background (any finite value).  sigma > 0 (BlendParams.sigma); gamma does not enter. */
+int mvr_mesh_soft_depth_forward(int B, int M, int H, int W, int K, float sigma, float depth_background, const int* pix_to_face,
+                                const float* zbuf, const float* dists, float* depth, void* stream);
+/* its backward through the rasterizer (grad_zbuf, grad_dists, clipped barycentrics, near-plane clipping, as
+ * mvr_mesh_soft_backward): grad_depth (n,1,H,W) -> gR (n,3,3), gT (n,3), WRITTEN (fixed-order sums: bit-reproducible, and the
+ * same with or without grad_verts); grad_verts (Vtot,3) or NULL, ACCUMULATED with atomics (caller zero-fills).  The depth does
+ * not depend on the camera centres or the colours.  z_clip, blur_radius, K, flags and sigma: those of the forward;
+ * MVR_IMAGES_BF16 is rejected (-11).  The workspace is mvr_mesh_workspace_bytes(B, M, H, W, K, ...). */
+int mvr_mesh_soft_depth_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
+                                 int64_t total_verts, int64_t total_faces, int max_verts, const float* R, const float* T,
+                                 float k00, float k11, float z_clip, float blur_radius, int H, int W, int K, int flags,
+                                 float sigma, float depth_background, const int* pix_to_face, const float* grad_depth,
+                                 float* gR, float* gT, float* grad_verts, void* workspace, size_t workspace_bytes, void* stream);
 
 /* -- point clouds --------------------------------------------------------------------------- */
 /* scratch for one forward or backward call (forward: pixel table + per-view projected points, tile lists, or for K not

@@ -5,7 +5,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvr_b200.so")
 
-ABI_VERSION = 14
+ABI_VERSION = 15
 PERSPECTIVE_CORRECT = 1
 CULL_BACKFACES = 2
 COMPOSITE_ALPHA = 4
@@ -60,6 +60,9 @@ SIGNATURES = {
                                     _i, _f, _f, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mvr_mesh_soft_backward_rgb": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _f, _f, _f, _f, _i, _i, _i,
                                         _i, _i, _f, _f, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp]),
+    "mvr_mesh_soft_depth_forward": (_i, [_i, _i, _i, _i, _i, _f, _f, _vp, _vp, _vp, _vp, _vp]),
+    "mvr_mesh_soft_depth_backward": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp, _vp, _f, _f, _f, _f, _i, _i, _i, _i, _f, _f,
+                                          _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mvr_mesh_backward": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp, _vp, _vp, _vp, _i, _vp, _f, _f, _f, _i, _i, _i, _i,
                                _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mvr_mesh_backward_rgb": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp, _vp, _vp, _vp, _i, _vp, _f, _f, _f, _i, _i, _i, _i,

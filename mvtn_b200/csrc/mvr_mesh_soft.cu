@@ -13,6 +13,8 @@
 //             chain through R, plus Phong's interpolated-position term) and d/d their unit normals (Phong, soft_phong only),
 //             scattered with one plain atomicAdd per value (as [upstream] RasterizeMeshesBackward): the vertex gradients are
 //             tolerance-level, their summation order is not fixed.  The camera arithmetic is the same in both instances.
+//   soft depth ([upstream] SoftDepthShader): mesh_soft_depth_kernel blends the same K fragments into one depth plane;
+//             mesh_soft_depth_backward_kernel<GV> chains its adjoint through soft_fragment_backward (no colour term).
 // Tolerance-compared against the torch restatement (oracle/torch_ref.py render_mesh_view_soft + vertex_normals, autograd): not
 // on MVTN's default path, written for clarity rather than tuned.
 #include "mvr_mesh.cuh"
@@ -367,6 +369,97 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
   if (!(lane & 1)) out[lane >> 1] = mine;
 }
 
+// [upstream] SoftDepthShader over the K fragments of a pixel, -1 entries skipped:  p_k = sigmoid(-dists_k / sigma),
+// c_k = sum_{j <= k} p_j, m_k = min(c_k, 1);  depth = sum_k (m_k - m_prev) z_k + (1 - m_last) bg.  Past the first entry with
+// c > 1 every weight is 0, so the loop stops there.  A pixel with no fragment gets exactly bg.
+// grid: x = 256-pixel chunks of the image, y = view m, z = object b
+__global__ void __launch_bounds__(MVR_THREADS) mesh_soft_depth_kernel(const int* __restrict__ pix_to_face, const float* __restrict__ zbuf,
+                                                                      const float* __restrict__ dists, int M, int HW, int K, float sigma,
+                                                                      float bg, float* __restrict__ depth) {
+  const int n = blockIdx.z * M + blockIdx.y, pix = blockIdx.x * MVR_THREADS + threadIdx.x;
+  if (pix >= HW) return;
+  const size_t fo = ((size_t)n * HW + pix) * K;
+  float c = 0.f, mprev = 0.f, d = 0.f;
+  for (int k = 0; k < K; ++k) {
+    if (pix_to_face[fo + k] < 0) continue;
+    c += sigmoidf_(-dists[fo + k] / sigma);
+    const float m = fminf(c, 1.0f);
+    d += (m - mprev) * zbuf[fo + k];
+    mprev = m;
+    if (c > 1.0f) break;
+  }
+  depth[(size_t)n * HW + pix] = d + (1.0f - mprev) * bg;
+}
+
+// Backward of mesh_soft_depth_kernel, thread and tile layout of mesh_soft_backward_kernel (one 16-float camera partial per
+// warp).  With g = d loss / d depth of the pixel: d/d z_k = g (m_k - m_prev); k_end = the last entry with c_k <= 1 (torch's
+// clamp passes the gradient at equality), Z_stop = z of the next entry after it, or bg;  d/d p_j = g (z_j - Z_stop) for
+// j <= k_end, 0 past it.  c is non-decreasing, so no entry past k_end + 1 carries a gradient.  The fragments are recomputed
+// from the projected vertices (soft_fragment) and handed to soft_fragment_backward without colour; gC stays 0.
+template <bool GV>
+__global__ void __launch_bounds__(MVR_THREADS) mesh_soft_depth_backward_kernel(const MeshParams p, const SoftParams sp,
+                                                                               const float* __restrict__ grad_depth, float bg,
+                                                                               float* __restrict__ partials, int parts_per_view, int tiles_x) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.z, m = blockIdx.y, n = b * p.M + m, cta = blockIdx.x;
+  int tyb, txb;
+  tile_rc(cta, tiles_x, tyb, txb);
+  const int xi = txb * 32 + lane;
+  const int HW = p.H * p.W, K = p.K;
+  const int f0 = p.face_off[b], voff = p.vert_off[b], V = p.vert_off[b + 1] - voff;
+  const float4* pvn = p.pv + (size_t)p.M * voff + (size_t)m * V;
+  const bool persp = p.flags & MVR_PERSPECTIVE_CORRECT, clipb = p.flags & MVR_CLIP_BARYCENTRIC;
+  const bool clip_on = may_clip(p.wsflags);
+  const ShadeCtx sc = {};      // no colour term
+  const float gcz[3] = {0.f, 0.f, 0.f};
+  float acc[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  for (int j = 0; j < 4; ++j) {
+    const int yi = tyb * 32 + warp + 8 * j;
+    if (xi >= p.W || yi >= p.H) continue;
+    const int pix = yi * p.W + xi;
+    const float g = grad_depth[(size_t)n * HW + pix];
+    if (g == 0.f) continue;
+    const float xf = __ldg(p.tab + xi), yf = __ldg(p.tab + p.W + yi);
+    const int* list = p.pix_to_face + ((size_t)n * HW + pix) * K;
+    // pass 1: Z_stop (k_end is implicit: the entries with c <= 1 form a prefix of the list)
+    float zstop = bg, c = 0.f;
+    for (int k = 0; k < K; ++k) {
+      const int fid = list[k];
+      if (fid < 0) continue;
+      const Face fc = gather_face(pvn, __ldg(p.faces4 + f0 + fid));
+      ClipSub cs; SoftFrag fr;
+      if (!soft_fragment(p, fc, persp, clipb, clip_on, xf, yf, clip_on ? rank_in_list(list, k, fid) : 0, cs, fr)) continue;
+      c += sigmoidf_(-fr.h.sd / sp.sigma);
+      if (c > 1.0f) { zstop = fr.h.pz; break; }
+    }
+    // pass 2: each fragment up to and including the one after k_end
+    float mprev = 0.f;
+    c = 0.f;
+    for (int k = 0; k < K; ++k) {
+      const int fid = list[k];
+      if (fid < 0) continue;
+      const int4 fi = __ldg(p.faces4 + f0 + fid);
+      const Face fc = gather_face(pvn, fi);
+      ClipSub cs; SoftFrag fr;
+      if (!soft_fragment(p, fc, persp, clipb, clip_on, xf, yf, clip_on ? rank_in_list(list, k, fid) : 0, cs, fr)) continue;
+      const float prob = sigmoidf_(-fr.h.sd / sp.sigma);
+      c += prob;
+      const float mk = fminf(c, 1.0f);
+      const float gz = g * (mk - mprev);
+      mprev = mk;
+      const float gsd = c <= 1.0f ? g * (fr.h.pz - zstop) * (-1.0f / sp.sigma) * prob * (1.0f - prob) : 0.f;
+      if (gz != 0.f || gsd != 0.f)
+        soft_fragment_backward<GV>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, gz, gsd, false, acc);
+      if (c > 1.0f) break;
+    }
+  }
+  float* out = partials + ((size_t)n * parts_per_view + (size_t)cta * NWARPS + warp) * 16;
+  const float mine = warp_sum16_transposed(acc);
+  if (!(lane & 1)) out[lane >> 1] = mine;
+}
+
 }  // namespace mvr
 
 using namespace mvr;
@@ -488,4 +581,64 @@ extern "C" int mvr_mesh_soft_backward_rgb(const void* geometry, const int* vert_
   return mesh_soft_backward_impl(geometry, vert_off, face_off, B, M, total_verts, total_faces, max_verts, R, T, Cc, light, light_stride,
                                  obj_rgb, bg_rgb, k00, k11, z_clip, blur_radius, H, W, K, flags, mode, sigma, gamma, znear, zfar,
                                  pix_to_face, grad_rgba, gR, gT, gC, grad_verts, grad_normals, workspace, workspace_bytes, stream, grad_rgb);
+}
+
+extern "C" int mvr_mesh_soft_depth_forward(int B, int M, int H, int W, int K, float sigma, float depth_background, const int* pix_to_face,
+                                           const float* zbuf, const float* dists, float* depth, void* stream) {
+  int rc = check_mesh_common("mvr_mesh_soft_depth_forward", B, M, H, W, K, 0, 0, 0);
+  if (rc) return rc;
+  if ((int64_t)B * M == 0) return 0;
+  if (!pix_to_face || !zbuf || !dists || !depth) { set_error("mvr_mesh_soft_depth_forward: null pointer"); return -5; }
+  if (!(sigma > 0.f) || !isfinite(depth_background)) { set_error("mvr_mesh_soft_depth_forward: sigma must be > 0 and depth_background finite"); return -7; }
+  const dim3 grid((unsigned)(((size_t)H * W + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
+  MVR_LAUNCH(mesh_soft_depth_kernel, grid, MVR_THREADS, 0, (cudaStream_t)stream, pix_to_face, zbuf, dists, M, H * W, K, sigma,
+             depth_background, depth);
+  return check_launch("mesh_soft_depth_kernel");
+}
+
+extern "C" int mvr_mesh_soft_depth_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M, int64_t total_verts,
+                                            int64_t total_faces, int max_verts, const float* R, const float* T, float k00, float k11,
+                                            float z_clip, float blur_radius, int H, int W, int K, int flags, float sigma, float depth_background,
+                                            const int* pix_to_face, const float* grad_depth, float* gR, float* gT, float* grad_verts,
+                                            void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_mesh_common("mvr_mesh_soft_depth_backward", B, M, H, W, K, total_verts, total_faces, max_verts);
+  if (rc) return rc;
+  const int64_t N = (int64_t)B * M;
+  if (N == 0) return 0;
+  if (!geometry || !vert_off || !face_off || !R || !T || !pix_to_face || !grad_depth || !gR || !gT || !workspace) { set_error("mvr_mesh_soft_depth_backward: null pointer"); return -5; }
+  if (!(sigma > 0.f) || !isfinite(depth_background)) { set_error("mvr_mesh_soft_depth_backward: sigma must be > 0 and depth_background finite"); return -7; }
+  if (!(blur_radius >= 0.f)) { set_error("mvr_mesh_soft_depth_backward: blur_radius must be >= 0"); return -9; }
+  if (flags & MVR_IMAGES_BF16) { set_error("mvr_mesh_soft_depth_backward: the depth is fp32"); return -11; }
+  const WsLayout w = ws_layout(B, M, H, W, K, total_verts, total_faces);
+  if (workspace_bytes < w.total) { set_error("mvr_mesh_soft_depth_backward: workspace too small (%zu < %zu)", workspace_bytes, w.total); return -8; }
+  const GeomLayout g = geom_layout(total_verts, total_faces);
+  cudaStream_t st = (cudaStream_t)stream;
+  char* wb = (char*)workspace;
+  // project again with the forward's z_clip, as mesh_soft_backward_impl does
+  rc = launch_project("mesh_project_kernel", g, w, geometry, vert_off, R, T, B, M, H, W, max_verts, k00, k11, z_clip, true, workspace, st);
+  if (rc) return rc;
+  MeshParams p;
+  fill_params(p, geometry, vert_off, face_off, B, M, total_verts, total_faces, R, T, nullptr, nullptr, 0, nullptr, nullptr, k00, k11, H, W, K,
+              flags, pix_to_face);
+  p.pv = (float4*)(wb + w.pv); p.tab = (float*)(wb + w.tab); p.wsflags = (int*)(wb + w.flags);
+  p.z_clip = z_clip;
+  p.blur_radius = blur_radius > 0.f ? blur_radius : 0.f; p.blur_r = sqrtf(p.blur_radius);
+  SoftParams sp = {1, sigma, 0.f, 0.f, 0.f, 0.f, nullptr, nullptr, nullptr, nullptr, nullptr, grad_verts, nullptr, nullptr, nullptr};
+  const int tiles_x = (W + 31) / 32;
+  const dim3 grid((unsigned)w.bwd_ctas_per_view, (unsigned)M, (unsigned)B);
+  if (grad_verts)
+    MVR_LAUNCH((mesh_soft_depth_backward_kernel<true>), grid, MVR_THREADS, 0, st, p, sp, grad_depth, depth_background, (float*)(wb + w.partials),
+               w.bwd_parts_per_view, tiles_x);
+  else
+    MVR_LAUNCH((mesh_soft_depth_backward_kernel<false>), grid, MVR_THREADS, 0, st, p, sp, grad_depth, depth_background, (float*)(wb + w.partials),
+               w.bwd_parts_per_view, tiles_x);
+  rc = check_launch("mesh_soft_depth_backward_kernel");
+  if (rc) return rc;
+  MeshBwdParams q;
+  q.azim = q.elev = q.dist = nullptr; q.g_azim = q.g_elev = q.g_dist = nullptr;
+  // the finish kernel only sums the partials (its hard clipped-pixel pass kept off as in mesh_soft_backward_impl)
+  q.partials = (float*)(wb + w.partials); q.parts_per_view = w.bwd_parts_per_view; q.wsflags = (int*)(wb + w.flags) + WSF_CLIP + 1;
+  q.B = B; q.M = M; q.H = H; q.W = W; q.K = K; q.flags = flags; q.z_clip = -1.f; q.grad_verts = nullptr; q.grad_normals = nullptr;
+  q.grad_rgb = nullptr; q.rgb_partials = nullptr; q.rgb_views = nullptr;
+  return launch_mesh_backward_finish(q, (int)N, gR, gT, nullptr, st);
 }

@@ -1068,6 +1068,67 @@ class _MeshDepth(torch.autograd.Function):
         return (gR, gT, gC, gV) + (None,) * 9
 
 
+class _MeshSoftDepth(torch.autograd.Function):
+    """Blurred rasterizer (K fragments per pixel, signed edge distances, clipped barycentrics) + soft depth blend as one autograd
+    node: (R, T, C, verts) -> depth (n,1,H,W).  [upstream] MeshRasterizer(blur_radius, faces_per_pixel) + SoftDepthShader:
+    prob = sigmoid(-dists / sigma), the cumulative sum of the probabilities clamped at 1 weighs each fragment's zbuf, and what
+    is left of 1 weighs depth_background.  Differentiable w.r.t. R, T and `verts` (mvr_mesh_soft_depth_backward), across
+    silhouette edges; the depth does not depend on the camera centres (their gradient is 0) or the colours."""
+
+    @staticmethod
+    def forward(ctx, R, T, Cc, verts, geom: PackedMeshes, M, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags, blur_radius,
+                sigma, depth_background):
+        lib = L.load()
+        if obj_rgb is None and not geom.per_vertex_rgb:      # the rasterizer's hard-shaded image is not returned: any colour
+            obj_rgb = bg_rgb
+        cfg, saved, _hard, extras = _mesh_forward_launch(geom, M, R, T, Cc, light, obj_rgb, bg_rgb, k00, k11, z_clip, H, W, K, flags,
+                                                         True, None, None, blur_radius=blur_radius)
+        p2f, counters, zbuf, bary, dists = extras
+        Rs, Ts = saved[0], saved[1]
+        dev = geom.device
+        N = geom.B * M
+        depth = torch.empty((N, 1, H, W), dtype=torch.float32, device=dev)
+        with _on(dev):
+            L.check(lib.mvr_mesh_soft_depth_forward(geom.B, M, H, W, K, sigma, depth_background, _ptr(p2f), _ptr(zbuf), _ptr(dists),
+                                                    _ptr(depth), _stream(dev)), "mvr_mesh_soft_depth_forward")
+        ctx.set_materialize_grads(False)
+        ctx.geom, ctx.M = geom, M
+        ctx.cfg = (k00, k11, z_clip, blur_radius, H, W, K, cfg[5], sigma, depth_background)
+        ctx.save_for_backward(Rs, Ts, p2f)
+        ctx.mark_non_differentiable(p2f, counters, zbuf, bary, dists)
+        return depth, p2f, counters, zbuf, bary, dists
+
+    @staticmethod
+    def backward(ctx, g_depth, *_unused):
+        if g_depth is None:
+            return (None,) * 19
+        lib = L.load()
+        geom, M = ctx.geom, ctx.M
+        R, T, p2f = ctx.saved_tensors
+        k00, k11, z_clip, blur_radius, H, W, K, fl, sigma, depth_background = ctx.cfg
+        dev = geom.device
+        N = geom.B * M
+        g_depth = _f32c(g_depth)
+        g = torch.empty(12 * N, dtype=torch.float32, device=dev)
+        gR, gT = g[: 9 * N].view(N, 3, 3), g[9 * N:].view(N, 3)
+        gV = torch.zeros((geom.total_verts, 3), dtype=torch.float32, device=dev) if ctx.needs_input_grad[3] else None
+        ws = workspace(dev, lib.mvr_mesh_workspace_bytes(geom.B, M, H, W, K, geom.total_verts, geom.total_faces))
+        with _on(dev):
+            L.check(lib.mvr_mesh_soft_depth_backward(_ptr(geom.geometry), _ptr(geom.vert_off), _ptr(geom.face_off), geom.B, M,
+                                                     geom.total_verts, geom.total_faces, geom.max_verts, _ptr(R), _ptr(T), k00, k11,
+                                                     z_clip, blur_radius, H, W, K, fl, sigma, depth_background, _ptr(p2f),
+                                                     _ptr(g_depth), _ptr(gR), _ptr(gT), _ptr(gV), _ptr(ws), ws.numel(), _stream(dev)),
+                    "mvr_mesh_soft_depth_backward")
+        gC = torch.zeros((N, 3), dtype=torch.float32, device=dev) if ctx.needs_input_grad[2] else None
+        return (gR, gT, gC, gV) + (None,) * 15
+
+
+def _check_soft_depth_options(normalize, out_dtype, keep_alpha=False):
+    if normalize is not None or out_dtype not in (None, torch.float32) or keep_alpha:
+        raise ValueError("shader='soft_depth' returns one fp32 depth channel: normalize / out_dtype / keep_alpha are not supported "
+                         "with it")
+
+
 def _check_depth_options(normalize, out_dtype, blur_radius=0.0):
     if normalize is not None or out_dtype not in (None, torch.float32) or blur_radius > 0:
         raise ValueError("shader='hard_depth' returns the fp32 depth of the hard rasterizer: normalize / out_dtype / blur_radius > 0 "
@@ -1111,7 +1172,12 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
     (bit for bit the rasterizer's zbuf[..., 0]) and `depth_background` (default 100, the cameras' zfar) where no face covers it.
     The nearest fragment does not depend on K: the depth always rasterizes with K = 1 and faces_per_pixel is ignored.
     Differentiable w.r.t. R, T and `verts` (not across silhouette edges; background pixels carry no gradient); it does not depend
-    on the colours or the light.  normalize / out_dtype / blur_radius > 0 raise."""
+    on the colours or the light.  normalize / out_dtype / blur_radius > 0 raise.
+    shader="soft_depth" ([upstream] SoftDepthShader): (B*M,1,H,W) fp32 from the K = faces_per_pixel fragments of the blurred
+    rasterizer (blur_radius, clip_barycentric_coords as for the soft shaders): with prob = sigmoid(-dists / sigma) over a pixel's
+    fragments nearest first, each zbuf is weighted by the step of min(cumsum(prob), 1) and what is left of 1 by
+    `depth_background` (default 100; gamma does not enter).  Differentiable w.r.t. R, T and `verts` across silhouette edges, with
+    the soft fragments dict alongside.  normalize / out_dtype raise."""
     H_, W_ = _hw(image_size)
     k00, k11 = fov_projection_scale(fov, znear, aspect=1.0)
     if z_clip is None:
@@ -1125,9 +1191,15 @@ def render_meshes(geom: PackedMeshes, M: int, R, T, Cc, light, obj_rgb, bg_rgb, 
         depth, p2f, counters = _MeshDepth.apply(R, T, Cc, verts, geom, M, k00, k11, float(z_clip), H, W, flags, float(depth_background))
         frag = {"pix_to_face": p2f, "counters": counters}
         return depth, frag
+    if shader == "soft_depth":
+        _check_soft_depth_options(normalize, out_dtype)
+        flags |= L.CLIP_BARYCENTRIC if clip_barycentric_coords else 0
+        out = _MeshSoftDepth.apply(R, T, Cc, verts, geom, M, light, obj_rgb, bg_rgb, k00, k11, float(z_clip), H, W, int(faces_per_pixel),
+                                   flags, float(blur_radius), float(sigma), float(depth_background))
+        return out[0], {"pix_to_face": out[1], "counters": out[2], "zbuf": out[3], "bary_coords": out[4], "dists": out[5]}
     if shader != "hard_phong":
         if shader not in SOFT_SHADERS:
-            raise ValueError("shader must be 'hard_phong', 'hard_depth', 'soft_phong' or 'soft_silhouette'")
+            raise ValueError("shader must be 'hard_phong', 'hard_depth', 'soft_phong', 'soft_silhouette' or 'soft_depth'")
         if normalize is not None or out_dtype not in (None, torch.float32):
             raise ValueError("the soft shaders return fp32 RGBA: normalize / out_dtype are not supported with them")
         flags |= L.CLIP_BARYCENTRIC if clip_barycentric_coords else 0

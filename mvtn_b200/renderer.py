@@ -152,6 +152,12 @@ class MVRenderer(nn.Module):
             require grad, the meshes' vertex tensors or the points (not across silhouette edges; background pixels carry none); the
             depth does not depend on the colour.  normalize, out_dtype=torch.bfloat16 and blur_radius > 0 raise ValueError.  Depth
             steps run eagerly (never from CUDA graphs).
+        shader="soft_depth" / faces_per_pixel / blur_radius / blend_sigma / depth_background (mesh path; [upstream] SoftDepthShader):
+            rendered_images is (B, M, 1, H, W) fp32, the faces_per_pixel fragments of the blurred rasterizer blended by the
+            cumulative sum of sigmoid(-dists / blend_sigma) clamped at 1, depth_background taking what is left.  Unlike
+            "hard_depth", gradients cross silhouette edges and reach background pixels, so an unmasked loss against a target depth
+            map moves the views and, when they require grad, the vertices.  normalize, out_dtype=torch.bfloat16 and keep_alpha=True
+            raise ValueError; the point path raises.  Runs eagerly (never from CUDA graphs).
         shader / blur_radius / blend_sigma / blend_gamma / keep_alpha: mesh path -- "soft_phong" (SoftPhongShader) or
             "soft_silhouette" (SoftSilhouetteShader) blend the faces_per_pixel fragments of the blurred rasterizer (the
             shaders renderer.py:4-6 imports; SURVEY 8f N3); images keep 3 channels as renderer.py:112 unless keep_alpha.
@@ -171,6 +177,8 @@ class MVRenderer(nn.Module):
         super().__init__()
         if shader == "hard_depth":
             ops._check_depth_options(normalize, out_dtype, blur_radius)
+        if shader == "soft_depth":
+            ops._check_soft_depth_options(normalize, out_dtype, keep_alpha)
         self.depth_background = float(depth_background)
         self.stage_overlap = bool(stage_overlap)
         self.shader, self.blur_radius, self.blend_sigma, self.blend_gamma, self.keep_alpha = shader, blur_radius, blend_sigma, blend_gamma, keep_alpha
@@ -277,7 +285,8 @@ class MVRenderer(nn.Module):
         fixed_light = None if lights is None else _device_vec(lights, device)
 
         depth = self.shader == "hard_depth"
-        soft = self.shader != "hard_phong" and not depth
+        soft_depth = self.shader == "soft_depth"
+        soft = self.shader != "hard_phong" and not depth and not soft_depth
 
         def render(R, T, C, dist_, C_light):
             geom.finish()
@@ -286,6 +295,12 @@ class MVRenderer(nn.Module):
                 return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
                                          cull_backfaces=self.cull_backfaces, perspective_correct=self.perspective_correct,
                                          verts=getattr(geom, "grad_verts", None), shader="hard_depth",
+                                         depth_background=self.depth_background)
+            if soft_depth:
+                return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
+                                         faces_per_pixel=self.faces_per_pixel, cull_backfaces=self.cull_backfaces,
+                                         perspective_correct=self.perspective_correct, verts=getattr(geom, "grad_verts", None),
+                                         shader="soft_depth", blur_radius=self.blur_radius, sigma=self.blend_sigma,
                                          depth_background=self.depth_background)
             if soft:
                 return ops.render_meshes(geom, self.nb_views, R, T, C, light, obj, bg, self.image_size,
@@ -301,7 +316,7 @@ class MVRenderer(nn.Module):
         try:
             out = None
             flag = None
-            if getattr(geom, "grad_verts", None) is None and grad_rgb is None and not soft and not depth:
+            if getattr(geom, "grad_verts", None) is None and grad_rgb is None and not soft and not depth and not soft_depth:
                 # fast path: cameras + rasterizer as ONE autograd node (ops.render_meshes_from_angles); the validity flag
                 # is still awaited through an event recorded between the camera kernel and the rasterizer
                 az, el, di = self._views(azim, elev, dist, device)
@@ -325,7 +340,7 @@ class MVRenderer(nn.Module):
         self.last_fragments = frag
         B = geom.B
         H, W = ops._hw(self.image_size)
-        if depth:
+        if depth or soft_depth:
             rendered_images = images.view(B, self.nb_views, 1, H, W)
         elif soft:      # RGBA from the soft shaders; renderer.py:112 keeps [..., 0:3]
             rendered_images = images.view(B, self.nb_views, 4, H, W)
@@ -336,6 +351,8 @@ class MVRenderer(nn.Module):
         return rendered_images, FoVPerspectiveCameras(R, T, C)
 
     def render_points(self, points, color, azim, elev, dist, background_color=(0.0, 0.0, 0.0)):
+        if self.shader == "soft_depth":
+            raise ValueError("shader='soft_depth' renders meshes only (pc_rendering=False)")
         device = self._device(azim)
         if points.shape[0] != azim.shape[0]:
             raise ValueError(f"{points.shape[0]} clouds but azim has batch {azim.shape[0]}")
