@@ -260,7 +260,8 @@ int mvr_mesh_depth_backward(const void* geometry, const int* vert_off, const int
 /* mode 0: [upstream] blending.softmax_rgb_blend over per-fragment Phong colours (SoftPhongShader; sigma, gamma = BlendParams,
  * znear / zfar = the camera's 1 / 100); mode 1: blending.sigmoid_alpha_blend (SoftSilhouetteShader: RGB = 1, alpha = 1 -
  * prod(1 - sigmoid(-dists / sigma))).  Input: the fragments mvr_mesh_forward wrote with K = faces_per_pixel and
- * blur_radius > 0 (pix_to_face, zbuf, bary, dists: (n,H,W,K[,3])); output rgba (n,4,H,W) fp32. */
+ * blur_radius > 0 (pix_to_face, zbuf, bary, dists: (n,H,W,K[,3])); output rgba (n,4,H,W) fp32.  sigma >= FLT_MIN: a
+ * subnormal sigma, where 1 / sigma overflows, is refused with -7 as sigma <= 0 is; gamma > 0, zfar > znear. */
 int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
                                 int64_t total_verts, int64_t total_faces, const float* Cc, const float* light,
                                 int light_stride, const float* obj_rgb, const float* bg_rgb, int H, int W, int K, int flags,
@@ -275,7 +276,8 @@ int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert_off, const
  * z_clip and blur_radius must be those of the mvr_mesh_forward call that produced it: a fragment of a face crossing the
  * near plane z_clip is recomputed on the clipped sub-triangle the forward kept, and the chain runs through the clipping
  * ([upstream] clip.py) to the vertices of the original face.  -1 entries of a pixel's K-list are skipped, as
- * mvr_mesh_soft_blend_forward does. */
+ * mvr_mesh_soft_blend_forward does.  sigma, gamma, znear, zfar: checked as by mvr_mesh_soft_blend_forward (a subnormal
+ * sigma is refused). */
 int mvr_mesh_soft_backward(const void* geometry, const int* vert_off, const int* face_off, int B, int M,
                            int64_t total_verts, int64_t total_faces, int max_verts, const float* R, const float* T,
                            const float* Cc, const float* light, int light_stride, const float* obj_rgb,
@@ -296,7 +298,8 @@ int mvr_mesh_soft_backward_rgb(const void* geometry, const int* vert_off, const 
 /* The K fragments mvr_mesh_forward wrote with K = faces_per_pixel and blur_radius > 0 (pix_to_face, zbuf, dists: (n,H,W,K)),
  * blended into depth (n,1,H,W) fp32: over the valid entries of a pixel in list order, p_k = sigmoid(-dists_k / sigma),
  * c_k = sum_{j <= k} p_j, m_k = min(c_k, 1); depth = sum_k (m_k - m_prev) zbuf_k + (1 - m_last) depth_background.  A pixel with
- * no fragment holds depth_background (any finite value).  sigma > 0 (BlendParams.sigma); gamma does not enter. */
+ * no fragment holds depth_background (any finite value).  sigma >= FLT_MIN (BlendParams.sigma; a subnormal sigma is refused,
+ * as by the other soft entry points); gamma does not enter. */
 int mvr_mesh_soft_depth_forward(int B, int M, int H, int W, int K, float sigma, float depth_background, const int* pix_to_face,
                                 const float* zbuf, const float* dists, float* depth, void* stream);
 /* its backward through the rasterizer (grad_zbuf, grad_dists, clipped barycentrics, near-plane clipping, as

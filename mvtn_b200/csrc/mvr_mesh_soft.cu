@@ -17,6 +17,8 @@
 //             mesh_soft_depth_backward_kernel<GV> chains its adjoint through soft_fragment_backward (no colour term).
 // Tolerance-compared against the torch restatement (oracle/torch_ref.py render_mesh_view_soft + vertex_normals, autograd): not
 // on MVTN's default path, written for clarity rather than tuned.
+#include <cfloat>
+
 #include "mvr_mesh.cuh"
 
 namespace mvr {
@@ -354,7 +356,9 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_backward_kernel(const M
           gzi = gE * E / sp.gamma;
           gzmax -= gzi;
         }
-        const float gsd = gprob * (-1.0f / sp.sigma) * prob * (1.0f - prob);
+        // sigmoid backward first, then the 1 / sigma (upstream's order): a saturated fragment's p (1 - p) = 0 gives 0 even where
+        // gprob / sigma would overflow
+        const float gsd = gprob * (prob * (1.0f - prob)) / -sp.sigma;
         soft_fragment_backward<GV, GC>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcol, -gzi * zscale, gsd, sp.mode == 0, acc, rgbacc);
       }
     }
@@ -449,7 +453,9 @@ __global__ void __launch_bounds__(MVR_THREADS) mesh_soft_depth_backward_kernel(c
       const float mk = fminf(c, 1.0f);
       const float gz = g * (mk - mprev);
       mprev = mk;
-      const float gsd = c <= 1.0f ? g * (fr.h.pz - zstop) * (-1.0f / sp.sigma) * prob * (1.0f - prob) : 0.f;
+      // g (z_k - Z_stop) times p (1 - p), then divided by sigma: multiplied first, the large factors overflow to inf before a
+      // saturated fragment's p (1 - p) = 0 could cancel them (NaN at sigma ~1e-37, inf at a background ~1e35)
+      const float gsd = c <= 1.0f ? (g * (fr.h.pz - zstop)) * (prob * (1.0f - prob)) / -sp.sigma : 0.f;
       if (gz != 0.f || gsd != 0.f)
         soft_fragment_backward<GV>(p, sp, n, voff, fi, fc, fr, cs, persp, clipb, xf, yf, sc, gcz, gz, gsd, false, acc);
       if (c > 1.0f) break;
@@ -491,7 +497,8 @@ extern "C" int mvr_mesh_soft_blend_forward(const void* geometry, const int* vert
   if ((int64_t)B * M == 0) return 0;
   if (!geometry || !vert_off || !face_off || !Cc || !light || !bg_rgb || !pix_to_face || !zbuf || !bary || !dists || !rgba) { set_error("mvr_mesh_soft_blend_forward: null pointer"); return -5; }
   if (!(flags & MVR_RGB_PER_ELEMENT) && !obj_rgb) { set_error("mvr_mesh_soft_blend_forward: obj_rgb is NULL"); return -6; }
-  if (mode < 0 || mode > 1 || !(sigma > 0.f) || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_blend_forward: bad mode / sigma / gamma / z range"); return -7; }
+  if (!(sigma >= FLT_MIN)) { set_error("mvr_mesh_soft_blend_forward: sigma must be a normal float > 0 (>= FLT_MIN)"); return -7; }
+  if (mode < 0 || mode > 1 || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_blend_forward: bad mode / gamma / z range"); return -7; }
   MeshParams p;
   fill_params(p, geometry, vert_off, face_off, B, M, total_verts, total_faces, nullptr, nullptr, Cc, light, light_stride, obj_rgb, bg_rgb, 0.f, 0.f, H, W, K, flags, pix_to_face);
   SoftParams sp = {mode, sigma, gamma, znear, zfar, 0.f, zbuf, bary, dists, rgba, nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -513,7 +520,8 @@ static int mesh_soft_backward_impl(const void* geometry, const int* vert_off, co
   if (N == 0) return 0;
   if (!geometry || !vert_off || !face_off || !R || !T || !Cc || !light || !bg_rgb || !pix_to_face || !grad_rgba || !gR || !gT || !gC || !workspace) { set_error("mvr_mesh_soft_backward: null pointer"); return -5; }
   if (!(flags & MVR_RGB_PER_ELEMENT) && !obj_rgb) { set_error("mvr_mesh_soft_backward: obj_rgb is NULL"); return -6; }
-  if (mode < 0 || mode > 1 || !(sigma > 0.f) || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_backward: bad mode / sigma / gamma / z range"); return -7; }
+  if (!(sigma >= FLT_MIN)) { set_error("mvr_mesh_soft_backward: sigma must be a normal float > 0 (>= FLT_MIN)"); return -7; }
+  if (mode < 0 || mode > 1 || !(gamma > 0.f) || !(zfar > znear)) { set_error("mvr_mesh_soft_backward: bad mode / gamma / z range"); return -7; }
   if (!(blur_radius >= 0.f)) { set_error("mvr_mesh_soft_backward: blur_radius must be >= 0"); return -9; }
   const WsLayout w = ws_layout(B, M, H, W, K, total_verts, total_faces);
   if (workspace_bytes < w.total) { set_error("mvr_mesh_soft_backward: workspace too small (%zu < %zu)", workspace_bytes, w.total); return -8; }
@@ -589,7 +597,7 @@ extern "C" int mvr_mesh_soft_depth_forward(int B, int M, int H, int W, int K, fl
   if (rc) return rc;
   if ((int64_t)B * M == 0) return 0;
   if (!pix_to_face || !zbuf || !dists || !depth) { set_error("mvr_mesh_soft_depth_forward: null pointer"); return -5; }
-  if (!(sigma > 0.f) || !isfinite(depth_background)) { set_error("mvr_mesh_soft_depth_forward: sigma must be > 0 and depth_background finite"); return -7; }
+  if (!(sigma >= FLT_MIN) || !isfinite(depth_background)) { set_error("mvr_mesh_soft_depth_forward: sigma must be a normal float > 0 (>= FLT_MIN) and depth_background finite"); return -7; }
   const dim3 grid((unsigned)(((size_t)H * W + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
   MVR_LAUNCH(mesh_soft_depth_kernel, grid, MVR_THREADS, 0, (cudaStream_t)stream, pix_to_face, zbuf, dists, M, H * W, K, sigma,
              depth_background, depth);
@@ -606,7 +614,7 @@ extern "C" int mvr_mesh_soft_depth_backward(const void* geometry, const int* ver
   const int64_t N = (int64_t)B * M;
   if (N == 0) return 0;
   if (!geometry || !vert_off || !face_off || !R || !T || !pix_to_face || !grad_depth || !gR || !gT || !workspace) { set_error("mvr_mesh_soft_depth_backward: null pointer"); return -5; }
-  if (!(sigma > 0.f) || !isfinite(depth_background)) { set_error("mvr_mesh_soft_depth_backward: sigma must be > 0 and depth_background finite"); return -7; }
+  if (!(sigma >= FLT_MIN) || !isfinite(depth_background)) { set_error("mvr_mesh_soft_depth_backward: sigma must be a normal float > 0 (>= FLT_MIN) and depth_background finite"); return -7; }
   if (!(blur_radius >= 0.f)) { set_error("mvr_mesh_soft_depth_backward: blur_radius must be >= 0"); return -9; }
   if (flags & MVR_IMAGES_BF16) { set_error("mvr_mesh_soft_depth_backward: the depth is fp32"); return -11; }
   const WsLayout w = ws_layout(B, M, H, W, K, total_verts, total_faces);

@@ -156,8 +156,10 @@ class MVRenderer(nn.Module):
             rendered_images is (B, M, 1, H, W) fp32, the faces_per_pixel fragments of the blurred rasterizer blended by the
             cumulative sum of sigmoid(-dists / blend_sigma) clamped at 1, depth_background taking what is left.  Unlike
             "hard_depth", gradients cross silhouette edges and reach background pixels, so an unmasked loss against a target depth
-            map moves the views and, when they require grad, the vertices.  normalize, out_dtype=torch.bfloat16 and keep_alpha=True
-            raise ValueError; the point path raises.  Runs eagerly (never from CUDA graphs).
+            map moves the views and, when they require grad, the vertices.  The depth does not depend on the colour: a colour that
+            requires grad (per object or per vertex) leaves the depth unchanged and gets no gradient (its .grad stays None).
+            normalize, out_dtype=torch.bfloat16 and keep_alpha=True raise ValueError; the point path raises.  Runs eagerly (never
+            from CUDA graphs, cuda_graph=True included).
         shader / blur_radius / blend_sigma / blend_gamma / keep_alpha: mesh path -- "soft_phong" (SoftPhongShader) or
             "soft_silhouette" (SoftSilhouetteShader) blend the faces_per_pixel fragments of the blurred rasterizer (the
             shaders renderer.py:4-6 imports; SURVEY 8f N3); images keep 3 channels as renderer.py:112 unless keep_alpha.

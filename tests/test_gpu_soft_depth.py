@@ -83,9 +83,10 @@ def blend_with_decision(p2f, zbuf, dists, sigma, background, live):
 
 
 class Scene:
-    def __init__(self, oracle, c, bg=BGD):
+    def __init__(self, oracle, c, bg=BGD, meshes=None):
+        """meshes: (verts, faces) pairs to use instead of c["meshes"]' synth.make_mesh ones (c must then give the views)."""
         self.c, self.bg = c, bg
-        self.meshes = [synth.make_mesh(nf, seed) for nf, seed in c["meshes"]]
+        self.meshes = meshes or [synth.make_mesh(nf, seed) for nf, seed in c["meshes"]]
         self.B, self.M, (self.H, self.W), self.K = len(self.meshes), c["M"], c["HW"], c["K"]
         self.persp, self.cull, self.near, self.clip = c.get("persp", True), c.get("cull", False), c.get("near", False), c.get("clip")
         self.views = c.get("views") or synth.learned_spherical_views(self.B, self.M, c["meshes"][0][1] + 1)
@@ -98,7 +99,7 @@ class Scene:
         self.g = torch.randn(self.B * self.M, 1, self.H, self.W, generator=torch.Generator().manual_seed(5))
         self.z_clip = 0.5 if self.near else None
 
-    def render(self, dev, verts=None, cameras=None):
+    def render(self, dev, verts=None, cameras=None, flags=0):
         geom = ops.PackedMeshes.from_packed(self.vp.to(dev), torch.cat([f for _, f in self.meshes]).to(dev), self.nv, self.nf,
                                             vert_rgb=self.vrgb)
         Rd, Td, Cd = cameras or (torch.from_numpy(x).to(dev) for x in (self.R, self.T, self.Cc))
@@ -106,7 +107,7 @@ class Scene:
         return ops.render_meshes(geom, self.M, Rd, Td, Cd, torch.ones(1, 3, device=dev), torch.ones(3, device=dev),
                                  torch.zeros(3, device=dev), (self.H, self.W), faces_per_pixel=self.K, shader="soft_depth",
                                  blur_radius=c["blur"], sigma=c["sigma"], perspective_correct=self.persp, cull_backfaces=self.cull,
-                                 clip_barycentric_coords=self.clip, verts=verts, depth_background=self.bg)
+                                 clip_barycentric_coords=self.clip, verts=verts, depth_background=self.bg, _extra_flags=flags)
 
     def reference(self, oracle, gpu_dists):
         """fp64 autograd of render_mesh_view_soft_depth on the reference rasterizer's fragment lists, on the kernels' fp32 IEEE
