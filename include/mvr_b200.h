@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MVR_ABI_VERSION 15
+#define MVR_ABI_VERSION 16
 
 /* flags */
 #define MVR_PERSPECTIVE_CORRECT 1  /* [upstream] RasterizationSettings.perspective_correct (FoV persp.: True) */
@@ -367,6 +367,30 @@ int mvr_points_depth_backward(const float* points, int B, int Np, int M, const f
                               double radius, int H, int W, int flags, const int* idx, const uint32_t* hit_mask,
                               const float* grad_depth, float* gR, float* gT, float* g_inv_dist, float* grad_points,
                               void* workspace, size_t workspace_bytes, void* stream);
+/* Splat depth of a point cloud ([upstream] SoftDepthShader's blend with the splat weight in place of the sigmoid): over the K =
+ * points_per_pixel nearest points of a pixel, in the (z, index) order of mvr_points_forward's idx at the same K, nearest first:
+ * alpha_k = 1 - d2_k / r^2 (d2: squared NDC distance of the point's projection to the pixel centre; r^2 the double radius * radius
+ * rounded to fp32, the compositors' weight radius; not clamped), c_k = sum_{j <= k} alpha_j, m_k = min(c_k, 1);
+ * depth = sum_k (m_k - m_prev) z_k + (1 - m_last) depth_background, z_k the point's view-space z (the rasterizer's zbuf), the sum
+ * stopping after the first entry with c_k > 1.  A pixel with no point holds depth_background (any finite value, else -7).
+ * Outputs: depth (n,1,H,W) fp32, idx (n,H,W,K) (-1 empty; aligned to 4*K bytes for K = 2, 4, else -10), hit_mask (required: the
+ * backward reads it).  flags: MVR_SCALE_IS_DIST only; MVR_IMAGES_BF16, MVR_IDX_SPARSE, MVR_COMPOSITE_ALPHA and MVR_RGB_PER_ELEMENT
+ * are rejected (-11).  The workspace is mvr_points_workspace_bytes(B, Np, M, H, W, K, radius) (smaller: -8).  Every check is made
+ * before any launch. */
+int mvr_points_splat_depth_forward(const float* points, int B, int Np, int M, const float* R, const float* T,
+                                   const float* inv_dist, double radius, float depth_background, int H, int W, int K,
+                                   int flags, float* depth, int* idx, uint32_t* hit_mask,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+/* its backward, with g = grad_depth of the pixel: d/d z_k = g (m_k - m_prev); Z_stop = z of the first entry with c > 1, else
+ * depth_background; d/d alpha_j = g (z_j - Z_stop) for the entries with c_j <= 1, 0 past them; d alpha / d d2 = -1 / r^2.
+ * -> gR (n,3,3), gT (n,3), g_inv_dist (n) (d/d dist with MVR_SCALE_IS_DIST), WRITTEN (fixed-order sums: bit-reproducible, and the
+ * same with or without grad_points); grad_points (B,Np,3) or NULL, ACCUMULATED with atomics (caller zero-fills).  Arguments as the
+ * forward's, whose idx and hit_mask it reads. */
+int mvr_points_splat_depth_backward(const float* points, int B, int Np, int M, const float* R, const float* T,
+                                    const float* inv_dist, double radius, float depth_background, int H, int W, int K,
+                                    int flags, const int* idx, const uint32_t* hit_mask, const float* grad_depth,
+                                    float* gR, float* gT, float* g_inv_dist, float* grad_points,
+                                    void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

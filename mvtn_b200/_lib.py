@@ -5,7 +5,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvr_b200.so")
 
-ABI_VERSION = 15
+ABI_VERSION = 16
 PERSPECTIVE_CORRECT = 1
 CULL_BACKFACES = 2
 COMPOSITE_ALPHA = 4
@@ -84,6 +84,9 @@ SIGNATURES = {
     "mvr_points_depth_forward": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _d, _f, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mvr_points_depth_backward": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _d, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                        _sz, _vp]),
+    "mvr_points_splat_depth_forward": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _d, _f, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mvr_points_splat_depth_backward": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _d, _f, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp,
+                                             _vp, _vp, _sz, _vp]),
 }
 
 _lib = None

@@ -16,6 +16,9 @@
 //             idx / grad_images, with all threads busy: compositor backward -> d dist2 -> d ndc.xy ->
 //             (dR, dT, d(1/dist)) reduced to one partial per CTA, summed in fixed order; optional
 //             per-point / colour gradients via atomics.
+//   splat depth (mvr_points_splat_depth_*): SPLAT instances of the same forward kernels blend the K layers' z by the splat
+//             weight alpha = 1 - d2 / r2 into one depth plane (no feature loads); points_splat_backward_kernel is its adjoint,
+//             with the compaction of points_backward_kernel and the same fixed-order reduction.
 #include <cooperative_groups.h>
 #include <cstdlib>
 
@@ -38,7 +41,7 @@ struct PointsParams {
   int vec_bg;                    // W % 4 == 0 and 16-byte aligned images: the tile kernel paints the background 4 pixels per store
   void* images; int* idx; float* zbuf; float* dists2; unsigned int* hit_mask;
   OutNorm onorm;
-  float depth_bg;                // hard depth (mvr_points_depth_forward): the value of an uncovered pixel; `images` is (n,1,H,W) fp32
+  float depth_bg;                // hard / splat depth: the value of an uncovered pixel; `images` is (n,1,H,W) fp32
 };
 
 __device__ __forceinline__ void project_point(const float* __restrict__ pts, int pi, float s, const Camera& cam,
@@ -164,8 +167,8 @@ __global__ void __launch_bounds__(MVR_THREADS) points_scatter_kernel(const Point
   }
 }
 
-// A pixel no point covers: empty fragment slots and the background colour.
-template <int KT>
+// A pixel no point covers: empty fragment slots and the background colour (SPLAT: depth_bg into the one depth plane).
+template <int KT, bool SPLAT = false>
 __device__ __forceinline__ void store_background_pixel(const PointsParams& p, int n, int xi, int yi) {
   const int K = KT > 0 ? KT : p.K;
   const size_t HW = (size_t)p.H * p.W;
@@ -181,6 +184,7 @@ __device__ __forceinline__ void store_background_pixel(const PointsParams& p, in
       if (p.zbuf) p.zbuf[po + l] = -1.f;
       if (p.dists2) p.dists2[po + l] = -1.f;
     }
+  if (SPLAT) { reinterpret_cast<float*>(p.images)[(size_t)n * HW + pix] = p.depth_bg; return; }
   store_rgb(p.images, p.flags & MVR_IMAGES_BF16, (size_t)n * 3 * HW + pix, HW, __ldg(p.bg_rgb), __ldg(p.bg_rgb + 1),
             __ldg(p.bg_rgb + 2), p.onorm);
 }
@@ -190,7 +194,10 @@ __device__ __forceinline__ void store_background_pixel(const PointsParams& p, in
 // image stores.
 // PP: the view's projected points are in the workspace (tiled path: p.pp, written by the binning kernel with the very
 // project_point below, so the values are the same bits) -- one 16-byte load instead of three loads and the transform.
-template <int KT, bool PP = false>
+// SPLAT (splat depth, no features): over the layers nearest first c_k = sum_{j <= k} alpha_j, m_k = min(c_k, 1);
+// depth = sum_k (m_k - m_prev) z_k + (1 - m_last) depth_bg into the one plane `images`, the blend stopping after the first
+// c > 1 (every later weight is 0); alpha is not clamped.  idx is written for every layer.
+template <int KT, bool PP = false, bool SPLAT = false>
 __device__ __forceinline__ void composite_hit_pixel(const PointsParams& p, const unsigned long long* kreg,
                                                     const unsigned long long* kp, const Camera& cam, float s, int b, int n,
                                                     int xi, int yi) {
@@ -207,6 +214,8 @@ __device__ __forceinline__ void composite_hit_pixel(const PointsParams& p, const
   float a0 = 0.f, a1 = 0.f, a2 = 0.f, aw = alpha_mode ? 1.f : 0.f;
   int ids[KT > 0 ? KT : 1];
   bool open = true;      // layers are contiguous: the first EMPTY key ends them
+  float sc = 0.f, sm = 0.f, sd = 0.f;      // SPLAT: running alpha sum, its clamp at the previous layer, the blended depth
+  bool live = true;                        // SPLAT: no layer so far has taken c past 1
 #pragma unroll
   for (int l = 0; l < K; ++l) {
     const unsigned long long key = KT > 0 ? kreg[KT > 0 ? l : 0] : kp[l];
@@ -222,15 +231,25 @@ __device__ __forceinline__ void composite_hit_pixel(const PointsParams& p, const
       d2 = dx * dx + dy * dy;
       z = __uint_as_float((unsigned int)(key >> 32));
       const float a = 1.f - d2 / p.r2_weight;
-      const float* f = feat + (per_point_rgb ? 3 * (size_t)q : 0);
-      const float f0 = __ldg(f), f1 = __ldg(f + 1), f2 = __ldg(f + 2);
-      if (alpha_mode) {   // out += cum * alpha * f ; cum *= (1 - alpha)
-        const float ca = aw * a;
-        a0 += ca * f0; a1 += ca * f1; a2 += ca * f2;
-        aw = aw * (1.f - a);
-      } else {            // numerators and the alpha sum
-        a0 += a * f0; a1 += a * f1; a2 += a * f2;
-        aw += a;
+      if (SPLAT) {
+        if (live) {
+          sc += a;
+          const float m = fminf(sc, 1.0f);
+          sd += (m - sm) * z;
+          sm = m;
+          live = !(sc > 1.0f);
+        }
+      } else {
+        const float* f = feat + (per_point_rgb ? 3 * (size_t)q : 0);
+        const float f0 = __ldg(f), f1 = __ldg(f + 1), f2 = __ldg(f + 2);
+        if (alpha_mode) {   // out += cum * alpha * f ; cum *= (1 - alpha)
+          const float ca = aw * a;
+          a0 += ca * f0; a1 += ca * f1; a2 += ca * f2;
+          aw = aw * (1.f - a);
+        } else {            // numerators and the alpha sum
+          a0 += a * f0; a1 += a * f1; a2 += a * f2;
+          aw += a;
+        }
       }
     }
     if (KT == 4) ids[KT > 0 ? l : 0] = q; else p.idx[po + l] = q;
@@ -238,6 +257,7 @@ __device__ __forceinline__ void composite_hit_pixel(const PointsParams& p, const
     if (p.dists2) p.dists2[po + l] = d2;
   }
   if (KT == 4) *reinterpret_cast<int4*>(p.idx + po) = make_int4(ids[0], ids[KT > 1 ? 1 : 0], ids[KT > 2 ? 2 : 0], ids[KT > 3 ? 3 : 0]);
+  if (SPLAT) { reinterpret_cast<float*>(p.images)[(size_t)n * HW + pix] = sd + (1.0f - sm) * p.depth_bg; return; }
   float o0 = a0, o1 = a1, o2 = a2;
   if (!alpha_mode) { const float t = fmaxf(aw, 1e-4f); o0 = a0 / t; o1 = a1 / t; o2 = a2 / t; }
   store_rgb(p.images, p.flags & MVR_IMAGES_BF16, (size_t)n * 3 * HW + pix, HW, o0, o1, o2, p.onorm);
@@ -245,7 +265,7 @@ __device__ __forceinline__ void composite_hit_pixel(const PointsParams& p, const
 
 // Everything that happens to ONE pixel once its K ascending keys are known: hit-mask bit (warp ballot: call with all
 // 32 lanes, lane = x within a 32-pixel row word `mask_word`), then the background or the composited pixel.
-template <int KT>
+template <int KT, bool SPLAT = false>
 __device__ __forceinline__ void composite_and_store(const PointsParams& p, const unsigned long long* kreg,
                                                     const unsigned long long* kp, int b, int n, int xi, int yi,
                                                     int mask_word, bool inside) {
@@ -256,13 +276,14 @@ __device__ __forceinline__ void composite_and_store(const PointsParams& p, const
     if ((threadIdx.x & 31) == 0 && yi < p.H) p.hit_mask[((size_t)n * p.H + yi) * p.mask_words + mask_word] = mword;
   }
   if (!inside) return;
-  if (!hit) { store_background_pixel<KT>(p, n, xi, yi); return; }
+  if (!hit) { store_background_pixel<KT, SPLAT>(p, n, xi, yi); return; }
   const Camera cam = load_camera(p.R, p.T, n);
-  composite_hit_pixel<KT>(p, kreg, kp, cam, view_scale(p.inv_dist, p.flags, n), b, n, xi, yi);
+  composite_hit_pixel<KT, false, SPLAT>(p, kreg, kp, cam, view_scale(p.inv_dist, p.flags, n), b, n, xi, yi);
 }
 
 // grid: x = 32x8-pixel tiles, y = view m, z = object b.  KT = K when K <= PK_MAX_REG (keys in registers), 0 = generic
-template <int KT>
+// SPLAT: splat depth (see composite_hit_pixel)
+template <int KT, bool SPLAT = false>
 __global__ void __launch_bounds__(MVR_THREADS) points_resolve_kernel(const PointsParams p, int tiles_x) {
   const int b = blockIdx.z, n = b * p.M + blockIdx.y;
   const int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
@@ -289,7 +310,7 @@ __global__ void __launch_bounds__(MVR_THREADS) points_resolve_kernel(const Point
       for (int l = 0; l < KT; ++l) kreg[l] = kp[l];
     }
   }
-  composite_and_store<KT>(p, kreg, kp, b, n, xi, yi, tx, inside);
+  composite_and_store<KT, SPLAT>(p, kreg, kp, b, n, xi, yi, tx, inside);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -479,7 +500,9 @@ __device__ __forceinline__ void insert_key_smem(unsigned long long* s_keys, int 
 // MINB: minimum CTAs per SM for the register allocator; 0 = unconstrained
 // DEPTH (KT = 1, no zbuf / dists2): the nearest point's z -- the key's -- or p.depth_bg into the (n,1,H,W) plane `images`, idx and
 // the hit mask; no compositing.
-template <int KT, int MINB, bool DEPTH = false>
+// SPLAT: splat depth -- idx of every layer, the hit mask and the alpha blend of the layers' z (composite_hit_pixel) or p.depth_bg
+// into the (n,1,H,W) plane `images`; no feature loads.
+template <int KT, int MINB, bool DEPTH = false, bool SPLAT = false>
 __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const PointsParams p) {
   pdl_enter();
   extern __shared__ unsigned long long s_keys[];              // [KT][1024]
@@ -589,9 +612,10 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
     unsigned int* mask_v = p.hit_mask ? p.hit_mask + (size_t)n * p.H * p.mask_words + tx : nullptr;
     const bool bf16 = p.flags & MVR_IMAGES_BF16;
     const bool sparse_idx = (p.flags & MVR_IDX_SPARSE) && mask_v;
-    float* img_f = reinterpret_cast<float*>(p.images) + (size_t)n * (DEPTH ? 1 : 3) * HW;
+    float* img_f = reinterpret_cast<float*>(p.images) + (size_t)n * (DEPTH || SPLAT ? 1 : 3) * HW;
     __nv_bfloat16* img_h = reinterpret_cast<__nv_bfloat16*>(p.images) + (size_t)n * 3 * HW;
-    float g0 = DEPTH ? p.depth_bg : __ldg(p.bg_rgb), g1 = DEPTH ? 0.f : __ldg(p.bg_rgb + 1), g2 = DEPTH ? 0.f : __ldg(p.bg_rgb + 2);
+    float g0 = DEPTH || SPLAT ? p.depth_bg : __ldg(p.bg_rgb), g1 = DEPTH || SPLAT ? 0.f : __ldg(p.bg_rgb + 1),
+          g2 = DEPTH || SPLAT ? 0.f : __ldg(p.bg_rgb + 2);
     if (p.onorm.on) { g0 = (g0 - p.onorm.m0) * p.onorm.s0; g1 = (g1 - p.onorm.m1) * p.onorm.s1; g2 = (g2 - p.onorm.m2) * p.onorm.s2; }
     const __nv_bfloat16 h0 = __float2bfloat16_rn(g0), h1 = __float2bfloat16_rn(g1), h2 = __float2bfloat16_rn(g2);
     const int hw = (int)HW, xi = x0 + lane;
@@ -601,7 +625,7 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
       const int yv = y0 + (tid >> 3), xv = x0 + ((tid & 7) << 2);
       if (yv < p.H && xv < p.W) {
         const int pv = yv * p.W + xv;
-        if (DEPTH) {
+        if (DEPTH || SPLAT) {
           *reinterpret_cast<float4*>(img_f + pv) = make_float4(g0, g0, g0, g0);
         } else if (bf16) {
           const unsigned int u0 = __bfloat16_as_ushort(h0), u1 = __bfloat16_as_ushort(h1), u2 = __bfloat16_as_ushort(h2);
@@ -649,7 +673,7 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
           for (int l = 0; l < KT; ++l) p.dists2[frag_o + KT * pix + l] = -1.f;
         }
         if (!p.vec_bg) {
-          if (DEPTH) img_f[pix] = g0;
+          if (DEPTH || SPLAT) img_f[pix] = g0;
           else if (bf16) { img_h[pix] = h0; img_h[pix + hw] = h1; img_h[pix + 2 * hw] = h2; }
           else { img_f[pix] = g0; img_f[pix + hw] = g1; img_f[pix + 2 * hw] = g2; }
         }
@@ -676,7 +700,7 @@ __global__ void __launch_bounds__(MVR_THREADS, MINB) points_tile_kernel(const Po
       unsigned long long kreg[KT];
 #pragma unroll
       for (int k = 0; k < KT; ++k) kreg[k] = s_keys[k * 1024 + q];
-      composite_hit_pixel<KT, true>(p, kreg, nullptr, cam, s, b, n, x0 + (q & 31), y0 + (q >> 5));
+      composite_hit_pixel<KT, true, SPLAT>(p, kreg, nullptr, cam, s, b, n, x0 + (q & 31), y0 + (q >> 5));
     }
   }
 }
@@ -691,6 +715,7 @@ struct PointsBwdParams {
   float* partials;        // (N, ctas_per_view, 16): one per 32x32 tile
   float* grad_points; float* grad_rgb;
   OutNorm onorm;
+  float depth_bg;         // splat depth: the background of the blend
 };
 
 // (dR, dT, d scale) contributions of one fragment layer whose d out / d alpha is `ga`
@@ -981,6 +1006,181 @@ __global__ void __launch_bounds__(MVR_THREADS) points_depth_backward_kernel(cons
   }
 }
 
+// One splat-depth layer: d/d alpha = ga -> d/d (px, py) as points_backward_layer, d/d z = gz as points_depth_backward_kernel, taken
+// together as dp = (gpx, gpy, gz) on p_view = (s X) R + T: dR[i][j] += s X_i dp_j, dT += dp, d s += X . (R dp), dX += s R dp (three
+// atomics per layer instead of six).
+__device__ __forceinline__ void points_splat_layer(const PointsBwdParams& p, const Camera& cam, float s, float inv_r2, int b, int pid,
+                                                   float X0, float X1, float X2, float dx, float dy, float ga, float gz, float (&acc)[16]) {
+  const float gd2 = -ga * inv_r2;
+  const float gpx = 2.f * gd2 * dx, gpy = 2.f * gd2 * dy;
+  const float Xs0 = X0 * s, Xs1 = X1 * s, Xs2 = X2 * s;
+  acc[0] = fmaf(Xs0, gpx, acc[0]); acc[1] = fmaf(Xs0, gpy, acc[1]); acc[2] = fmaf(Xs0, gz, acc[2]);
+  acc[3] = fmaf(Xs1, gpx, acc[3]); acc[4] = fmaf(Xs1, gpy, acc[4]); acc[5] = fmaf(Xs1, gz, acc[5]);
+  acc[6] = fmaf(Xs2, gpx, acc[6]); acc[7] = fmaf(Xs2, gpy, acc[7]); acc[8] = fmaf(Xs2, gz, acc[8]);
+  acc[9] += gpx; acc[10] += gpy; acc[11] += gz;
+  const float gx0 = cam.r[0] * gpx + cam.r[1] * gpy + cam.r[2] * gz, gx1 = cam.r[3] * gpx + cam.r[4] * gpy + cam.r[5] * gz,
+              gx2 = cam.r[6] * gpx + cam.r[7] * gpy + cam.r[8] * gz;
+  acc[12] += gx0 * X0 + gx1 * X1 + gx2 * X2;
+  if (p.grad_points) {
+    float* o = p.grad_points + 3 * ((size_t)b * p.Np + pid);
+    atomicAdd(o, gx0 * s); atomicAdd(o + 1, gx1 * s); atomicAdd(o + 2, gx2 * s);
+  }
+}
+
+// Splat depth backward.  Grid, covered-pixel compaction (from the hit mask) and partials as points_backward_kernel.  Per pixel, with
+// g = d loss / d depth: pass 1 finds Z_stop = z of the first layer whose running alpha sum c passes 1, else depth_bg; pass 2 gives
+// each layer d/d z_k = g (m_k - m_prev) and d/d alpha_k = g (z_k - Z_stop) while c_k <= 1 (torch's clamp passes the gradient at
+// c = 1), 0 past it, and stops after the layer that took c past 1, as the forward does.  The layers' z and alpha are recomputed
+// with the forward's fp32 arithmetic (the same bits), so both passes take the forward's decisions.  KT in {1, 2, 4}: the layers stay
+// in registers between the passes; KT = 0 serves any K with the layers re-read and re-projected.
+template <int KT>
+__global__ void __launch_bounds__(MVR_THREADS) points_splat_backward_kernel(const PointsBwdParams p) {
+  constexpr int NW = MVR_THREADS / 32;               // warps (= tiles of a column) per CTA
+  __shared__ unsigned short s_list[NW * 1024];       // warp << 10 | row << 5 | x of every covered pixel of the CTA's tiles
+  __shared__ int s_wtot[NW];
+  __shared__ float s_part[NW][16];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.z, n = b * p.M + blockIdx.y;
+  const int tgy = blockIdx.x / p.tiles_x, txb = blockIdx.x - tgy * p.tiles_x;
+  const int tyb = tgy * NW + warp;
+  const float* pts = p.points + 3 * (size_t)b * p.Np;
+  const float* gd = reinterpret_cast<const float*>(p.grad_images);
+  // ---- covered pixels of row (tile row * 32 + lane), compacted into s_list ----
+  unsigned int word = 0u;
+  if (tyb < p.tiles_y && tyb * 32 + lane < p.H) word = __ldg(p.hit_mask + ((size_t)n * p.H + tyb * 32 + lane) * p.mask_words + txb);
+  const int cnt = __popc(word);
+  int pre = cnt;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, pre, o);
+    if (lane >= o) pre += v;
+  }
+  if (lane == 31) s_wtot[warp] = pre;
+  __syncthreads();
+  int base = 0, total = 0;
+  for (int w = 0; w < NW; ++w) { const int c = s_wtot[w]; if (w < warp) base += c; total += c; }
+  float* out = p.partials + ((size_t)n * p.ctas_per_view + blockIdx.x) * 16;
+  if (total == 0) {                                  // background only (block-uniform)
+    if (tid < 16) out[tid] = 0.f;
+    return;
+  }
+  {
+    int at = base + pre - cnt;
+    unsigned int wv = word;
+    while (wv) {
+      const int x = __ffs(wv) - 1;
+      wv &= wv - 1u;
+      s_list[at++] = (unsigned short)((warp << 10) | (lane << 5) | x);
+    }
+  }
+  __syncthreads();
+  float acc[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  const Camera cam = load_camera(p.R, p.T, n);
+  const float s = view_scale(p.inv_dist, p.flags, n);
+  const float inv_r2 = 1.f / p.r2_weight;
+  constexpr int KR = KT > 0 ? KT : 1;
+  auto pixel_of = [&](int i, int& xi, int& yi) {
+    const int code = s_list[i];
+    yi = (tgy * NW + (code >> 10)) * 32 + ((code >> 5) & 31); xi = txb * 32 + (code & 31);
+  };
+  // the pixel's K point ids (one vector load) and its cotangent, fetched one iteration ahead
+  auto fetch = [&](int i, int (&pid)[KR], float& g) {
+    int xi, yi; pixel_of(i, xi, yi);
+    const size_t pix = ((size_t)n * p.H + yi) * p.W + xi;
+    if (KT == 4) { const int4 v = __ldg(reinterpret_cast<const int4*>(p.idx) + pix); pid[0] = v.x; pid[1 % KR] = v.y; pid[2 % KR] = v.z; pid[3 % KR] = v.w; }
+    else if (KT == 2) { const int2 v = __ldg(reinterpret_cast<const int2*>(p.idx) + pix); pid[0] = v.x; pid[1 % KR] = v.y; }
+    else if (KT == 1) pid[0] = __ldg(p.idx + pix);
+    g = __ldg(gd + pix);
+  };
+  int pid_n[KR] = {}; float g_n = 0.f;
+  if (tid < total) fetch(tid, pid_n, g_n);
+  for (int it = tid; it < total; it += MVR_THREADS) {
+    int pid[KR];
+#pragma unroll
+    for (int k = 0; k < KR; ++k) pid[k] = pid_n[k];
+    const float g = g_n;
+    int xi, yi; pixel_of(it, xi, yi);
+    if (it + MVR_THREADS < total) fetch(it + MVR_THREADS, pid_n, g_n);
+    if (g == 0.f) continue;
+    const float xf = pix_to_ndc(p.W - 1 - xi, p.W, p.H), yf = pix_to_ndc(p.H - 1 - yi, p.H, p.W);
+    if (KT > 0) {
+      int nk = 0;
+#pragma unroll
+      for (int k = 0; k < KR; ++k) if (nk == k && pid[k] >= 0) nk = k + 1;      // the filled slots are a prefix
+      float X[KR][3], z[KR], a[KR], dx[KR], dy[KR];
+#pragma unroll
+      for (int k = 0; k < KR; ++k) {
+        const size_t q = k < nk ? (size_t)pid[k] : 0;      // (slot 0 is filled: the pixel is covered)
+        X[k][0] = __ldg(pts + 3 * q); X[k][1] = __ldg(pts + 3 * q + 1); X[k][2] = __ldg(pts + 3 * q + 2);
+      }
+      float zstop = p.depth_bg, c = 0.f;
+      bool live = true;
+#pragma unroll
+      for (int k = 0; k < KR; ++k) {
+        float px, py; world_to_view(cam, X[k][0] * s, X[k][1] * s, X[k][2] * s, px, py, z[k]);
+        dx[k] = px - xf; dy[k] = py - yf;
+        a[k] = 1.f - (dx[k] * dx[k] + dy[k] * dy[k]) / p.r2_weight;      // exactly the forward's alpha
+        if (live && k < nk) {
+          c += a[k];
+          if (c > 1.0f) { zstop = z[k]; live = false; }
+        }
+      }
+      float mprev = 0.f;
+      c = 0.f;
+#pragma unroll
+      for (int k = 0; k < KR; ++k) {
+        if (k < nk) {
+          c += a[k];
+          const float mk = fminf(c, 1.0f);
+          const float gz = g * (mk - mprev);
+          mprev = mk;
+          const float ga = c <= 1.0f ? g * (z[k] - zstop) : 0.f;
+          points_splat_layer(p, cam, s, inv_r2, b, pid[k], X[k][0], X[k][1], X[k][2], dx[k], dy[k], ga, gz, acc);
+          if (c > 1.0f) break;
+        }
+      }
+    } else {
+      const int* ip = p.idx + (((size_t)n * p.H + yi) * p.W + xi) * p.K;
+      float zstop = p.depth_bg, c = 0.f;
+      for (int k = 0; k < p.K; ++k) {
+        const int q = __ldg(ip + k);
+        if (q < 0) break;
+        float px, py, pz; project_point(pts, q, s, cam, px, py, pz);
+        const float ddx = px - xf, ddy = py - yf;
+        c += 1.f - (ddx * ddx + ddy * ddy) / p.r2_weight;
+        if (c > 1.0f) { zstop = pz; break; }
+      }
+      float mprev = 0.f;
+      c = 0.f;
+      for (int k = 0; k < p.K; ++k) {
+        const int q = __ldg(ip + k);
+        if (q < 0) break;
+        const float X0 = __ldg(pts + 3 * (size_t)q), X1 = __ldg(pts + 3 * (size_t)q + 1), X2 = __ldg(pts + 3 * (size_t)q + 2);
+        float px, py, pz; world_to_view(cam, X0 * s, X1 * s, X2 * s, px, py, pz);
+        const float ddx = px - xf, ddy = py - yf;
+        c += 1.f - (ddx * ddx + ddy * ddy) / p.r2_weight;
+        const float mk = fminf(c, 1.0f);
+        const float gz = g * (mk - mprev);
+        mprev = mk;
+        const float ga = c <= 1.0f ? g * (pz - zstop) : 0.f;
+        points_splat_layer(p, cam, s, inv_r2, b, q, X0, X1, X2, ddx, ddy, ga, gz, acc);
+        if (c > 1.0f) break;
+      }
+    }
+  }
+  // one partial per CTA: warp totals, then the warps in fixed order; the reduce kernel sums the CTAs in fixed order
+  const float mine = warp_sum16_transposed(acc);
+  if (!(lane & 1)) s_part[warp][lane >> 1] = mine;
+  __syncthreads();
+  if (tid < 16) {
+    float v = 0.f;
+    for (int w = 0; w < NW; ++w) v += s_part[w][tid];
+    out[tid] = v;
+  }
+}
+
 // grad_rgb_uniform: the (3,) gradient of the single point colour, or NULL (per-point colours / not wanted)
 __global__ void points_backward_reduce_kernel(const float* __restrict__ partials, int N, int n_parts,
                                               float* __restrict__ gR, float* __restrict__ gT, float* __restrict__ gs,
@@ -1035,6 +1235,12 @@ __global__ void points_backward_reduce_angles_kernel(const float* __restrict__ p
     g_azim[n] = ga; g_elev[n] = ge; g_dist[n] = gd + (-g[12] * (inv * inv));
   }
 }
+
+// The splat-depth forward instances, under names of their own: the launch profiler matches the spelling at the launch site by prefix,
+// and "points_tile_kernel<4," or "points_resolve_kernel<0>" name the colour instances.
+template <int KT, int MINB>
+constexpr void (*points_splat_tile_kernel)(const PointsParams) = points_tile_kernel<KT, MINB, false, true>;
+constexpr void (*points_splat_resolve_kernel)(const PointsParams, int) = points_resolve_kernel<0, true>;
 
 }  // namespace mvr
 
@@ -1367,4 +1573,120 @@ extern "C" int mvr_points_backward_angles(const float* points, const float* rgb,
   if (!azim) { set_error("mvr_points_backward_angles: null pointer"); return -6; }
   return points_backward_impl(points, rgb, B, Np, M, R, T, dist, radius, H, W, K, flags, out_mean_std, idx, hit_mask, grad_images, gR, gT,
                               nullptr, grad_points, grad_rgb, workspace, workspace_bytes, stream, azim, elev, g_azim, g_elev, g_dist);
+}
+
+// Splat depth: the K nearest points of mvr_points_forward blended by their splat weight (see composite_hit_pixel); binning as
+// mvr_points_forward, then the SPLAT tile kernel (K in {1, 2, 4, 8}) or the global key plane and the SPLAT resolve kernel.
+extern "C" int mvr_points_splat_depth_forward(const float* points, int B, int Np, int M, const float* R, const float* T,
+                                              const float* inv_dist, double radius, float depth_background, int H, int W, int K,
+                                              int flags, float* depth, int* idx, uint32_t* hit_mask, void* workspace,
+                                              size_t workspace_bytes, void* stream) {
+  const char* who = "mvr_points_splat_depth_forward";
+  int rc = check_points_common(who, B, Np, M, H, W, K, radius);
+  if (rc) return rc;
+  const int64_t N = (int64_t)B * M;
+  if (N == 0) return 0;
+  if ((Np > 0 && !points) || !R || !T || !inv_dist || !depth || !idx || !hit_mask || !workspace) { set_error("%s: null pointer", who); return -6; }
+  if (flags & (MVR_IMAGES_BF16 | MVR_IDX_SPARSE | MVR_COMPOSITE_ALPHA | MVR_RGB_PER_ELEMENT)) {
+    set_error("%s: the depth is fp32, idx dense and there is no colour: flags take MVR_SCALE_IS_DIST only", who); return -11;
+  }
+  if (!isfinite(depth_background)) { set_error("%s: depth_background must be finite", who); return -7; }
+  if ((K == 2 || K == 4) && ((uintptr_t)idx & (uintptr_t)(4 * K - 1))) { set_error("%s: idx must be aligned to 4*K = %d bytes", who, 4 * K); return -10; }
+  const PointsWs w = points_ws(B, Np, M, H, W, K, radius);
+  if (workspace_bytes < w.total) { set_error("%s: workspace too small (%zu < %zu)", who, workspace_bytes, w.total); return -8; }
+  if (w.tiled && Np > 0 && (long long)w.list_cap >= 0x7fffffffLL) { set_error("%s: point lists too large", who); return -12; }
+  char* wb = (char*)workspace;
+  PointsParams p = {};
+  p.points = points; p.R = R; p.T = T; p.inv_dist = inv_dist;
+  p.radius = (float)radius;
+  p.r2_raster = p.radius * p.radius;
+  p.r2_weight = (float)(radius * radius);
+  p.B = B; p.Np = Np; p.M = M; p.H = H; p.W = W; p.K = K; p.flags = flags & MVR_SCALE_IS_DIST; p.mask_words = w.mask_words;
+  p.keys = (unsigned long long*)(wb + w.keys);
+  p.tab = (const float*)(wb + w.tab);
+  p.pp = (float4*)(wb + w.pp); p.pw = (int2*)(wb + w.pw);
+  p.tile_cnt = (int*)(wb + w.tile_cnt); p.tile_off = (int*)(wb + w.tile_off); p.tile_cur = (int*)(wb + w.tile_cur);
+  p.list = (int*)(wb + w.list);
+  p.tiles_x = w.tiles_x; p.tiles_y = w.tiles_y; p.ntiles = w.ntiles; p.list_cap = w.list_cap;
+  p.vec_bg = (W % 4 == 0) && ((uintptr_t)depth % 16 == 0);
+  p.images = depth; p.idx = idx; p.hit_mask = hit_mask;
+  p.depth_bg = depth_background;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (w.tiled) {
+    rc = launch_points_binning(p, w, wb, st);
+    if (rc) return rc;
+    const dim3 tile_grid((unsigned)w.ntiles, (unsigned)M, (unsigned)B);
+    const size_t smem = (size_t)K * 1024 * sizeof(unsigned long long);
+    switch (K) {      // MINB as the colour instances (see mvr_points_forward)
+      case 1: MVR_LAUNCH_PDL((points_splat_tile_kernel<1, 0>), tile_grid, MVR_THREADS, smem, st, p); break;
+      case 2: MVR_LAUNCH_PDL((points_splat_tile_kernel<2, 0>), tile_grid, MVR_THREADS, smem, st, p); break;
+      case 4: MVR_LAUNCH_PDL((points_splat_tile_kernel<4, 5>), tile_grid, MVR_THREADS, smem, st, p); break;
+      default: {
+        const cudaError_t e = cudaFuncSetAttribute(points_splat_tile_kernel<8, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e)); return (int)e; }
+        MVR_LAUNCH_PDL((points_splat_tile_kernel<8, 3>), tile_grid, MVR_THREADS, smem, st, p);
+      }
+    }
+    return check_launch("points_splat_tile_kernel");
+  }
+  if (Np > 0) MVR_LAUNCH(pixel_table_kernel, 1, MVR_THREADS, 0, st, (float*)(wb + w.tab), H, W);
+  const cudaError_t e = cudaMemsetAsync(p.keys, 0xFF, (size_t)N * H * W * K * 8, st);      // every key = EMPTY
+  if (e != cudaSuccess) { set_error("%s: cudaMemsetAsync: %s", who, cudaGetErrorString(e)); return (int)e; }
+  if (Np > 0) {
+    const dim3 point_grid((unsigned)((Np + MVR_THREADS - 1) / MVR_THREADS), (unsigned)M, (unsigned)B);
+    MVR_LAUNCH(points_scatter_kernel, point_grid, MVR_THREADS, 0, st, p);
+    rc = check_launch("points_scatter_kernel");
+    if (rc) return rc;
+  }
+  const int tiles_x = (W + 31) / 32, tiles_y = (H + 7) / 8;
+  MVR_LAUNCH(points_splat_resolve_kernel, dim3((unsigned)(tiles_x * tiles_y), (unsigned)M, (unsigned)B), MVR_THREADS, 0, st, p, tiles_x);
+  return check_launch("points_splat_resolve_kernel");
+}
+
+extern "C" int mvr_points_splat_depth_backward(const float* points, int B, int Np, int M, const float* R, const float* T,
+                                               const float* inv_dist, double radius, float depth_background, int H, int W, int K,
+                                               int flags, const int* idx, const uint32_t* hit_mask, const float* grad_depth,
+                                               float* gR, float* gT, float* g_inv_dist, float* grad_points, void* workspace,
+                                               size_t workspace_bytes, void* stream) {
+  const char* who = "mvr_points_splat_depth_backward";
+  int rc = check_points_common(who, B, Np, M, H, W, K, radius);
+  if (rc) return rc;
+  const int64_t N = (int64_t)B * M;
+  if (N == 0) return 0;
+  if ((Np > 0 && !points) || !R || !T || !inv_dist || !idx || !hit_mask || !grad_depth || !gR || !gT || !g_inv_dist || !workspace) {
+    set_error("%s: null pointer", who); return -6;
+  }
+  if (flags & (MVR_IMAGES_BF16 | MVR_IDX_SPARSE | MVR_COMPOSITE_ALPHA | MVR_RGB_PER_ELEMENT)) {
+    set_error("%s: the depth is fp32, idx dense and there is no colour: flags take MVR_SCALE_IS_DIST only", who); return -11;
+  }
+  if (!isfinite(depth_background)) { set_error("%s: depth_background must be finite", who); return -7; }
+  const PointsWs w = points_ws(B, Np, M, H, W, K, radius);
+  const size_t need = (size_t)N * w.ctas_per_view * 16 * sizeof(float);
+  if (workspace_bytes < need) { set_error("%s: workspace too small (%zu < %zu)", who, workspace_bytes, need); return -8; }
+  PointsBwdParams p = {};
+  p.points = points; p.R = R; p.T = T; p.inv_dist = inv_dist;
+  p.r2_weight = (float)(radius * radius);
+  p.B = B; p.Np = Np; p.M = M; p.H = H; p.W = W; p.K = K; p.flags = flags & MVR_SCALE_IS_DIST;
+  p.tiles_x = w.tiles_x; p.tiles_y = w.tiles_y; p.mask_words = w.mask_words;
+  p.idx = idx; p.grad_images = grad_depth; p.hit_mask = hit_mask;
+  p.partials = (float*)((char*)workspace + w.partials);
+  p.grad_points = grad_points;
+  p.depth_bg = depth_background;
+  cudaStream_t st = (cudaStream_t)stream;
+  p.ctas_per_view = w.tiles_x * ((p.tiles_y + MVR_THREADS / 32 - 1) / (MVR_THREADS / 32));      // one CTA per column of 8 tiles
+  const dim3 grid((unsigned)p.ctas_per_view, (unsigned)M, (unsigned)B);
+  // the register-resident variants read a pixel's K ids as one vector: they need idx aligned to K ints
+  const int kt = ((K == 1 || K == 2 || K == 4) && ((uintptr_t)idx & (size_t)(4 * K - 1)) == 0) ? K : 0;
+  switch (kt) {
+    case 1: MVR_LAUNCH((points_splat_backward_kernel<1>), grid, MVR_THREADS, 0, st, p); break;
+    case 2: MVR_LAUNCH((points_splat_backward_kernel<2>), grid, MVR_THREADS, 0, st, p); break;
+    case 4: MVR_LAUNCH((points_splat_backward_kernel<4>), grid, MVR_THREADS, 0, st, p); break;
+    default: MVR_LAUNCH((points_splat_backward_kernel<0>), grid, MVR_THREADS, 0, st, p); break;
+  }
+  rc = check_launch("points_splat_backward_kernel");
+  if (rc) return rc;
+  const int wpb = 8;
+  MVR_LAUNCH_PDL(points_backward_reduce_kernel, (unsigned)((N + wpb - 1) / wpb), wpb * 32, 0, st, (const float*)p.partials, (int)N,
+                 p.ctas_per_view, gR, gT, g_inv_dist, inv_dist, p.flags, (float*)nullptr);
+  return check_launch("points_backward_reduce_kernel");
 }

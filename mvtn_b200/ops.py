@@ -1438,6 +1438,68 @@ class _PointsDepth(torch.autograd.Function):
         return (gR, gT, gs.reshape(scale_shape), None if gP is None else gP.reshape(points_shape)) + (None,) * 6
 
 
+class _PointsSplatDepth(torch.autograd.Function):
+    """Splat depth of point clouds as one autograd node: (R, T, scale, points) -> depth (n,1,H,W), idx (n,H,W,K).  Over the K nearest
+    points of a pixel (mvr_points_forward's idx at the same K), nearest first, alpha_k = 1 - d2_k / r^2 is cumulated and clamped
+    at 1, each z_k is weighted by the step of that clamped sum and depth_background by what is left ([upstream] SoftDepthShader's
+    blend with the splat weight in place of the sigmoid).  Differentiable w.r.t. R, T, the scale (1 / dist, or dist itself under
+    SCALE_IS_DIST) and `points`, across splat edges."""
+
+    @staticmethod
+    def forward(ctx, R, T, scale, points, M, radius, H, W, K, flags, depth_background):
+        lib = L.load()
+        _require_cuda(points, "points")
+        dev = points.device
+        pts = _f32c(points)
+        if pts.dim() != 3 or pts.shape[2] != 3:
+            raise ValueError("points must be (B,N,3)")
+        B, Np, _ = pts.shape
+        N = B * M
+        R, T, sc = _f32c(R), _f32c(T), _f32c(scale).reshape(-1)
+        if R.shape[0] != N or sc.numel() != N:
+            raise ValueError(f"expected {N} cameras (B*M)")
+        depth = torch.empty((N, 1, H, W), dtype=torch.float32, device=dev)
+        idx = torch.empty((N, H, W, K), dtype=torch.int32, device=dev)
+        mask = torch.empty(max(lib.mvr_points_hit_mask_words(B, M, H, W), 1), dtype=torch.int32, device=dev)
+        ws = workspace(dev, lib.mvr_points_workspace_bytes(B, Np, M, H, W, K, float(radius)))
+        with _on(dev):
+            L.check(lib.mvr_points_splat_depth_forward(_ptr(pts), B, Np, M, _ptr(R), _ptr(T), _ptr(sc), float(radius),
+                                                       depth_background, H, W, K, flags, _ptr(depth), _ptr(idx), _ptr(mask),
+                                                       _ptr(ws), ws.numel(), _stream(dev)), "mvr_points_splat_depth_forward")
+        ctx.set_materialize_grads(False)
+        ctx.cfg = (B, Np, M, float(radius), H, W, K, flags, depth_background, scale.shape, points.shape)
+        ctx.save_for_backward(R, T, sc, pts, idx, mask)
+        ctx.mark_non_differentiable(idx)
+        return depth, idx
+
+    @staticmethod
+    def backward(ctx, g_depth, *_unused):
+        if g_depth is None:
+            return (None,) * 11
+        lib = L.load()
+        R, T, sc, pts, idx, mask = ctx.saved_tensors
+        B, Np, M, radius, H, W, K, flags, depth_background, scale_shape, points_shape = ctx.cfg
+        dev = pts.device
+        N = B * M
+        g_depth = _f32c(g_depth)
+        g = torch.empty(13 * N, dtype=torch.float32, device=dev)
+        gR, gT, gs = g[: 9 * N].view(N, 3, 3), g[9 * N: 12 * N].view(N, 3), g[12 * N:]
+        gP = torch.zeros_like(pts) if ctx.needs_input_grad[3] else None
+        ws = workspace(dev, lib.mvr_points_workspace_bytes(B, Np, M, H, W, K, radius))
+        with _on(dev):
+            L.check(lib.mvr_points_splat_depth_backward(_ptr(pts), B, Np, M, _ptr(R), _ptr(T), _ptr(sc), radius, depth_background,
+                                                        H, W, K, flags, _ptr(idx), _ptr(mask), _ptr(g_depth), _ptr(gR), _ptr(gT),
+                                                        _ptr(gs), _ptr(gP), _ptr(ws), ws.numel(), _stream(dev)),
+                    "mvr_points_splat_depth_backward")
+        return (gR, gT, gs.reshape(scale_shape), None if gP is None else gP.reshape(points_shape)) + (None,) * 7
+
+
+def _check_splat_depth_options(normalize, out_dtype, keep_alpha=False):
+    if normalize is not None or out_dtype not in (None, torch.float32) or keep_alpha:
+        raise ValueError("shader='splat_depth' returns one fp32 depth channel: normalize / out_dtype / keep_alpha are not supported "
+                         "with it")
+
+
 def render_points_from_angles(points, rgb, M: int, azim, elev, dist, radius: float, bg_rgb, image_size, points_per_pixel=1,
                               compositor="norm", normalize=None, out_dtype=None, after_cameras=None):
     """look_at_view_transform + render_points(dist=...) in one autograd node (see _PointsRenderFromAngles).
@@ -1462,11 +1524,16 @@ def render_points(points, rgb, M: int, R, T, inv_dist, radius: float, bg_rgb, im
     normalize / out_dtype: as in render_meshes (consumer-side fusion).
     shader="hard_depth": (B*M,1,H,W) fp32, the view-space depth of each pixel's nearest point (bit for bit the rasterizer's
     zbuf[..., 0]), `depth_background` (default 100) where no point covers it; rgb, points_per_pixel and compositor do not change it
-    (it always rasterizes with K = 1).  Differentiable w.r.t. R, T, the scale and `points`.  normalize / out_dtype raise."""
+    (it always rasterizes with K = 1).  Differentiable w.r.t. R, T, the scale and `points`.  normalize / out_dtype raise.
+    shader="splat_depth": (B*M,1,H,W) fp32 from the K = points_per_pixel nearest points of each pixel (idx in the fragments dict):
+    nearest first, alpha_k = 1 - dists_k / radius^2 (not clamped) is cumulated and clamped at 1, each point's z is weighted by the
+    step of that sum and `depth_background` (default 100) by what is left; a pixel no point covers holds `depth_background`.
+    Differentiable w.r.t. R, T, the scale and `points` across splat edges (the weights carry the gradient of the points' in-plane
+    positions); rgb and compositor do not change it.  normalize / out_dtype raise."""
     if compositor not in ("norm", "alpha"):
         raise ValueError("compositor must be 'norm' or 'alpha'")
-    if shader not in ("composite", "hard_depth"):
-        raise ValueError("shader must be 'composite' or 'hard_depth'")
+    if shader not in ("composite", "hard_depth", "splat_depth"):
+        raise ValueError("shader must be 'composite', 'hard_depth' or 'splat_depth'")
     flags = L.COMPOSITE_ALPHA if compositor == "alpha" else 0
     if (inv_dist is None) == (dist is None):
         raise ValueError("pass exactly one of inv_dist and dist")
@@ -1479,6 +1546,11 @@ def render_points(points, rgb, M: int, R, T, inv_dist, radius: float, bg_rgb, im
         depth, idx = _PointsDepth.apply(R, T, inv_dist, points, M, radius, H, W, flags & L.SCALE_IS_DIST, float(depth_background))
         frag = {"idx": idx}
         return depth, frag
+    if shader == "splat_depth":
+        _check_splat_depth_options(normalize, out_dtype)
+        depth, idx = _PointsSplatDepth.apply(R, T, inv_dist, points, M, radius, H, W, int(points_per_pixel), flags & L.SCALE_IS_DIST,
+                                             float(depth_background))
+        return depth, {"idx": idx}
     out = _PointsRender.apply(R, T, inv_dist, points, rgb, M, radius, bg_rgb, H, W,
                               int(points_per_pixel), flags, bool(fragments), _out_norm(normalize), out_dtype)
     if fragments:

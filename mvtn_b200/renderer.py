@@ -158,8 +158,16 @@ class MVRenderer(nn.Module):
             "hard_depth", gradients cross silhouette edges and reach background pixels, so an unmasked loss against a target depth
             map moves the views and, when they require grad, the vertices.  The depth does not depend on the colour: a colour that
             requires grad (per object or per vertex) leaves the depth unchanged and gets no gradient (its .grad stays None).
-            normalize, out_dtype=torch.bfloat16 and keep_alpha=True raise ValueError; the point path raises.  Runs eagerly (never
-            from CUDA graphs, cuda_graph=True included).
+            normalize, out_dtype=torch.bfloat16 and keep_alpha=True raise ValueError; the point path raises (its soft depth is
+            "splat_depth").  Runs eagerly (never from CUDA graphs, cuda_graph=True included).
+        shader="splat_depth" / points_per_pixel / points_radius / depth_background (point path): rendered_images is (B, M, 1, H, W)
+            fp32, the z of each pixel's points_per_pixel nearest points blended by the cumulative sum of their splat weights
+            1 - d^2 / points_radius^2 clamped at 1, depth_background taking what is left -- the "soft_depth" formula with the
+            splat weight in place of the sigmoid.  Unlike "hard_depth", the weights carry the gradient of the points' in-plane
+            positions, so an unmasked loss against a target depth map moves the views sideways and, when they require grad, the
+            points.  The colour and the compositor do not change it, and a colour that requires grad gets no gradient.  normalize,
+            out_dtype=torch.bfloat16 and keep_alpha=True raise ValueError; the mesh path raises.  Runs eagerly (never from CUDA
+            graphs, cuda_graph=None and True included).
         shader / blur_radius / blend_sigma / blend_gamma / keep_alpha: mesh path -- "soft_phong" (SoftPhongShader) or
             "soft_silhouette" (SoftSilhouetteShader) blend the faces_per_pixel fragments of the blurred rasterizer (the
             shaders renderer.py:4-6 imports; SURVEY 8f N3); images keep 3 channels as renderer.py:112 unless keep_alpha.
@@ -181,6 +189,8 @@ class MVRenderer(nn.Module):
             ops._check_depth_options(normalize, out_dtype, blur_radius)
         if shader == "soft_depth":
             ops._check_soft_depth_options(normalize, out_dtype, keep_alpha)
+        if shader == "splat_depth":
+            ops._check_splat_depth_options(normalize, out_dtype, keep_alpha)
         self.depth_background = float(depth_background)
         self.stage_overlap = bool(stage_overlap)
         self.shader, self.blur_radius, self.blend_sigma, self.blend_gamma, self.keep_alpha = shader, blur_radius, blend_sigma, blend_gamma, keep_alpha
@@ -262,6 +272,8 @@ class MVRenderer(nn.Module):
         return out, R, T, C
 
     def render_meshes(self, meshes, color, azim, elev, dist, lights, background_color=(1.0, 1.0, 1.0)):
+        if self.shader == "splat_depth":
+            raise ValueError("shader='splat_depth' renders point clouds only (pc_rendering=True)")
         device = self._device(azim)
         # deferred: the meshes are staged (gather + H2D + mvr_mesh_prepare) inside render(), AFTER the camera kernel and
         # the constants below have been enqueued, so that the rasterizer launch follows the geometry with as little host
@@ -354,14 +366,15 @@ class MVRenderer(nn.Module):
 
     def render_points(self, points, color, azim, elev, dist, background_color=(0.0, 0.0, 0.0)):
         if self.shader == "soft_depth":
-            raise ValueError("shader='soft_depth' renders meshes only (pc_rendering=False)")
+            raise ValueError("shader='soft_depth' renders meshes only (pc_rendering=False); the point path's soft depth is "
+                             "shader='splat_depth'")
         device = self._device(azim)
         if points.shape[0] != azim.shape[0]:
             raise ValueError(f"{points.shape[0]} clouds but azim has batch {azim.shape[0]}")
         bg = _device_vec(background_color, device)
         rgb = torch.as_tensor(color, dtype=torch.float32)
         rgb_grad = _requires_grad(rgb)
-        depth = self.shader == "hard_depth"
+        depth = self.shader in ("hard_depth", "splat_depth")
         use_graph = self.cuda_graph and not depth      # depth steps run eagerly
         if use_graph is None and not depth:      # auto: only where the step is launch-bound (DESIGN.md section 5)
             use_graph = (points.shape[0] * self.nb_views <= GRAPH_AUTO_MAX_VIEWS and not torch.cuda.is_current_stream_capturing())
@@ -381,7 +394,8 @@ class MVRenderer(nn.Module):
             # renderer.py:142 point_cloud.scale_(1/dist): the reciprocal is taken inside the kernels (dist=)
             if depth:
                 return ops.render_points(pts, rgb, self.nb_views, R, T, None, self.points_radius, bg, self.image_size,
-                                         dist=dist_, shader="hard_depth", depth_background=self.depth_background)
+                                         points_per_pixel=self.points_per_pixel, dist=dist_, shader=self.shader,
+                                         depth_background=self.depth_background)
             return ops.render_points(pts, rgb, self.nb_views, R, T, None, self.points_radius, bg, self.image_size,
                                      points_per_pixel=self.points_per_pixel, compositor=self.compositor,
                                      normalize=self.normalize, out_dtype=self.out_dtype, dist=dist_)
